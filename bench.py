@@ -2,7 +2,7 @@
 """Benchmark of the batched step hot path (BASELINE.json metric: env-steps/s, DeepRMSA-v0 NSFNET,
 65536 envs per GPU, obs + reward + done on device).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one env.step of the whole batch (one env-step for each of the 65536 envs of every rank)
@@ -11,6 +11,10 @@ with the uniform random policy drawn on the device.  The K timed steps run as ON
 [K, N, ...] device buffers), repeated R times; the median repetition is reported (the list is in the
 line).  Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for value / e2e / roofline /
 cpu_baseline.
+
+--dump-outputs DIR writes what the last timed step returned (rank 0's envs) as DIR/<name>.npy.  Traffic and
+actions come from seeded Philox streams, so the same arguments give the same inputs on every run and two
+builds can be compared output for output.
 """
 import argparse
 import json
@@ -20,6 +24,8 @@ import threading
 import time
 
 import numpy as np
+
+sys.dont_write_bytecode = True      # the benchmark may run from a read-only tree: it writes nothing there
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "optical-rl-gym_b200")):
@@ -41,6 +47,25 @@ def read_peaks():
             return float(json.load(f)["hbm_gbs"]), "measured"
     except Exception:  # noqa: BLE001
         return 6650.0, "fallback"
+
+
+DUMP_LIMIT = 64 << 20           # bytes written by --dump-outputs
+
+
+def dump_outputs(path, arrays):
+    """Writes each [N, ...] device tensor as path/<name>.npy in float32 (the integer outputs are exact in it).  Above
+    DUMP_LIMIT bytes the same fixed, seeded sample of envs is kept in every array; its indices go to env_index.npy."""
+    arrays = {k: v.float().cpu().numpy() for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a[0].nbytes for a in arrays.values())
+    budget = DUMP_LIMIT - 4096                  # room for the .npy headers
+    if n * row_bytes > budget:
+        keep = np.sort(np.random.default_rng(0).choice(n, budget // (row_bytes + 8), replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+        arrays["env_index"] = keep.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 class ClockSampler:
@@ -238,6 +263,8 @@ def run_secondary(args):
             ev1.record()
             torch.cuda.synchronize()
             rep_ms.append(ev0.elapsed_time(ev1))
+        last = (K - 1) % chunk          # the last timed step, kept before the launches below overwrite the buffers
+        dump = {"reward": rew[last].clone(), "done": done[last].clone(), "action": act[last].clone()} if args.dump_outputs else None
         t_end = time.perf_counter() + 0.25
         while time.perf_counter() < t_end:
             k_steps(chunk)
@@ -261,6 +288,8 @@ def run_secondary(args):
         "cpu_baseline": None, "e2e": None, "gpu_launches": (K + chunk - 1) // chunk * (1 if persistent else 2 * chunk),
         "clocks": sampler.summary(), "accept_rate": float(cnt[1]) / float(cnt[0]),
         "envs_with_errors": int((env.error_flags() != 0).sum()), "state_MB": env.state_bytes / 1e6}))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dump)
 
 
 E2E_CHUNK = int(os.environ.get("ORLG_E2E_CHUNK", "2"))   # steps per pipeline stage of the end-to-end leg (orlg_rollout_host)
@@ -279,7 +308,11 @@ def main():
                     help="c2 = the headline (BASELINE configs[2]); the others print a secondary line for that config")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's obs / reward / done / action of rank 0's envs to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the device path; --impl reference has none")
     args.warmup = max(args.warmup, 3)
     args.reps = max(args.reps, 1)
     rank = int(os.environ.get("RANK", 0))
@@ -354,6 +387,9 @@ def main():
             if world > 1:
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)        # max over ranks, per repetition
             rep_ms.append(float(t.item()))
+        last = (K - 1) % chunk          # the last timed step, kept before the launches below overwrite the buffers
+        dump = {"obs": obs[last].clone(), "reward": rew[last].clone(), "done": done[last].clone(),
+                "action": act[last].clone()} if args.dump_outputs and rank == 0 else None
         # keep the GPU under the same load a little longer so that the clock sampler sees it
         t_end = time.perf_counter() + 0.25
         while time.perf_counter() < t_end:
@@ -576,6 +612,8 @@ def main():
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+    if dump is not None:
+        dump_outputs(args.dump_outputs, dump)
     if out is not None:
         print(json.dumps(out))
 

@@ -12,7 +12,6 @@ import helpers
 from optical_rl_gym_b200 import topology as T
 
 GOLD = helpers.GOLDEN_DIR
-REF_TOPO = "/root/reference/examples/topologies"
 
 
 def assert_same_tables(a, b, skip=("name",)):
@@ -60,19 +59,6 @@ def test_txt_reader_edge_cases(tmp_path):
     bad.write_text("2\n1\n1 5 10\n")
     with pytest.raises(ValueError):
         T.get_topology(bad)
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_TOPO), reason="reference tree only exists in the build container")
-def test_reference_files_and_pickles_agree():
-    """The shipped pickles, un-pickled WITHOUT the reference package, equal what our readers build from the
-    shipped .txt / .xml files, and equal the committed goldens."""
-    for stem, src, gold in (("nsfnet_chen", "nsfnet_chen.txt", "nsfnet_tables.npz"),
-                            ("germany50", "germany50.xml", "topo_germany50_tables.npz")):
-        pick = T.load_reference_pickle(os.path.join(REF_TOPO, stem + "_5-paths_6-modulations.h5"))
-        mine = T.get_topology(os.path.join(REF_TOPO, src))
-        want = T.TopologyTables.load(os.path.join(GOLD, gold))
-        assert_same_tables(mine, pick)
-        assert_same_tables(mine, want, skip=("name", "link_nodes") if stem == "nsfnet_chen" else ("name",))
 
 
 def test_germany50_golden_is_consistent():
@@ -131,18 +117,6 @@ def test_mlp_policy_loads_sb3_archive_and_matches_numpy_forward(tmp_path, shared
     assert np.array_equal(a[clear, 0], logits.argmax(1)[clear])
     s = pol.act(torch.as_tensor(obs), deterministic=False, generator=torch.Generator().manual_seed(1))
     assert s.min() >= 0 and s.max() < 5
-
-
-@pytest.mark.skipif(not os.path.isdir("/root/reference/examples/stable_baselines3/bkp"), reason="build container only")
-def test_mlp_policy_loads_the_shipped_agent():
-    torch = pytest.importorskip("torch")
-    from optical_rl_gym_b200.policy import MlpPolicy
-
-    pol = MlpPolicy.from_sb3_zip("/root/reference/examples/stable_baselines3/bkp/deeprmsa-ppo-trained/best_model.zip")
-    assert [m.out_features for m in pol.shared_net if hasattr(m, "out_features")] == [128] * 5
-    obs = torch.as_tensor(helpers.load_golden("deeprmsa_default_random")["obs"][0, :64])
-    a = pol.act(obs)
-    assert a.shape == (64, 1) and int(a.min()) >= 0 and int(a.max()) <= 4
 
 
 def test_monitor_file_format_matches_sb3(tmp_path):
