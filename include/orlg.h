@@ -112,6 +112,18 @@ int orlg_mask_words(const orlg_env *env);   /* 32-bit words per (core, link) in 
 int orlg_heap_capacity(const orlg_env *env);
 int64_t orlg_state_bytes(const orlg_env *env);
 
+/* Which compiled kernel instances the handle runs (fixed at orlg_create, except last_rollout_persistent). */
+typedef struct orlg_kernel_info {
+    int32_t wide;              /* > 32 links, > 128 slots or > 8 paths: CSR link lists, multi-word masks */
+    int32_t fast;              /* DeepRMSA: the per-step fast kernel (deeprmsa_fast_kernel) */
+    int32_t hot;               /* ... and its steady-state specialisation is allowed */
+    int32_t rollout_kernel;    /* the persistent rollout kernel applies to this configuration */
+    int32_t rollout_lanes;     /* envs per warp of the rollout kernel: 8 or 32 (environment ORLG_RO_LPW at orlg_create) */
+    int32_t link_template;     /* link count the non-wide kernels are compiled for: 22 (NSFNET), 0 = read at run time */
+    int32_t last_rollout_persistent;   /* 1: the last orlg_rollout* call ran the persistent kernel, 0: per-step launches or none yet */
+} orlg_kernel_info_t;
+int orlg_kernel_info(const orlg_env *env, orlg_kernel_info_t *out);
+
 /* ---- traffic -------------------------------------------------------------------------- */
 /* env.seed(seed) (optical_network_env.py:205-210): new key of the counter-based request stream from the next
  * request on; the state of the environments is not touched (like the reference, which only replaces its rng). */

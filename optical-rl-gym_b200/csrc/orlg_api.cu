@@ -46,6 +46,8 @@ struct orlg_env {
     bool fast;                    // DeepRMSA fast kernel applicable (NSFNET-class: 22 links, k <= 5)
     bool hot;                     // ... and its steady-state specialisation (deeprmsa_fast_kernel<.., HOT = true>)
     bool ro_ok;                   // the persistent rollout kernel applies (DeepRMSA / RMSA / RWA on NSFNET-class topologies)
+    int ro_lpw;                   // envs per warp of the rollout kernel (8 or 32): fixed per handle, the event slabs follow it
+    bool ro_last_persistent = false;   // the last orlg_rollout* call ran the persistent kernel (orlg_kernel_info)
     CUtensorMap mask_map;         // TMA view of the mask tensor: [C*E rows][n x 16 bytes], box = E rows x 512 bytes
     bool wide;                    // beyond 32 links / 128 slots / 8 paths: CSR link lists, multi-word masks
     size_t fast_smem;
@@ -258,12 +260,16 @@ int launch_step(const orlg_env *env, const StepIO &io, int mode, cudaStream_t s)
 }
 
 // envs per warp of the rollout kernel: a batch that would leave most SMs with one or two warps is spread over more warps
-// with fewer lanes in use (less divergence per warp, more warps to hide latency); fixed per handle (the event slabs follow it)
-int rollout_lpw(const orlg_env *env) {
-    static const int forced = [] { const char *v = std::getenv("ORLG_RO_LPW"); const int w = v ? std::atoi(v) : 0; return (w == 8 || w == 32) ? w : 0; }();
-    if (forced) return forced;
-    return env->p.n >= 16384 ? 32 : 8;
+// with fewer lanes in use (less divergence per warp, more warps to hide latency).  Chosen by orlg_create (ORLG_RO_LPW = 8 or
+// 32 overrides it for the handles created while it is set) and fixed per handle: the event slabs follow it.
+int choose_rollout_lpw(int n) {
+    const char *v = std::getenv("ORLG_RO_LPW");
+    const int w = v ? std::atoi(v) : 0;
+    if (w == 8 || w == 32) return w;
+    return n >= 16384 ? 32 : 8;
 }
+
+int rollout_lpw(const orlg_env *env) { return env->ro_lpw; }
 
 void rollout_state_args(const orlg_env *env, RolloutArgs *ra) {
     const size_t n = (size_t)env->p.n;
@@ -387,6 +393,7 @@ int orlg_create(const orlg_config *cfg, const orlg_tables *t, int device, orlg_e
     env->device = device;
     env->state_bytes = 0;
     env->wide = wide;
+    env->ro_lpw = choose_rollout_lpw(cfg->num_envs);
     Params &p = env->p;
     std::memset(&p, 0, sizeof(p));
     p.kind = cfg->kind; p.n = cfg->num_envs; p.N = t->num_nodes; p.E = t->num_links; p.C = C; p.S = cfg->num_slots;
@@ -660,6 +667,18 @@ int orlg_obs_dim(const orlg_env *env) { return env->p.obs_dim; }
 int orlg_mask_words(const orlg_env *env) { return NW * env->p.nwv; }
 int orlg_heap_capacity(const orlg_env *env) { return env->p.heap_cap; }
 int64_t orlg_state_bytes(const orlg_env *env) { return env->state_bytes; }
+
+int orlg_kernel_info(const orlg_env *env, orlg_kernel_info_t *out) {
+    if (!env || !out) return fail(ORLG_E_INVALID, "null handle or output");
+    out->wide = env->wide;
+    out->fast = env->fast;
+    out->hot = env->hot;
+    out->rollout_kernel = env->ro_ok;
+    out->rollout_lanes = rollout_lpw(env);
+    out->link_template = !env->wide && env->p.E == 22 ? 22 : 0;     // the ET choice of launch_fast / rollout_impl
+    out->last_rollout_persistent = env->ro_last_persistent;
+    return ORLG_OK;
+}
 
 int orlg_seed(orlg_env *env, uint64_t seed) {
     if (!env) return fail(ORLG_E_INVALID, "null handle");
@@ -1016,8 +1035,10 @@ static int rollout_impl(orlg_env *env, int steps, int policy, void *obs_dev, flo
         if (e != cudaSuccess) return fail(ORLG_E_CUDA, std::string("rollout launch: ") + cudaGetErrorString(e));
         p.lockstep_ridx += (unsigned)steps;
         env->ro_valid = true;
+        env->ro_last_persistent = true;
         return ORLG_OK;
     }
+    env->ro_last_persistent = false;
     if (packed_dev) return fail(ORLG_E_UNSUPPORTED, "packed records exist for the persistent DeepRMSA rollout kernel only (k = 5, j = 1, float32)");
     // generic: the same T steps as separate policy + step launches
     {

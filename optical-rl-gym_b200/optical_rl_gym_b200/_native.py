@@ -29,6 +29,11 @@ class Config(C.Structure):
                 ("mean_iat", C.c_double), ("worst_xt", C.c_double)]
 
 
+class KernelInfo(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("wide", "fast", "hot", "rollout_kernel", "rollout_lanes", "link_template",
+                                         "last_rollout_persistent")]
+
+
 class Tables(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("num_nodes", "num_links", "k_paths", "num_paths", "num_mods", "num_bit_rates")] + [
         (n, C.c_void_p) for n in ("pair_first", "pair_count", "path_hops", "path_se", "path_mod", "path_link_ptr",
@@ -67,6 +72,7 @@ def lib():
         getattr(L, name).argtypes = [vp]
     L.orlg_state_bytes.argtypes = [vp]
     L.orlg_state_bytes.restype = i64
+    L.orlg_kernel_info.argtypes = [vp, C.POINTER(KernelInfo)]
     L.orlg_host_dma_fraction.argtypes = [vp]
     L.orlg_host_dma_fraction.restype = C.c_double
     L.orlg_set_trace.argtypes = [vp, vp, i64]
@@ -113,7 +119,7 @@ def check(rc):
 
 
 EXPORTED = ["orlg_create", "orlg_destroy", "orlg_last_error", "orlg_version", "orlg_action_dim", "orlg_obs_dim",
-            "orlg_mask_words", "orlg_heap_capacity", "orlg_state_bytes", "orlg_seed", "orlg_set_trace", "orlg_reset", "orlg_step",
+            "orlg_mask_words", "orlg_heap_capacity", "orlg_state_bytes", "orlg_kernel_info", "orlg_seed", "orlg_set_trace", "orlg_reset", "orlg_step",
             "orlg_observation", "orlg_observation_int", "orlg_heuristic", "orlg_random_actions", "orlg_get_counters",
             "orlg_get_requests", "orlg_export_state", "orlg_error_flags", "orlg_reduce_counters", "orlg_enable_stats",
             "orlg_num_bit_rates", "orlg_bit_rate_blocking", "orlg_matrix_obs_dim", "orlg_matrix_observation",

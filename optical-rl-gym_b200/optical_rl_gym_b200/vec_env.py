@@ -514,6 +514,18 @@ class OpticalVecEnv:
         self.seed(sd["seed"])
 
     # ------------------------------------------------------------------ introspection
+    def kernel_info(self) -> dict:
+        """Which compiled kernel instances this batch runs (``orlg_kernel_info``): ``wide``, ``fast``, ``hot``,
+        ``rollout_kernel`` (bools), ``rollout_lanes`` (envs per warp of the rollout kernel, 8 or 32), ``link_template``
+        (22: the NSFNET instance, 0: link count read at run time) and ``last_rollout_persistent`` (whether the last
+        :meth:`rollout` / :meth:`rollout_packed` / :meth:`rollout_host` ran the persistent kernel)."""
+        info = nat.KernelInfo()
+        nat.check(self._lib.orlg_kernel_info(self._h, C.byref(info)))
+        out = {name: int(getattr(info, name)) for name, _ in nat.KernelInfo._fields_}
+        for name in ("wide", "fast", "hot", "rollout_kernel", "last_rollout_persistent"):
+            out[name] = bool(out[name])
+        return out
+
     @property
     def decisions(self):
         return self._decision

@@ -30,6 +30,28 @@ def golden_tables():
     return TopologyTables.load(os.path.join(GOLDEN_DIR, "nsfnet_tables.npz"))
 
 
+# Non-NSFNET topologies within the non-wide kernels' limits (<= 32 links, 5 paths per pair): the kernels read their link
+# count at run time there (link template 0) instead of using the 22-link NSFNET instance.
+SYNTHETIC = {"E20": (12, 8), "E32": (16, 16)}       # name -> (ring nodes, chords); 20 and 32 links
+_TABLES = {}
+
+
+def tables(name):
+    """"nsfnet" (22 links), "E20" / "E32" (seeded ring + chords graphs, k = 5, seed 3), "small_xml" (10 nodes, 15 links,
+    k = 3); built once per process."""
+    if name not in _TABLES:
+        from optical_rl_gym_b200.topology import synthetic_ring_chords
+
+        if name == "nsfnet":
+            _TABLES[name] = golden_tables()
+        elif name == "small_xml":
+            _TABLES[name] = TopologyTables.load(os.path.join(GOLDEN_DIR, "topo_small_xml_tables.npz"))
+        else:
+            nodes, chords = SYNTHETIC[name]
+            _TABLES[name] = synthetic_ring_chords(nodes, chords, k_paths=5, seed=3)
+    return _TABLES[name]
+
+
 def sim_kwargs(meta):
     """Reference env_args (as recorded) -> the keyword set shared by the oracle and the product
     (defaults per env class: optical_network_env.py:14-25, rmsa_env.py:29-46, deeprmsa_env.py:10-21,

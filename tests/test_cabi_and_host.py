@@ -38,6 +38,7 @@ def test_struct_layouts_match_header():
     assert ctypes.sizeof(_native.Config) == 104          # 2*i32, i64, 12*i32, u64, 4*f64 (with padding)
     assert _native.Config.seed.offset % 8 == 0 and _native.Config.env_id_base.offset == 8
     assert ctypes.sizeof(_native.Tables) == 6 * 4 + 15 * 8
+    assert ctypes.sizeof(_native.KernelInfo) == 7 * 4
     assert _native.REQUEST_DTYPE.itemsize == 32
     assert [_native.REQUEST_DTYPE.fields[n][1] for n in ("arrival", "holding", "src", "dst", "bit_rate")] == [0, 8, 16, 20, 24]
 

@@ -125,18 +125,47 @@ PHILOX_CASES = [
     ("RMCSA-v0", dict(episode_length=50, load=400, mean_service_holding_time=25, num_spectrum_resources=100,
                       num_spatial_resources=3, worst_xt=-84.7, allow_rejection=True), "random", 48, 300),
 ]
+# The DeepRMSA fast kernel with its link count read at run time (link template 0): synthetic graphs of 20 and 32 links
+# (helpers.tables) and the 15-link, 3-path topo_small_xml.  env_args["topology"] names the tables (default NSFNET);
+# env_args["variant"] the instance: "f64" (default) float64 observations with the decision output, "hot" the steady-state
+# instance (float32 observations, no decision output), "general" the float32 instance (ORLG_NO_HOT) with decisions.
+_DEEP_BLOCKING = dict(episode_length=37, mean_service_holding_time=40.0, num_spectrum_resources=64)
+PHILOX_CASES += [
+    ("DeepRMSA-v0", dict(_DEEP_BLOCKING, topology="E20", variant="hot"), "random", 93, 300),
+    ("DeepRMSA-v0", dict(_DEEP_BLOCKING, topology="E32", variant="hot", allow_rejection=True), "sap", 93, 300),
+    ("DeepRMSA-v0", dict(_DEEP_BLOCKING, topology="E20", variant="general", allow_rejection=True), "sap", 93, 300),
+    ("DeepRMSA-v0", dict(_DEEP_BLOCKING, topology="E32", variant="general"), "random", 93, 300),
+    ("DeepRMSA-v0", dict(_DEEP_BLOCKING, topology="E20"), "random", 93, 300),
+    ("DeepRMSA-v0", dict(_DEEP_BLOCKING, topology="E32", allow_rejection=True), "sap", 93, 300),
+    ("DeepRMSA-v0", dict(_DEEP_BLOCKING, topology="E20", j=2, allow_rejection=True), "sap", 93, 300),
+    ("DeepRMSA-v0", dict(_DEEP_BLOCKING, topology="E32", j=2), "random", 93, 300),
+    ("DeepRMSA-v0", dict(_DEEP_BLOCKING, topology="small_xml"), "random", 93, 300),
+    ("DeepRMSA-v0", dict(_DEEP_BLOCKING, topology="small_xml", variant="general", allow_rejection=True), "sap", 93, 300),
+]
 
 
 @pytest.mark.parametrize("kind,env_args,policy,n_envs,T", PHILOX_CASES)
-def test_cuda_matches_oracle_on_philox_traffic(kind, env_args, policy, n_envs, T):
+def test_cuda_matches_oracle_on_philox_traffic(monkeypatch, kind, env_args, policy, n_envs, T):
     from optical_rl_gym_b200 import OpticalVecEnv
     from oracle import oracle
 
-    tables = helpers.golden_tables()
+    env_args = dict(env_args)
+    topo, variant = env_args.pop("topology", "nsfnet"), env_args.pop("variant", "f64")
+    tables = helpers.tables(topo)
     seed, base = 77, 1000
     meta = dict(kind=kind, env_args=env_args)
-    env = OpticalVecEnv(kind, n_envs, tables, traffic="philox", record_decisions=True, obs_dtype=torch.float64,
-                        env_id_base=base, seed=seed, **env_args)
+    if variant == "general":
+        monkeypatch.setenv("ORLG_NO_HOT", "1")
+    f64, decisions = variant == "f64", variant != "hot"
+    env = OpticalVecEnv(kind, n_envs, tables, traffic="philox", record_decisions=decisions,
+                        obs_dtype=torch.float64 if f64 else torch.float32, env_id_base=base, seed=seed, **env_args)
+    monkeypatch.delenv("ORLG_NO_HOT", raising=False)
+    info = env.kernel_info()
+    assert info["link_template"] == (22 if topo == "nsfnet" else 0), info
+    if topo != "nsfnet":
+        assert info["fast"], info
+    if variant != "f64":
+        assert info["hot"] == (variant == "hot"), info
     okw = helpers.sim_kwargs(meta)
     if env_args.get("bit_rate_selection") == "discrete":
         okw["bit_rates"] = [10, 40, 100]
@@ -153,14 +182,18 @@ def test_cuda_matches_oracle_on_philox_traffic(kind, env_args, policy, n_envs, T
         a = env.sample_actions() if pol is not None else env.heuristic(hid)
         want_a = np.stack([r["actions"][t] for r in ref])
         assert np.array_equal(a.cpu().numpy(), want_a), ("actions", t)
-        obs, reward, done, info = env.step(a)
-        d = env.decisions.cpu().numpy()
-        want_d = np.stack([r["decisions"][t] for r in ref])
-        assert np.array_equal(d[:, :4], want_d), ("decision", t, d[:4], want_d[:4])
+        obs, reward, done, _ = env.step(a)
+        if decisions:
+            d = env.decisions.cpu().numpy()
+            want_d = np.stack([r["decisions"][t] for r in ref])
+            assert np.array_equal(d[:, :4], want_d), ("decision", t, d[:4], want_d[:4])
         assert np.array_equal(reward.cpu().numpy().astype(np.float64), np.array([r["rewards"][t] for r in ref])), t
         assert np.array_equal(done.cpu().numpy(), np.array([r["dones"][t] for r in ref])), ("done", t)
-        if kind == "DeepRMSA-v0":
+        if kind == "DeepRMSA-v0" and f64:
             assert np.array_equal(obs.cpu().numpy(), np.stack([r["obs"][t] for r in ref])), ("obs", t)
+        elif kind == "DeepRMSA-v0":
+            np.testing.assert_allclose(obs.cpu().numpy(), np.stack([r["obs"][t] for r in ref]), rtol=OBS_RTOL, atol=0,
+                                       err_msg="obs f32 step %d" % t)
     # final state
     m, alloc, now, nheap = env.export_state(allocation=True)
     avail = env.available_slots().cpu().numpy()
