@@ -204,6 +204,38 @@ int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers,
 int orlg_policy_act(orlg_policy *pol, const float *obs_dev, int n, int32_t *actions_dev, float *logits_dev, orlg_stream stream);
 int orlg_policy_destroy(orlg_policy *pol);
 
+/* What PPO's collect_rollouts needs from the same fused kernel: the action, log softmax(logits)[action] and the value head.
+ * Deterministic: the argmax (first maximum), as orlg_policy_act.  Sampling: one Philox4x32-10 block per row with key = seed and
+ * counter = (c0, 0, row_id_base + row, 3) (stream 3, DESIGN.md section 5); u = (word 0 >> 8) * 2^-24; the action is the
+ * smallest a with u * S < e_0 + ... + e_a, e_a = expf(l_a - max l), S = sum of e_a (the last action if rounding leaves none).
+ * A draw is therefore a function of (seed, c0, row id, observation) only. */
+typedef struct orlg_policy_draw {
+    uint64_t seed;               /* Philox key of the action draws */
+    const uint32_t *counter_dev; /* per row: counter word 0 (the env's request index); NULL = `counter` for every row */
+    uint32_t counter;
+    int32_t deterministic;       /* 1: argmax, as model.predict(deterministic=True); 0: sample from softmax(logits) */
+    int64_t row_id_base;         /* counter word 2 of row r = row_id_base + r (the global env id) */
+} orlg_policy_draw;
+/* actions_dev int32 [n], log_prob_dev f32 [n], value_dev f32 [n]: any may be NULL */
+int orlg_policy_sample(orlg_policy *pol, const float *obs_dev, int n, const orlg_policy_draw *draw, int32_t *actions_dev,
+                       float *log_prob_dev, float *value_dev, orlg_stream stream);
+
+/* A PPO rollout buffer in one call: steps x { a, log p(a), V(obs) = policy(obs); obs, r, done = env.step(a) } for DeepRMSA-v0
+ * with float32 observations (per step the sampling kernel, an optional critic launch and the step kernel, chained by
+ * programmatic dependent launch).
+ *   obs_dev      f32 [steps + 1, N, obs_dim]  required: obs[0] = observation of the pending request, obs[t+1] = what step t returned
+ *   actions_dev  i32 [steps, N]      log_prob_dev f32 [steps, N]      value_dev f32 [steps + 1, N] (value[steps] = bootstrap value)
+ *   reward_dev   f32 [steps, N]      done_dev     u8  [steps, N]      (all but obs may be NULL)
+ *   critic       NULL = the actor's value head; else a handle whose value head is the critic's (separate SB3 >= 1.8 trunk)
+ * The draws are keyed by (seed, global env id, the env's request index): results do not depend on sharding, on how a rollout is
+ * split into calls, or on a checkpoint taken between calls.  deterministic = 1: argmax actions. */
+int orlg_rollout_policy(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
+                        float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
+                        float *reward_dev, uint8_t *done_dev, orlg_stream stream);
+/* requests drawn so far by every env of the handle (all step together): counter word 0 of the draws orlg_rollout_policy
+ * makes at its next step.  Host state, no device access. */
+int64_t orlg_request_index(const orlg_env *env);
+
 /* Float statistics of `info` (rmsa_env.py:229-264, 439-543, 699-744; RMSA-v0 / DeepRMSA-v0, <= 32 links,
  * <= 128 slots): after this call every orlg_step also writes, per env, float64
  *   stats_dev[env][0..3] = network_compactness, network_compactness_difference,

@@ -1452,7 +1452,8 @@ int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers,
     pol->pp.bias = reinterpret_cast<const float *>(pol->b_dev);
     pol->pp.obs_dim = obs_dim; pol->pp.n_actions = n_actions;
     pol->smem = bytes + (size_t)PL_GROUPS * PL_TILE * PL_H * 2 + bias.size() * 4 + 64;
-    if (cudaFuncSetAttribute(mlp_policy_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pol->smem) != cudaSuccess) {
+    if (cudaFuncSetAttribute(mlp_policy_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pol->smem) != cudaSuccess ||
+        cudaFuncSetAttribute(mlp_policy_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pol->smem) != cudaSuccess) {
         cudaFree(pol->w_dev); cudaFree(pol->b_dev); delete pol;
         return fail(ORLG_E_CUDA, "cudaFuncSetAttribute(policy kernel shared memory) failed");
     }
@@ -1460,18 +1461,102 @@ int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers,
     return ORLG_OK;
 }
 
+}  // extern "C"
+
+// one launch of the fused policy kernel over n rows: a persistent CTA per SM (each walks PL_GROUPS tile streams)
+template <bool SAMPLE>
+static int launch_policy(const orlg_policy *pol, const float *obs_dev, int n, int32_t *actions_dev, float *logits_dev,
+                         const PolicyDraw &dr, cudaStream_t s) {
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, pol->device);
+    const int pairs = ((n + PL_TILE - 1) / PL_TILE + PL_GROUPS - 1) / PL_GROUPS;
+    cudaLaunchConfig_t cfg = pdl_config(pairs < sms ? pairs : sms, PL_WG * PL_GROUPS, pol->smem, s);
+    int *actions = actions_dev;
+    CUDA_OK(cudaLaunchKernelEx(&cfg, mlp_policy_kernel<SAMPLE>, pol->pp, obs_dev, n, actions, logits_dev, dr));
+    return ORLG_OK;
+}
+
+extern "C" {
+
 int orlg_policy_act(orlg_policy *pol, const float *obs_dev, int n, int32_t *actions_dev, float *logits_dev, orlg_stream stream) {
     if (!pol || !obs_dev || !actions_dev || n < 0) return fail(ORLG_E_INVALID, "null policy or buffer");
     if (n == 0) return ORLG_OK;
     DeviceGuard guard(pol->device);
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, pol->device);
-    const int pairs = ((n + PL_TILE - 1) / PL_TILE + PL_GROUPS - 1) / PL_GROUPS;       // each CTA walks PL_GROUPS tile streams
-    cudaLaunchConfig_t cfg = pdl_config(pairs < sms ? pairs : sms, PL_WG * PL_GROUPS, pol->smem, (cudaStream_t)stream);
-    int *actions = actions_dev;
-    CUDA_OK(cudaLaunchKernelEx(&cfg, mlp_policy_kernel, pol->pp, obs_dev, n, actions, logits_dev));
-    return ORLG_OK;
+    PolicyDraw dr;
+    std::memset(&dr, 0, sizeof(dr));
+    return launch_policy<false>(pol, obs_dev, n, actions_dev, logits_dev, dr, (cudaStream_t)stream);
 }
+
+static PolicyDraw policy_draw(const orlg_policy_draw &d, float *log_prob_dev, float *value_dev) {
+    PolicyDraw dr;
+    std::memset(&dr, 0, sizeof(dr));
+    dr.seed = d.seed;
+    dr.counter_dev = d.counter_dev;
+    dr.counter = d.counter;
+    dr.deterministic = d.deterministic ? 1 : 0;
+    dr.row_id_base = d.row_id_base;
+    dr.log_prob = log_prob_dev;
+    dr.value = value_dev;
+    return dr;
+}
+
+int orlg_policy_sample(orlg_policy *pol, const float *obs_dev, int n, const orlg_policy_draw *draw, int32_t *actions_dev,
+                       float *log_prob_dev, float *value_dev, orlg_stream stream) {
+    if (!pol || !obs_dev || !draw || n < 0) return fail(ORLG_E_INVALID, "null policy, observation buffer or draw");
+    if (n == 0) return ORLG_OK;
+    DeviceGuard guard(pol->device);
+    return launch_policy<true>(pol, obs_dev, n, actions_dev, nullptr, policy_draw(*draw, log_prob_dev, value_dev), (cudaStream_t)stream);
+}
+
+int orlg_rollout_policy(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
+                        float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
+                        float *reward_dev, uint8_t *done_dev, orlg_stream stream) {
+    if (!env || !actor) return fail(ORLG_E_INVALID, "null env or actor handle");
+    const Params &p = env->p;
+    if (p.kind != ORLG_DEEPRMSA) return fail(ORLG_E_UNSUPPORTED, "orlg_rollout_policy drives DeepRMSA-v0 (the env kind with a tensor observation)");
+    if (p.obs_f64) return fail(ORLG_E_UNSUPPORTED, "orlg_rollout_policy needs float32 observations (the policy kernel reads float32)");
+    if (actor->pp.obs_dim != p.obs_dim)
+        return fail(ORLG_E_INVALID, "actor obs_dim " + std::to_string(actor->pp.obs_dim) + " != env obs_dim " + std::to_string(p.obs_dim));
+    const int n_act = p.k * p.J + p.allow_rejection;
+    if (actor->pp.n_actions != n_act)
+        return fail(ORLG_E_INVALID, "actor n_actions " + std::to_string(actor->pp.n_actions) + " != k * j + allow_rejection = " + std::to_string(n_act));
+    if (critic && critic->pp.obs_dim != p.obs_dim)
+        return fail(ORLG_E_INVALID, "critic obs_dim " + std::to_string(critic->pp.obs_dim) + " != env obs_dim " + std::to_string(p.obs_dim));
+    if (actor->device != env->device || (critic && critic->device != env->device))
+        return fail(ORLG_E_INVALID, "policy and env handles live on different devices");
+    if (!obs_dev) return fail(ORLG_E_INVALID, "orlg_rollout_policy needs obs_dev (the policy reads it)");
+    if (steps < 0) return fail(ORLG_E_INVALID, "steps must be >= 0");
+    if (p.traffic == ORLG_TRAFFIC_TRACE && p.trace == nullptr) return fail(ORLG_E_INVALID, "trace traffic selected but orlg_set_trace was not called");
+    DeviceGuard guard(env->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    int rc = ensure_canonical(env, s);          // the handle may have been stepped by the persistent rollout kernel
+    if (!rc) rc = orlg_observation(env, obs_dev, stream);
+    if (rc) return rc;
+    if (!actions_dev && steps > 0 && !env->ro_actions) {
+        rc = dev_alloc(env, &env->ro_actions, (size_t)p.n, false);
+        if (rc) return rc;
+    }
+    const size_t n = (size_t)p.n, row = n * (size_t)p.obs_dim;
+    orlg_policy_draw d;
+    d.seed = seed; d.counter_dev = p.req_index; d.counter = 0; d.deterministic = deterministic; d.row_id_base = p.env_id_base;
+    for (int t = 0; t < steps; t++) {
+        const float *o = obs_dev + (size_t)t * row;
+        int32_t *a = actions_dev ? actions_dev + (size_t)t * n : env->ro_actions;
+        float *v = value_dev ? value_dev + (size_t)t * n : nullptr;
+        rc = launch_policy<true>(actor, o, p.n, a, nullptr, policy_draw(d, log_prob_dev ? log_prob_dev + (size_t)t * n : nullptr,
+                                                                       critic ? nullptr : v), s);
+        if (!rc && critic && v) rc = launch_policy<true>(critic, o, p.n, nullptr, nullptr, policy_draw(d, nullptr, v), s);
+        if (!rc) rc = step_impl(env, a, -1, nullptr, obs_dev + (size_t)(t + 1) * row, reward_dev ? reward_dev + (size_t)t * n : nullptr,
+                                done_dev ? done_dev + (size_t)t * n : nullptr, nullptr, nullptr, stream);
+        if (rc) return rc;
+    }
+    if (value_dev)                              // the bootstrap value of the last observation
+        rc = launch_policy<true>(critic ? critic : actor, obs_dev + (size_t)steps * row, p.n, nullptr, nullptr,
+                                 policy_draw(d, nullptr, value_dev + (size_t)steps * n), s);
+    return rc;
+}
+
+int64_t orlg_request_index(const orlg_env *env) { return env ? (int64_t)env->p.lockstep_ridx : -1; }
 
 int orlg_policy_destroy(orlg_policy *pol) {
     if (!pol) return ORLG_OK;

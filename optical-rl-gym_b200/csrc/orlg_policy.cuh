@@ -10,7 +10,8 @@
 // tcgen05.mma (M = 128, N = 128, K = 16 per instruction) with A = the tile's activations (bf16, shared memory),
 // B = the layer's weights, D = fp32 accumulators in TMEM; the four warps then read their 32 TMEM lanes back with
 // tcgen05.ld, add the bias, apply tanh and write the next layer's A operand.  Nothing but the observation rows and
-// the actions touches HBM.
+// the actions touches HBM.  A second instance (mlp_policy_kernel<true>) ends in a sampling epilogue: the action drawn from
+// softmax(logits) with Philox stream 3, its log-probability and the value (PPO's rollout collection, orlg_policy_sample).
 #pragma once
 #include <cuda_bf16.h>
 #include "orlg_deeprmsa_fast.cuh"
@@ -28,6 +29,19 @@ struct PolicyParams {
     int w_bytes;                      // multiple of 16
     const float *bias;                // [5 * 128 + 16]
     int obs_dim, n_actions;           // 54, 5
+};
+
+// The sampling epilogue (mlp_policy_kernel<true>, orlg_policy_sample): one Philox4x32-10 block per row, key = seed,
+// counter = (c0, 0, row_id_base + row, 3) -- stream 3 of DESIGN.md section 5 -- where c0 = counter_dev[row] (the env's
+// request index) or `counter`.  Every output may be NULL.
+struct PolicyDraw {
+    unsigned long long seed;
+    const unsigned *counter_dev;
+    unsigned counter;
+    int deterministic;                // 1: argmax (first maximum); 0: inverse-CDF draw from softmax(logits)
+    long long row_id_base;
+    float *log_prob;                  // [n] log softmax(logits)[action]
+    float *value;                     // [n] the value head
 };
 
 // Shared-memory operand layout (no swizzle): 8 x 8 bf16 core matrices of 128 contiguous bytes (row r of the core matrix at
@@ -100,6 +114,61 @@ __device__ __forceinline__ void pl_tmem_ld16(unsigned taddr, float (&v)[16]) {
     for (int i = 0; i < 16; i++) v[i] = __uint_as_float(r[i]);
 }
 
+// Output layer of the sampling instance, one thread = one row, all in registers (static indices over the 15 possible logits):
+// l_a = acc_a + bias_a, m = max l, e_a = expf(l_a - m), S = e_0 + ... in index order; the action is the argmax (deterministic)
+// or the smallest a with u S < e_0 + ... + e_a for u = (Philox word 0 >> 8) 2^-24 (the last action if rounding leaves none);
+// log_prob = l_a - m - logf(S).  expf / logf, not the intrinsics: 15 values per row.
+__device__ __forceinline__ void pl_sample_epilogue(const PolicyParams &pp, const PolicyDraw &dr, const float (&v)[16], const float *b,
+                                                   int env, int *actions) {
+    constexpr int NA = PL_NOUT - 1;
+    const int na = pp.n_actions;
+    float l[NA], m = v[0] + b[0];
+#pragma unroll
+    for (int a = 0; a < NA; a++) {
+        l[a] = v[a] + b[a];
+        if (a < na && l[a] > m) m = l[a];
+    }
+    float value = 0.0f;
+#pragma unroll
+    for (int a = 1; a < PL_NOUT; a++)
+        if (a == na) value = v[a] + b[a];
+    if (dr.value) dr.value[env] = value;
+    if (!actions && !dr.log_prob) return;                           // a critic launch: the value only
+    float e[NA], S = 0.0f;
+#pragma unroll
+    for (int a = 0; a < NA; a++) {
+        e[a] = a < na ? expf(l[a] - m) : 0.0f;
+        S += e[a];                                                   // (+ 0.0f beyond n_actions: exact)
+    }
+    int pick = 0;
+    if (dr.deterministic) {
+        float bv = l[0];
+#pragma unroll
+        for (int a = 1; a < NA; a++)
+            if (a < na && l[a] > bv) { bv = l[a]; pick = a; }
+    } else {
+        uint32_t c[4] = {dr.counter_dev ? dr.counter_dev[env] : dr.counter, 0u, (uint32_t)(unsigned long long)(dr.row_id_base + env), 3u};
+        philox4x32_10(c, (uint32_t)dr.seed, (uint32_t)(dr.seed >> 32));
+        const float us = (float)(c[0] >> 8) * 0x1p-24f * S;
+        float acc = 0.0f;
+        bool found = false;
+        pick = na - 1;
+#pragma unroll
+        for (int a = 0; a < NA; a++) {
+            if (a < na) {
+                acc += e[a];
+                if (!found && us < acc) { pick = a; found = true; }
+            }
+        }
+    }
+    float lp = l[0];
+#pragma unroll
+    for (int a = 1; a < NA; a++)
+        if (a == pick) lp = l[a];
+    if (actions) actions[env] = pick;
+    if (dr.log_prob) dr.log_prob[env] = lp - m - logf(S);
+}
+
 // Two groups of EIGHT warps per CTA, each walking its own stream of 128-environment tiles with its own A buffer, TMEM accumulator
 // and mbarrier (they only share the weights): one group's tensor-core work and TMEM reads overlap the other's epilogue math.
 // Inside a group warp w reads TMEM lanes 32 (w % 4) .. + 31 (the hardware's lane quarter of a warp) and takes columns
@@ -112,9 +181,12 @@ __device__ __forceinline__ void pl_group_sync(int group) {          // named bar
     asm volatile("bar.sync %0, %1;" ::"r"(group + 1), "n"(PL_WG) : "memory");
 }
 
+// SAMPLE = false: orlg_policy_act (argmax, optional logits; `dr` unused).  SAMPLE = true: orlg_policy_sample (the epilogue
+// of PolicyDraw; `actions` may be NULL, `logits_out` is unused).
+template <bool SAMPLE>
 __global__ void __launch_bounds__(PL_WG * PL_GROUPS, 1)
 mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const int n, int *__restrict__ actions,
-                  float *__restrict__ logits_out /* [n, 6] = 5 logits + value, or NULL */) {
+                  float *__restrict__ logits_out /* [n, 6] = 5 logits + value, or NULL */, const PolicyDraw dr) {
     extern __shared__ __align__(128) unsigned char psm[];
     const int group = threadIdx.x / PL_WG, tid = threadIdx.x % PL_WG, warp = (tid >> 5) & 3;     // warp = TMEM lane quarter of this warp
     const int half = tid >> 7;        // which 64 of the 128 columns (K elements of the next layer) this thread produces
@@ -268,7 +340,9 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
                 if (half == 0) {                                   // warp-uniform: the four warps of the first half hold the 128 rows
                     float v[16];
                     pl_tmem_ld16(t_lane, v);
-                    if (env < n) {
+                    if (SAMPLE) {
+                        if (env < n) pl_sample_epilogue(pp, dr, v, b, env, actions);
+                    } else if (env < n) {
                         int best = 0;
                         float bv = v[0] + b[0];
 #pragma unroll

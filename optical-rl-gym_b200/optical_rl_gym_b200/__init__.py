@@ -2,7 +2,8 @@
 from .topology import (TopologyTables, get_topology, load_reference_pickle, nsfnet, read_sndlib_topology,  # noqa: F401
                        read_txt_file, synthetic_ring_chords)
 
-_LAZY = {"OpticalVecEnv": "vec_env", "make": "vec_env", "StepInfo": "vec_env", "COUNTER_NAMES": "vec_env"}
+_LAZY = {"OpticalVecEnv": "vec_env", "make": "vec_env", "StepInfo": "vec_env", "COUNTER_NAMES": "vec_env",
+         "PolicyRollout": "vec_env"}
 
 
 def __getattr__(name):      # torch / CUDA are imported lazily so that the topology tools work anywhere

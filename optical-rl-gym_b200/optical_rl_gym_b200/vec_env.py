@@ -12,7 +12,7 @@ reference's ``reset(only_episode_counters=True)`` (``rmsa_env.py:284-330``).
 from __future__ import annotations
 
 import ctypes as C
-from typing import Optional
+from typing import NamedTuple, Optional
 
 import numpy as np
 import torch
@@ -97,6 +97,16 @@ class StepInfo:
 
     def items(self):
         return [(k, self[k]) for k in self._keys]
+
+
+class PolicyRollout(NamedTuple):
+    """A PPO rollout buffer filled on the device by :meth:`OpticalVecEnv.rollout_policy` (T steps of N envs)."""
+    obs: torch.Tensor          # float32 [T + 1, N, obs_dim]: obs[0] = the pending request's observation, obs[t + 1] = step t's
+    actions: torch.Tensor      # int32 [T, N]
+    log_prob: torch.Tensor     # float32 [T, N]: log softmax(logits)[action]
+    value: torch.Tensor        # float32 [T + 1, N]: V(obs[t]); value[T] = the bootstrap value of the last observation
+    reward: torch.Tensor       # float32 [T, N]
+    done: torch.Tensor         # uint8 [T, N]
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -390,6 +400,44 @@ class OpticalVecEnv:
         with torch.cuda.device(self._dev_index):
             nat.check(self._lib.orlg_rollout(self._h, T, pol, _ptr(obs), _ptr(reward), _ptr(done), _ptr(actions), self._stream()))
         return obs, reward, done, actions
+
+    def rollout_policy(self, policy, steps: int, *, deterministic: bool = False, seed: Optional[int] = None,
+                       out: Optional[PolicyRollout] = None) -> PolicyRollout:
+        """``steps`` iterations of ``a, log p(a), V(obs) = policy(obs); obs, r, done = env.step(a)`` in ONE native call
+        (``orlg_rollout_policy``): a :class:`PolicyRollout` of device tensors, what SB3's ``collect_rollouts`` gathers.
+        ``policy`` is an :class:`~optical_rl_gym_b200.policy.MlpPolicy` on this device (its current weights; the value comes
+        from its critic trunk when it has one).  Actions are drawn from softmax(logits) (``deterministic=True``: argmax) with
+        Philox stream 3 keyed by ``seed`` (default: the env's seed), the global env id and the env's request index, so the
+        result does not depend on the number of GPUs, on how the rollout is split into calls or on a checkpoint in between.
+        ``out`` reuses the buffers of an earlier call.  DeepRMSA-v0 with float32 observations."""
+        T, n, dev = int(steps), self.num_envs, self.device
+        if T < 0:
+            raise ValueError("steps must be >= 0")
+        if out is None:
+            out = PolicyRollout(torch.empty((T + 1, n, self.obs_dim), dtype=torch.float32, device=dev),
+                                torch.empty((T, n), dtype=torch.int32, device=dev),
+                                torch.empty((T, n), dtype=torch.float32, device=dev),
+                                torch.empty((T + 1, n), dtype=torch.float32, device=dev),
+                                torch.empty((T, n), dtype=torch.float32, device=dev),
+                                torch.empty((T, n), dtype=torch.uint8, device=dev))
+        want = (((T + 1, n, self.obs_dim), torch.float32), ((T, n), torch.int32), ((T, n), torch.float32),
+                ((T + 1, n), torch.float32), ((T, n), torch.float32), ((T, n), torch.uint8))
+        for name, tns, (shape, dt) in zip(PolicyRollout._fields, out, want):
+            if tuple(tns.shape) != shape or tns.dtype != dt or tns.device != dev or not tns.is_contiguous():
+                raise ValueError("out.%s must be a contiguous %s tensor %s on %s, got %s %s %s" % (
+                    name, dt, shape, dev, tuple(tns.shape), tns.dtype, tns.device))
+        actor, critic = policy._native_handles(self._dev_index)
+        key = self.rand_seed if seed is None else int(seed)
+        with torch.cuda.device(self._dev_index):
+            nat.check(self._lib.orlg_rollout_policy(self._h, T, actor, critic, key & (2 ** 64 - 1), int(bool(deterministic)),
+                                                    *[_ptr(t) for t in out], self._stream()))
+        return out
+
+    @property
+    def request_index(self) -> int:
+        """Requests drawn so far by every env (they step together): counter word 0 of the action draws of the next
+        :meth:`rollout_policy` step, for a Python loop that wants the same keying (``MlpPolicy.sample_native(counter=...)``)."""
+        return int(self._lib.orlg_request_index(self._h))
 
     def rollout_packed(self, steps: int, policy="random", out=None):
         """Like :meth:`rollout`, but ONE 32-byte record per env-step (int32 ``[T, N, 8]`` on the device): the integer
