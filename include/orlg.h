@@ -181,15 +181,9 @@ int orlg_expand_packed(const uint32_t *packed_host, int64_t rows, int num_nodes,
 /* orlg_rollout with HOST buffers (pageable or pinned): the steps run in chunks on the device while the previous chunk's
  * records cross PCIe and are expanded by a persistent pool of `threads` host threads (<= 0: all cores).  obs_host f32
  * [steps, num_envs, obs_dim] etc.; any output may be NULL.  With ORLG_POLICY_REPLAY actions_host is the INPUT: the action of
- * every env at every step, copied to the device chunk by chunk ahead of the kernel that consumes it.
- * Opt-in (environment ORLG_HOST_DMA_FRACTION=<share> or ORLG_HOST_DMA=auto) and only when obs_host is page-locked
- * (cudaHostAlloc / cudaHostRegister / torch pin_memory): the float32 rows of the first envs of every step are copied by DMA
- * straight into it while the host threads expand the records of the others; "auto" adapts the share to the measured copy and
- * decode rates (orlg_host_dma_fraction). */
+ * every env at every step, copied to the device chunk by chunk ahead of the kernel that consumes it. */
 int orlg_rollout_host(orlg_env *env, int steps, int policy, float *obs_host, float *reward_host, uint8_t *done_host,
                       int32_t *actions_host, int chunk_steps, int threads, orlg_stream stream);
-/* share of the envs whose observation rows the last orlg_rollout_host calls delivered by DMA (0 when the buffer was pageable) */
-double orlg_host_dma_fraction(const orlg_env *env);
 
 /* ---- the PPO agent of the reference's notebook, evaluated on the device ------------------------------------------ */
 /* model.predict(obs, deterministic=True) of the agent the reference trains and ships (examples/stable_baselines3/

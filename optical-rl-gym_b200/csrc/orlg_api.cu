@@ -4,7 +4,6 @@
 #include <condition_variable>
 #include <cstdio>
 #include <cstdlib>
-#include <chrono>
 #include <cstring>
 #include <emmintrin.h>
 #include <functional>
@@ -72,12 +71,6 @@ struct orlg_env {
     cudaStream_t ro_copy_stream = nullptr;         // D2H of chunk c overlaps the kernel of chunk c + 1
     int32_t *ro_act_dev[RO_HOST_BUFFERS] = {};     // ORLG_POLICY_REPLAY: the host's action chunks on the device
     size_t ro_act_rows = 0;
-    // ... and, when the caller's observation buffer is pinned, the float32 rows of the first envs of every step go straight
-    // into it by DMA while the host threads expand the records of the others (the split follows the two measured rates)
-    float *ro_obs_dev[RO_HOST_BUFFERS] = {};
-    size_t ro_obs_rows = 0;
-    cudaEvent_t ro_cp_ev[RO_HOST_BUFFERS] = {};    // start of the chunk's copies (copy stream, timed)
-    double ro_dma_frac = -1.0;                     // share of the envs whose rows travel by DMA (< 0: not initialised)
     int *ro_actions = nullptr;    // [n, action_dim] scratch of the generic (kernel-per-step) rollout
 };
 
@@ -180,10 +173,9 @@ void launch_step_kind(const orlg_env *env, const StepIO &io, int mode, cudaStrea
 
 // launch configuration with the programmatic-stream-serialization attribute (griddepcontrol in the kernels)
 cudaLaunchConfig_t pdl_config(int blocks, int threads, size_t smem, cudaStream_t s) {
-    static const bool off = std::getenv("ORLG_NO_PDL") != nullptr;
     static thread_local cudaLaunchAttribute g_pdl_attr[1];          // one host thread per handle (orlg.h)
     g_pdl_attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    g_pdl_attr[0].val.programmaticStreamSerializationAllowed = off ? 0 : 1;
+    g_pdl_attr[0].val.programmaticStreamSerializationAllowed = 1;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)blocks);
     cfg.blockDim = dim3((unsigned)threads);
@@ -540,7 +532,7 @@ int orlg_create(const orlg_config *cfg, const orlg_tables *t, int device, orlg_e
     env->fast = false;
     env->hot = false;
     env->ro_ok = false;
-    if (!wide && cfg->kind != ORLG_RMCSA && p.k <= 5 && P <= 65535 && se_max <= 15 && !std::getenv("ORLG_FORCE_GENERIC")) {
+    if (!wide && cfg->kind != ORLG_RMCSA && p.k <= 5 && P <= 65535 && se_max <= 15) {
         std::vector<unsigned char> blob;
         auto put = [&blob](const void *src, size_t bytes) {
             size_t off = (blob.size() + 15) / 16 * 16;
@@ -654,8 +646,6 @@ int orlg_destroy(orlg_env *env) {
         if (env->ro_pk_ev[i]) cudaEventDestroy(env->ro_pk_ev[i]);
         if (env->ro_k_ev[i]) cudaEventDestroy(env->ro_k_ev[i]);
         if (env->ro_act_dev[i]) cudaFree(env->ro_act_dev[i]);
-        if (env->ro_obs_dev[i]) cudaFree(env->ro_obs_dev[i]);
-        if (env->ro_cp_ev[i]) cudaEventDestroy(env->ro_cp_ev[i]);
     }
     if (env->ro_copy_stream) cudaStreamDestroy(env->ro_copy_stream);
     delete env;
@@ -1005,7 +995,7 @@ static int rollout_impl(orlg_env *env, int steps, int policy, void *obs_dev, flo
     else if (p.kind == ORLG_DEEPRMSA) policy_ok = policy == ORLG_POLICY_RANDOM || policy == ORLG_POLICY_REPLAY || policy == ORLG_HEUR_SP_FF || policy == ORLG_HEUR_SAP_FF;
     else if (p.kind == ORLG_RMSA) policy_ok = policy != ORLG_HEUR_SAP_LF;
     else policy_ok = true;
-    const bool persistent = env->ro_ok && !p.stats && !p.obs_f64 && !p.br_hist && policy_ok && !std::getenv("ORLG_NO_ROLLOUT_KERNEL");
+    const bool persistent = env->ro_ok && !p.stats && !p.obs_f64 && !p.br_hist && policy_ok;
     RolloutArgs ra;
     std::memset(&ra, 0, sizeof(ra));
     int wpc = 0;
@@ -1052,7 +1042,7 @@ static int rollout_impl(orlg_env *env, int steps, int policy, void *obs_dev, flo
     }
     const size_t obs_row = (size_t)p.obs_dim * (p.obs_f64 ? 8 : 4);
     // wide kernels: the heuristic runs in the step kernel's prologue (one launch per step; the chosen path's masks are read once)
-    bool fuse = env->wide && policy >= 0 && !std::getenv("ORLG_NO_FUSED_HEURISTIC");
+    bool fuse = env->wide && policy >= 0;
     if (fuse && ((p.kind == ORLG_RMSA && policy == ORLG_HEUR_SAP_LF) || (p.kind == ORLG_DEEPRMSA && policy > ORLG_HEUR_SAP_FF))) fuse = false;
     for (int t = 0; t < steps; t++) {
         int32_t *a = actions_dev ? actions_dev + (size_t)t * p.n * adim : env->ro_actions;
@@ -1227,10 +1217,8 @@ void expand_rows(const ExpandTables &tb, const uint32_t *pk, int64_t r0, int64_t
 }
 }  // namespace
 
-// rows = [step][env] records of `n_envs` envs per step; the observation rows of envs [0, n_skip) of every step are NOT written
-// (orlg_rollout_host delivers them by DMA), their reward / done / action are.
-static int expand_packed_split(const uint32_t *packed_host, int64_t rows, int num_nodes, int num_slots, float *obs_host, float *reward_host,
-                               uint8_t *done_host, int32_t *action_host, int threads, int64_t n_envs, int64_t n_skip) {
+int orlg_expand_packed(const uint32_t *packed_host, int64_t rows, int num_nodes, int num_slots, float *obs_host, float *reward_host,
+                       uint8_t *done_host, int32_t *action_host, int threads) {
     if (!packed_host || rows < 0 || num_nodes < 2 || num_nodes > 255 || num_slots < 1) return fail(ORLG_E_INVALID, "bad arguments");
     int nt = threads > 0 ? threads : (int)std::thread::hardware_concurrency();
     if (nt < 1) nt = 1;
@@ -1239,27 +1227,14 @@ static int expand_packed_split(const uint32_t *packed_host, int64_t rows, int nu
     const int64_t blocks = (rows + JOB - 1) / JOB;
     if ((int64_t)nt > blocks) nt = (int)blocks;
     auto job = [&](int64_t b) {
-        int64_t r0 = b * JOB;
+        const int64_t r0 = b * JOB;
         const int64_t r1 = r0 + JOB < rows ? r0 + JOB : rows;
-        if (n_skip <= 0 || !obs_host) { expand_rows(tb, packed_host, r0, r1, num_nodes, obs_host, reward_host, done_host, action_host); return; }
-        while (r0 < r1) {                  // pieces that lie entirely inside / outside the DMA share of their step
-            const int64_t e = r0 % n_envs;
-            const bool skip = e < n_skip;
-            const int64_t lim = skip ? n_skip - e : n_envs - e;
-            const int64_t r2 = r0 + lim < r1 ? r0 + lim : r1;
-            expand_rows(tb, packed_host, r0, r2, num_nodes, skip ? nullptr : obs_host, reward_host, done_host, action_host);
-            r0 = r2;
-        }
+        expand_rows(tb, packed_host, r0, r1, num_nodes, obs_host, reward_host, done_host, action_host);
     };
     if (nt <= 1) { for (int64_t b = 0; b < blocks; b++) job(b); return ORLG_OK; }
     std::lock_guard<std::mutex> lk(g_pool_mu);
     g_pool.run(nt, blocks, job);
     return ORLG_OK;
-}
-
-int orlg_expand_packed(const uint32_t *packed_host, int64_t rows, int num_nodes, int num_slots, float *obs_host, float *reward_host,
-                       uint8_t *done_host, int32_t *action_host, int threads) {
-    return expand_packed_split(packed_host, rows, num_nodes, num_slots, obs_host, reward_host, done_host, action_host, threads, rows > 0 ? rows : 1, 0);
 }
 
 int orlg_rollout_host(orlg_env *env, int steps, int policy, float *obs_host, float *reward_host, uint8_t *done_host,
@@ -1299,68 +1274,21 @@ int orlg_rollout_host(orlg_env *env, int steps, int policy, float *obs_host, flo
     const int nchunks = (steps + chunk - 1) / chunk;
     const size_t D = (size_t)p.obs_dim;
     cudaStream_t sc = env->ro_copy_stream;
-    // Hybrid delivery of the observation rows.  The host threads expand the records at the host's streaming-store bandwidth;
-    // PCIe is idle meanwhile (the records are 32 of the 253 bytes a row set weighs).  When the caller's observation buffer is
-    // page-locked, the rows of envs [0, n_dma) of every step are written by the kernel as float32 (the same bits the decoder
-    // produces) and copied by DMA straight into the caller's buffer (one 2-D copy per chunk), the host expands the others.
-    // OPT-IN (ORLG_HOST_DMA_FRACTION=<share>, or ORLG_HOST_DMA=auto: the share follows the measured copy and decode rates of the
-    // previous chunks): on the boxes this was measured on (PCIe at 47 GB/s, 16 host cores) the DMA writes and the decoder's
-    // streaming stores compete for the same host memory bandwidth and the best share gains 2 % (profiles/r2_experiments.md).
-    bool pinned = false;
-    const char *dma_fixed = std::getenv("ORLG_HOST_DMA_FRACTION"), *dma_mode = std::getenv("ORLG_HOST_DMA");
-    const bool dma_auto = dma_mode && std::strcmp(dma_mode, "auto") == 0;
-    if (obs_host && p.kind == ORLG_DEEPRMSA && p.n >= 8192 && (dma_fixed || dma_auto)) {
-        cudaPointerAttributes at;
-        if (cudaPointerGetAttributes(&at, obs_host) == cudaSuccess) pinned = at.type == cudaMemoryTypeHost;
-        else cudaGetLastError();
-    }
-    if (pinned) {
-        if (env->ro_obs_rows < rows) {
-            for (int i = 0; i < NB; i++) {
-                if (env->ro_obs_dev[i]) cudaFree(env->ro_obs_dev[i]);
-                env->ro_obs_dev[i] = nullptr;
-                if (cudaMalloc(&env->ro_obs_dev[i], rows * D * sizeof(float)) != cudaSuccess) return fail(ORLG_E_NOMEM, "cudaMalloc (observation chunks) failed");
-            }
-            env->ro_obs_rows = rows;
-        }
-        for (int i = 0; i < NB; i++)
-            if (!env->ro_cp_ev[i]) {
-                CUDA_OK(cudaEventCreate(&env->ro_cp_ev[i]));
-                if (env->ro_pk_ev[i]) cudaEventDestroy(env->ro_pk_ev[i]);
-                CUDA_OK(cudaEventCreate(&env->ro_pk_ev[i]));             // timed from here on
-            }
-        if (env->ro_dma_frac < 0.0) env->ro_dma_frac = 0.2;
-        if (dma_fixed) { const double f = std::atof(dma_fixed); if (f >= 0.0 && f <= 0.95) env->ro_dma_frac = f; }
-    }
-    const bool adapt = pinned && !dma_fixed;
-    constexpr int64_t GRAN = 2048;                       // the decoder's job size: a job is either all DMA or all decode
-    int64_t ndma_of[NB] = {};
-    auto dma_envs = [&]() -> int64_t {
-        if (!pinned) return 0;
-        int64_t v = (int64_t)(env->ro_dma_frac * (double)p.n) / GRAN * GRAN;
-        return v < 0 ? 0 : (v > p.n ? (int64_t)p.n : v);
-    };
-    // chunk c: [user stream] H2D of its actions, the rollout kernel -> [copy stream] D2H of its records (+ DMA rows).  The kernel
+    // chunk c: [user stream] H2D of its actions, the rollout kernel -> [copy stream] D2H of its records.  The kernel
     // of chunk c + 1 overlaps the copy of chunk c; buffer b = c % NB is reused by chunk c + NB, whose kernel waits for the copy
     // of chunk c (event) and which is only enqueued after the host has decoded chunk c (program order below).
     auto enqueue = [&](int c) -> int {
         const int b = c % NB, t0 = c * chunk, tc = steps - t0 < chunk ? steps - t0 : chunk;
-        const int64_t nd = dma_envs();
-        ndma_of[b] = nd;
         if (replay)
             CUDA_OK(cudaMemcpyAsync(env->ro_act_dev[b], actions_host + (size_t)t0 * p.n * adim, (size_t)tc * p.n * adim * sizeof(int32_t),
                                     cudaMemcpyHostToDevice, s));
         if (c >= NB) CUDA_OK(cudaStreamWaitEvent(s, env->ro_pk_ev[b], 0));
-        int rc = rollout_impl(env, tc, policy, nd > 0 ? env->ro_obs_dev[b] : nullptr, nullptr, nullptr, replay ? env->ro_act_dev[b] : nullptr,
+        int rc = rollout_impl(env, tc, policy, nullptr, nullptr, nullptr, replay ? env->ro_act_dev[b] : nullptr,
                               reinterpret_cast<uint32_t *>(env->ro_pk_dev[b]), stream);
         if (rc) return rc;
         CUDA_OK(cudaEventRecord(env->ro_k_ev[b], s));
         CUDA_OK(cudaStreamWaitEvent(sc, env->ro_k_ev[b], 0));
-        if (pinned) CUDA_OK(cudaEventRecord(env->ro_cp_ev[b], sc));
         CUDA_OK(cudaMemcpyAsync(env->ro_pk_host[b], env->ro_pk_dev[b], (size_t)tc * p.n * 32, cudaMemcpyDeviceToHost, sc));
-        if (nd > 0)
-            CUDA_OK(cudaMemcpy2DAsync(obs_host + (size_t)t0 * p.n * D, (size_t)p.n * D * sizeof(float), env->ro_obs_dev[b],
-                                      (size_t)p.n * D * sizeof(float), (size_t)nd * D * sizeof(float), (size_t)tc, cudaMemcpyDeviceToHost, sc));
         CUDA_OK(cudaEventRecord(env->ro_pk_ev[b], sc));
         return ORLG_OK;
     };
@@ -1370,33 +1298,15 @@ int orlg_rollout_host(orlg_env *env, int steps, int policy, float *obs_host, flo
         const int b = c % NB, t0 = c * chunk, tc = steps - t0 < chunk ? steps - t0 : chunk;
         CUDA_OK(cudaEventSynchronize(env->ro_pk_ev[b]));
         const size_t off = (size_t)t0 * p.n;
-        const auto w0 = std::chrono::steady_clock::now();
-        int rc = expand_packed_split(reinterpret_cast<const uint32_t *>(env->ro_pk_host[b]), (int64_t)tc * p.n, p.N, p.S,
-                                     obs_host ? obs_host + off * D : nullptr, reward_host ? reward_host + off : nullptr,
-                                     done_host ? done_host + off : nullptr, (actions_host && !replay) ? actions_host + off : nullptr, threads,
-                                     (int64_t)p.n, ndma_of[b]);
+        int rc = orlg_expand_packed(reinterpret_cast<const uint32_t *>(env->ro_pk_host[b]), (int64_t)tc * p.n, p.N, p.S,
+                                    obs_host ? obs_host + off * D : nullptr, reward_host ? reward_host + off : nullptr,
+                                    done_host ? done_host + off : nullptr, (actions_host && !replay) ? actions_host + off : nullptr, threads);
         if (rc) return rc;
-        if (adapt && tc == chunk) {
-            // bytes per millisecond of the two paths on this chunk -> the share at which both would take the same time
-            const double t_dec = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - w0).count();
-            float t_cp = 0.0f;
-            if (cudaEventElapsedTime(&t_cp, env->ro_cp_ev[b], env->ro_pk_ev[b]) == cudaSuccess && t_cp > 0.0f && t_dec > 0.0) {
-                const double O = (double)tc * p.n * D * 4.0, P = (double)tc * p.n * 32.0, f = (double)ndma_of[b] / (double)p.n;
-                const double r_d = (P + f * O) / (double)t_cp, r_c = ((1.0 - f) * O + P) / t_dec;
-                double f_new = (O / r_c - P / r_d) / (O / r_d + O / r_c);
-                f_new = f_new < 0.0 ? 0.0 : (f_new > 0.9 ? 0.9 : f_new);
-                env->ro_dma_frac = 0.5 * env->ro_dma_frac + 0.5 * f_new;
-            } else {
-                cudaGetLastError();
-            }
-        }
     }
     // the user's stream must not run ahead of the copies that still read the record buffers (a later call reuses them)
     CUDA_OK(cudaStreamWaitEvent(s, env->ro_pk_ev[(nchunks - 1) % NB], 0));
     return ORLG_OK;
 }
-
-double orlg_host_dma_fraction(const orlg_env *env) { return env && env->ro_dma_frac > 0.0 ? env->ro_dma_frac : 0.0; }
 
 // ---------------------------------------------------------------- the shipped PPO agent (orlg_policy.cuh)
 struct orlg_policy {

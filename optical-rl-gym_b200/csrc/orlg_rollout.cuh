@@ -31,10 +31,6 @@
 #pragma once
 #include "orlg_deeprmsa_fast.cuh"
 
-#ifndef ORLG_RO_BULK
-#define ORLG_RO_BULK 1          // observation tile leaves by one bulk (TMA) store per warp; 0 = coalesced 16-byte stores
-#endif
-
 namespace orlg {
 
 constexpr int RO_WCAP = 64;            // window entries per env
@@ -771,7 +767,7 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
                                 rec_flags & 0xffffu, 0u);
         }
         if (KIND == ORLG_DEEPRMSA && ra.obs) {
-            // ---- the warp's 32 rows = one contiguous run of obs[t]: written to a pool tile, copied out with coalesced 16-byte stores
+            // ---- the warp's 32 rows = one contiguous run of obs[t]: written to a pool tile, copied out by one bulk (TMA) store
             const unsigned tile = ro_tile_acquire(pool_free, lane);
             unsigned char *stage = pool + (size_t)tile * ra.tile_bytes;
             RPH_MARK(4);             // tile acquisition
@@ -807,7 +803,6 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
             {
                 float *g = ra.obs + ((size_t)t * p.n + env0) * p.obs_dim;
                 const int total_el = nvalid * p.obs_dim;
-#if ORLG_RO_BULK
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                 __syncwarp();
                 if ((reinterpret_cast<size_t>(g) & 15) == 0 && (total_el & 3) == 0) {
@@ -821,18 +816,6 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
                     const float *sv = reinterpret_cast<const float *>(stage);
                     for (int q = lane; q < total_el; q += 32) g[q] = sv[q];
                 }
-#else
-                __syncwarp();
-                if ((reinterpret_cast<size_t>(g) & 15) == 0 && (total_el & 3) == 0) {
-                    const uint4 *sv = reinterpret_cast<const uint4 *>(stage);
-                    uint4 *gv = reinterpret_cast<uint4 *>(g);
-#pragma unroll 7
-                    for (int q = lane; q < total_el / 4; q += 32) gv[q] = sv[q];
-                } else {
-                    const float *sv = reinterpret_cast<const float *>(stage);
-                    for (int q = lane; q < total_el; q += 32) g[q] = sv[q];
-                }
-#endif
             }
             ro_tile_release(pool_free, tile, lane);
         }

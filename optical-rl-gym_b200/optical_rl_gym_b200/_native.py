@@ -78,8 +78,6 @@ def lib():
     L.orlg_state_bytes.argtypes = [vp]
     L.orlg_state_bytes.restype = i64
     L.orlg_kernel_info.argtypes = [vp, C.POINTER(KernelInfo)]
-    L.orlg_host_dma_fraction.argtypes = [vp]
-    L.orlg_host_dma_fraction.restype = C.c_double
     L.orlg_set_trace.argtypes = [vp, vp, i64]
     L.orlg_seed.argtypes = [vp, C.c_uint64]
     L.orlg_reset.argtypes = [vp, i32, vp, vp]
@@ -132,5 +130,5 @@ EXPORTED = ["orlg_create", "orlg_destroy", "orlg_last_error", "orlg_version", "o
             "orlg_observation", "orlg_observation_int", "orlg_heuristic", "orlg_random_actions", "orlg_get_counters",
             "orlg_get_requests", "orlg_export_state", "orlg_error_flags", "orlg_reduce_counters", "orlg_enable_stats",
             "orlg_num_bit_rates", "orlg_bit_rate_blocking", "orlg_matrix_obs_dim", "orlg_matrix_observation",
-            "orlg_path_only_first_fit", "orlg_rollout", "orlg_state_save_bytes", "orlg_state_save", "orlg_state_load", "orlg_policy_create", "orlg_policy_act", "orlg_policy_destroy", "orlg_rollout_packed", "orlg_expand_packed", "orlg_rollout_host", "orlg_host_dma_fraction", "orlg_action_hist_dim", "orlg_action_probability",
+            "orlg_path_only_first_fit", "orlg_rollout", "orlg_state_save_bytes", "orlg_state_save", "orlg_state_load", "orlg_policy_create", "orlg_policy_act", "orlg_policy_destroy", "orlg_rollout_packed", "orlg_expand_packed", "orlg_rollout_host", "orlg_action_hist_dim", "orlg_action_probability",
             "orlg_enable_link_stats", "orlg_link_stats", "orlg_policy_sample", "orlg_rollout_policy", "orlg_request_index"]

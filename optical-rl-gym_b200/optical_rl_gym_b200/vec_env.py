@@ -468,9 +468,7 @@ class OpticalVecEnv:
     def rollout_host(self, steps: int, policy="random", *, obs=None, reward=None, done=None, actions=None, chunk: int = 8,
                      threads: int = 0):
         """:meth:`rollout` with the results delivered in HOST memory (numpy arrays, pageable is fine): the device runs chunk
-        c + 1 while chunk c's packed records cross PCIe and the host threads expand them (``orlg_rollout_host``).  Opt-in
-        (``ORLG_HOST_DMA=auto`` or ``ORLG_HOST_DMA_FRACTION=<share>`` in the environment) and with a page-locked ``obs``
-        (``torch.empty(..., pin_memory=True).numpy()``), part of every step's rows is written by DMA straight into it.
+        c + 1 while chunk c's packed records cross PCIe and the host threads expand them (``orlg_rollout_host``).
         ``policy="replay"``: ``actions`` (int32 ``[steps, num_envs]``, host) is the input action sequence."""
         T, n = int(steps), self.num_envs
         if policy == "replay":
@@ -490,10 +488,6 @@ class OpticalVecEnv:
                                                   done.ctypes.data_as(C.c_void_p), actions.ctypes.data_as(C.c_void_p),
                                                   int(chunk), int(threads), self._stream()))
         return obs, reward, done, actions
-
-    def host_dma_fraction(self) -> float:
-        """Share of the envs whose observation rows :meth:`rollout_host` currently delivers by DMA (0: pageable buffers)."""
-        return float(self._lib.orlg_host_dma_fraction(self._h))
 
     def observation(self):
         if not self.obs_dim:
