@@ -1,4 +1,5 @@
 // orlg_api.cu -- the C ABI (include/orlg.h) on top of the step kernels.  Links cudart only.
+#include <algorithm>
 #include <atomic>
 #include <cmath>
 #include <condition_variable>
@@ -11,6 +12,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "orlg_deeprmsa_fast.cuh"
@@ -37,21 +39,70 @@ static int fail(int code, const std::string &msg) {
 
 constexpr int RO_HOST_BUFFERS = 3;       // orlg_rollout_host: record buffers in flight (device runs two chunks ahead of the decoder)
 
+namespace {
+// orlg_rollout_host: packed records on the device and in pinned host memory, the copy stream with its events, and the device
+// copies of replayed action chunks.  Allocated by the first call, grown by later calls that need more rows.
+struct HostPipeline {
+    uint4 *pk_dev[RO_HOST_BUFFERS] = {};
+    uint4 *pk_host[RO_HOST_BUFFERS] = {};
+    size_t pk_rows = 0;                        // rows (env-steps) each buffer holds
+    cudaEvent_t pk_ev[RO_HOST_BUFFERS] = {};   // records of the chunk are in pinned host memory (copy stream)
+    cudaEvent_t k_ev[RO_HOST_BUFFERS] = {};    // the chunk's kernel is done (user stream)
+    cudaStream_t copy_stream = nullptr;        // D2H of chunk c overlaps the kernel of chunk c + 1
+    int32_t *act_dev[RO_HOST_BUFFERS] = {};    // ORLG_POLICY_REPLAY: the host's action chunks on the device
+    size_t act_rows = 0;
+
+    int reserve(size_t rows, bool replay, size_t action_dim) {
+        if (pk_rows < rows) {                  // (re)allocate the record buffers (device + pinned host)
+            for (int i = 0; i < RO_HOST_BUFFERS; i++) {
+                if (pk_dev[i]) cudaFree(pk_dev[i]);
+                if (pk_host[i]) cudaFreeHost(pk_host[i]);
+                pk_dev[i] = nullptr; pk_host[i] = nullptr;
+                if (cudaMalloc(&pk_dev[i], rows * 32) != cudaSuccess) return fail(ORLG_E_NOMEM, "cudaMalloc (packed records) failed");
+                if (cudaHostAlloc(&pk_host[i], rows * 32, cudaHostAllocDefault) != cudaSuccess) return fail(ORLG_E_NOMEM, "cudaHostAlloc (packed records) failed");
+                if (!pk_ev[i]) CUDA_OK(cudaEventCreateWithFlags(&pk_ev[i], cudaEventDisableTiming));
+                if (!k_ev[i]) CUDA_OK(cudaEventCreateWithFlags(&k_ev[i], cudaEventDisableTiming));
+            }
+            pk_rows = rows;
+        }
+        if (!copy_stream) CUDA_OK(cudaStreamCreateWithFlags(&copy_stream, cudaStreamNonBlocking));
+        if (replay && act_rows < rows) {       // device copies of the action chunks
+            for (int i = 0; i < RO_HOST_BUFFERS; i++) {
+                if (act_dev[i]) cudaFree(act_dev[i]);
+                act_dev[i] = nullptr;
+                if (cudaMalloc(&act_dev[i], rows * action_dim * sizeof(int32_t)) != cudaSuccess) return fail(ORLG_E_NOMEM, "cudaMalloc (action chunks) failed");
+            }
+            act_rows = rows;
+        }
+        return ORLG_OK;
+    }
+    ~HostPipeline() {
+        for (int i = 0; i < RO_HOST_BUFFERS; i++) {
+            if (pk_dev[i]) cudaFree(pk_dev[i]);
+            if (pk_host[i]) cudaFreeHost(pk_host[i]);
+            if (pk_ev[i]) cudaEventDestroy(pk_ev[i]);
+            if (k_ev[i]) cudaEventDestroy(k_ev[i]);
+            if (act_dev[i]) cudaFree(act_dev[i]);
+        }
+        if (copy_stream) cudaStreamDestroy(copy_stream);
+    }
+};
+}  // namespace
+
+// Owns every device resource of a handle.  Deleted on the handle's device (orlg_destroy).
 struct orlg_env {
     Params p;
     orlg_config cfg;
     int device;
-    int km;                       // KM template instance (5 or 8)
-    bool fast;                    // DeepRMSA fast kernel applicable (NSFNET-class: 22 links, k <= 5)
-    bool hot;                     // ... and its steady-state specialisation (deeprmsa_fast_kernel<.., HOT = true>)
-    bool ro_ok;                   // the persistent rollout kernel applies (DeepRMSA / RMSA / RWA on NSFNET-class topologies)
+    bool fast = false;            // DeepRMSA fast kernel applicable (NSFNET-class: 22 links, k <= 5)
+    bool hot = false;             // ... and its steady-state specialisation qualifies (hot_launch)
+    bool ro_ok = false;           // the persistent rollout kernel qualifies (rollout_kernel_applies)
     int ro_lpw;                   // envs per warp of the rollout kernel (8 or 32): fixed per handle, the event slabs follow it
     bool ro_last_persistent = false;   // the last orlg_rollout* call ran the persistent kernel (orlg_kernel_info)
     CUtensorMap mask_map;         // TMA view of the mask tensor: [C*E rows][n x 16 bytes], box = E rows x 512 bytes
     bool wide;                    // beyond 32 links / 128 slots / 8 paths: CSR link lists, multi-word masks
     size_t fast_smem;
-    size_t obs_smem;
-    int64_t state_bytes;
+    int64_t state_bytes = 0;
     std::vector<void *> allocs;
     // the per-environment STATE arrays among them (orlg_state_save / orlg_state_load), in allocation order
     std::vector<std::pair<void *, size_t>> state_allocs;
@@ -62,16 +113,10 @@ struct orlg_env {
     double *ro_st_f64 = nullptr;               // [2 + RO_SIDE][n] table minimum, horizon, side-buffer times
     unsigned long long *ro_st_u64 = nullptr;   // [RO_SIDE][n] side-buffer payloads
     bool ro_valid = false;                     // the events live in the rollout-private storage (canonical tables are stale)
-    // orlg_rollout_host: double-buffered packed records on the device and in pinned host memory
-    uint4 *ro_pk_dev[RO_HOST_BUFFERS] = {};
-    uint4 *ro_pk_host[RO_HOST_BUFFERS] = {};
-    size_t ro_pk_rows = 0;                     // rows (env-steps) each buffer holds
-    cudaEvent_t ro_pk_ev[RO_HOST_BUFFERS] = {};    // records of the chunk are in pinned host memory (copy stream)
-    cudaEvent_t ro_k_ev[RO_HOST_BUFFERS] = {};     // the chunk's kernel is done (user stream)
-    cudaStream_t ro_copy_stream = nullptr;         // D2H of chunk c overlaps the kernel of chunk c + 1
-    int32_t *ro_act_dev[RO_HOST_BUFFERS] = {};     // ORLG_POLICY_REPLAY: the host's action chunks on the device
-    size_t ro_act_rows = 0;
+    HostPipeline host_pipe;
     int *ro_actions = nullptr;    // [n, action_dim] scratch of the generic (kernel-per-step) rollout
+
+    ~orlg_env() { for (void *ptr : allocs) cudaFree(ptr); }
 };
 
 namespace {
@@ -91,8 +136,8 @@ int dev_alloc(orlg_env *env, T **out, size_t count, bool zero = true) {
     void *ptr = nullptr;
     size_t bytes = sizeof(T) * (count ? count : 1);
     if (cudaMalloc(&ptr, bytes) != cudaSuccess) return fail(ORLG_E_NOMEM, "cudaMalloc failed for " + std::to_string(bytes) + " bytes");
-    if (zero && cudaMemset(ptr, 0, bytes) != cudaSuccess) return fail(ORLG_E_CUDA, "cudaMemset failed");
     env->allocs.push_back(ptr);
+    if (zero && cudaMemset(ptr, 0, bytes) != cudaSuccess) return fail(ORLG_E_CUDA, "cudaMemset failed");
     if (env->alloc_is_state) env->state_allocs.emplace_back(ptr, bytes);
     env->state_bytes += (int64_t)bytes;
     *out = reinterpret_cast<T *>(ptr);
@@ -163,11 +208,13 @@ bool encode_mask_map(orlg_env *env) {
                                            CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+size_t step_obs_smem(const Params &p) { return (size_t)STEP_THREADS * p.obs_dim * (p.obs_f64 ? 8 : 4); }
+
 template <int KIND>
 void launch_step_kind(const orlg_env *env, const StepIO &io, int mode, cudaStream_t s) {
     const int blocks = (env->p.n + STEP_THREADS - 1) / STEP_THREADS;
-    const size_t smem = (KIND == ORLG_DEEPRMSA && io.obs) ? env->obs_smem : 0;
-    if (env->km == 5) step_kernel<KIND, 5><<<blocks, STEP_THREADS, smem, s>>>(env->p, io, mode);
+    const size_t smem = (KIND == ORLG_DEEPRMSA && io.obs) ? step_obs_smem(env->p) : 0;
+    if (env->p.k <= 5) step_kernel<KIND, 5><<<blocks, STEP_THREADS, smem, s>>>(env->p, io, mode);
     else step_kernel<KIND, KMAX><<<blocks, STEP_THREADS, smem, s>>>(env->p, io, mode);
 }
 
@@ -186,67 +233,84 @@ cudaLaunchConfig_t pdl_config(int blocks, int threads, size_t smem, cudaStream_t
     return cfg;
 }
 
-template <int JT, bool OBS64>
+// ---- kernel-instance decisions: each is made here and nowhere else
+
+// f(std::integral_constant<int, KIND>()) for the env kind
+template <typename F>
+void for_kind(int kind, F &&f) {
+    switch (kind) {
+    case ORLG_RWA: f(std::integral_constant<int, ORLG_RWA>()); break;
+    case ORLG_RMSA: f(std::integral_constant<int, ORLG_RMSA>()); break;
+    case ORLG_DEEPRMSA: f(std::integral_constant<int, ORLG_DEEPRMSA>()); break;
+    default: f(std::integral_constant<int, ORLG_RMCSA>()); break;
+    }
+}
+
+// f(std::integral_constant<int, W>()) for the 128-slot mask words per (core, link) of the wide kernels
+template <typename F>
+void for_words(int nwv, F &&f) {
+    switch (nwv) {
+    case 1: f(std::integral_constant<int, 1>()); break;
+    case 2: f(std::integral_constant<int, 2>()); break;
+    case 3: f(std::integral_constant<int, 3>()); break;
+    default: f(std::integral_constant<int, 4>()); break;
+    }
+}
+
+// link-count template of the fast and rollout kernels: 22 (NSFNET) is compiled in, 0 reads the link count at run time
+int link_template(const orlg_env *env) { return !env->wide && env->p.E == 22 ? 22 : 0; }
+
+// the steady-state instance (HOT = true) of the fast kernel runs for this launch: the handle qualifies (orlg_create) and the
+// launch is a float32 Philox step that writes observation, reward and done and nothing else
+bool hot_launch(const orlg_env *env, const StepIO &io, int mode) {
+    return env->hot && env->p.J == 1 && !env->p.obs_f64 && mode == MODE_STEP && env->p.traffic == ORLG_TRAFFIC_PHILOX &&
+           io.obs && io.reward && io.done && !io.decision && !io.obs_int;
+}
+
+// nullptr when the env kind has heuristic `which`, else why it is refused
+constexpr const char *heuristic_refusal(int kind, int which) {
+    return kind == ORLG_RMSA && which == ORLG_HEUR_SAP_LF         ? "last-fit exists for RWA only"
+           : kind == ORLG_DEEPRMSA && which > ORLG_HEUR_SAP_FF ? "DeepRMSA has SP-FF and SAP-FF only"
+                                                                : nullptr;
+}
+
+// the persistent rollout kernel runs this policy on this handle (given a shared-memory plan, rollout_plan)
+bool rollout_kernel_applies(const orlg_env *env, int policy) {
+    const Params &p = env->p;
+    const bool policy_ok = p.traffic == ORLG_TRAFFIC_TRACE ? policy == ORLG_POLICY_REPLAY
+                           : policy == ORLG_POLICY_RANDOM || policy == ORLG_POLICY_REPLAY || !heuristic_refusal(p.kind, policy);
+    return env->ro_ok && !p.stats && !p.obs_f64 && !p.br_hist && policy_ok;
+}
+
+// the fast-kernel instances launch_fast picks from, [j != 1][float64 obs][link template 0] then HOT [link template 0]
+using FastKernel = void (*)(Params, StepIO, int, CUtensorMap);
+const FastKernel FAST_KERNELS[] = {
+    deeprmsa_fast_kernel<22, 5, 1, false>, deeprmsa_fast_kernel<0, 5, 1, false>, deeprmsa_fast_kernel<22, 5, 1, true>, deeprmsa_fast_kernel<0, 5, 1, true>,
+    deeprmsa_fast_kernel<22, 5, 0, false>, deeprmsa_fast_kernel<0, 5, 0, false>, deeprmsa_fast_kernel<22, 5, 0, true>, deeprmsa_fast_kernel<0, 5, 0, true>,
+    deeprmsa_fast_kernel<22, 5, 1, false, true>, deeprmsa_fast_kernel<0, 5, 1, false, true>};
+
 void launch_fast(const orlg_env *env, const StepIO &io, int mode, cudaStream_t s) {
     const int blocks = (env->p.n + FAST_THREADS - 1) / FAST_THREADS;
-    if (JT == 1 && !OBS64 && env->hot && mode == MODE_STEP && env->p.traffic == ORLG_TRAFFIC_PHILOX && io.obs && io.reward &&
-        io.done && !io.decision && !io.obs_int) {
+    const bool hot = hot_launch(env, io, mode);
+    const int et = link_template(env) == 22 ? 0 : 1;
+    const FastKernel kernel = FAST_KERNELS[hot ? 8 + et : (env->p.J == 1 ? 0 : 4) + (env->p.obs_f64 ? 2 : 0) + et];
+    if (hot) {
         // programmatic dependent launch: the prologue overlaps the tail of the preceding kernel of the stream
         cudaLaunchConfig_t cfg = pdl_config(blocks, FAST_THREADS, env->fast_smem, s);
-        if (env->p.E == 22) cudaLaunchKernelEx(&cfg, deeprmsa_fast_kernel<22, 5, 1, false, true>, env->p, io, mode, env->mask_map);
-        else cudaLaunchKernelEx(&cfg, deeprmsa_fast_kernel<0, 5, 1, false, true>, env->p, io, mode, env->mask_map);
+        cudaLaunchKernelEx(&cfg, kernel, env->p, io, mode, env->mask_map);
         return;
     }
-    if (env->p.E == 22) deeprmsa_fast_kernel<22, 5, JT, OBS64><<<blocks, FAST_THREADS, env->fast_smem, s>>>(env->p, io, mode, env->mask_map);
-    else deeprmsa_fast_kernel<0, 5, JT, OBS64><<<blocks, FAST_THREADS, env->fast_smem, s>>>(env->p, io, mode, env->mask_map);
-}
-
-template <int KIND>
-void launch_wide_kind(const orlg_env *env, const StepIO &io, int mode, cudaStream_t s) {
-    const int blocks = (env->p.n + ORLG_WIDE_THREADS - 1) / ORLG_WIDE_THREADS;
-    switch (env->p.nwv) {
-    case 1: step_wide_kernel<KIND, 1><<<blocks, ORLG_WIDE_THREADS, 0, s>>>(env->p, io, mode); break;
-    case 2: step_wide_kernel<KIND, 2><<<blocks, ORLG_WIDE_THREADS, 0, s>>>(env->p, io, mode); break;
-    case 3: step_wide_kernel<KIND, 3><<<blocks, ORLG_WIDE_THREADS, 0, s>>>(env->p, io, mode); break;
-    default: step_wide_kernel<KIND, 4><<<blocks, ORLG_WIDE_THREADS, 0, s>>>(env->p, io, mode); break;
-    }
-}
-
-template <int KIND>
-void launch_heuristic_wide(const orlg_env *env, int which, int *actions, cudaStream_t s) {
-    const int blocks = (env->p.n + 127) / 128;
-    switch (env->p.nwv) {
-    case 1: heuristic_wide_kernel<KIND, 1><<<blocks, 128, 0, s>>>(env->p, which, actions); break;
-    case 2: heuristic_wide_kernel<KIND, 2><<<blocks, 128, 0, s>>>(env->p, which, actions); break;
-    case 3: heuristic_wide_kernel<KIND, 3><<<blocks, 128, 0, s>>>(env->p, which, actions); break;
-    default: heuristic_wide_kernel<KIND, 4><<<blocks, 128, 0, s>>>(env->p, which, actions); break;
-    }
+    kernel<<<blocks, FAST_THREADS, env->fast_smem, s>>>(env->p, io, mode, env->mask_map);
 }
 
 int launch_step(const orlg_env *env, const StepIO &io, int mode, cudaStream_t s) {
+    const Params &p = env->p;
     if (env->wide) {
-        switch (env->p.kind) {
-        case ORLG_RWA: launch_wide_kind<ORLG_RWA>(env, io, mode, s); break;
-        case ORLG_RMSA: launch_wide_kind<ORLG_RMSA>(env, io, mode, s); break;
-        case ORLG_DEEPRMSA: launch_wide_kind<ORLG_DEEPRMSA>(env, io, mode, s); break;
-        default: launch_wide_kind<ORLG_RMCSA>(env, io, mode, s); break;
-        }
-        CUDA_OK(cudaGetLastError());
-        return ORLG_OK;
-    }
-    if (env->fast && !env->p.stats) {
-        if (env->p.J == 1) { if (env->p.obs_f64) launch_fast<1, true>(env, io, mode, s); else launch_fast<1, false>(env, io, mode, s); }
-        else { if (env->p.obs_f64) launch_fast<0, true>(env, io, mode, s); else launch_fast<0, false>(env, io, mode, s); }
-        CUDA_OK(cudaGetLastError());
-        return ORLG_OK;
-    }
-    switch (env->p.kind) {
-    case ORLG_RWA: launch_step_kind<ORLG_RWA>(env, io, mode, s); break;
-    case ORLG_RMSA: launch_step_kind<ORLG_RMSA>(env, io, mode, s); break;
-    case ORLG_DEEPRMSA: launch_step_kind<ORLG_DEEPRMSA>(env, io, mode, s); break;
-    case ORLG_RMCSA: launch_step_kind<ORLG_RMCSA>(env, io, mode, s); break;
-    default: return fail(ORLG_E_INVALID, "unknown env kind");
-    }
+        const int blocks = (p.n + ORLG_WIDE_THREADS - 1) / ORLG_WIDE_THREADS;
+        for_kind(p.kind, [&](auto K) { for_words(p.nwv, [&](auto W) {
+            step_wide_kernel<decltype(K)::value, decltype(W)::value><<<blocks, ORLG_WIDE_THREADS, 0, s>>>(p, io, mode); }); });
+    } else if (env->fast && !p.stats) launch_fast(env, io, mode, s);
+    else for_kind(p.kind, [&](auto K) { launch_step_kind<decltype(K)::value>(env, io, mode, s); });
     CUDA_OK(cudaGetLastError());
     return ORLG_OK;
 }
@@ -261,11 +325,9 @@ int choose_rollout_lpw(int n) {
     return n >= 16384 ? 32 : 8;
 }
 
-int rollout_lpw(const orlg_env *env) { return env->ro_lpw; }
-
 void rollout_state_args(const orlg_env *env, RolloutArgs *ra) {
     const size_t n = (size_t)env->p.n;
-    ra->lpw = rollout_lpw(env);
+    ra->lpw = env->ro_lpw;
     ra->ev = env->ro_ev;
     ra->st_ntab = env->ro_st_u32; ra->st_wh = env->ro_st_u32 + n; ra->st_wn = env->ro_st_u32 + 2 * n; ra->st_ncanon = env->ro_st_u32 + 3 * n;
     ra->st_tmin = env->ro_st_f64; ra->st_hzn = env->ro_st_f64 + n; ra->st_side_t = env->ro_st_f64 + 2 * n;
@@ -289,8 +351,7 @@ int ensure_canonical(orlg_env *env, cudaStream_t s) {
 // its mask tile + side buffer, plus a pool of observation tiles
 bool rollout_plan(const orlg_env *env, int *wpc_out, RolloutArgs *ra, size_t *smem_out) {
     const Params &p = env->p;
-    const int lpw = rollout_lpw(env);
-    const int warps = (p.n + lpw - 1) / lpw;
+    const int warps = (p.n + env->ro_lpw - 1) / env->ro_lpw;
     int wpc = (warps + 147) / 148;
     if (wpc > RO_MAX_THREADS / 32) wpc = RO_MAX_THREADS / 32;
     if (wpc < 1) wpc = 1;
@@ -333,8 +394,8 @@ cudaError_t launch_rollout_kind(const orlg_env *env, const RolloutArgs &ra, int 
     } else if (policy == ORLG_POLICY_RANDOM) ORLG_RO_LAUNCH(RO_POLICY_RANDOM, false);
     else if (policy == ORLG_HEUR_SP_FF) ORLG_RO_LAUNCH(RO_POLICY_SP_FF, false);
     else if (policy == ORLG_HEUR_SAP_FF) ORLG_RO_LAUNCH(RO_POLICY_SAP_FF, false);
-    else if (policy == ORLG_HEUR_LLP_FF) { if (KIND != ORLG_DEEPRMSA) ORLG_RO_LAUNCH(RO_POLICY_LLP_FF, false); }
-    else if (policy == ORLG_HEUR_SAP_LF) { if (KIND == ORLG_RWA) ORLG_RO_LAUNCH(RO_POLICY_SAP_LF, false); }
+    else if (policy == ORLG_HEUR_LLP_FF) { if (!heuristic_refusal(KIND, ORLG_HEUR_LLP_FF)) ORLG_RO_LAUNCH(RO_POLICY_LLP_FF, false); }
+    else if (policy == ORLG_HEUR_SAP_LF) { if (!heuristic_refusal(KIND, ORLG_HEUR_SAP_LF)) ORLG_RO_LAUNCH(RO_POLICY_SAP_LF, false); }
 #undef ORLG_RO_LAUNCH
 #undef ORLG_RO_LAUNCH1
     return e;
@@ -349,166 +410,161 @@ cudaError_t launch_rollout(const orlg_env *env, const RolloutArgs &ra, int polic
     default: return cudaErrorInvalidValue;
     }
 }
-}  // namespace
 
-extern "C" {
+int slots_needed(int bit_rate, int se, double channel_width) {   // get_number_slots (rmsa_env.py:610-621), same float expression
+    return (int)std::ceil((double)bit_rate / ((double)se * channel_width)) + 1;
+}
 
-const char *orlg_last_error(void) { return g_err.c_str(); }
-int orlg_version(void) { return ORLG_VERSION; }
-
-int orlg_create(const orlg_config *cfg, const orlg_tables *t, int device, orlg_env **out) {
-    if (!cfg || !t || !out) return fail(ORLG_E_INVALID, "null argument");
-    *out = nullptr;
-    if (cfg->kind < ORLG_RWA || cfg->kind > ORLG_RMCSA) return fail(ORLG_E_INVALID, "unknown env kind");
-    if (cfg->num_envs <= 0) return fail(ORLG_E_INVALID, "num_envs must be positive");
-    if (cfg->num_slots > 512 || cfg->num_slots <= 0) return fail(ORLG_E_UNSUPPORTED, "1..512 slots per link");
-    if (t->num_links < 1 || t->num_links > 65535) return fail(ORLG_E_UNSUPPORTED, "1..65535 links");
-    if (t->num_nodes > 255 || t->num_nodes < 2) return fail(ORLG_E_UNSUPPORTED, "2..255 nodes");
-    if (t->k_paths > 16 || t->k_paths < 1) return fail(ORLG_E_UNSUPPORTED, "k_paths must be 1..16");
-    const bool wide = t->num_links > 32 || cfg->num_slots > MAX_SLOTS || t->k_paths > KMAX;
-    if (t->num_paths >= (1 << 20)) return fail(ORLG_E_UNSUPPORTED, "too many paths");
-    const int C = cfg->kind == ORLG_RMCSA ? cfg->num_cores : 1;
+// Step 1.  Every refusal of a configuration, in a fixed order: an input with several faults is always refused for the same
+// one.  Nothing is allocated; the device query is the only CUDA call.  Fills the scalar launch parameters, whether the wide
+// kernels serve the handle, and the largest spectral efficiency (the extent of the slot-count tables).
+int configure(const orlg_config &cfg, const orlg_tables &t, int device, Params &p, bool &wide, int &se_max) {
+    if (cfg.kind < ORLG_RWA || cfg.kind > ORLG_RMCSA) return fail(ORLG_E_INVALID, "unknown env kind");
+    if (cfg.num_envs <= 0) return fail(ORLG_E_INVALID, "num_envs must be positive");
+    if (cfg.num_slots > 512 || cfg.num_slots <= 0) return fail(ORLG_E_UNSUPPORTED, "1..512 slots per link");
+    if (t.num_links < 1 || t.num_links > 65535) return fail(ORLG_E_UNSUPPORTED, "1..65535 links");
+    if (t.num_nodes > 255 || t.num_nodes < 2) return fail(ORLG_E_UNSUPPORTED, "2..255 nodes");
+    if (t.k_paths > 16 || t.k_paths < 1) return fail(ORLG_E_UNSUPPORTED, "k_paths must be 1..16");
+    if (t.num_paths >= (1 << 20)) return fail(ORLG_E_UNSUPPORTED, "too many paths");
+    const int C = cfg.kind == ORLG_RMCSA ? cfg.num_cores : 1;
     if (C < 1 || C > 31) return fail(ORLG_E_UNSUPPORTED, "1..31 cores");
-    const int J = cfg->kind == ORLG_DEEPRMSA ? cfg->j : 1;
+    const int J = cfg.kind == ORLG_DEEPRMSA ? cfg.j : 1;
     if (J < 1 || J > 16) return fail(ORLG_E_INVALID, "j must be 1..16");
-    if (cfg->episode_length < 1 || cfg->episode_length >= (1 << 22)) return fail(ORLG_E_UNSUPPORTED, "episode_length must be < 2^22");
-    if (!(cfg->mean_holding > 0) || !(cfg->mean_iat > 0)) return fail(ORLG_E_INVALID, "holding / inter-arrival times must be positive");
-    if (cfg->kind != ORLG_RWA && t->num_bit_rates == 0 && cfg->bit_rate_hi < cfg->bit_rate_lo)
+    if (cfg.episode_length < 1 || cfg.episode_length >= (1 << 22)) return fail(ORLG_E_UNSUPPORTED, "episode_length must be < 2^22");
+    if (!(cfg.mean_holding > 0) || !(cfg.mean_iat > 0)) return fail(ORLG_E_INVALID, "holding / inter-arrival times must be positive");
+    if (cfg.kind != ORLG_RWA && t.num_bit_rates == 0 && cfg.bit_rate_hi < cfg.bit_rate_lo)
         return fail(ORLG_E_INVALID, "bit_rate_higher_bound < bit_rate_lower_bound");
-    if (cfg->kind == ORLG_RMCSA && t->num_mods < 1) return fail(ORLG_E_INVALID, "RMCSA needs a modulation table");
+    if (cfg.kind == ORLG_RMCSA && t.num_mods < 1) return fail(ORLG_E_INVALID, "RMCSA needs a modulation table");
 
     int n_dev = 0;
     if (cudaGetDeviceCount(&n_dev) != cudaSuccess || device < 0 || device >= n_dev) return fail(ORLG_E_CUDA, "no such CUDA device");
-    DeviceGuard guard(device);
-    orlg_env *env = new orlg_env();
-    env->cfg = *cfg;
-    env->device = device;
-    env->state_bytes = 0;
-    env->wide = wide;
-    env->ro_lpw = choose_rollout_lpw(cfg->num_envs);
-    Params &p = env->p;
+    wide = t.num_links > 32 || cfg.num_slots > MAX_SLOTS || t.k_paths > KMAX;
     std::memset(&p, 0, sizeof(p));
-    p.kind = cfg->kind; p.n = cfg->num_envs; p.N = t->num_nodes; p.E = t->num_links; p.C = C; p.S = cfg->num_slots;
-    p.k = t->k_paths; p.J = J; p.M = t->num_mods;
-    p.episode_length = cfg->episode_length; p.allow_rejection = cfg->allow_rejection ? 1 : 0;
-    p.auto_reset = cfg->auto_reset ? 1 : 0; p.traffic = cfg->traffic; p.obs_f64 = cfg->obs_dtype == ORLG_OBS_F64;
-    p.n_bit_rates = t->num_bit_rates;
-    p.br_lo = cfg->bit_rate_lo; p.br_span = cfg->bit_rate_hi - cfg->bit_rate_lo + 1;
-    int br_max = cfg->kind == ORLG_RWA ? 0 : (cfg->bit_rate_hi > 1023 ? cfg->bit_rate_hi : 1023);   // traces may carry any rate <= 1023
-    for (int i = 0; i < t->num_bit_rates; i++) br_max = t->bit_rates[i] > br_max ? t->bit_rates[i] : br_max;
-    if (br_max < 0 || br_max > 65535) { delete env; return fail(ORLG_E_UNSUPPORTED, "bit rates must be 0..65535"); }
+    p.kind = cfg.kind; p.n = cfg.num_envs; p.N = t.num_nodes; p.E = t.num_links; p.C = C; p.S = cfg.num_slots;
+    p.k = t.k_paths; p.J = J; p.M = t.num_mods;
+    p.episode_length = cfg.episode_length; p.allow_rejection = cfg.allow_rejection ? 1 : 0;
+    p.auto_reset = cfg.auto_reset ? 1 : 0; p.traffic = cfg.traffic; p.obs_f64 = cfg.obs_dtype == ORLG_OBS_F64;
+    p.n_bit_rates = t.num_bit_rates;
+    p.br_lo = cfg.bit_rate_lo; p.br_span = cfg.bit_rate_hi - cfg.bit_rate_lo + 1;
+    int br_max = cfg.kind == ORLG_RWA ? 0 : (cfg.bit_rate_hi > 1023 ? cfg.bit_rate_hi : 1023);   // traces may carry any rate <= 1023
+    for (int i = 0; i < t.num_bit_rates; i++) br_max = t.bit_rates[i] > br_max ? t.bit_rates[i] : br_max;
+    if (br_max < 0 || br_max > 65535) return fail(ORLG_E_UNSUPPORTED, "bit rates must be 0..65535");
     p.br_max = br_max;
-    p.seed = cfg->seed; p.env_id_base = cfg->env_id_base;
-    p.mean_holding = cfg->mean_holding; p.mean_iat = cfg->mean_iat;
-    p.obs_dim = cfg->kind == ORLG_DEEPRMSA ? 1 + 2 * p.N + (2 * J + 3) * p.k : 0;
+    p.seed = cfg.seed; p.env_id_base = cfg.env_id_base;
+    p.mean_holding = cfg.mean_holding; p.mean_iat = cfg.mean_iat;
+    p.obs_dim = cfg.kind == ORLG_DEEPRMSA ? 1 + 2 * p.N + (2 * J + 3) * p.k : 0;
     p.node_top_step = 1;                   // highest power of two <= N - 1: binary search over the node CDF
     while (p.node_top_step * 2 <= p.N - 1) p.node_top_step *= 2;
     p.cand_stride = ((p.k * J + 7) / 8) * 8;
     p.nwv = wide ? (p.S + 127) / 128 : 1;
     p.wstride = wide ? (p.nwv == 3 ? 4 : p.nwv) : 0;      // 3-word entries padded to 64 bytes: one DRAM burst per (env, core, link)
-    env->km = p.k <= 5 ? 5 : KMAX;
-    env->obs_smem = (size_t)STEP_THREADS * p.obs_dim * (p.obs_f64 ? 8 : 4);
-    if (env->obs_smem > 200 * 1024) { delete env; return fail(ORLG_E_UNSUPPORTED, "observation too large for the staging tile"); }
+    if (step_obs_smem(p) > 200 * 1024) return fail(ORLG_E_UNSUPPORTED, "observation too large for the staging tile");
 
     // heap capacity: live services ~ Poisson(load) at most (M/M/inf bound); hard bound E*S*C/2 slots pairs
-    int cap = cfg->heap_capacity;
+    int cap = cfg.heap_capacity;
     if (cap <= 0) {
-        double load = cfg->mean_holding / cfg->mean_iat;
+        double load = cfg.mean_holding / cfg.mean_iat;
         double want = load + 8.0 * std::sqrt(load) + 16.0;
-        double hard = cfg->kind == ORLG_RWA ? (double)p.E * p.S * C : (double)p.E * p.S * C / 2.0;
+        double hard = cfg.kind == ORLG_RWA ? (double)p.E * p.S * C : (double)p.E * p.S * C / 2.0;
         cap = (int)std::ceil(want < hard ? want : hard);
     }
     cap = ((cap + EV_GROUP - 1) / EV_GROUP) * EV_GROUP;
     // up to 4096 live services per env (RWA's physical bound on NSFNET is E * W = 1760).  A derived capacity is capped
     // there (overflow is flagged per env, ORLG_ERR_HEAP_OVERFLOW); an explicit request beyond it is refused.
-    if (cfg->heap_capacity > 256 * EV_GROUP) {
-        delete env;
-        return fail(ORLG_E_UNSUPPORTED, "heap_capacity above 4096 live services per environment");
-    }
+    if (cfg.heap_capacity > 256 * EV_GROUP) return fail(ORLG_E_UNSUPPORTED, "heap_capacity above 4096 live services per environment");
     if (cap > 256 * EV_GROUP) cap = 256 * EV_GROUP;
     p.ev_groups = ((cap / EV_GROUP + 15) / 16) * 16;
     p.heap_cap = cap;
 
-    // ---- tables
-    int rc = ORLG_OK;
-    const int NN = p.N * p.N, P = t->num_paths;
-    std::vector<int> pair_first(t->pair_first, t->pair_first + NN);
-    std::vector<unsigned char> pair_count(NN);
-    for (int i = 0; i < NN; i++) pair_count[i] = (unsigned char)(t->pair_count[i] < 0 ? 0 : (t->pair_count[i] > p.k ? p.k : t->pair_count[i]));
-    std::vector<unsigned> linkmask(P), meta(P);
-    int se_max = 1;
+    se_max = 1;
+    for (int r = 0; r < t.num_paths; r++) {
+        for (int h = t.path_link_ptr[r]; h < t.path_link_ptr[r + 1]; h++)
+            if (t.path_links[h] < 0 || t.path_links[h] >= p.E) return fail(ORLG_E_INVALID, "path link index out of range");
+        if (t.path_hops[r] > 255 || t.path_link_ptr[r + 1] - t.path_link_ptr[r] != t.path_hops[r]) return fail(ORLG_E_INVALID, "inconsistent path hop counts");
+        se_max = t.path_se[r] > se_max ? t.path_se[r] : se_max;
+    }
+    for (int m = 0; m < t.num_mods; m++) se_max = t.mod_se[m] > se_max ? t.mod_se[m] : se_max;
+    // slot counts are 8-bit table entries / payload fields: harmless above 200 only while 200 slots can never fit
+    bool unrepresentable = false;
+    auto check = [&](int b) {
+        for (int se = 1; se <= se_max; se++) { const int n = slots_needed(b, se, cfg.channel_width); unrepresentable |= n > 200 && n <= p.S; }
+    };
+    if (cfg.kind != ORLG_RWA && t.num_bit_rates > 0) for (int i = 0; i < t.num_bit_rates; i++) check(t.bit_rates[i]);
+    else if (cfg.kind != ORLG_RWA) for (int b = cfg.bit_rate_lo < 0 ? 0 : cfg.bit_rate_lo; b <= cfg.bit_rate_hi; b++) check(b);
+    if (unrepresentable)
+        return fail(ORLG_E_UNSUPPORTED, "a request of this configuration may need 201.." + std::to_string(p.S) + " slots: at most 200 slots per service are representable");
+    return ORLG_OK;
+}
+
+// the host copies of the lookup tables that the fast-kernel blob and the instance selection read after the upload
+struct HostTables {
+    std::vector<int> pair_first;
+    std::vector<unsigned char> pair_count, nslots;     // nslots: [se][bit rate]
+    std::vector<unsigned> linkmask, meta, node_thr;
+};
+
+// Step 2.  The lookup tables (paths, slot counts, reach, traffic CDFs): built on the host, uploaded.
+int upload_tables(orlg_env *env, const orlg_config &cfg, const orlg_tables &t, int se_max, HostTables &h) {
+    Params &p = env->p;
+    const int NN = p.N * p.N, P = t.num_paths, br_max = p.br_max;
+    h.pair_first.assign(t.pair_first, t.pair_first + NN);
+    h.pair_count.resize(NN);
+    for (int i = 0; i < NN; i++) h.pair_count[i] = (unsigned char)(t.pair_count[i] < 0 ? 0 : (t.pair_count[i] > p.k ? p.k : t.pair_count[i]));
+    h.linkmask.resize(P); h.meta.resize(P);
     for (int r = 0; r < P; r++) {
         unsigned lm = 0;
-        for (int h = t->path_link_ptr[r]; h < t->path_link_ptr[r + 1]; h++) {
-            if (t->path_links[h] < 0 || t->path_links[h] >= p.E) { delete env; return fail(ORLG_E_INVALID, "path link index out of range"); }
-            if (!wide) lm |= 1u << t->path_links[h];
-        }
-        if (t->path_hops[r] > 255 || t->path_link_ptr[r + 1] - t->path_link_ptr[r] != t->path_hops[r]) { delete env; return fail(ORLG_E_INVALID, "inconsistent path hop counts"); }
-        linkmask[r] = lm;
-        int se = t->path_se[r] < 1 ? 1 : t->path_se[r];
-        meta[r] = (unsigned)(t->path_hops[r] & 0xff) | ((unsigned)(se & 0xff) << 8) | ((unsigned)(t->path_mod[r] & 0xff) << 16);
-        se_max = se > se_max ? se : se_max;
+        if (!env->wide) for (int h0 = t.path_link_ptr[r]; h0 < t.path_link_ptr[r + 1]; h0++) lm |= 1u << t.path_links[h0];
+        h.linkmask[r] = lm;
+        int se = t.path_se[r] < 1 ? 1 : t.path_se[r];
+        h.meta[r] = (unsigned)(t.path_hops[r] & 0xff) | ((unsigned)(se & 0xff) << 8) | ((unsigned)(t.path_mod[r] & 0xff) << 16);
     }
-    std::vector<unsigned char> mod_se(t->num_mods > 0 ? t->num_mods : 1, 1);
-    for (int m = 0; m < t->num_mods; m++) { mod_se[m] = (unsigned char)t->mod_se[m]; se_max = t->mod_se[m] > se_max ? t->mod_se[m] : se_max; }
-    // get_number_slots (rmsa_env.py:610-621): ceil(bit_rate / (SE * channel_width)) + 1, same float expression
-    std::vector<unsigned char> nslots((size_t)(se_max + 1) * (br_max + 1), 1);
-    bool slots_unrepresentable = false;
+    std::vector<unsigned char> mod_se(t.num_mods > 0 ? t.num_mods : 1, 1);
+    for (int m = 0; m < t.num_mods; m++) mod_se[m] = (unsigned char)t.mod_se[m];
+    h.nslots.assign((size_t)(se_max + 1) * (br_max + 1), 1);
     for (int se = 1; se <= se_max; se++)
         for (int b = 0; b <= br_max; b++) {
-            int n = (int)std::ceil((double)b / ((double)se * cfg->channel_width)) + 1;
-            if (n > 200) {             // 8-bit table entry / payload field; harmless only while 200 slots can never fit
-                const bool configured = t->num_bit_rates > 0 ? false : (b >= cfg->bit_rate_lo && b <= cfg->bit_rate_hi);
-                if (n <= p.S && configured) slots_unrepresentable = true;
-                n = 200;
-            }
-            nslots[(size_t)se * (br_max + 1) + b] = (unsigned char)n;
+            const int n = slots_needed(b, se, cfg.channel_width);
+            h.nslots[(size_t)se * (br_max + 1) + b] = (unsigned char)(n > 200 ? 200 : n);
         }
-    for (int i = 0; i < t->num_bit_rates; i++)
-        for (int se = 1; se <= se_max; se++) {
-            const int n = (int)std::ceil((double)t->bit_rates[i] / ((double)se * cfg->channel_width)) + 1;
-            if (n > 200 && n <= p.S) slots_unrepresentable = true;
-        }
-    if (slots_unrepresentable && cfg->kind != ORLG_RWA) {
-        delete env;
-        return fail(ORLG_E_UNSUPPORTED, "a request of this configuration may need 201.." + std::to_string(p.S) + " slots: at most 200 slots per service are representable");
-    }
-    std::vector<double> reach((size_t)(t->num_mods > 0 ? t->num_mods : 1) * (br_max + 1), 0.0);
-    if (cfg->kind == ORLG_RMCSA)
-        for (int m = 0; m < t->num_mods; m++)
+    std::vector<double> reach((size_t)(t.num_mods > 0 ? t.num_mods : 1) * (br_max + 1), 0.0);
+    if (cfg.kind == ORLG_RMCSA)
+        for (int m = 0; m < t.num_mods; m++)
             for (int b = 0; b <= br_max; b++)
-                reach[(size_t)m * (br_max + 1) + b] = b == 0 ? 1e300 : reach_km(t->mod_osnr[m], t->mod_xt[m], t->mod_se[m], b, cfg->worst_xt);
-    std::vector<double> plen(t->path_length, t->path_length + P);
-    std::vector<unsigned> node_thr = thresholds(t->node_prob, p.N);
-    std::vector<unsigned> br_thr = t->num_bit_rates > 0 ? thresholds(t->bit_rate_prob, t->num_bit_rates) : std::vector<unsigned>(1, 0u);
+                reach[(size_t)m * (br_max + 1) + b] = b == 0 ? 1e300 : reach_km(t.mod_osnr[m], t.mod_xt[m], t.mod_se[m], b, cfg.worst_xt);
+    std::vector<double> plen(t.path_length, t.path_length + P);
+    h.node_thr = thresholds(t.node_prob, p.N);
+    std::vector<unsigned> br_thr = t.num_bit_rates > 0 ? thresholds(t.bit_rate_prob, t.num_bit_rates) : std::vector<unsigned>(1, 0u);
     std::vector<int> link_order(p.E);
-    for (int l = 0; l < p.E; l++) link_order[l] = t->link_order ? t->link_order[l] : l;
-    std::vector<int> bit_rates(t->num_bit_rates > 0 ? t->num_bit_rates : 1, 0);
-    for (int i = 0; i < t->num_bit_rates; i++) bit_rates[i] = t->bit_rates[i];
+    for (int l = 0; l < p.E; l++) link_order[l] = t.link_order ? t.link_order[l] : l;
+    std::vector<int> bit_rates(t.num_bit_rates > 0 ? t.num_bit_rates : 1, 0);
+    for (int i = 0; i < t.num_bit_rates; i++) bit_rates[i] = t.bit_rates[i];
+    std::vector<int> lptr(t.path_link_ptr, t.path_link_ptr + P + 1);
+    std::vector<unsigned short> l16(lptr[P] > 0 ? lptr[P] : 1, 0);
+    for (int i = 0; i < lptr[P]; i++) l16[i] = (unsigned short)t.path_links[i];
 
-    if (!rc) rc = dev_upload(env, &p.pair_first, pair_first);
-    if (!rc) rc = dev_upload(env, &p.pair_count, pair_count);
-    if (!rc) rc = dev_upload(env, &p.path_linkmask, linkmask);
-    if (!rc) rc = dev_upload(env, &p.path_meta, meta);
+    int rc = dev_upload(env, &p.pair_first, h.pair_first);
+    if (!rc) rc = dev_upload(env, &p.pair_count, h.pair_count);
+    if (!rc) rc = dev_upload(env, &p.path_linkmask, h.linkmask);
+    if (!rc) rc = dev_upload(env, &p.path_meta, h.meta);
     if (!rc) rc = dev_upload(env, &p.path_length, plen);
-    {
-        std::vector<int> lptr(t->path_link_ptr, t->path_link_ptr + P + 1);
-        std::vector<unsigned short> l16(lptr[P] > 0 ? lptr[P] : 1, 0);
-        for (int h = 0; h < lptr[P]; h++) l16[h] = (unsigned short)t->path_links[h];
-        if (!rc) rc = dev_upload(env, &p.path_link_ptr, lptr);
-        if (!rc) rc = dev_upload(env, &p.path_links16, l16);
-    }
-    if (!rc) rc = dev_upload(env, &p.nslots, nslots);
+    if (!rc) rc = dev_upload(env, &p.path_link_ptr, lptr);
+    if (!rc) rc = dev_upload(env, &p.path_links16, l16);
+    if (!rc) rc = dev_upload(env, &p.nslots, h.nslots);
     if (!rc) rc = dev_upload(env, &p.mod_se, mod_se);
     if (!rc) rc = dev_upload(env, &p.reach, reach);
-    if (!rc) rc = dev_upload(env, &p.node_thr, node_thr);
+    if (!rc) rc = dev_upload(env, &p.node_thr, h.node_thr);
     if (!rc) rc = dev_upload(env, &p.br_thr, br_thr);
     if (!rc) rc = dev_upload(env, &p.bit_rates, bit_rates);
     if (!rc) rc = dev_upload(env, &p.link_order, link_order);
-    // ---- state
-    env->alloc_is_state = true;
+    return rc;
+}
+
+// Step 3.  The per-environment state arrays (orlg_state_save / orlg_state_load keep them, in this order).
+int alloc_state(orlg_env *env, const orlg_tables &t) {
+    Params &p = env->p;
     const size_t n = (size_t)p.n;
-    if (!rc) rc = dev_alloc(env, &p.masks, (size_t)C * p.E * (wide ? p.wstride : p.nwv) * n);
+    env->alloc_is_state = true;
+    int rc = dev_alloc(env, &p.masks, (size_t)p.C * p.E * (env->wide ? p.wstride : p.nwv) * n);
     if (!rc) rc = dev_alloc(env, &p.now, n);
     if (!rc) rc = dev_alloc(env, &p.cur_hold, n);
     if (!rc) rc = dev_alloc(env, &p.cur_req, n);
@@ -521,133 +577,144 @@ int orlg_create(const orlg_config *cfg, const orlg_tables *t, int device, orlg_e
     if (!rc) rc = dev_alloc(env, &p.ev_gmin, n * (size_t)p.ev_groups);
     if (!rc) rc = dev_alloc(env, &p.ev_tail, n);
     if (!rc) rc = dev_alloc(env, &p.cand, n * (size_t)p.cand_stride);
-    if (!rc && wide && cfg->kind == ORLG_DEEPRMSA) rc = dev_alloc(env, &p.cand16, n * (size_t)p.cand_stride);
+    if (!rc && env->wide && p.kind == ORLG_DEEPRMSA) rc = dev_alloc(env, &p.cand16, n * (size_t)p.cand_stride);
     if (!rc) rc = dev_alloc(env, &p.errors, n);
-    if (!rc && cfg->kind == ORLG_RMSA && t->num_bit_rates > 0) rc = dev_alloc(env, &p.br_hist, 2 * (size_t)t->num_bit_rates * n);
-    if (!rc && cfg->kind == ORLG_RWA) rc = dev_alloc(env, &p.act_hist, (size_t)(p.k + p.S + 2 * p.allow_rejection) * n);
+    if (!rc && p.kind == ORLG_RMSA && t.num_bit_rates > 0) rc = dev_alloc(env, &p.br_hist, 2 * (size_t)t.num_bit_rates * n);
+    if (!rc && p.kind == ORLG_RWA) rc = dev_alloc(env, &p.act_hist, (size_t)(p.k + p.S + 2 * p.allow_rejection) * n);
     env->alloc_is_state = false;
-    if (rc) { orlg_destroy(env); return rc; }
+    return rc;
+}
 
-    // ---- fast DeepRMSA kernel: small tables packed for shared-memory staging
-    env->fast = false;
-    env->hot = false;
-    env->ro_ok = false;
-    if (!wide && cfg->kind != ORLG_RMCSA && p.k <= 5 && P <= 65535 && se_max <= 15) {
-        std::vector<unsigned char> blob;
-        auto put = [&blob](const void *src, size_t bytes) {
-            size_t off = (blob.size() + 15) / 16 * 16;
-            blob.resize(off + bytes);
-            std::memcpy(blob.data() + off, src, bytes);
-            return (int)off;
-        };
-        std::vector<unsigned short> pf16(NN);
-        for (int i = 0; i < NN; i++) pf16[i] = (unsigned short)(pair_first[i] < 0 ? 0 : pair_first[i]);
-        std::vector<unsigned char> pse(P);
-        for (int r = 0; r < P; r++) pse[r] = (unsigned char)((meta[r] >> 8) & 0xff);
-        std::vector<unsigned char> ns128((size_t)(se_max + 1) * 128, 1);
+// Step 4.  The small tables packed for shared-memory staging by the fast DeepRMSA kernel and the rollout kernel (p.tab_blob),
+// and the shared-memory size of the fast kernel.  Nothing is uploaded when the topology does not fit that form.
+int upload_fast_blob(orlg_env *env, const orlg_tables &t, const HostTables &h, int se_max) {
+    Params &p = env->p;
+    const int NN = p.N * p.N, P = t.num_paths, br_max = p.br_max;
+    if (env->wide || p.kind == ORLG_RMCSA || p.k > 5 || P > 65535 || se_max > 15) return ORLG_OK;
+    std::vector<unsigned char> blob;
+    auto put = [&blob](const void *src, size_t bytes) {
+        size_t off = (blob.size() + 15) / 16 * 16;
+        blob.resize(off + bytes);
+        std::memcpy(blob.data() + off, src, bytes);
+        return (int)off;
+    };
+    std::vector<unsigned short> pf16(NN);
+    for (int i = 0; i < NN; i++) pf16[i] = (unsigned short)(h.pair_first[i] < 0 ? 0 : h.pair_first[i]);
+    std::vector<unsigned char> pse(P);
+    for (int r = 0; r < P; r++) pse[r] = (unsigned char)((h.meta[r] >> 8) & 0xff);
+    std::vector<unsigned char> ns128((size_t)(se_max + 1) * 128, 1);
+    for (int se = 1; se <= se_max; se++)
+        for (int b = 0; b < 128 && b <= br_max; b++) ns128[(size_t)se * 128 + b] = h.nslots[(size_t)se * (br_max + 1) + b];
+    std::vector<float> pos(p.S + 1), nsl(32);
+    for (int v = 0; v <= p.S; v++) pos[v] = (float)(2 * v - p.S) / (float)p.S;      // IEEE f32 division == __fdiv_rn
+    for (int v = 0; v < 32; v++) nsl[v] = (float)(2 * v - 11) / 7.0f;
+    p.off_pair_first = put(pf16.data(), pf16.size() * 2);
+    p.off_pair_count = put(h.pair_count.data(), h.pair_count.size());
+    p.off_path_lm = put(h.linkmask.data(), h.linkmask.size() * 4);
+    p.off_path_se = put(pse.data(), pse.size());
+    std::vector<unsigned long long> pll(P, 0ULL);      // hop list: 5 bits per link index, hop count in bits 60..63
+    for (int r = 0; r < P; r++) {
+        const int h0 = t.path_link_ptr[r], hn = t.path_link_ptr[r + 1] - h0;
+        if (hn > 12) return ORLG_OK;
+        unsigned long long v = (unsigned long long)hn << 60;
+        for (int i = 0; i < hn; i++) v |= (unsigned long long)(t.path_links[h0 + i] & 31) << (5 * i);
+        pll[r] = v;
+    }
+    p.off_path_ll = put(pll.data(), pll.size() * 8);
+    p.off_nslots = put(ns128.data(), ns128.size());
+    p.off_node_thr = put(h.node_thr.data(), h.node_thr.size() * 4);
+    p.off_pos = put(pos.data(), pos.size() * 4);
+    p.off_nsl = put(nsl.data(), nsl.size() * 4);
+    std::vector<float> rcp4(p.S / 2 + 2, 0.0f);               // 1 / (4 r): at most (S + 1) / 2 free runs on a path
+    for (size_t r = 1; r < rcp4.size(); r++) rcp4[r] = 1.0f / (float)(4 * r);
+    p.off_rcp4 = put(rcp4.data(), rcp4.size() * 4);
+    std::vector<unsigned> dbl(17, 0u);                          // shift-AND doubling: shifts of the 4 rounds for n <= 16
+    for (int nn = 1; nn <= 16; nn++) {
+        int len = 1;
+        for (int it = 0; it < 4; it++) {
+            int sh = len < nn - len ? len : nn - len;
+            if (sh < 0) sh = 0;
+            dbl[nn] |= (unsigned)sh << (8 * it);
+            len += sh;
+        }
+    }
+    p.off_dbl = put(dbl.data(), dbl.size() * 4);
+    blob.resize((blob.size() + 127) / 128 * 128);          // the warp areas behind it are TMA destinations (128-byte aligned)
+    if (blob.size() > 24 * 1024 || blob.size() + (size_t)FAST_THREADS * 16 * 32 > 100 * 1024) return ORLG_OK;
+    std::vector<uint4> blob4(blob.size() / 16);
+    std::memcpy(blob4.data(), blob.data(), blob.size());
+    int rc = dev_upload(env, &p.tab_blob, blob4);
+    if (rc) return rc;
+    p.tab_vec = (int)blob4.size();
+    size_t per_thread = (size_t)p.obs_dim * (p.obs_f64 ? 8 : 4);      // observation tile overlays the mask area
+    if (per_thread < (size_t)p.E * 16) per_thread = (size_t)p.E * 16;
+    p.warp_area_bytes = (int)((per_thread * 32 + 127) / 128 * 128);
+    env->fast_smem = blob.size() + (size_t)(FAST_THREADS / 32) * p.warp_area_bytes + 8 * (FAST_THREADS / 32 + 1);   // + per-warp mbarriers + the table barrier
+    return ORLG_OK;
+}
+
+// Step 5.  Which kernel instances the handle may run (the per-launch half is in hot_launch / rollout_kernel_applies), and
+// the shared-memory size of each of them.
+int select_instances(orlg_env *env, const orlg_config &cfg, const HostTables &h, int se_max) {
+    const Params &p = env->p;
+    if (p.tab_blob) {
+        cudaError_t ea = cudaSuccess;
+        if (env->fast_smem > 48 * 1024)
+            for (FastKernel k : FAST_KERNELS)
+                if (ea == cudaSuccess) ea = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->fast_smem);
+        env->fast = p.kind == ORLG_DEEPRMSA && ea == cudaSuccess;
+        // continuous bit rates below 128 Gb/s whose slot counts all fit the 4-round shift-AND
+        int n_hi = 0;
         for (int se = 1; se <= se_max; se++)
-            for (int b = 0; b < 128 && b <= br_max; b++) ns128[(size_t)se * 128 + b] = nslots[(size_t)se * (br_max + 1) + b];
-        std::vector<float> pos(p.S + 1), nsl(32);
-        for (int v = 0; v <= p.S; v++) pos[v] = (float)(2 * v - p.S) / (float)p.S;      // IEEE f32 division == __fdiv_rn
-        for (int v = 0; v < 32; v++) nsl[v] = (float)(2 * v - 11) / 7.0f;
-        p.off_pair_first = put(pf16.data(), pf16.size() * 2);
-        p.off_pair_count = put(pair_count.data(), pair_count.size());
-        p.off_path_lm = put(linkmask.data(), linkmask.size() * 4);
-        p.off_path_se = put(pse.data(), pse.size());
-        std::vector<unsigned long long> pll(P, 0ULL);      // hop list: 5 bits per link index, hop count in bits 60..63
-        bool ll_ok = true;
-        for (int r = 0; r < P; r++) {
-            const int h0 = t->path_link_ptr[r], hn = t->path_link_ptr[r + 1] - h0;
-            if (hn > 12) { ll_ok = false; break; }
-            unsigned long long v = (unsigned long long)hn << 60;
-            for (int h = 0; h < hn; h++) v |= (unsigned long long)(t->path_links[h0 + h] & 31) << (5 * h);
-            pll[r] = v;
-        }
-        p.off_path_ll = put(pll.data(), pll.size() * 8);
-        p.off_nslots = put(ns128.data(), ns128.size());
-        p.off_node_thr = put(node_thr.data(), node_thr.size() * 4);
-        p.off_pos = put(pos.data(), pos.size() * 4);
-        p.off_nsl = put(nsl.data(), nsl.size() * 4);
-        std::vector<float> rcp4(p.S / 2 + 2, 0.0f);               // 1 / (4 r): at most (S + 1) / 2 free runs on a path
-        for (size_t r = 1; r < rcp4.size(); r++) rcp4[r] = 1.0f / (float)(4 * r);
-        p.off_rcp4 = put(rcp4.data(), rcp4.size() * 4);
-        std::vector<unsigned> dbl(17, 0u);                          // shift-AND doubling: shifts of the 4 rounds for n <= 16
-        for (int nn = 1; nn <= 16; nn++) {
-            int len = 1;
-            for (int it = 0; it < 4; it++) {
-                int sh = len < nn - len ? len : nn - len;
-                if (sh < 0) sh = 0;
-                dbl[nn] |= (unsigned)sh << (8 * it);
-                len += sh;
-            }
-        }
-        p.off_dbl = put(dbl.data(), dbl.size() * 4);
-        blob.resize((blob.size() + 127) / 128 * 128);          // the warp areas behind it are TMA destinations (128-byte aligned)
-        if (ll_ok && blob.size() <= 24 * 1024 && blob.size() + (size_t)FAST_THREADS * 16 * 32 <= 100 * 1024) {
-            std::vector<uint4> blob4(blob.size() / 16);
-            std::memcpy(blob4.data(), blob.data(), blob.size());
-            rc = dev_upload(env, &p.tab_blob, blob4);
-            if (rc) { orlg_destroy(env); return rc; }
-            p.tab_vec = (int)blob4.size();
-            env->fast = cfg->kind == ORLG_DEEPRMSA;
-            size_t per_thread = (size_t)p.obs_dim * (p.obs_f64 ? 8 : 4);      // observation tile overlays the mask area
-            if (per_thread < (size_t)p.E * 16) per_thread = (size_t)p.E * 16;
-            p.warp_area_bytes = (int)((per_thread * 32 + 127) / 128 * 128);
-            env->fast_smem = blob.size() + (size_t)(FAST_THREADS / 32) * p.warp_area_bytes + 8 * (FAST_THREADS / 32 + 1);   // + per-warp mbarriers + the table barrier
-            cudaError_t ea = cudaSuccess;
-            if (env->fast_smem > 48 * 1024) {
-                ea = cudaFuncSetAttribute(deeprmsa_fast_kernel<22, 5, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->fast_smem);
-                if (ea == cudaSuccess) ea = cudaFuncSetAttribute(deeprmsa_fast_kernel<0, 5, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->fast_smem);
-                if (ea == cudaSuccess) ea = cudaFuncSetAttribute(deeprmsa_fast_kernel<22, 5, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->fast_smem);
-                if (ea == cudaSuccess) ea = cudaFuncSetAttribute(deeprmsa_fast_kernel<0, 5, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->fast_smem);
-                if (ea == cudaSuccess) ea = cudaFuncSetAttribute(deeprmsa_fast_kernel<22, 5, 0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->fast_smem);
-                if (ea == cudaSuccess) ea = cudaFuncSetAttribute(deeprmsa_fast_kernel<0, 5, 0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->fast_smem);
-                if (ea == cudaSuccess) ea = cudaFuncSetAttribute(deeprmsa_fast_kernel<22, 5, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->fast_smem);
-                if (ea == cudaSuccess) ea = cudaFuncSetAttribute(deeprmsa_fast_kernel<0, 5, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->fast_smem);
-            }
-            if (ea == cudaSuccess && env->fast_smem > 48 * 1024) {
-                ea = cudaFuncSetAttribute(deeprmsa_fast_kernel<22, 5, 1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->fast_smem);
-                if (ea == cudaSuccess) ea = cudaFuncSetAttribute(deeprmsa_fast_kernel<0, 5, 1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->fast_smem);
-            }
-            if (ea != cudaSuccess) env->fast = false;
-            // steady-state specialisation: continuous bit rates below 128 Gb/s whose slot counts all fit the 4-round
-            // shift-AND, exactly KM candidate paths per pair, j = 1, 8-byte candidate cache, even observation width
-            int n_hi = 0;
-            for (int se = 1; se <= se_max; se++)
-                for (int b = 0; b <= cfg->bit_rate_hi && b <= br_max; b++)
-                    n_hi = nslots[(size_t)se * (br_max + 1) + b] > n_hi ? nslots[(size_t)se * (br_max + 1) + b] : n_hi;
-            env->hot = env->fast && J == 1 && p.k == 5 && p.cand_stride == 8 && t->num_bit_rates == 0 && cfg->bit_rate_hi < 128 &&
-                       cfg->bit_rate_lo >= 0 && n_hi <= 16 && (p.obs_dim & 1) == 0 && p.E <= 256 && !std::getenv("ORLG_NO_HOT");
-            if (env->hot && !encode_mask_map(env)) env->hot = false;
-            // the persistent rollout kernel (orlg_rollout.cuh): DeepRMSA-v0 under the HOT conditions; RMSA-v0 with continuous
-            // bit rates below 128 Gb/s whose slot counts fit the 4-round shift-AND; RWA-v0 (one wavelength per lightpath)
-            const bool small_n = t->num_bit_rates == 0 && cfg->bit_rate_hi < 128 && cfg->bit_rate_lo >= 0 && n_hi <= 16;
-            env->ro_ok = cfg->kind == ORLG_DEEPRMSA ? env->hot
-                         : (ea == cudaSuccess && p.E <= 32 && (cfg->kind == ORLG_RWA || small_n) && !std::getenv("ORLG_NO_HOT"));
-        }
+            for (int b = 0; b <= cfg.bit_rate_hi && b <= p.br_max; b++) n_hi = std::max<int>(n_hi, h.nslots[(size_t)se * (p.br_max + 1) + b]);
+        const bool small_n = p.n_bit_rates == 0 && cfg.bit_rate_hi < 128 && cfg.bit_rate_lo >= 0 && n_hi <= 16;
+        const bool no_hot = std::getenv("ORLG_NO_HOT") != nullptr;
+        // steady-state specialisation: small slot counts, exactly KM candidate paths per pair, j = 1, 8-byte candidate
+        // cache, even observation width
+        env->hot = env->fast && p.J == 1 && p.k == 5 && p.cand_stride == 8 && small_n && (p.obs_dim & 1) == 0 && p.E <= 256 && !no_hot;
+        if (env->hot && !encode_mask_map(env)) env->hot = false;
+        // the persistent rollout kernel (orlg_rollout.cuh): DeepRMSA-v0 under the HOT conditions; RMSA-v0 with small slot
+        // counts; RWA-v0 (one wavelength per lightpath)
+        env->ro_ok = p.kind == ORLG_DEEPRMSA ? env->hot
+                     : (ea == cudaSuccess && p.E <= 32 && (p.kind == ORLG_RWA || small_n) && !no_hot);
     }
+    if (const size_t obs_smem = step_obs_smem(p); obs_smem > 48 * 1024) {
+        cudaError_t e1 = cudaFuncSetAttribute(step_kernel<ORLG_DEEPRMSA, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)obs_smem);
+        cudaError_t e2 = cudaFuncSetAttribute(step_kernel<ORLG_DEEPRMSA, KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)obs_smem);
+        if (e1 != cudaSuccess || e2 != cudaSuccess) return fail(ORLG_E_CUDA, "cudaFuncSetAttribute(shared memory) failed");
+    }
+    return ORLG_OK;
+}
+}  // namespace
 
-    if (env->obs_smem > 48 * 1024) {
-        cudaError_t e1 = cudaFuncSetAttribute(step_kernel<ORLG_DEEPRMSA, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->obs_smem);
-        cudaError_t e2 = cudaFuncSetAttribute(step_kernel<ORLG_DEEPRMSA, KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->obs_smem);
-        if (e1 != cudaSuccess || e2 != cudaSuccess) { orlg_destroy(env); return fail(ORLG_E_CUDA, "cudaFuncSetAttribute(shared memory) failed"); }
-    }
-    *out = env;
+extern "C" {
+
+const char *orlg_last_error(void) { return g_err.c_str(); }
+int orlg_version(void) { return ORLG_VERSION; }
+
+int orlg_create(const orlg_config *cfg, const orlg_tables *t, int device, orlg_env **out) {
+    if (!cfg || !t || !out) return fail(ORLG_E_INVALID, "null argument");
+    *out = nullptr;
+    Params p; bool wide; int se_max;
+    int rc = configure(*cfg, *t, device, p, wide, se_max);
+    if (rc) return rc;
+    DeviceGuard guard(device);
+    std::unique_ptr<orlg_env, int (*)(orlg_env *)> env(new orlg_env(), orlg_destroy);
+    env->p = p; env->cfg = *cfg; env->device = device; env->wide = wide;
+    env->ro_lpw = choose_rollout_lpw(cfg->num_envs);
+    HostTables h;
+    rc = upload_tables(env.get(), *cfg, *t, se_max, h);
+    if (!rc) rc = alloc_state(env.get(), *t);
+    if (!rc) rc = upload_fast_blob(env.get(), *t, h, se_max);
+    if (!rc) rc = select_instances(env.get(), *cfg, h, se_max);
+    if (rc) return rc;
+    *out = env.release();
     return ORLG_OK;
 }
 
 int orlg_destroy(orlg_env *env) {
     if (!env) return ORLG_OK;
     DeviceGuard guard(env->device);
-    for (void *ptr : env->allocs) cudaFree(ptr);
-    for (int i = 0; i < RO_HOST_BUFFERS; i++) {
-        if (env->ro_pk_dev[i]) cudaFree(env->ro_pk_dev[i]);
-        if (env->ro_pk_host[i]) cudaFreeHost(env->ro_pk_host[i]);
-        if (env->ro_pk_ev[i]) cudaEventDestroy(env->ro_pk_ev[i]);
-        if (env->ro_k_ev[i]) cudaEventDestroy(env->ro_k_ev[i]);
-        if (env->ro_act_dev[i]) cudaFree(env->ro_act_dev[i]);
-    }
-    if (env->ro_copy_stream) cudaStreamDestroy(env->ro_copy_stream);
     delete env;
     return ORLG_OK;
 }
@@ -664,8 +731,8 @@ int orlg_kernel_info(const orlg_env *env, orlg_kernel_info_t *out) {
     out->fast = env->fast;
     out->hot = env->hot;
     out->rollout_kernel = env->ro_ok;
-    out->rollout_lanes = rollout_lpw(env);
-    out->link_template = !env->wide && env->p.E == 22 ? 22 : 0;     // the ET choice of launch_fast / rollout_impl
+    out->rollout_lanes = env->ro_lpw;
+    out->link_template = link_template(env);
     out->last_rollout_persistent = env->ro_last_persistent;
     return ORLG_OK;
 }
@@ -695,10 +762,7 @@ int orlg_reset(orlg_env *env, int full, void *obs_dev, orlg_stream stream) {
     io.policy = -1;
     io.obs = env->p.obs_dim ? obs_dev : nullptr;
     if (full) env->ro_valid = false;           // everything is reset below: nothing to convert back
-    else {
-        int rc0 = ensure_canonical(env, (cudaStream_t)stream);
-        if (rc0) return rc0;
-    }
+    else if (int rc0 = ensure_canonical(env, (cudaStream_t)stream)) return rc0;
     if (full) {
         fill_events_kernel<<<592, 256, 0, (cudaStream_t)stream>>>(env->p);
         CUDA_OK(cudaGetLastError());
@@ -711,10 +775,7 @@ int orlg_reset(orlg_env *env, int full, void *obs_dev, orlg_stream stream) {
 // orlg_step; fused_policy >= 0 (wide kernels only): the heuristic is evaluated inside the step kernel, actions_dev receives it
 static int step_impl(orlg_env *env, const int32_t *actions_dev, int fused_policy, int32_t *actions_out, void *obs_dev, float *reward_dev,
                      uint8_t *done_dev, int32_t *decision_dev, int64_t *info_dev, orlg_stream stream) {
-    {
-        int rc0 = ensure_canonical(env, (cudaStream_t)stream);
-        if (rc0) return rc0;
-    }
+    if (int rc0 = ensure_canonical(env, (cudaStream_t)stream)) return rc0;
     StepIO io;
     io.policy = fused_policy;
     io.actions_out = actions_out;
@@ -765,28 +826,12 @@ int orlg_heuristic(orlg_env *env, int which, int32_t *actions_dev, orlg_stream s
     if (which < 0 || which > ORLG_HEUR_SAP_LF) return fail(ORLG_E_INVALID, "unknown heuristic");
     const int threads = 128, blocks = (env->p.n + threads - 1) / threads;
     cudaStream_t s = (cudaStream_t)stream;
-    if (env->wide) {
-        if (env->p.kind == ORLG_RMSA && which == ORLG_HEUR_SAP_LF) return fail(ORLG_E_UNSUPPORTED, "last-fit exists for RWA only");
-        if (env->p.kind == ORLG_DEEPRMSA && which > ORLG_HEUR_SAP_FF) return fail(ORLG_E_UNSUPPORTED, "DeepRMSA has SP-FF and SAP-FF only");
-        switch (env->p.kind) {
-        case ORLG_RWA: launch_heuristic_wide<ORLG_RWA>(env, which, actions_dev, s); break;
-        case ORLG_RMSA: launch_heuristic_wide<ORLG_RMSA>(env, which, actions_dev, s); break;
-        case ORLG_DEEPRMSA: launch_heuristic_wide<ORLG_DEEPRMSA>(env, which, actions_dev, s); break;
-        default: launch_heuristic_wide<ORLG_RMCSA>(env, which, actions_dev, s); break;
-        }
-        CUDA_OK(cudaGetLastError());
-        return ORLG_OK;
-    }
-    switch (env->p.kind) {
-    case ORLG_RWA: heuristic_kernel<ORLG_RWA><<<blocks, threads, 0, s>>>(env->p, which, actions_dev); break;
-    case ORLG_RMSA:
-        if (which == ORLG_HEUR_SAP_LF) return fail(ORLG_E_UNSUPPORTED, "last-fit exists for RWA only");
-        heuristic_kernel<ORLG_RMSA><<<blocks, threads, 0, s>>>(env->p, which, actions_dev); break;
-    case ORLG_DEEPRMSA:
-        if (which > ORLG_HEUR_SAP_FF) return fail(ORLG_E_UNSUPPORTED, "DeepRMSA has SP-FF and SAP-FF only");
-        heuristic_kernel<ORLG_DEEPRMSA><<<blocks, threads, 0, s>>>(env->p, which, actions_dev); break;
-    case ORLG_RMCSA: heuristic_kernel<ORLG_RMCSA><<<blocks, threads, 0, s>>>(env->p, which, actions_dev); break;
-    }
+    if (const char *why = heuristic_refusal(env->p.kind, which)) return fail(ORLG_E_UNSUPPORTED, why);
+    for_kind(env->p.kind, [&](auto K) {
+        if (env->wide) for_words(env->p.nwv, [&](auto W) {
+            heuristic_wide_kernel<decltype(K)::value, decltype(W)::value><<<blocks, threads, 0, s>>>(env->p, which, actions_dev); });
+        else heuristic_kernel<decltype(K)::value><<<blocks, threads, 0, s>>>(env->p, which, actions_dev);
+    });
     CUDA_OK(cudaGetLastError());
     return ORLG_OK;
 }
@@ -807,8 +852,7 @@ static int run_export(orlg_env *env, uint32_t *masks, int32_t *alloc, double *no
     DeviceGuard guard(env->device);
     const int threads = 128, blocks = (env->p.n + threads - 1) / threads;
     if (alloc) {                               // the allocation matrix is rebuilt from the release-event table
-        int rc0 = ensure_canonical(env, (cudaStream_t)stream);
-        if (rc0) return rc0;
+        if (int rc0 = ensure_canonical(env, (cudaStream_t)stream)) return rc0;
     }
     if (env->wide && (masks || alloc)) {
         export_wide_kernel<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->p, masks, alloc);
@@ -969,12 +1013,7 @@ int orlg_path_only_first_fit(orlg_env *env, const int32_t *path_actions_dev, int
         return fail(ORLG_E_UNSUPPORTED, "PathOnlyFirstFitAction exists for RMSA-v0 and RWA-v0 (the RMCSA one raises upstream)");
     const int blocks = (env->p.n + 127) / 128;
     cudaStream_t s = (cudaStream_t)stream;
-    switch (env->p.nwv) {
-    case 1: path_only_first_fit_kernel<1><<<blocks, 128, 0, s>>>(env->p, path_actions_dev, actions_dev); break;
-    case 2: path_only_first_fit_kernel<2><<<blocks, 128, 0, s>>>(env->p, path_actions_dev, actions_dev); break;
-    case 3: path_only_first_fit_kernel<3><<<blocks, 128, 0, s>>>(env->p, path_actions_dev, actions_dev); break;
-    default: path_only_first_fit_kernel<4><<<blocks, 128, 0, s>>>(env->p, path_actions_dev, actions_dev); break;
-    }
+    for_words(env->p.nwv, [&](auto W) { path_only_first_fit_kernel<decltype(W)::value><<<blocks, 128, 0, s>>>(env->p, path_actions_dev, actions_dev); });
     CUDA_OK(cudaGetLastError());
     return ORLG_OK;
 }
@@ -990,21 +1029,13 @@ static int rollout_impl(orlg_env *env, int steps, int policy, void *obs_dev, flo
     if (steps == 0) return ORLG_OK;
     Params &p = env->p;
     cudaStream_t s = (cudaStream_t)stream;
-    bool policy_ok;
-    if (p.traffic == ORLG_TRAFFIC_TRACE) policy_ok = policy == ORLG_POLICY_REPLAY;
-    else if (p.kind == ORLG_DEEPRMSA) policy_ok = policy == ORLG_POLICY_RANDOM || policy == ORLG_POLICY_REPLAY || policy == ORLG_HEUR_SP_FF || policy == ORLG_HEUR_SAP_FF;
-    else if (p.kind == ORLG_RMSA) policy_ok = policy != ORLG_HEUR_SAP_LF;
-    else policy_ok = true;
-    const bool persistent = env->ro_ok && !p.stats && !p.obs_f64 && !p.br_hist && policy_ok;
     RolloutArgs ra;
     std::memset(&ra, 0, sizeof(ra));
     int wpc = 0;
     size_t smem = 0;
-    if (persistent && rollout_plan(env, &wpc, &ra, &smem)) {
+    if (rollout_kernel_applies(env, policy) && rollout_plan(env, &wpc, &ra, &smem)) {
         if (!env->ro_ev) {
-            const size_t n = (size_t)p.n;
-            const size_t lpw = (size_t)rollout_lpw(env);
-            const size_t warps = (n + lpw - 1) / lpw;
+            const size_t n = (size_t)p.n, warps = (n + env->ro_lpw - 1) / env->ro_lpw;
             int rc = dev_alloc(env, &env->ro_ev, warps * 32 * ((size_t)p.heap_cap + 2 * RO_WCAP), false);
             if (!rc) rc = dev_alloc(env, &env->ro_st_u32, 4 * n, false);
             if (!rc) rc = dev_alloc(env, &env->ro_st_f64, (2 + RO_SIDE) * n, false);
@@ -1021,7 +1052,7 @@ static int rollout_impl(orlg_env *env, int steps, int policy, void *obs_dev, flo
         if (packed_dev && p.kind != ORLG_DEEPRMSA) return fail(ORLG_E_UNSUPPORTED, "packed records describe the DeepRMSA observation");
         rollout_state_args(env, &ra);
         ra.resume = env->ro_valid ? 1 : 0;
-        cudaError_t e = p.E == 22 ? launch_rollout<22>(env, ra, policy, wpc, smem, s) : launch_rollout<0>(env, ra, policy, wpc, smem, s);
+        cudaError_t e = link_template(env) == 22 ? launch_rollout<22>(env, ra, policy, wpc, smem, s) : launch_rollout<0>(env, ra, policy, wpc, smem, s);
         if (e != cudaSuccess) return fail(ORLG_E_CUDA, std::string("rollout launch: ") + cudaGetErrorString(e));
         p.lockstep_ridx += (unsigned)steps;
         env->ro_valid = true;
@@ -1031,38 +1062,27 @@ static int rollout_impl(orlg_env *env, int steps, int policy, void *obs_dev, flo
     env->ro_last_persistent = false;
     if (packed_dev) return fail(ORLG_E_UNSUPPORTED, "packed records exist for the persistent DeepRMSA rollout kernel only (k = 5, j = 1, float32)");
     // generic: the same T steps as separate policy + step launches
-    {
-        int rc = ensure_canonical(env, s);
-        if (rc) return rc;
-    }
+    int rc = ensure_canonical(env, s);
+    if (rc) return rc;
     const int adim = orlg_action_dim(env);
     if (policy != ORLG_POLICY_REPLAY && !actions_dev && !env->ro_actions) {
-        int rc = dev_alloc(env, &env->ro_actions, (size_t)p.n * adim, false);
+        rc = dev_alloc(env, &env->ro_actions, (size_t)p.n * adim, false);
         if (rc) return rc;
     }
     const size_t obs_row = (size_t)p.obs_dim * (p.obs_f64 ? 8 : 4);
     // wide kernels: the heuristic runs in the step kernel's prologue (one launch per step; the chosen path's masks are read once)
-    bool fuse = env->wide && policy >= 0;
-    if (fuse && ((p.kind == ORLG_RMSA && policy == ORLG_HEUR_SAP_LF) || (p.kind == ORLG_DEEPRMSA && policy > ORLG_HEUR_SAP_FF))) fuse = false;
-    for (int t = 0; t < steps; t++) {
+    const bool fuse = env->wide && policy >= 0 && !heuristic_refusal(p.kind, policy);
+    for (int t = 0; t < steps && !rc; t++) {
         int32_t *a = actions_dev ? actions_dev + (size_t)t * p.n * adim : env->ro_actions;
-        if (fuse) {
-            int rc = step_impl(env, nullptr, policy, actions_dev ? a : nullptr,
-                               (obs_dev && p.obs_dim) ? reinterpret_cast<unsigned char *>(obs_dev) + (size_t)t * p.n * obs_row : nullptr,
-                               reward_dev ? reward_dev + (size_t)t * p.n : nullptr, done_dev ? done_dev + (size_t)t * p.n : nullptr,
-                               nullptr, nullptr, stream);
-            if (rc) return rc;
-            continue;
-        }
-        int rc = policy == ORLG_POLICY_REPLAY ? ORLG_OK
-                 : (policy == ORLG_POLICY_RANDOM ? orlg_random_actions(env, a, stream) : orlg_heuristic(env, policy, a, stream));
-        if (rc) return rc;
-        rc = orlg_step(env, a, (obs_dev && p.obs_dim) ? reinterpret_cast<unsigned char *>(obs_dev) + (size_t)t * p.n * obs_row : nullptr,
-                       reward_dev ? reward_dev + (size_t)t * p.n : nullptr, done_dev ? done_dev + (size_t)t * p.n : nullptr,
-                       nullptr, nullptr, stream);
-        if (rc) return rc;
+        void *o = (obs_dev && p.obs_dim) ? reinterpret_cast<unsigned char *>(obs_dev) + (size_t)t * p.n * obs_row : nullptr;
+        float *r = reward_dev ? reward_dev + (size_t)t * p.n : nullptr;
+        uint8_t *d = done_dev ? done_dev + (size_t)t * p.n : nullptr;
+        if (fuse) rc = step_impl(env, nullptr, policy, actions_dev ? a : nullptr, o, r, d, nullptr, nullptr, stream);
+        else if (policy != ORLG_POLICY_REPLAY)
+            rc = policy == ORLG_POLICY_RANDOM ? orlg_random_actions(env, a, stream) : orlg_heuristic(env, policy, a, stream);
+        if (!rc && !fuse) rc = orlg_step(env, a, o, r, d, nullptr, nullptr, stream);
     }
-    return ORLG_OK;
+    return rc;
 }
 
 
@@ -1249,62 +1269,43 @@ int orlg_rollout_host(orlg_env *env, int steps, int policy, float *obs_host, flo
     const int chunk = chunk_steps > 0 ? chunk_steps : 4;
     const size_t rows = (size_t)chunk * p.n;
     constexpr int NB = RO_HOST_BUFFERS, AHEAD = RO_HOST_BUFFERS - 1;      // the device runs up to AHEAD chunks ahead of the host decoder
-    if (env->ro_pk_rows < rows) {                       // (re)allocate the record buffers (device + pinned host)
-        for (int i = 0; i < NB; i++) {
-            if (env->ro_pk_dev[i]) cudaFree(env->ro_pk_dev[i]);
-            if (env->ro_pk_host[i]) cudaFreeHost(env->ro_pk_host[i]);
-            env->ro_pk_dev[i] = nullptr; env->ro_pk_host[i] = nullptr;
-            if (cudaMalloc(&env->ro_pk_dev[i], rows * 32) != cudaSuccess) return fail(ORLG_E_NOMEM, "cudaMalloc (packed records) failed");
-            if (cudaHostAlloc(&env->ro_pk_host[i], rows * 32, cudaHostAllocDefault) != cudaSuccess) return fail(ORLG_E_NOMEM, "cudaHostAlloc (packed records) failed");
-            if (!env->ro_pk_ev[i]) CUDA_OK(cudaEventCreateWithFlags(&env->ro_pk_ev[i], cudaEventDisableTiming));
-            if (!env->ro_k_ev[i]) CUDA_OK(cudaEventCreateWithFlags(&env->ro_k_ev[i], cudaEventDisableTiming));
-        }
-        env->ro_pk_rows = rows;
-    }
-    if (!env->ro_copy_stream) CUDA_OK(cudaStreamCreateWithFlags(&env->ro_copy_stream, cudaStreamNonBlocking));
     const size_t adim = (size_t)orlg_action_dim(env);
-    if (replay && env->ro_act_rows < rows) {             // device copies of the action chunks
-        for (int i = 0; i < NB; i++) {
-            if (env->ro_act_dev[i]) cudaFree(env->ro_act_dev[i]);
-            env->ro_act_dev[i] = nullptr;
-            if (cudaMalloc(&env->ro_act_dev[i], rows * adim * sizeof(int32_t)) != cudaSuccess) return fail(ORLG_E_NOMEM, "cudaMalloc (action chunks) failed");
-        }
-        env->ro_act_rows = rows;
-    }
+    HostPipeline &hp = env->host_pipe;
+    if (int rc0 = hp.reserve(rows, replay, adim)) return rc0;
     const int nchunks = (steps + chunk - 1) / chunk;
     const size_t D = (size_t)p.obs_dim;
-    cudaStream_t sc = env->ro_copy_stream;
+    cudaStream_t sc = hp.copy_stream;
     // chunk c: [user stream] H2D of its actions, the rollout kernel -> [copy stream] D2H of its records.  The kernel
     // of chunk c + 1 overlaps the copy of chunk c; buffer b = c % NB is reused by chunk c + NB, whose kernel waits for the copy
     // of chunk c (event) and which is only enqueued after the host has decoded chunk c (program order below).
     auto enqueue = [&](int c) -> int {
         const int b = c % NB, t0 = c * chunk, tc = steps - t0 < chunk ? steps - t0 : chunk;
         if (replay)
-            CUDA_OK(cudaMemcpyAsync(env->ro_act_dev[b], actions_host + (size_t)t0 * p.n * adim, (size_t)tc * p.n * adim * sizeof(int32_t),
+            CUDA_OK(cudaMemcpyAsync(hp.act_dev[b], actions_host + (size_t)t0 * p.n * adim, (size_t)tc * p.n * adim * sizeof(int32_t),
                                     cudaMemcpyHostToDevice, s));
-        if (c >= NB) CUDA_OK(cudaStreamWaitEvent(s, env->ro_pk_ev[b], 0));
-        int rc = rollout_impl(env, tc, policy, nullptr, nullptr, nullptr, replay ? env->ro_act_dev[b] : nullptr,
-                              reinterpret_cast<uint32_t *>(env->ro_pk_dev[b]), stream);
+        if (c >= NB) CUDA_OK(cudaStreamWaitEvent(s, hp.pk_ev[b], 0));
+        int rc = rollout_impl(env, tc, policy, nullptr, nullptr, nullptr, replay ? hp.act_dev[b] : nullptr,
+                              reinterpret_cast<uint32_t *>(hp.pk_dev[b]), stream);
         if (rc) return rc;
-        CUDA_OK(cudaEventRecord(env->ro_k_ev[b], s));
-        CUDA_OK(cudaStreamWaitEvent(sc, env->ro_k_ev[b], 0));
-        CUDA_OK(cudaMemcpyAsync(env->ro_pk_host[b], env->ro_pk_dev[b], (size_t)tc * p.n * 32, cudaMemcpyDeviceToHost, sc));
-        CUDA_OK(cudaEventRecord(env->ro_pk_ev[b], sc));
+        CUDA_OK(cudaEventRecord(hp.k_ev[b], s));
+        CUDA_OK(cudaStreamWaitEvent(sc, hp.k_ev[b], 0));
+        CUDA_OK(cudaMemcpyAsync(hp.pk_host[b], hp.pk_dev[b], (size_t)tc * p.n * 32, cudaMemcpyDeviceToHost, sc));
+        CUDA_OK(cudaEventRecord(hp.pk_ev[b], sc));
         return ORLG_OK;
     };
     for (int c = 0; c < AHEAD && c < nchunks; c++) { int rc = enqueue(c); if (rc) return rc; }
     for (int c = 0; c < nchunks; c++) {
         if (c + AHEAD < nchunks) { int rc = enqueue(c + AHEAD); if (rc) return rc; }
         const int b = c % NB, t0 = c * chunk, tc = steps - t0 < chunk ? steps - t0 : chunk;
-        CUDA_OK(cudaEventSynchronize(env->ro_pk_ev[b]));
+        CUDA_OK(cudaEventSynchronize(hp.pk_ev[b]));
         const size_t off = (size_t)t0 * p.n;
-        int rc = orlg_expand_packed(reinterpret_cast<const uint32_t *>(env->ro_pk_host[b]), (int64_t)tc * p.n, p.N, p.S,
+        int rc = orlg_expand_packed(reinterpret_cast<const uint32_t *>(hp.pk_host[b]), (int64_t)tc * p.n, p.N, p.S,
                                     obs_host ? obs_host + off * D : nullptr, reward_host ? reward_host + off : nullptr,
                                     done_host ? done_host + off : nullptr, (actions_host && !replay) ? actions_host + off : nullptr, threads);
         if (rc) return rc;
     }
     // the user's stream must not run ahead of the copies that still read the record buffers (a later call reuses them)
-    CUDA_OK(cudaStreamWaitEvent(s, env->ro_pk_ev[(nchunks - 1) % NB], 0));
+    CUDA_OK(cudaStreamWaitEvent(s, hp.pk_ev[(nchunks - 1) % NB], 0));
     return ORLG_OK;
 }
 
@@ -1313,7 +1314,9 @@ struct orlg_policy {
     PolicyParams pp;
     int device;
     size_t smem;
-    void *w_dev, *b_dev;
+    void *w_dev = nullptr, *b_dev = nullptr;
+
+    ~orlg_policy() { cudaFree(w_dev); cudaFree(b_dev); }
 };
 
 static unsigned short f32_to_bf16(float f) {          // round to nearest even
@@ -1349,25 +1352,21 @@ int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers,
     for (int r = 0; r < n_actions + 1; r++)                     // action_net rows, then value_net
         for (int k = 0; k < PL_H; k++) blob[(off + pl_operand_offset(PL_NOUT, r, k)) / 2] = f32_to_bf16(w[(size_t)r * PL_H + k]);
     for (int r = 0; r < n_actions + 1; r++) bias[PL_LAYERS * PL_H + r] = b[r];
-    orlg_policy *pol = new orlg_policy();
-    pol->device = device; pol->w_dev = nullptr; pol->b_dev = nullptr;
+    std::unique_ptr<orlg_policy, int (*)(orlg_policy *)> pol(new orlg_policy(), orlg_policy_destroy);
+    pol->device = device;
     if (cudaMalloc(&pol->w_dev, bytes) != cudaSuccess || cudaMalloc(&pol->b_dev, bias.size() * 4) != cudaSuccess ||
         cudaMemcpy(pol->w_dev, blob.data(), bytes, cudaMemcpyHostToDevice) != cudaSuccess ||
-        cudaMemcpy(pol->b_dev, bias.data(), bias.size() * 4, cudaMemcpyHostToDevice) != cudaSuccess) {
-        cudaFree(pol->w_dev); cudaFree(pol->b_dev); delete pol;
+        cudaMemcpy(pol->b_dev, bias.data(), bias.size() * 4, cudaMemcpyHostToDevice) != cudaSuccess)
         return fail(ORLG_E_NOMEM, "policy weight upload failed");
-    }
     pol->pp.w_blob = reinterpret_cast<const uint4 *>(pol->w_dev);
     pol->pp.w_bytes = (int)bytes;
     pol->pp.bias = reinterpret_cast<const float *>(pol->b_dev);
     pol->pp.obs_dim = obs_dim; pol->pp.n_actions = n_actions;
     pol->smem = bytes + (size_t)PL_GROUPS * PL_TILE * PL_H * 2 + bias.size() * 4 + 64;
     if (cudaFuncSetAttribute(mlp_policy_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pol->smem) != cudaSuccess ||
-        cudaFuncSetAttribute(mlp_policy_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pol->smem) != cudaSuccess) {
-        cudaFree(pol->w_dev); cudaFree(pol->b_dev); delete pol;
+        cudaFuncSetAttribute(mlp_policy_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pol->smem) != cudaSuccess)
         return fail(ORLG_E_CUDA, "cudaFuncSetAttribute(policy kernel shared memory) failed");
-    }
-    *out = pol;
+    *out = pol.release();
     return ORLG_OK;
 }
 
@@ -1471,7 +1470,6 @@ int64_t orlg_request_index(const orlg_env *env) { return env ? (int64_t)env->p.l
 int orlg_policy_destroy(orlg_policy *pol) {
     if (!pol) return ORLG_OK;
     DeviceGuard guard(pol->device);
-    cudaFree(pol->w_dev); cudaFree(pol->b_dev);
     delete pol;
     return ORLG_OK;
 }
