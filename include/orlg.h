@@ -185,12 +185,17 @@ int orlg_expand_packed(const uint32_t *packed_host, int64_t rows, int num_nodes,
 int orlg_rollout_host(orlg_env *env, int steps, int policy, float *obs_host, float *reward_host, uint8_t *done_host,
                       int32_t *actions_host, int chunk_steps, int threads, orlg_stream stream);
 
-/* ---- the PPO agent of the reference's notebook, evaluated on the device ------------------------------------------ */
-/* model.predict(obs, deterministic=True) of the agent the reference trains and ships (examples/stable_baselines3/
- * DeepRMSA.ipynb cell 13: PPO(MlpPolicy, env, policy_kwargs=dict(net_arch=5*[128])); bkp/deeprmsa-ppo-trained/best_model.zip):
- * obs -> 5 x (Linear 128 + tanh) -> action_net / value_net -> argmax.  One fused kernel on the tensor cores (bf16 operands,
- * fp32 accumulation).  weights: HOST float32, the nn.Linear matrices [out, in] row-major one after the other (5 trunk layers,
- * action_net, value_net); biases likewise. */
+/* ---- SB3 MlpPolicy agents (the PPO agent of the reference's notebook among them), evaluated on the device ---------- */
+/* model.predict(obs, deterministic=True) of an SB3 MlpPolicy: obs -> n_hidden_layers x (Linear hidden + tanh) -> action_net /
+ * value_net -> argmax.  The agent the reference trains and ships (examples/stable_baselines3/DeepRMSA.ipynb cell 13:
+ * PPO(MlpPolicy, env, policy_kwargs=dict(net_arch=5*[128])); bkp/deeprmsa-ppo-trained/best_model.zip) is 5 x 128; SB3's PPO /
+ * A2C default trunk is 2 x 64.  One fused kernel on the tensor cores (bf16 operands, fp32 accumulation), all weights resident
+ * in shared memory.  Accepted: obs_dim even in 2..64, n_actions 1..15, hidden a multiple of 16 in 16..128, n_hidden_layers
+ * >= 1 with hidden * 64 * 2 + (n_hidden_layers - 1) * hidden^2 * 2 + 16 * hidden * 2 (weights) + 65536 (activations) +
+ * (n_hidden_layers * hidden + 16) * 4 + 64 <= 232448 bytes of shared memory (5 x 128 and 6 x 112 fit, 6 x 128 does not);
+ * anything else is ORLG_E_UNSUPPORTED.  weights: HOST float32, the nn.Linear matrices [out, in] row-major one after the other
+ * (the trunk layers, action_net, value_net); biases likewise.  5 x 128 runs a kernel instance compiled for it (environment
+ * ORLG_POLICY_GENERAL at create: the run-time instance the other architectures use, the same results bit for bit). */
 typedef struct orlg_policy orlg_policy;
 int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers, int n_actions, const float *weights,
                        const float *biases, orlg_policy **out);
@@ -220,7 +225,8 @@ int orlg_policy_sample(orlg_policy *pol, const float *obs_dev, int n, const orlg
  *   obs_dev      f32 [steps + 1, N, obs_dim]  required: obs[0] = observation of the pending request, obs[t+1] = what step t returned
  *   actions_dev  i32 [steps, N]      log_prob_dev f32 [steps, N]      value_dev f32 [steps + 1, N] (value[steps] = bootstrap value)
  *   reward_dev   f32 [steps, N]      done_dev     u8  [steps, N]      (all but obs may be NULL)
- *   critic       NULL = the actor's value head; else a handle whose value head is the critic's (separate SB3 >= 1.8 trunk)
+ *   critic       NULL = the actor's value head; else a handle whose value head is the critic's (separate SB3 >= 1.8 trunk,
+ *                which may have its own width and depth: n_actions = 1, value_net as both head rows)
  * The draws are keyed by (seed, global env id, the env's request index): results do not depend on sharding, on how a rollout is
  * split into calls, or on a checkpoint taken between calls.  deterministic = 1: argmax actions. */
 int orlg_rollout_policy(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,

@@ -1309,15 +1309,28 @@ int orlg_rollout_host(orlg_env *env, int steps, int policy, float *obs_host, flo
     return ORLG_OK;
 }
 
-// ---------------------------------------------------------------- the shipped PPO agent (orlg_policy.cuh)
+// ---------------------------------------------------------------- MLP policies on the tensor cores (orlg_policy.cuh)
 struct orlg_policy {
     PolicyParams pp;
     int device;
     size_t smem;
+    bool general;                     // ORLG_POLICY_GENERAL at orlg_policy_create: the run-time (H, L) instance also for 5 x 128
     void *w_dev = nullptr, *b_dev = nullptr;
 
     ~orlg_policy() { cudaFree(w_dev); cudaFree(b_dev); }
 };
+
+}  // extern "C"
+
+// The one place that picks the kernel instance of a handle: the shipped agent's 5 x 128 has one compiled for it, every other
+// architecture runs the instance that reads H and L from PolicyParams.
+template <bool SAMPLE>
+static decltype(&mlp_policy_kernel<SAMPLE, 0, 0>) policy_kernel(const orlg_policy *pol) {
+    if (pol->pp.H == 128 && pol->pp.L == 5 && !pol->general) return mlp_policy_kernel<SAMPLE, 128, 5>;
+    return mlp_policy_kernel<SAMPLE, 0, 0>;
+}
+
+extern "C" {
 
 static unsigned short f32_to_bf16(float f) {          // round to nearest even
     unsigned u;
@@ -1330,30 +1343,43 @@ int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers,
                        const float *biases, orlg_policy **out) {
     if (!weights || !biases || !out) return fail(ORLG_E_INVALID, "null argument");
     *out = nullptr;
-    if (hidden != PL_H || n_hidden_layers != PL_LAYERS || obs_dim < 2 || obs_dim > PL_K0 || (obs_dim & 1) || n_actions < 1 ||
-        n_actions + 1 > PL_NOUT)
-        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel is built for obs_dim <= 64 (even), 5 hidden layers of 128, <= 15 actions");
+    if (obs_dim < 2 || obs_dim > PL_K0 || (obs_dim & 1) || n_actions < 1 || n_actions + 1 > PL_NOUT)
+        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel is built for obs_dim <= 64 (even), <= 15 actions; got obs_dim " +
+                                            std::to_string(obs_dim) + ", " + std::to_string(n_actions) + " actions");
+    if (hidden < 16 || hidden > PL_HMAX || hidden % 16)
+        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs a hidden width that is a multiple of 16 in 16..128; got " +
+                                            std::to_string(hidden));
+    if (n_hidden_layers < 1)
+        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs at least one hidden layer; got " + std::to_string(n_hidden_layers));
+    const int H = hidden, L = n_hidden_layers;
+    const size_t smem = pl_smem_bytes(H, L);
+    if (smem > (size_t)PL_SMEM_MAX)         // all weights stay resident in shared memory
+        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs " + std::to_string(smem) + " bytes of shared memory, " +
+                                            std::to_string(PL_SMEM_MAX) + " available, for " + std::to_string(L) +
+                                            " hidden layers of " + std::to_string(H));
     int n_dev = 0;
     if (cudaGetDeviceCount(&n_dev) != cudaSuccess || device < 0 || device >= n_dev) return fail(ORLG_E_CUDA, "no such CUDA device");
     DeviceGuard guard(device);
-    // bf16 weights in the shared-memory operand layout of the kernel: layer l is an [N x K] K-major operand
-    size_t bytes = (size_t)PL_H * PL_K0 * 2 + (size_t)(PL_LAYERS - 1) * PL_H * PL_H * 2 + (size_t)PL_NOUT * PL_H * 2;
+    // bf16 weights in the shared-memory operand layout of the kernel: layer l is an [N x K] K-major operand, K = 64 (the
+    // padded observation) for layer 0, H after it
+    const size_t bytes = pl_weight_bytes(H, L);
     std::vector<unsigned short> blob(bytes / 2, 0);
-    std::vector<float> bias(PL_LAYERS * PL_H + PL_NOUT, 0.0f);
+    std::vector<float> bias((size_t)L * H + PL_NOUT, 0.0f);
     const float *w = weights, *b = biases;
     size_t off = 0;
-    for (int l = 0; l < PL_LAYERS; l++) {
-        const int K = l == 0 ? obs_dim : PL_H, Kp = l == 0 ? PL_K0 : PL_H;
-        for (int r = 0; r < PL_H; r++)
-            for (int k = 0; k < K; k++) blob[(off + pl_operand_offset(PL_H, r, k)) / 2] = f32_to_bf16(w[(size_t)r * K + k]);
-        for (int r = 0; r < PL_H; r++) bias[l * PL_H + r] = b[r];
-        w += (size_t)PL_H * K; b += PL_H; off += (size_t)PL_H * Kp * 2;
+    for (int l = 0; l < L; l++) {
+        const int K = l == 0 ? obs_dim : H, Kp = l == 0 ? PL_K0 : H;
+        for (int r = 0; r < H; r++)
+            for (int k = 0; k < K; k++) blob[(off + pl_operand_offset(H, r, k)) / 2] = f32_to_bf16(w[(size_t)r * K + k]);
+        for (int r = 0; r < H; r++) bias[(size_t)l * H + r] = b[r];
+        w += (size_t)H * K; b += H; off += (size_t)H * Kp * 2;
     }
     for (int r = 0; r < n_actions + 1; r++)                     // action_net rows, then value_net
-        for (int k = 0; k < PL_H; k++) blob[(off + pl_operand_offset(PL_NOUT, r, k)) / 2] = f32_to_bf16(w[(size_t)r * PL_H + k]);
-    for (int r = 0; r < n_actions + 1; r++) bias[PL_LAYERS * PL_H + r] = b[r];
+        for (int k = 0; k < H; k++) blob[(off + pl_operand_offset(PL_NOUT, r, k)) / 2] = f32_to_bf16(w[(size_t)r * H + k]);
+    for (int r = 0; r < n_actions + 1; r++) bias[(size_t)L * H + r] = b[r];
     std::unique_ptr<orlg_policy, int (*)(orlg_policy *)> pol(new orlg_policy(), orlg_policy_destroy);
     pol->device = device;
+    pol->general = std::getenv("ORLG_POLICY_GENERAL") != nullptr;
     if (cudaMalloc(&pol->w_dev, bytes) != cudaSuccess || cudaMalloc(&pol->b_dev, bias.size() * 4) != cudaSuccess ||
         cudaMemcpy(pol->w_dev, blob.data(), bytes, cudaMemcpyHostToDevice) != cudaSuccess ||
         cudaMemcpy(pol->b_dev, bias.data(), bias.size() * 4, cudaMemcpyHostToDevice) != cudaSuccess)
@@ -1362,9 +1388,17 @@ int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers,
     pol->pp.w_bytes = (int)bytes;
     pol->pp.bias = reinterpret_cast<const float *>(pol->b_dev);
     pol->pp.obs_dim = obs_dim; pol->pp.n_actions = n_actions;
-    pol->smem = bytes + (size_t)PL_GROUPS * PL_TILE * PL_H * 2 + bias.size() * 4 + 64;
-    if (cudaFuncSetAttribute(mlp_policy_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pol->smem) != cudaSuccess ||
-        cudaFuncSetAttribute(mlp_policy_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pol->smem) != cudaSuccess)
+    pol->pp.H = H; pol->pp.L = L;
+    pol->smem = smem;
+    // the attribute only raises a kernel's limit: a larger policy made earlier on this device keeps its launches valid
+    int have_act = 0, have_sample = 0;
+    cudaFuncAttributes fa;
+    if (cudaFuncGetAttributes(&fa, policy_kernel<false>(pol.get())) == cudaSuccess) have_act = fa.maxDynamicSharedSizeBytes;
+    if (cudaFuncGetAttributes(&fa, policy_kernel<true>(pol.get())) == cudaSuccess) have_sample = fa.maxDynamicSharedSizeBytes;
+    if ((have_act < (int)smem &&
+         cudaFuncSetAttribute(policy_kernel<false>(pol.get()), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) ||
+        (have_sample < (int)smem &&
+         cudaFuncSetAttribute(policy_kernel<true>(pol.get()), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess))
         return fail(ORLG_E_CUDA, "cudaFuncSetAttribute(policy kernel shared memory) failed");
     *out = pol.release();
     return ORLG_OK;
@@ -1381,7 +1415,7 @@ static int launch_policy(const orlg_policy *pol, const float *obs_dev, int n, in
     const int pairs = ((n + PL_TILE - 1) / PL_TILE + PL_GROUPS - 1) / PL_GROUPS;
     cudaLaunchConfig_t cfg = pdl_config(pairs < sms ? pairs : sms, PL_WG * PL_GROUPS, pol->smem, s);
     int *actions = actions_dev;
-    CUDA_OK(cudaLaunchKernelEx(&cfg, mlp_policy_kernel<SAMPLE>, pol->pp, obs_dev, n, actions, logits_dev, dr));
+    CUDA_OK(cudaLaunchKernelEx(&cfg, policy_kernel<SAMPLE>(pol), pol->pp, obs_dev, n, actions, logits_dev, dr));
     return ORLG_OK;
 }
 

@@ -1,14 +1,15 @@
-// orlg_policy.cuh -- the PPO agent the reference trains and ships (examples/stable_baselines3/DeepRMSA.ipynb cell 13:
-// PPO(MlpPolicy, env, policy_kwargs=dict(net_arch=5*[128])); bkp/deeprmsa-ppo-trained/best_model.zip), evaluated for a
-// whole batch of observations in ONE fused kernel: model.predict(obs, deterministic=True).
+// orlg_policy.cuh -- an SB3 MlpPolicy (a tanh trunk of L hidden layers of width H, then action_net / value_net), evaluated
+// for a whole batch of observations in ONE fused kernel: model.predict(obs, deterministic=True).  The agent the reference
+// trains and ships (examples/stable_baselines3/DeepRMSA.ipynb cell 13: PPO(MlpPolicy, env, policy_kwargs=dict(net_arch=5*[128]));
+// bkp/deeprmsa-ppo-trained/best_model.zip) is H = 128, L = 5; SB3's default PPO / A2C trunk is H = 64, L = 2.
 //
-//   obs f32 [n, 54] -> 5 x (Linear 128 + tanh) -> action_net (5 logits) / value_net (1) -> argmax -> int32 action
+//   obs f32 [n, 54] -> L x (Linear H + tanh) -> action_net (5 logits) / value_net (1) -> argmax -> int32 action
 //
-// This IS a contraction (146 kFLOP per env, 9.6 GFLOP per 65536-env step), so it runs on the 5th-generation tensor
-// cores: a persistent CTA per SM keeps all six weight matrices (bf16, 148 KB) in shared memory in the UMMA K-major
-// core-matrix layout, and walks tiles of 128 environments.  Per tile and layer one elected thread issues
-// tcgen05.mma (M = 128, N = 128, K = 16 per instruction) with A = the tile's activations (bf16, shared memory),
-// B = the layer's weights, D = fp32 accumulators in TMEM; the four warps then read their 32 TMEM lanes back with
+// This IS a contraction (146 kFLOP per env at 5 x 128, 9.6 GFLOP per 65536-env step), so it runs on the 5th-generation
+// tensor cores: a persistent CTA per SM keeps all L + 1 weight matrices (bf16, 148 KB at 5 x 128) in shared memory in the
+// UMMA K-major core-matrix layout, and walks tiles of 128 environments.  Per tile and layer one elected thread issues
+// tcgen05.mma (M = 128, N = H, K = 16 per instruction) with A = the tile's activations (bf16, shared memory),
+// B = the layer's weights, D = fp32 accumulators in TMEM; the warps then read their 32 TMEM lanes back with
 // tcgen05.ld, add the bias, apply tanh and write the next layer's A operand.  Nothing but the observation rows and
 // the actions touches HBM.  A second instance (mlp_policy_kernel<true>) ends in a sampling epilogue: the action drawn from
 // softmax(logits) with Philox stream 3, its log-probability and the value (PPO's rollout collection, orlg_policy_sample).
@@ -19,17 +20,25 @@
 namespace orlg {
 
 constexpr int PL_TILE = 128;          // environments per tile = UMMA M
-constexpr int PL_H = 128;             // hidden width
+constexpr int PL_HMAX = 128;          // widest hidden layer: the TMEM columns and the A buffer of a tile group
 constexpr int PL_K0 = 64;             // observation width padded to a multiple of 16 (54 -> 64)
 constexpr int PL_NOUT = 16;           // output layer padded: 5 logits + 1 value
-constexpr int PL_LAYERS = 5;          // hidden layers
+constexpr int PL_SMEM_MAX = 232448;   // dynamic shared memory a block may opt in to on sm_100 (227 KB)
 
 struct PolicyParams {
-    const uint4 *w_blob;              // all weights, bf16, already in the shared-memory operand layout (see policy_pack_weights)
-    int w_bytes;                      // multiple of 16
-    const float *bias;                // [5 * 128 + 16]
+    const uint4 *w_blob;              // all weights, bf16, already in the shared-memory operand layout (orlg_policy_create)
+    int w_bytes;                      // H * 64 * 2 + (L - 1) * H * H * 2 + 16 * H * 2
+    const float *bias;                // [L * H + 16]
     int obs_dim, n_actions;           // 54, 5
+    int H, L;                         // hidden width (multiple of 16, 16..128) and number of hidden layers (>= 1)
 };
+
+// bytes of weights and of dynamic shared memory of a policy with hidden width H and L hidden layers
+inline size_t pl_weight_bytes(int H, int L) { return (size_t)H * PL_K0 * 2 + (size_t)(L - 1) * H * H * 2 + (size_t)PL_NOUT * H * 2; }
+constexpr int PL_GROUPS = 2;          // tile groups per CTA
+inline size_t pl_smem_bytes(int H, int L) {
+    return pl_weight_bytes(H, L) + (size_t)PL_GROUPS * PL_TILE * PL_HMAX * 2 + ((size_t)L * H + PL_NOUT) * 4 + 64;
+}
 
 // The sampling epilogue (mlp_policy_kernel<true>, orlg_policy_sample): one Philox4x32-10 block per row, key = seed,
 // counter = (c0, 0, row_id_base + row, 3) -- stream 3 of DESIGN.md section 5 -- where c0 = counter_dev[row] (the env's
@@ -91,7 +100,7 @@ __device__ __forceinline__ void pl_tmem_ld32(unsigned taddr, float (&v)[32]) {
     for (int i = 0; i < 32; i++) v[i] = __uint_as_float(r[i]);
 }
 // the same without the wait: several loads in flight, one pl_tmem_wait() before the first use
-__device__ __forceinline__ void pl_tmem_ld32_nowait(unsigned taddr, unsigned (&r)[32]) {
+__device__ __forceinline__ void pl_tmem_ld32_nowait(unsigned taddr, unsigned *r) {
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 "
                  "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
                  "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
@@ -172,28 +181,29 @@ __device__ __forceinline__ void pl_sample_epilogue(const PolicyParams &pp, const
 // Two groups of EIGHT warps per CTA, each walking its own stream of 128-environment tiles with its own A buffer, TMEM accumulator
 // and mbarrier (they only share the weights): one group's tensor-core work and TMEM reads overlap the other's epilogue math.
 // Inside a group warp w reads TMEM lanes 32 (w % 4) .. + 31 (the hardware's lane quarter of a warp) and takes columns
-// 64 (w / 4) .. + 63: thread t owns row t % 128 and one half of its columns, so the epilogue of a layer (128 x 128 tanh, the
-// chain that bounds this kernel) is spread over 8 warps with both of a thread's TMEM loads in flight before the first use.
-// smem: [weights w_bytes][2 x A tile 128 x 128 bf16 = 64 KB][bias floats][mbarriers][tmem base]
-constexpr int PL_GROUPS = 2;
+// (H / 2) (w / 4) .. + H / 2 - 1: thread t owns row t % 128 and one half of its columns, so the epilogue of a layer (128 x H
+// tanh, the chain that bounds this kernel) is spread over 8 warps with all of a thread's TMEM loads in flight before the first use.
+// smem: [weights w_bytes][2 x A tile 128 x 128 bf16 = 64 KB][bias floats][mbarriers][tmem base]  (pl_smem_bytes)
 constexpr int PL_WG = 256;            // threads per group
 __device__ __forceinline__ void pl_group_sync(int group) {          // named barrier of one group (ids 1, 2; 0 = __syncthreads)
     asm volatile("bar.sync %0, %1;" ::"r"(group + 1), "n"(PL_WG) : "memory");
 }
 
 // SAMPLE = false: orlg_policy_act (argmax, optional logits; `dr` unused).  SAMPLE = true: orlg_policy_sample (the epilogue
-// of PolicyDraw; `actions` may be NULL, `logits_out` is unused).
-template <bool SAMPLE>
+// of PolicyDraw; `actions` may be NULL, `logits_out` is unused).  HC, LC: the hidden width and depth fixed at compile time
+// (they must equal pp.H, pp.L), or 0: read from pp at run time.
+template <bool SAMPLE, int HC, int LC>
 __global__ void __launch_bounds__(PL_WG * PL_GROUPS, 1)
 mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const int n, int *__restrict__ actions,
-                  float *__restrict__ logits_out /* [n, 6] = 5 logits + value, or NULL */, const PolicyDraw dr) {
+                  float *__restrict__ logits_out /* [n, n_actions + 1] = logits + value, or NULL */, const PolicyDraw dr) {
     extern __shared__ __align__(128) unsigned char psm[];
+    const int H = HC ? HC : pp.H, L = LC ? LC : pp.L;
     const int group = threadIdx.x / PL_WG, tid = threadIdx.x % PL_WG, warp = (tid >> 5) & 3;     // warp = TMEM lane quarter of this warp
-    const int half = tid >> 7;        // which 64 of the 128 columns (K elements of the next layer) this thread produces
+    const int half = tid >> 7;        // which half of the H columns (K elements of the next layer) this thread produces
     unsigned char *s_w = psm;
-    unsigned char *s_a = psm + pp.w_bytes + (size_t)group * PL_TILE * PL_H * 2;
-    float *s_bias = reinterpret_cast<float *>(psm + pp.w_bytes + (size_t)PL_GROUPS * PL_TILE * PL_H * 2);
-    unsigned long long *bars = reinterpret_cast<unsigned long long *>(s_bias + PL_LAYERS * PL_H + PL_NOUT);   // [0] weights, [1 + g] mma of group g
+    unsigned char *s_a = psm + pp.w_bytes + (size_t)group * PL_TILE * PL_HMAX * 2;
+    float *s_bias = reinterpret_cast<float *>(psm + pp.w_bytes + (size_t)PL_GROUPS * PL_TILE * PL_HMAX * 2);
+    unsigned long long *bars = reinterpret_cast<unsigned long long *>(s_bias + L * H + PL_NOUT);   // [0] weights, [1 + g] mma of group g
     unsigned *s_tmem = reinterpret_cast<unsigned *>(bars + 1 + PL_GROUPS);
 
     pdl_launch_dependents();
@@ -210,8 +220,8 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
                            "r"(bytes), "r"((unsigned)__cvta_generic_to_shared(&bars[0])) : "memory");
         }
     }
-    for (int i = threadIdx.x; i < PL_LAYERS * PL_H + PL_NOUT; i += PL_WG * PL_GROUPS) s_bias[i] = pp.bias[i];
-    if (threadIdx.x < 32) {     // TMEM: 128 columns (one 128 x 128 fp32 accumulator tile) per warpgroup
+    for (int i = threadIdx.x; i < L * H + PL_NOUT; i += PL_WG * PL_GROUPS) s_bias[i] = pp.bias[i];
+    if (threadIdx.x < 32) {     // TMEM: 128 columns (one 128 x 128 fp32 accumulator tile, of which H are used) per tile group
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
                      ::"r"((unsigned)__cvta_generic_to_shared(s_tmem)), "r"(128u * PL_GROUPS) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
@@ -219,8 +229,7 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const unsigned tmem_base = *s_tmem;
-    const unsigned tmem = tmem_base + (unsigned)group * 128u;           // this warpgroup's accumulator columns
+    const unsigned tmem = *s_tmem + (unsigned)group * 128u;           // this warpgroup's accumulator columns
     const unsigned t_lane = tmem + ((unsigned)(warp * 32) << 16);       // this warp's 32 TMEM lanes
     mbar_wait(&bars[0], 0);           // weights have landed
     pdl_wait();                       // the observations come from the previous kernel of the stream
@@ -287,9 +296,9 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
             }
         }
         int w_off = 0;                 // byte offset of the current layer's weights in s_w
-        for (int layer = 0; layer <= PL_LAYERS; layer++) {
-            const int K = layer == 0 ? PL_K0 : PL_H;
-            const int N = layer == PL_LAYERS ? PL_NOUT : PL_H;
+        for (int layer = 0; layer <= L; layer++) {
+            const int K = layer == 0 ? PL_K0 : H;
+            const int N = layer == L ? PL_NOUT : H;
             // activations written by the generic proxy -> visible to the tensor core (async proxy); previous TMEM reads done
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -309,26 +318,29 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
             mbar_wait(bar, phase);
             phase ^= 1u;
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const float *b = s_bias + layer * PL_H;
-            if (layer < PL_LAYERS) {
-                // ---- epilogue: bias + tanh, next layer's A operand (bf16) back into shared memory; this thread's 64 columns
-                unsigned r0[32], r1[32];
-                const int cb = half * 64;
-                pl_tmem_ld32_nowait(t_lane + (unsigned)cb, r0);
-                pl_tmem_ld32_nowait(t_lane + (unsigned)cb + 32u, r1);
+            const float *b = s_bias + layer * H;
+            if (layer < L) {
+                // ---- epilogue: bias + tanh, next layer's A operand (bf16) back into shared memory.  This thread's H / 2
+                // columns are m chunks of 8 (register r[8 j ..] = column cb + 8 j ..).  Both .x32 loads are issued whatever H
+                // is -- columns cb .. cb + 63 lie inside the group's 128 TMEM columns, chunks from m on are not used: loads
+                // sized to H (.x16 / .x8, or a second .x32 only when H > 64) give a register two possible definitions, which
+                // costs some 17 registers and spills at the 128 that 512 threads leave.
+                const int m = H >> 4;
+                const int cb = half * (H >> 1);
+                unsigned r[64];
+                pl_tmem_ld32_nowait(t_lane + (unsigned)cb, r);
+                pl_tmem_ld32_nowait(t_lane + (unsigned)cb + 32u, r + 32);
                 pl_tmem_wait();
 #pragma unroll
-                for (int hh = 0; hh < 2; hh++) {
-#pragma unroll
-                    for (int j = 0; j < 4; j++) {
-                        const int c0 = cb + 32 * hh + 8 * j;
+                for (int j = 0; j < 8; j++) {
+                    if (j < m) {
+                        const int c0 = cb + 8 * j;
                         const float4 b0 = *reinterpret_cast<const float4 *>(b + c0), b1 = *reinterpret_cast<const float4 *>(b + c0 + 4);
                         const float bb[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
                         unsigned w4[4];
 #pragma unroll
                         for (int q = 0; q < 4; q++) {
-                            const float v0 = __uint_as_float(hh ? r1[8 * j + 2 * q] : r0[8 * j + 2 * q]);
-                            const float v1 = __uint_as_float(hh ? r1[8 * j + 2 * q + 1] : r0[8 * j + 2 * q + 1]);
+                            const float v0 = __uint_as_float(r[8 * j + 2 * q]), v1 = __uint_as_float(r[8 * j + 2 * q + 1]);
                             __nv_bfloat162 h = __floats2bfloat162_rn(pl_tanh(v0 + bb[2 * q]), pl_tanh(v1 + bb[2 * q + 1]));
                             w4[q] = *reinterpret_cast<unsigned *>(&h);
                         }
@@ -364,7 +376,7 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (threadIdx.x < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(128u * PL_GROUPS) : "memory");
+    if (threadIdx.x < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*s_tmem), "r"(128u * PL_GROUPS) : "memory");
 }
 
 }  // namespace orlg

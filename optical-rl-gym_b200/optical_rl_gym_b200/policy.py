@@ -1,14 +1,17 @@
 """On-device MLP policy for the "PPO-policy actions" variant of the headline config (SURVEY.md row f4).
 
-Architecture of the agent the reference trains and ships
-(examples/stable_baselines3/DeepRMSA.ipynb: ``PPO(MlpPolicy, env, policy_kwargs=dict(net_arch=5*[128]))``;
-examples/stable_baselines3/bkp/deeprmsa-ppo-trained/best_model.zip): observation 54 -> 5 x (Linear 128 + tanh)
-shared trunk -> ``action_net`` (5 logits) and ``value_net`` (1).  ``from_sb3_zip`` reads ``policy.pth`` out of
-such an archive (a plain ``state_dict``; Stable-Baselines3 itself is not needed).
+An SB3 ``MlpPolicy``: a trunk of tanh ``Linear`` layers -> ``action_net`` (logits) and ``value_net`` (1).  The agent the
+reference trains and ships (examples/stable_baselines3/DeepRMSA.ipynb: ``PPO(MlpPolicy, env,
+policy_kwargs=dict(net_arch=5*[128]))``; examples/stable_baselines3/bkp/deeprmsa-ppo-trained/best_model.zip) is observation
+54 -> 5 x (Linear 128 + tanh) shared trunk -> 5 logits; an agent trained with SB3's PPO / A2C defaults has separate actor and
+critic trunks of 2 x (Linear 64 + tanh).  ``from_sb3_zip`` reads ``policy.pth`` out of such an archive (a plain
+``state_dict``; Stable-Baselines3 itself is not needed).
 
 Two forward paths: :meth:`forward` (plain torch float32, the numerics reference) and :meth:`act_native` -- the whole
 ``model.predict(obs, deterministic=True)`` as ONE fused sm_100a kernel of liborlg.so (``orlg_policy_act``: bf16
 ``tcgen05.mma`` with TMEM accumulators, weights resident in shared memory, tanh + argmax epilogue, int32 actions out).
+The kernel takes any trunk of one width H (a multiple of 16 in 16..128) and any depth whose weights fit in shared memory
+(5 x 128 and 6 x 112 do, 6 x 128 does not), observations up to 64 wide and up to 15 actions.
 :meth:`sample_native` is the same kernel with a sampling epilogue (``orlg_policy_sample``): sampled or argmax actions, their
 log-probabilities and the value estimate, as PPO's rollout collection needs them.  The native weights follow the module:
 an in-place update (``optimizer.step()``, ``load_state_dict``) rebuilds them at the next call.
@@ -40,13 +43,16 @@ class MlpPolicy(torch.nn.Module):
         or with separate actor/critic trunks (``mlp_extractor.policy_net`` / ``mlp_extractor.value_net``, SB3 >= 1.8: the
         actor's trunk becomes ``shared_net``, the critic's is kept as ``critic_net``: ``forward``, :meth:`sample_native` and
         ``OpticalVecEnv.rollout_policy`` return its value (a second native handle evaluates it); the value column of
-        :meth:`act_native`'s ``logits`` is the actor trunk's)."""
+        :meth:`act_native`'s ``logits`` is the actor trunk's, or NaN when ``value_net`` does not fit the actor's trunk).
+        ``value_net`` is sized from the checkpoint: with separate trunks it takes the critic's last width."""
         shared = any(k.startswith("mlp_extractor.shared_net.") for k in sd)
         trunk = "mlp_extractor.shared_net." if shared else "mlp_extractor.policy_net."
         idx = sorted({int(k[len(trunk):].split(".")[0]) for k in sd if k.startswith(trunk)})
         widths = [sd["%s%d.weight" % (trunk, i)].shape[0] for i in idx]
         obs_dim = sd["%s%d.weight" % (trunk, idx[0])].shape[1]
         pol = cls(obs_dim, sd["action_net.weight"].shape[0], widths)
+        if sd["value_net.weight"].shape[1] != pol.value_net.in_features:
+            pol.value_net = torch.nn.Linear(sd["value_net.weight"].shape[1], 1)
         mine = {}
         for j, i in enumerate(idx):
             mine["shared_net.%d.weight" % (2 * j)] = sd["%s%d.weight" % (trunk, i)]
@@ -78,12 +84,21 @@ class MlpPolicy(torch.nn.Module):
         """What the native handles are built from: ``{"actor": spec, "critic": spec | None}`` with ``spec`` =
         ``(trunk Linear layers, head Linear layers, obs_dim)``.  The actor's heads are ``action_net`` then ``value_net``.  With
         a separate critic trunk (SB3 >= 1.8) the critic handle evaluates that trunk; its one-row action head is ``value_net``
-        as well (its actions are never requested), so its value output is ``value_net(critic_net(obs))``."""
+        as well (its actions are never requested), so its value output is ``value_net(critic_net(obs))``.  When the critic's
+        trunk is wider or narrower than the actor's, ``value_net`` does not fit the actor's trunk: the actor's value row is
+        then a stand-in with zero weights and a NaN bias (the actor handle's value is never used with a critic handle)."""
         lins = [m for m in self.shared_net if isinstance(m, torch.nn.Linear)]
-        specs = {"actor": (lins, [self.action_net, self.value_net], lins[0].in_features), "critic": None}
+        value_head = self.value_net
+        if self.critic_net is not None and lins and self.value_net.in_features != lins[-1].out_features:
+            value_head = torch.nn.Linear(lins[-1].out_features, 1)
+            with torch.no_grad():
+                value_head.weight.zero_()
+                value_head.bias.fill_(float("nan"))
+        obs_dim = lins[0].in_features if lins else self.action_net.in_features
+        specs = {"actor": (lins, [self.action_net, value_head], obs_dim), "critic": None}
         if self.critic_net is not None:
             clins = [m for m in self.critic_net if isinstance(m, torch.nn.Linear)]
-            specs["critic"] = (clins, [self.value_net, self.value_net], clins[0].in_features)
+            specs["critic"] = (clins, [self.value_net, self.value_net], clins[0].in_features if clins else obs_dim)
         return specs
 
     @staticmethod
@@ -95,11 +110,20 @@ class MlpPolicy(torch.nn.Module):
         from . import _native as nat
 
         lins, heads, obs_dim = spec
+        # orlg_policy_create reads every layer as [H, H] after the first and the heads as [rows, H]: other shapes would be read
+        # past the end of the arrays below, so they are refused here
+        if not lins:
+            raise ValueError("the fused policy kernel needs at least one hidden layer; the trunk is empty")
+        H = lins[0].out_features
+        if any(m.out_features != H for m in lins) or any(m.in_features != H for m in list(lins[1:]) + list(heads)):
+            raise ValueError("the fused policy kernel needs one hidden width for the whole trunk; got layer widths %s, layer "
+                             "inputs %s and head inputs %s" % ([m.out_features for m in lins], [m.in_features for m in lins],
+                                                               [m.in_features for m in heads]))
         mats = list(lins) + list(heads)
         w = np.concatenate([m.weight.detach().float().cpu().numpy().reshape(-1) for m in mats]).astype(np.float32)
         b = np.concatenate([m.bias.detach().float().cpu().numpy().reshape(-1) for m in mats]).astype(np.float32)
         h = C.c_void_p()
-        nat.check(nat.lib().orlg_policy_create(device_index, obs_dim, lins[0].out_features, len(lins), heads[0].out_features,
+        nat.check(nat.lib().orlg_policy_create(device_index, obs_dim, H, len(lins), heads[0].out_features,
                                                w.ctypes.data_as(C.c_void_p), b.ctypes.data_as(C.c_void_p), C.byref(h)))
         return h
 
@@ -181,7 +205,10 @@ class MlpPolicy(torch.nn.Module):
     @torch.no_grad()
     def act_native(self, obs: torch.Tensor, out: torch.Tensor = None, logits: torch.Tensor = None) -> torch.Tensor:
         """Deterministic actions int32 ``[N, 1]`` from float32 CUDA observations ``[N, obs_dim]`` through the fused tensor-core
-        kernel; ``logits`` (optional float32 ``[N, n_actions + 1]``) receives the logits and the value estimate."""
+        kernel; ``logits`` (optional float32 ``[N, n_actions + 1]``) receives the logits and the value estimate of the actor's
+        trunk (NaN when the critic's separate trunk has another width: :meth:`sample_native` gives the critic's value).  Any
+        trunk of one width H, a multiple of 16 in 16..128, whose weights fit in shared memory (see the module docstring);
+        other architectures raise ``ValueError`` (widths) or ``NativeError`` (shapes outside the kernel)."""
         import ctypes as C
 
         from . import _native as nat
