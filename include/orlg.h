@@ -236,13 +236,16 @@ int orlg_rollout_policy(orlg_env *env, int steps, orlg_policy *actor, orlg_polic
  * makes at its next step.  Host state, no device access. */
 int64_t orlg_request_index(const orlg_env *env);
 
-/* Float statistics of `info` (rmsa_env.py:229-264, 439-543, 699-744; RMSA-v0 / DeepRMSA-v0, <= 32 links,
- * <= 128 slots): after this call every orlg_step also writes, per env, float64
+/* Float statistics of `info` (rmsa_env.py:229-264, 439-543, 699-744; RMSA-v0 / DeepRMSA-v0, any topology the handle
+ * takes: any link count, up to 512 slots): after this call every orlg_step also writes, per env, float64
  *   stats_dev[env][0..3] = network_compactness, network_compactness_difference,
  *                          avg_link_compactness, avg_link_utilization
  * bit-identical to the reference (same float64 operation order, releases applied in time order, numpy's
- * pairwise mean).  Call before orlg_reset(full = 1).  stats_dev = NULL disables it again.  The statistics
- * path uses the generic kernel (slower than the default path). */
+ * pairwise mean, recursive above 128 links).  Call before orlg_reset(full = 1).  stats_dev = NULL disables it again.  Bit
+ * rates must fit 16 bits (<= 65535).  NSFNET-class handles (<= 32 links, <= 128 slots) run the statistics on the generic
+ * kernel instead of the fast one; wide handles on the statistics instance of the wide step kernel, which updates each link
+ * with a load / store instead of fire-and-forget reductions.  Both are slower than the default path.  orlg_rollout on a
+ * handle with statistics on (fused heuristic, random or replay) runs the same kernels step by step. */
 int orlg_enable_stats(orlg_env *env, double *stats_dev);
 /* The time-averaged statistics the reference keeps ON the topology graph while it provisions and releases (never returned by
  * step, read by users through env.topology): per link `utilization`, `external_fragmentation`, `compactness`
@@ -251,7 +254,8 @@ int orlg_enable_stats(orlg_env *env, double *stats_dev);
  * rmsa_env.py:439-462, rmcsa_env.py:560-589; a no-op in rwa_env.py:351-363).  orlg_enable_link_stats(on = 1) before
  * orlg_reset(full = 1) turns them on for ANY env kind (orlg_enable_stats implies it); orlg_link_stats reads them as of the last
  * step: link_dev f64 [num_envs, links, 3] by link index, graph_dev f64 [num_envs, 2] (either may be NULL).  Bit-identical to
- * the reference (same float64 operation order, releases applied in time order).  Same limits and cost as orlg_enable_stats. */
+ * the reference (same float64 operation order, releases applied in time order; more than 24 releases in one step set
+ * ORLG_ERR_STATS_ORDER).  Any link count, up to 512 slots and 31 cores; same kernels and cost as orlg_enable_stats. */
 int orlg_enable_link_stats(orlg_env *env, int on);
 int orlg_link_stats(orlg_env *env, double *link_dev, double *graph_dev, orlg_stream stream);
 

@@ -308,7 +308,9 @@ int launch_step(const orlg_env *env, const StepIO &io, int mode, cudaStream_t s)
     if (env->wide) {
         const int blocks = (p.n + ORLG_WIDE_THREADS - 1) / ORLG_WIDE_THREADS;
         for_kind(p.kind, [&](auto K) { for_words(p.nwv, [&](auto W) {
-            step_wide_kernel<decltype(K)::value, decltype(W)::value><<<blocks, ORLG_WIDE_THREADS, 0, s>>>(p, io, mode); }); });
+            constexpr int KIND = decltype(K)::value, NWV = decltype(W)::value;
+            if (p.stats) step_wide_kernel<KIND, NWV, true><<<blocks, ORLG_WIDE_THREADS, 0, s>>>(p, io, mode);
+            else step_wide_kernel<KIND, NWV, false><<<blocks, ORLG_WIDE_THREADS, 0, s>>>(p, io, mode); }); });
     } else if (env->fast && !p.stats) launch_fast(env, io, mode, s);
     else for_kind(p.kind, [&](auto K) { launch_step_kind<decltype(K)::value>(env, io, mode, s); });
     CUDA_OK(cudaGetLastError());
@@ -919,7 +921,6 @@ int orlg_debug_rollout_timeline(unsigned long long *out, int n_warps) {
 
 static int stats_alloc(orlg_env *env) {
     Params &p = env->p;
-    if (env->wide || p.E > 128) return fail(ORLG_E_UNSUPPORTED, "statistics path handles <= 32 links and <= 128 slots");
     if (p.br_max > 65535) return fail(ORLG_E_UNSUPPORTED, "statistics path keeps bit rates in 16 bits");
     if (!p.link_util) {
         const size_t n = (size_t)p.n;
@@ -931,7 +932,10 @@ static int stats_alloc(orlg_env *env) {
         if (!rc) rc = dev_alloc(env, &p.graph_stats, 3 * n);
         if (!rc) rc = dev_alloc(env, &p.run_br, n);
         if (!rc) rc = dev_alloc(env, &p.ev_br, n * (size_t)p.heap_cap);
-        if (!rc) rc = dev_alloc(env, &p.sum_nh, n);
+        // wide kernels: the compactness terms follow sum_nh in its allocation (nc_totals / nc_links, orlg_step_wide.cuh), in
+        // units of 8 bytes: int2 [n][C], then unsigned [n][C*E]
+        const size_t nc = env->wide && p.kind != ORLG_RWA ? (size_t)p.C * n + ((size_t)p.C * p.E * n + 1) / 2 : 0;
+        if (!rc) rc = dev_alloc(env, &p.sum_nh, n + nc);
         env->alloc_is_state = false;
         if (rc) return rc;
     }

@@ -74,7 +74,7 @@ struct Params {
     double *graph_stats;               // [3][n] topology.graph["throughput"], ["compactness"], ["last_update"] (rmsa_env.py:439-462)
     long long *run_br;                 // [n] sum of bit_rate over graph["running_services"]
     unsigned short *ev_br;             // [n][heap_cap] bit rate of every live service (parallel to ev_pay)
-    long long *sum_nh;                 // [n] sum over running services of number_slots * hops
+    long long *sum_nh;                 // [n] sum over running services of number_slots * hops (wide handles: + nc_totals, nc_links)
     double *stats_out;                 // [n][4] network_compactness, its difference, avg link compactness, avg link utilisation
     const int *link_order;             // [E] link indices in topology.edges() order (np.mean over the links)
     // ---- discrete bit-rate selection (row f4: rmsa_env.py:88-110, 217-227, 268-273, 408-415, 579-581)
@@ -232,6 +232,12 @@ __device__ __forceinline__ LinkShape link_shape(const Bits &fr, int S) {
     return r;
 }
 
+// _get_network_compactness from its integer sums over the links: occupied = sum of spans, unused = free runs inside them
+__device__ __forceinline__ double compactness_value(const Params &p, long long occupied, long long unused, long long sum_nh) {
+    if (unused > 0) return __dmul_rn(__ddiv_rn((double)occupied, (double)sum_nh), __ddiv_rn((double)p.E, (double)unused));
+    return 1.0;
+}
+
 // _get_network_compactness (rmsa_env.py:699-744)
 // (rmcsa_env.py:825-871: the links of ONE core, number_slots * hops summed over all running services)
 __device__ __forceinline__ double network_compactness(const Params &p, int env, long long sum_nh, int core = 0) {
@@ -240,18 +246,18 @@ __device__ __forceinline__ double network_compactness(const Params &p, int env, 
         const LinkShape s = link_shape(bits_from(p.masks[(size_t)(core * p.E + l) * p.n + env]), p.S);
         occupied += s.span; unused += s.free_runs_in;
     }
-    if (unused > 0) return __dmul_rn(__ddiv_rn((double)occupied, (double)sum_nh), __ddiv_rn((double)p.E, (double)unused));
-    return 1.0;
+    return compactness_value(p, occupied, unused, sum_nh);
 }
 
 // _update_link_stats (rmsa_env.py:464-543, rmcsa_env.py:591-688, rwa_env.py:365-383: utilisation only) for link l whose (already
-// updated) mask -- of the core being touched -- is `fr`; the statistics are per LINK (RMCSA's cores share them)
-__device__ __forceinline__ void update_link_stats(const Params &p, int env, int l, const Bits &fr, double now) {
+// updated) mask -- of the core being touched -- has the shape `shape()`; the statistics are per LINK (RMCSA's cores share them)
+template <typename ShapeFn>
+__device__ __forceinline__ void update_link_stats_with(const Params &p, int env, int l, double now, ShapeFn shape) {
     const size_t i = (size_t)l * p.n + env;
     const double last_update = p.link_last[i];
     const double time_diff = __dadd_rn(now, -last_update);
     if (now > 0) {
-        const LinkShape s = link_shape(fr, p.S);
+        const LinkShape s = shape();
         const double cur_util = __ddiv_rn((double)(p.S - s.free_cnt), (double)p.S);
         p.link_util[i] = __ddiv_rn(__dadd_rn(__dmul_rn(p.link_util[i], last_update), __dmul_rn(cur_util, time_diff)), now);
         if (p.kind != ORLG_RWA) {
@@ -268,38 +274,72 @@ __device__ __forceinline__ void update_link_stats(const Params &p, int env, int 
     }
     p.link_last[i] = now;
 }
+__device__ __forceinline__ void update_link_stats(const Params &p, int env, int l, const Bits &fr, double now) {
+    update_link_stats_with(p, env, l, now, [&] { return link_shape(fr, p.S); });
+}
 
 // _update_network_stats (rmsa_env.py:439-462, rmcsa_env.py:560-589; a no-op for RWA): called by _provision_path only, after the
-// new service joined graph["running_services"]
-__device__ __forceinline__ void update_network_stats(const Params &p, int env, long long sum_nh, long long run_br, int core, double now) {
+// new service joined graph["running_services"]; `compactness()` is _get_network_compactness of the core being provisioned
+template <typename CompactnessFn>
+__device__ __forceinline__ void update_network_stats_with(const Params &p, int env, long long run_br, double now, CompactnessFn compactness) {
     double *g = p.graph_stats + env;
     const double last_update = g[2 * (size_t)p.n];
     const double time_diff = __dadd_rn(now, -last_update);
     if (now > 0) {
         g[0] = __ddiv_rn(__dadd_rn(__dmul_rn(g[0], last_update), __dmul_rn((double)run_br, time_diff)), now);
-        g[p.n] = __ddiv_rn(__dadd_rn(__dmul_rn(g[p.n], last_update), __dmul_rn(network_compactness(p, env, sum_nh, core), time_diff)), now);
+        g[p.n] = __ddiv_rn(__dadd_rn(__dmul_rn(g[p.n], last_update), __dmul_rn(compactness(), time_diff)), now);
     }
     g[2 * (size_t)p.n] = now;
 }
+__device__ __forceinline__ void update_network_stats(const Params &p, int env, long long sum_nh, long long run_br, int core, double now) {
+    update_network_stats_with(p, env, run_br, now, [&] { return network_compactness(p, env, sum_nh, core); });
+}
 
-// np.mean over the links in topology.edges() order: numpy's pairwise summation (8 partial sums), E <= 128
-__device__ __forceinline__ double mean_over_links(const Params &p, const double *per_link, int env) {
-    const int n = p.E;
+// numpy's pairwise summation of the n <= 128 links at positions [off, off + n) of topology.edges() order (8 partial sums)
+__device__ __forceinline__ double links_block_sum(const Params &p, const double *per_link, int env, int off, int n) {
+    const int *order = p.link_order + off;
     double res;
     if (n < 8) {
         res = 0.0;
-        for (int i = 0; i < n; i++) res = __dadd_rn(res, per_link[(size_t)p.link_order[i] * p.n + env]);
+        for (int i = 0; i < n; i++) res = __dadd_rn(res, per_link[(size_t)order[i] * p.n + env]);
     } else {
         double r[8];
 #pragma unroll
-        for (int j = 0; j < 8; j++) r[j] = per_link[(size_t)p.link_order[j] * p.n + env];
+        for (int j = 0; j < 8; j++) r[j] = per_link[(size_t)order[j] * p.n + env];
         int i;
         for (i = 8; i < n - (n % 8); i += 8) {
 #pragma unroll
-            for (int j = 0; j < 8; j++) r[j] = __dadd_rn(r[j], per_link[(size_t)p.link_order[i + j] * p.n + env]);
+            for (int j = 0; j < 8; j++) r[j] = __dadd_rn(r[j], per_link[(size_t)order[i + j] * p.n + env]);
         }
         res = __dadd_rn(__dadd_rn(__dadd_rn(r[0], r[1]), __dadd_rn(r[2], r[3])), __dadd_rn(__dadd_rn(r[4], r[5]), __dadd_rn(r[6], r[7])));
-        for (; i < n; i++) res = __dadd_rn(res, per_link[(size_t)p.link_order[i] * p.n + env]);
+        for (; i < n; i++) res = __dadd_rn(res, per_link[(size_t)order[i] * p.n + env]);
+    }
+    return res;
+}
+
+// np.mean over the links in topology.edges() order.  Above 128 links numpy's pairwise_sum splits a range of n at
+// n2 = n / 2 - (n / 2) % 8 and adds the sums of the two halves; that recursion runs here on an explicit stack (16 frames
+// reach far beyond the 65535 links a hop list can name).
+__device__ __forceinline__ double mean_over_links(const Params &p, const double *per_link, int env) {
+    const int n = p.E;
+    double res;
+    if (n <= 128) {
+        res = links_block_sum(p, per_link, env, 0, n);
+    } else {
+        int off[16], len[16], phase[16];     // phase 0: left half next, 1: right half next, 2: add the halves
+        double left[16];
+        int sp = 1;
+        off[0] = 0; len[0] = n; phase[0] = 0;
+        res = 0.0;
+        while (sp > 0) {
+            const int i = sp - 1;
+            if (len[i] <= 128) { res = links_block_sum(p, per_link, env, off[i], len[i]); sp--; continue; }
+            int n2 = len[i] / 2;
+            n2 -= n2 % 8;
+            if (phase[i] == 0) { phase[i] = 1; off[sp] = off[i]; len[sp] = n2; phase[sp] = 0; sp++; }
+            else if (phase[i] == 1) { phase[i] = 2; left[i] = res; off[sp] = off[i] + n2; len[sp] = len[i] - n2; phase[sp] = 0; sp++; }
+            else { res = __dadd_rn(left[i], res); sp--; }
+        }
     }
     return __ddiv_rn(res, (double)n);
 }

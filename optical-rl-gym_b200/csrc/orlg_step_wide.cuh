@@ -175,6 +175,118 @@ __device__ __forceinline__ void wide_path_update(const Params &p, int env, int r
 
 __device__ __forceinline__ int wide_nslots(const Params &p, int se, int br) { return p.nslots[se * (p.br_max + 1) + br]; }
 
+// ---------------------------------------------------------------- row f1 (float statistics) on the wide layout
+// longest run of ones: one pass over the words, ctz / clz at every run boundary (no shift-AND pass per slot)
+template <int NWV>
+__device__ __forceinline__ int wb_longest_run(const WBits<NWV> &a) {
+    int best = 0, cur = 0;                             // cur: the run that reaches the top of the words seen so far
+#pragma unroll
+    for (int i = 0; i < 4 * NWV; i++) {
+        const uint32_t x = a.w[i];
+        if (x == 0xFFFFFFFFu) { cur += 32; continue; }
+        best = max(best, cur + __ffs(~x) - 1);         // the run coming from below ends at the lowest 0 of x
+        const int top = __clz(~x);                     // ones reaching bit 31 start the next carried run
+        uint32_t y = (x & (x + 1u)) & (0xFFFFFFFFu >> top);   // the runs strictly inside x (bit 0 of y is 0)
+        while (y) {
+            const int s = __ffs(y) - 1, len = __ffs(~(y >> s)) - 1;      // s >= 1, so len <= 31
+            best = max(best, len);
+            y &= ~(((1u << len) - 1u) << s);
+        }
+        cur = top;
+    }
+    return max(best, cur);
+}
+
+// link_shape (orlg_kernels.cuh) of a multi-word mask: the same integers.  With two or more used runs the free runs outside
+// [ffs(used), fls(used) + 1) are exactly the one at slot 0 and the one at slot S - 1 (when those slots are free).
+template <int NWV>
+__device__ __forceinline__ LinkShape wb_link_shape(const WBits<NWV> &fr, int S) {
+    const WBits<NWV> valid = wb_range<NWV>(0, S), last = wb_range<NWV>(S - 1, S);
+    WBits<NWV> used;
+#pragma unroll
+    for (int i = 0; i < 4 * NWV; i++) used.w[i] = valid.w[i] & ~fr.w[i];
+    const WBits<NWV> ul = wb_shl1(used), fl = wb_shl1(fr);
+    LinkShape r;
+    int ur = 0, frn = 0;
+    uint32_t at_end = 0;
+#pragma unroll
+    for (int i = 0; i < 4 * NWV; i++) {
+        ur += __popc(used.w[i] & ~ul.w[i]);
+        frn += __popc(fr.w[i] & ~fl.w[i]);
+        at_end |= fr.w[i] & last.w[i];
+    }
+    const int f0 = fr.w[0] & 1u, f1 = at_end != 0;
+    r.free_cnt = wb_popc(fr);
+    r.used_runs = ur;
+    r.free_runs = frn;
+    r.longest_free = wb_longest_run(fr);
+    r.free_at_both_ends = f0 && f1;
+    r.span = 0; r.free_runs_in = 0;
+    if (ur > 1) {
+        r.span = wb_fls(used) + 1 - wb_ffs(used);
+        r.free_runs_in = frn - f0 - f1;
+    }
+    return r;
+}
+
+__device__ __forceinline__ int wide_hops(const Params &p, int row) { return p.path_link_ptr[row + 1] - p.path_link_ptr[row]; }
+
+// The integer terms of _get_network_compactness (rmsa_env.py:699-744), kept current so that the compactness needs no pass over
+// every link.  They live behind sum_nh in the same allocation (orlg_enable_stats on a wide handle other than RWA-v0), which
+// leaves the kernel parameter block -- and with it the code of every other kernel -- as it was:
+//     int2     [n][C]    per core, the sums over its links: x = occupied (spans), y = free runs inside the spans
+//     unsigned [n][C*E]  per (core, link): span | free runs inside the span << 16
+__device__ __forceinline__ int2 *nc_totals(const Params &p) { return reinterpret_cast<int2 *>(p.sum_nh + p.n); }
+__device__ __forceinline__ unsigned *nc_links(const Params &p) { return reinterpret_cast<unsigned *>(nc_totals(p) + (size_t)p.n * p.C); }
+
+// _get_network_compactness of one core from its kept integer sums (equal to a pass over every link: exact integers)
+__device__ __forceinline__ double wide_compactness(const Params &p, int env, int core, long long sum_nh) {
+    const int2 t = nc_totals(p)[(size_t)env * p.C + core];
+    return compactness_value(p, t.x, t.y, sum_nh);
+}
+
+// _provision_path / _release_path with the statistics (rmsa_env.py:381-396, 418-436): links in hop order, each entry loaded,
+// modified and stored by the thread that owns it, so _update_link_stats sees the link's new mask.  The link's compactness terms
+// (span, free runs inside it) are refreshed from the same shape and the core's sums adjusted by the difference.
+template <int KIND, int NWV>
+__device__ __forceinline__ void wide_path_update_stats(const Params &p, int env, int row, int core, int start, int n, bool set, double now) {
+    const WBits<NWV> rm = wb_range<NWV>(start, start + n);
+    const size_t vs = p.wstride ? 1 : (size_t)p.n;
+    int d_occ = 0, d_unused = 0;
+    for (int h = p.path_link_ptr[row]; h < p.path_link_ptr[row + 1]; h++) {
+        const int l = p.path_links16[h];
+        uint4 *m = p.masks + mask_index(p, core * p.E + l, 0, env);
+        WBits<NWV> b;
+#pragma unroll
+        for (int v = 0; v < NWV; v++) {
+            const uint4 x = __ldcg(m + v * vs);
+            b.w[4 * v] = x.x; b.w[4 * v + 1] = x.y; b.w[4 * v + 2] = x.z; b.w[4 * v + 3] = x.w;
+        }
+#pragma unroll
+        for (int i = 0; i < 4 * NWV; i++) b.w[i] = set ? (b.w[i] | rm.w[i]) : (b.w[i] & ~rm.w[i]);
+#pragma unroll
+        for (int v = 0; v < NWV; v++) m[v * vs] = make_uint4(b.w[4 * v], b.w[4 * v + 1], b.w[4 * v + 2], b.w[4 * v + 3]);
+        LinkShape s{};
+        if (KIND == ORLG_RWA) {
+            s.free_cnt = wb_popc(b);                   // rwa_env.py:365-383: utilisation only
+        } else {
+            s = wb_link_shape(b, p.S);
+            unsigned *t = nc_links(p) + ((size_t)env * p.C + core) * p.E + l;
+            const unsigned old = *t;
+            d_occ += s.span - (int)(old & 0xFFFFu);
+            d_unused += s.free_runs_in - (int)(old >> 16);
+            *t = (unsigned)s.span | ((unsigned)s.free_runs_in << 16);
+        }
+        update_link_stats_with(p, env, l, now, [&] { return s; });
+    }
+    if (KIND != ORLG_RWA) {
+        int2 *t = nc_totals(p) + (size_t)env * p.C + core;
+        int2 v = *t;
+        v.x += d_occ; v.y += d_unused;
+        *t = v;
+    }
+}
+
 // heuristic action sources (SURVEY a21) for the wide layout: the action of env's pending request (src, dst, br) into a[0..3]
 // Returns true when the action is KNOWN to fit (it was derived from the path's free mask just now), so that the fused step
 // does not have to read the masks a second time for is_path_free.
@@ -283,8 +395,14 @@ __global__ void heuristic_wide_kernel(const Params p, const int which, int *acti
 #ifndef ORLG_WIDE_MIN_BLOCKS
 #define ORLG_WIDE_MIN_BLOCKS 8
 #endif
-template <int KIND, int NWV>
-__global__ void __launch_bounds__(ORLG_WIDE_THREADS, ORLG_WIDE_MIN_BLOCKS) step_wide_kernel(const Params p, const StepIO io, const int mode) {
+// STATS = true: the float statistics of row f1 (orlg_enable_stats / orlg_enable_link_stats) are kept as well.  That instance
+// carries more live state (the shape of a link, the sorted releases) and is given 6 CTAs per SM (up to 168 registers): with 8
+// the RMCSA instance of 512 slots spills.
+#ifndef ORLG_WIDE_STATS_MIN_BLOCKS
+#define ORLG_WIDE_STATS_MIN_BLOCKS 6
+#endif
+template <int KIND, int NWV, bool STATS>
+__global__ void __launch_bounds__(ORLG_WIDE_THREADS, STATS ? ORLG_WIDE_STATS_MIN_BLOCKS : ORLG_WIDE_MIN_BLOCKS) step_wide_kernel(const Params p, const StepIO io, const int mode) {
     const int env = blockIdx.x * blockDim.x + threadIdx.x;
     if (env >= p.n) return;
     double now = p.now[env];
@@ -299,7 +417,8 @@ __global__ void __launch_bounds__(ORLG_WIDE_THREADS, ORLG_WIDE_MIN_BLOCKS) step_
     double hmin = p.heap_min[env];
     double tailmin = p.ev_tail[env];
     unsigned err = p.errors[env];
-    const Events ev = {p.ev_time + (size_t)env * p.heap_cap, p.ev_pay + (size_t)env * p.heap_cap, p.ev_gmin + (size_t)env * p.ev_groups};
+    Events ev = {p.ev_time + (size_t)env * p.heap_cap, p.ev_pay + (size_t)env * p.heap_cap, p.ev_gmin + (size_t)env * p.ev_groups};
+    if constexpr (STATS) ev.br = p.ev_br + (size_t)env * p.heap_cap;
     bool accepted = false, done = false;
 
     if (mode == MODE_FULL_RESET) {
@@ -373,9 +492,29 @@ __global__ void __launch_bounds__(ORLG_WIDE_THREADS, ORLG_WIDE_MIN_BLOCKS) step_
             }
         }
         if (accepted && nheap + 1 > (unsigned)p.heap_cap) { accepted = false; err |= ORLG_ERR_HEAP_OVERFLOW; }
+        bool info_stats = false;
+        long long snh = 0;
+        double prev_compactness = 0.0;
+        if constexpr (STATS) {
+            info_stats = (KIND == ORLG_RMSA || KIND == ORLG_DEEPRMSA) && p.stats_out;
+            snh = p.sum_nh[env];
+            if (info_stats) prev_compactness = wide_compactness(p, env, 0, snh);     // rmsa_env.py:168-170
+        }
         if (accepted) {
-            wide_path_update<NWV>(p, env, row, core, start, n, false);
-            events_push(ev, nheap, hmin, tailmin, __dadd_rn(now, hold), pack_service(row, start, n, core, sid));
+            if constexpr (STATS) {
+                wide_path_update_stats<KIND, NWV>(p, env, row, core, start, n, false, now);
+                snh += (long long)n * wide_hops(p, row);
+                p.sum_nh[env] = snh;
+                if (KIND != ORLG_RWA) {
+                    const long long rb = p.run_br[env] + br;
+                    p.run_br[env] = rb;
+                    update_network_stats_with(p, env, rb, now, [&] { return wide_compactness(p, env, core, snh); });
+                }
+                events_push(ev, nheap, hmin, tailmin, __dadd_rn(now, hold), pack_service(row, start, n, core, sid), (unsigned)br);
+            } else {
+                wide_path_update<NWV>(p, env, row, core, start, n, false);
+                events_push(ev, nheap, hmin, tailmin, __dadd_rn(now, hold), pack_service(row, start, n, core, sid));
+            }
             cnt[1] += 1; cnt[3] += 1;
             if (KIND != ORLG_RWA) { cnt[5] += br; cnt[7] += br; }
             if (KIND == ORLG_RMSA) br_hist_bump(p, env, 1, br);
@@ -393,6 +532,27 @@ __global__ void __launch_bounds__(ORLG_WIDE_THREADS, ORLG_WIDE_MIN_BLOCKS) step_
         if (io.info) {
 #pragma unroll
             for (int q = 0; q < 8; q++) io.info[(size_t)env * 8 + q] = cnt[q];
+        }
+        if constexpr (STATS) if (info_stats) {              // rmsa_env.py:229-264
+            const double cur = wide_compactness(p, env, 0, snh);
+            double *so = p.stats_out + (size_t)env * 4;
+            so[0] = cur;
+            so[1] = __dadd_rn(prev_compactness, -cur);
+            so[2] = mean_over_links(p, p.link_comp, env);
+            so[3] = mean_over_links(p, p.link_util, env);
+        }
+    }
+
+    if constexpr (STATS) if (mode == MODE_FULL_RESET) {
+        for (int l = 0; l < p.E; l++) {
+            const size_t i = (size_t)l * p.n + env;
+            p.link_util[i] = 0.0; p.link_comp[i] = 0.0; p.link_last[i] = 0.0; p.link_frag[i] = 0.0;
+        }
+        p.sum_nh[env] = 0; p.run_br[env] = 0;
+        for (int q = 0; q < 3; q++) p.graph_stats[(size_t)q * p.n + env] = 0.0;
+        if (KIND != ORLG_RWA) {
+            for (int l = 0; l < p.C * p.E; l++) nc_links(p)[(size_t)env * p.C * p.E + l] = 0u;
+            for (int c = 0; c < p.C; c++) nc_totals(p)[(size_t)env * p.C + c] = make_int2(0, 0);
         }
     }
 
@@ -415,6 +575,39 @@ __global__ void __launch_bounds__(ORLG_WIDE_THREADS, ORLG_WIDE_MIN_BLOCKS) step_
         if (KIND == ORLG_RMSA || KIND == ORLG_DEEPRMSA) { cnt[0] += 1; cnt[2] += 1; cnt[4] += br; cnt[6] += br; }
         if (KIND == ORLG_RMSA) br_hist_bump(p, env, 0, br);
         else if (KIND == ORLG_RMCSA) { cnt[4] += br; cnt[6] += br; }
+        if constexpr (STATS) {
+            // the reference releases in heap order (by time) and every release updates the statistics of its links: the due
+            // services are collected, sorted by release time and applied in that order (as in step_kernel)
+            constexpr int MAXR = 24;
+            double rt[MAXR];
+            unsigned long long rp[MAXR];
+            int nr = 0;
+            long long rel_br = 0;                                // bit rates leaving graph["running_services"]
+            long long snh = p.sum_nh[env];
+            events_release(ev, nheap, hmin, tailmin, now, apply_timed([&](unsigned long long pl, double t, unsigned sbr) {
+                rel_br += sbr;
+                if (nr < MAXR) { rt[nr] = t; rp[nr] = pl; nr++; }
+                else {                                           // overflow: masks stay exact, statistics order is not
+                    err |= ORLG_ERR_STATS_ORDER;
+                    wide_path_update_stats<KIND, NWV>(p, env, svc_row(pl), svc_core(pl), svc_start(pl), svc_slots(pl), true, now);
+                    snh -= (long long)svc_slots(pl) * wide_hops(p, svc_row(pl));
+                }
+            }));
+            if (rel_br) p.run_br[env] -= rel_br;
+            for (int a = 1; a < nr; a++) {                       // insertion sort by release time
+                const double t = rt[a];
+                const unsigned long long q = rp[a];
+                int b = a - 1;
+                while (b >= 0 && rt[b] > t) { rt[b + 1] = rt[b]; rp[b + 1] = rp[b]; b--; }
+                rt[b + 1] = t; rp[b + 1] = q;
+            }
+            for (int a = 0; a < nr; a++) {
+                const unsigned long long pl = rp[a];
+                wide_path_update_stats<KIND, NWV>(p, env, svc_row(pl), svc_core(pl), svc_start(pl), svc_slots(pl), true, now);
+                snh -= (long long)svc_slots(pl) * wide_hops(p, svc_row(pl));
+            }
+            p.sum_nh[env] = snh;
+        } else
         events_release(ev, nheap, hmin, tailmin, now, apply_payload([&](unsigned long long pl) {
             wide_path_update<NWV>(p, env, svc_row(pl), svc_core(pl), svc_start(pl), svc_slots(pl), true);
         }));

@@ -249,7 +249,8 @@ class OpticalVecEnv:
         self._out_ptrs = (_ptr(self._obs), _ptr(self._reward), _ptr(self._done), _ptr(self._decision), _ptr(self._info))
         self._actions = None
         self._trace = None
-        # float statistics of info (network / link compactness, utilisation): opt-in, uses the generic kernel
+        # float statistics of info (network / link compactness, utilisation): opt-in; the NSFNET class runs them on the generic
+        # kernel, wider topologies on the statistics instance of the wide kernel (any link count, up to 512 slots and 31 cores)
         self._stats = None
         self._link_stats = bool(link_stats)
         if link_stats and env_id in ("RMSA-v0", "DeepRMSA-v0"):
