@@ -166,6 +166,23 @@ enum { ORLG_POLICY_RANDOM = -1, ORLG_POLICY_REPLAY = -2 };   /* REPLAY: actions_
 int orlg_rollout(orlg_env *env, int steps, int policy, void *obs_dev, float *reward_dev, uint8_t *done_dev,
                  int32_t *actions_dev, orlg_stream stream);
 
+/* The fourth part of env.step's result, kept for every step of a rollout: row t of each output is what the step-by-step calls
+ * give after step t.  Any member may be NULL (not written).  Asking for an output the handle does not have is
+ * ORLG_E_UNSUPPORTED, with the message of the per-step entry point. */
+typedef struct orlg_info_out {
+    int64_t *counters_dev;              /* int64 [steps, num_envs, 8]: at step t exactly what orlg_step's info_dev receives */
+    double *stats_dev;                  /* f64 [steps, num_envs, 4]: orlg_enable_stats's values (handles with float statistics) */
+    double *bit_rate_blocking_dev;      /* f64 [steps, num_envs, orlg_num_bit_rates + 1]: orlg_bit_rate_blocking (discrete bit rates) */
+    double *action_probability_dev;     /* f64 [steps, num_envs, orlg_action_hist_dim]: orlg_action_probability (RWA-v0) */
+} orlg_info_out;
+/* orlg_rollout (= this call with info NULL) that also keeps every step's info.  The persistent kernel writes the counters
+ * itself (64 bytes per env-step); handles with statistics or discrete bit rates already run step by step, and so does an RWA-v0
+ * call that asks for action probabilities (about 90 doubles per env-step).  orlg_kernel_info's last_rollout_persistent reports
+ * which path ran.  Not offered for orlg_rollout_packed / orlg_rollout_host (a 32-byte record has no room, and int64 counters
+ * would triple the bytes that cross PCIe), nor the decision output of orlg_step. */
+int orlg_rollout_info(orlg_env *env, int steps, int policy, void *obs_dev, float *reward_dev, uint8_t *done_dev,
+                      int32_t *actions_dev, const orlg_info_out *info, orlg_stream stream);
+
 /* The same rollout with ONE 32-byte record per env-step instead of the float observation: uint32 [steps, num_envs, 8]
  *   w0..w4  per candidate path: first-block start (7 bits, 127 = none) | its length (7) | free slots (7) | free runs (6) | slots needed (5)
  *   w5      bit rate (8) | source << 8 | destination << 16 | candidate paths << 24 | accepted << 28 | done << 29  (request = the NEXT one)
@@ -232,6 +249,11 @@ int orlg_policy_sample(orlg_policy *pol, const float *obs_dev, int n, const orlg
 int orlg_rollout_policy(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
                         float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
                         float *reward_dev, uint8_t *done_dev, orlg_stream stream);
+/* orlg_rollout_policy (= this call with info NULL) that also keeps every step's info: counters_dev and stats_dev as in
+ * orlg_rollout_info (DeepRMSA-v0 has neither discrete bit rates nor action probabilities). */
+int orlg_rollout_policy_info(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
+                             float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
+                             float *reward_dev, uint8_t *done_dev, const orlg_info_out *info, orlg_stream stream);
 /* requests drawn so far by every env of the handle (all step together): counter word 0 of the draws orlg_rollout_policy
  * makes at its next step.  Host state, no device access. */
 int64_t orlg_request_index(const orlg_env *env);

@@ -274,12 +274,27 @@ constexpr const char *heuristic_refusal(int kind, int which) {
                                                                 : nullptr;
 }
 
-// the persistent rollout kernel runs this policy on this handle (given a shared-memory plan, rollout_plan)
-bool rollout_kernel_applies(const orlg_env *env, int policy) {
+// the persistent rollout kernel runs this policy on this handle (given a shared-memory plan, rollout_plan); it writes the
+// counters of info but not the RWA action probabilities (about 90 doubles per env-step): a call that wants them steps
+bool rollout_kernel_applies(const orlg_env *env, int policy, const orlg_info_out *info) {
     const Params &p = env->p;
     const bool policy_ok = p.traffic == ORLG_TRAFFIC_TRACE ? policy == ORLG_POLICY_REPLAY
                            : policy == ORLG_POLICY_RANDOM || policy == ORLG_POLICY_REPLAY || !heuristic_refusal(p.kind, policy);
-    return env->ro_ok && !p.stats && !p.obs_f64 && !p.br_hist && policy_ok;
+    return env->ro_ok && !p.stats && !p.obs_f64 && !p.br_hist && !(info && info->action_probability_dev) && policy_ok;
+}
+
+// refusals of the float entries of info, shared by the per-step entry points and the rollouts that keep every step's info
+constexpr const char *NO_STATS_INFO = "info has float statistics only after orlg_enable_stats (RMSA-v0 / DeepRMSA-v0)";
+constexpr const char *NO_BIT_RATES = "per-bit-rate statistics exist for RMSA-v0 with bit_rate_selection='discrete'";
+constexpr const char *NO_ACTION_HIST = "action probabilities are part of info for RWA-v0 only (rwa_env.py:148-151)";
+
+// nullptr when the handle has every output `info` asks for, else why it is refused
+const char *info_refusal(const Params &p, const orlg_info_out *info) {
+    if (!info) return nullptr;
+    if (info->stats_dev && !p.stats_out) return NO_STATS_INFO;
+    if (info->bit_rate_blocking_dev && !p.br_hist) return NO_BIT_RATES;
+    if (info->action_probability_dev && !p.act_hist) return NO_ACTION_HIST;
+    return nullptr;
 }
 
 // the fast-kernel instances launch_fast picks from, [j != 1][float64 obs][link template 0] then HOT [link template 0]
@@ -383,11 +398,12 @@ cudaError_t launch_rollout_kind(const orlg_env *env, const RolloutArgs &ra, int 
     cudaLaunchConfig_t cfg = pdl_config(blocks, threads, smem, s);
     cudaError_t e = cudaErrorInvalidValue;
     const bool trace = env->p.traffic == ORLG_TRAFFIC_TRACE;
-#define ORLG_RO_LAUNCH1(POL, TR, LP)                                                                                     \
+#define ORLG_RO_LAUNCH2(POL, TR, LP, INF)                                                                                \
     do {                                                                                                                 \
-        e = cudaFuncSetAttribute(deeprmsa_rollout_kernel<ET, POL, TR, KIND, LP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-        if (e == cudaSuccess) e = cudaLaunchKernelEx(&cfg, deeprmsa_rollout_kernel<ET, POL, TR, KIND, LP>, env->p, ra); \
+        e = cudaFuncSetAttribute(deeprmsa_rollout_kernel<ET, POL, TR, KIND, LP, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+        if (e == cudaSuccess) e = cudaLaunchKernelEx(&cfg, deeprmsa_rollout_kernel<ET, POL, TR, KIND, LP, INF>, env->p, ra); \
     } while (0)
+#define ORLG_RO_LAUNCH1(POL, TR, LP) do { if (ra.info) ORLG_RO_LAUNCH2(POL, TR, LP, true); else ORLG_RO_LAUNCH2(POL, TR, LP, false); } while (0)
 #define ORLG_RO_LAUNCH(POL, TR) do { if (ra.lpw == 32) ORLG_RO_LAUNCH1(POL, TR, 32); else ORLG_RO_LAUNCH1(POL, TR, 8); } while (0)
     if (policy == ORLG_POLICY_REPLAY) {
         if (trace) ORLG_RO_LAUNCH(RO_POLICY_REPLAY, true); else ORLG_RO_LAUNCH(RO_POLICY_REPLAY, false);
@@ -400,6 +416,7 @@ cudaError_t launch_rollout_kind(const orlg_env *env, const RolloutArgs &ra, int 
     else if (policy == ORLG_HEUR_SAP_LF) { if (!heuristic_refusal(KIND, ORLG_HEUR_SAP_LF)) ORLG_RO_LAUNCH(RO_POLICY_SAP_LF, false); }
 #undef ORLG_RO_LAUNCH
 #undef ORLG_RO_LAUNCH1
+#undef ORLG_RO_LAUNCH2
     return e;
 }
 
@@ -980,7 +997,7 @@ int orlg_num_bit_rates(const orlg_env *env) { return env->p.br_hist ? env->p.n_b
 int orlg_bit_rate_blocking(orlg_env *env, double *out_dev, orlg_stream stream) {
     if (!env || !out_dev) return fail(ORLG_E_INVALID, "null handle or buffer");
     DeviceGuard guard(env->device);
-    if (!env->p.br_hist) return fail(ORLG_E_UNSUPPORTED, "per-bit-rate statistics exist for RMSA-v0 with bit_rate_selection='discrete'");
+    if (!env->p.br_hist) return fail(ORLG_E_UNSUPPORTED, NO_BIT_RATES);
     bit_rate_blocking_kernel<<<(env->p.n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(env->p, out_dev);
     CUDA_OK(cudaGetLastError());
     return ORLG_OK;
@@ -990,7 +1007,7 @@ int orlg_action_hist_dim(const orlg_env *env) { return env->p.act_hist ? env->p.
 
 int orlg_action_probability(orlg_env *env, double *out_dev, orlg_stream stream) {
     if (!env || !out_dev) return fail(ORLG_E_INVALID, "null handle or buffer");
-    if (!env->p.act_hist) return fail(ORLG_E_UNSUPPORTED, "action probabilities are part of info for RWA-v0 only (rwa_env.py:148-151)");
+    if (!env->p.act_hist) return fail(ORLG_E_UNSUPPORTED, NO_ACTION_HIST);
     DeviceGuard guard(env->device);
     action_probability_kernel<<<(env->p.n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(env->p, out_dev);
     CUDA_OK(cudaGetLastError());
@@ -1022,14 +1039,30 @@ int orlg_path_only_first_fit(orlg_env *env, const int32_t *path_actions_dev, int
     return ORLG_OK;
 }
 
+// row t of the float outputs of info, after step t (the counters come through the step kernel's info_dev)
+static int info_row(orlg_env *env, const orlg_info_out *info, int t, orlg_stream stream) {
+    const Params &p = env->p;
+    const size_t n = (size_t)p.n;
+    if (info->stats_dev)
+        CUDA_OK(cudaMemcpyAsync(info->stats_dev + (size_t)t * n * 4, p.stats_out, n * 4 * sizeof(double), cudaMemcpyDeviceToDevice,
+                                (cudaStream_t)stream));
+    int rc = ORLG_OK;
+    if (info->bit_rate_blocking_dev)
+        rc = orlg_bit_rate_blocking(env, info->bit_rate_blocking_dev + (size_t)t * n * (p.n_bit_rates + 1), stream);
+    if (!rc && info->action_probability_dev)
+        rc = orlg_action_probability(env, info->action_probability_dev + (size_t)t * n * orlg_action_hist_dim(env), stream);
+    return rc;
+}
+
 static int rollout_impl(orlg_env *env, int steps, int policy, void *obs_dev, float *reward_dev, uint8_t *done_dev,
-                        int32_t *actions_dev, uint32_t *packed_dev, orlg_stream stream) {
+                        int32_t *actions_dev, uint32_t *packed_dev, const orlg_info_out *info, orlg_stream stream) {
     if (!env) return fail(ORLG_E_INVALID, "null handle");
     DeviceGuard guard(env->device);
     if (steps < 0) return fail(ORLG_E_INVALID, "steps must be >= 0");
     if (policy != ORLG_POLICY_RANDOM && policy != ORLG_POLICY_REPLAY && (policy < 0 || policy > ORLG_HEUR_SAP_LF)) return fail(ORLG_E_INVALID, "unknown policy");
     if (policy == ORLG_POLICY_REPLAY && !actions_dev) return fail(ORLG_E_INVALID, "ORLG_POLICY_REPLAY needs the action sequence in actions_dev");
     if (env->p.traffic == ORLG_TRAFFIC_TRACE && env->p.trace == nullptr) return fail(ORLG_E_INVALID, "trace traffic selected but orlg_set_trace was not called");
+    if (const char *why = info_refusal(env->p, info)) return fail(ORLG_E_UNSUPPORTED, why);
     if (steps == 0) return ORLG_OK;
     Params &p = env->p;
     cudaStream_t s = (cudaStream_t)stream;
@@ -1037,7 +1070,7 @@ static int rollout_impl(orlg_env *env, int steps, int policy, void *obs_dev, flo
     std::memset(&ra, 0, sizeof(ra));
     int wpc = 0;
     size_t smem = 0;
-    if (rollout_kernel_applies(env, policy) && rollout_plan(env, &wpc, &ra, &smem)) {
+    if (rollout_kernel_applies(env, policy, info) && rollout_plan(env, &wpc, &ra, &smem)) {
         if (!env->ro_ev) {
             const size_t n = (size_t)p.n, warps = (n + env->ro_lpw - 1) / env->ro_lpw;
             int rc = dev_alloc(env, &env->ro_ev, warps * 32 * ((size_t)p.heap_cap + 2 * RO_WCAP), false);
@@ -1053,6 +1086,7 @@ static int rollout_impl(orlg_env *env, int steps, int policy, void *obs_dev, flo
         ra.obs = reinterpret_cast<float *>(obs_dev);
         ra.reward = reward_dev; ra.done = done_dev; ra.actions = actions_dev;
         ra.packed = reinterpret_cast<uint4 *>(packed_dev);
+        ra.info = info ? reinterpret_cast<long long *>(info->counters_dev) : nullptr;
         if (packed_dev && p.kind != ORLG_DEEPRMSA) return fail(ORLG_E_UNSUPPORTED, "packed records describe the DeepRMSA observation");
         rollout_state_args(env, &ra);
         ra.resume = env->ro_valid ? 1 : 0;
@@ -1081,10 +1115,12 @@ static int rollout_impl(orlg_env *env, int steps, int policy, void *obs_dev, flo
         void *o = (obs_dev && p.obs_dim) ? reinterpret_cast<unsigned char *>(obs_dev) + (size_t)t * p.n * obs_row : nullptr;
         float *r = reward_dev ? reward_dev + (size_t)t * p.n : nullptr;
         uint8_t *d = done_dev ? done_dev + (size_t)t * p.n : nullptr;
-        if (fuse) rc = step_impl(env, nullptr, policy, actions_dev ? a : nullptr, o, r, d, nullptr, nullptr, stream);
+        int64_t *c = info && info->counters_dev ? info->counters_dev + (size_t)t * p.n * 8 : nullptr;
+        if (fuse) rc = step_impl(env, nullptr, policy, actions_dev ? a : nullptr, o, r, d, nullptr, c, stream);
         else if (policy != ORLG_POLICY_REPLAY)
             rc = policy == ORLG_POLICY_RANDOM ? orlg_random_actions(env, a, stream) : orlg_heuristic(env, policy, a, stream);
-        if (!rc && !fuse) rc = orlg_step(env, a, o, r, d, nullptr, nullptr, stream);
+        if (!rc && !fuse) rc = orlg_step(env, a, o, r, d, nullptr, c, stream);
+        if (!rc && info) rc = info_row(env, info, t, stream);
     }
     return rc;
 }
@@ -1092,12 +1128,17 @@ static int rollout_impl(orlg_env *env, int steps, int policy, void *obs_dev, flo
 
 int orlg_rollout(orlg_env *env, int steps, int policy, void *obs_dev, float *reward_dev, uint8_t *done_dev,
                  int32_t *actions_dev, orlg_stream stream) {
-    return rollout_impl(env, steps, policy, obs_dev, reward_dev, done_dev, actions_dev, nullptr, stream);
+    return rollout_impl(env, steps, policy, obs_dev, reward_dev, done_dev, actions_dev, nullptr, nullptr, stream);
+}
+
+int orlg_rollout_info(orlg_env *env, int steps, int policy, void *obs_dev, float *reward_dev, uint8_t *done_dev,
+                      int32_t *actions_dev, const orlg_info_out *info, orlg_stream stream) {
+    return rollout_impl(env, steps, policy, obs_dev, reward_dev, done_dev, actions_dev, nullptr, info, stream);
 }
 
 int orlg_rollout_packed(orlg_env *env, int steps, int policy, uint32_t *packed_dev, int32_t *actions_dev, orlg_stream stream) {
     if (!packed_dev) return fail(ORLG_E_INVALID, "null record buffer");
-    return rollout_impl(env, steps, policy, nullptr, nullptr, nullptr, actions_dev, packed_dev, stream);
+    return rollout_impl(env, steps, policy, nullptr, nullptr, nullptr, actions_dev, packed_dev, nullptr, stream);
 }
 
 // ---------------------------------------------------------------- host side of the packed records (no CUDA below this line)
@@ -1289,7 +1330,7 @@ int orlg_rollout_host(orlg_env *env, int steps, int policy, float *obs_host, flo
                                     cudaMemcpyHostToDevice, s));
         if (c >= NB) CUDA_OK(cudaStreamWaitEvent(s, hp.pk_ev[b], 0));
         int rc = rollout_impl(env, tc, policy, nullptr, nullptr, nullptr, replay ? hp.act_dev[b] : nullptr,
-                              reinterpret_cast<uint32_t *>(hp.pk_dev[b]), stream);
+                              reinterpret_cast<uint32_t *>(hp.pk_dev[b]), nullptr, stream);
         if (rc) return rc;
         CUDA_OK(cudaEventRecord(hp.k_ev[b], s));
         CUDA_OK(cudaStreamWaitEvent(sc, hp.k_ev[b], 0));
@@ -1458,6 +1499,13 @@ int orlg_policy_sample(orlg_policy *pol, const float *obs_dev, int n, const orlg
 int orlg_rollout_policy(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
                         float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
                         float *reward_dev, uint8_t *done_dev, orlg_stream stream) {
+    return orlg_rollout_policy_info(env, steps, actor, critic, seed, deterministic, obs_dev, actions_dev, log_prob_dev, value_dev,
+                                    reward_dev, done_dev, nullptr, stream);
+}
+
+int orlg_rollout_policy_info(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
+                             float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
+                             float *reward_dev, uint8_t *done_dev, const orlg_info_out *info, orlg_stream stream) {
     if (!env || !actor) return fail(ORLG_E_INVALID, "null env or actor handle");
     const Params &p = env->p;
     if (p.kind != ORLG_DEEPRMSA) return fail(ORLG_E_UNSUPPORTED, "orlg_rollout_policy drives DeepRMSA-v0 (the env kind with a tensor observation)");
@@ -1474,6 +1522,7 @@ int orlg_rollout_policy(orlg_env *env, int steps, orlg_policy *actor, orlg_polic
     if (!obs_dev) return fail(ORLG_E_INVALID, "orlg_rollout_policy needs obs_dev (the policy reads it)");
     if (steps < 0) return fail(ORLG_E_INVALID, "steps must be >= 0");
     if (p.traffic == ORLG_TRAFFIC_TRACE && p.trace == nullptr) return fail(ORLG_E_INVALID, "trace traffic selected but orlg_set_trace was not called");
+    if (const char *why = info_refusal(p, info)) return fail(ORLG_E_UNSUPPORTED, why);
     DeviceGuard guard(env->device);
     cudaStream_t s = (cudaStream_t)stream;
     int rc = ensure_canonical(env, s);          // the handle may have been stepped by the persistent rollout kernel
@@ -1494,7 +1543,9 @@ int orlg_rollout_policy(orlg_env *env, int steps, orlg_policy *actor, orlg_polic
                                                                        critic ? nullptr : v), s);
         if (!rc && critic && v) rc = launch_policy<true>(critic, o, p.n, nullptr, nullptr, policy_draw(d, nullptr, v), s);
         if (!rc) rc = step_impl(env, a, -1, nullptr, obs_dev + (size_t)(t + 1) * row, reward_dev ? reward_dev + (size_t)t * n : nullptr,
-                                done_dev ? done_dev + (size_t)t * n : nullptr, nullptr, nullptr, stream);
+                                done_dev ? done_dev + (size_t)t * n : nullptr, nullptr,
+                                info && info->counters_dev ? info->counters_dev + (size_t)t * n * 8 : nullptr, stream);
+        if (!rc && info) rc = info_row(env, info, t, stream);
         if (rc) return rc;
     }
     if (value_dev)                              // the bootstrap value of the last observation

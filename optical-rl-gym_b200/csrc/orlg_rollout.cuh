@@ -107,6 +107,7 @@ struct RolloutArgs {
     double *st_tmin, *st_hzn;                           // [n]
     double *st_side_t;                                  // [RO_SIDE][n]
     unsigned long long *st_side_p;                      // [RO_SIDE][n]
+    long long *info;             // [T][n][8]         the counters orlg_step's info_dev receives, every step (INFO instances)
 };
 
 // apply a release / an allocation to the path's links in the warp's shared-memory mask tile
@@ -328,7 +329,8 @@ __device__ __forceinline__ unsigned feat_pack(int st, int len, int total, int ru
 // the reference's first-fit heuristics evaluated on the cached free-slot masks of the candidate paths).
 // LPW: envs (lanes in use) per warp, 32 or 8 (compile-time: the 32-lane instances are the code they were before the small-batch
 // mapping existed -- a run-time lane count cost the headline instance 3 % through register allocation alone).
-template <int ET, int POLICY, bool TRACE = false, int KIND = ORLG_DEEPRMSA, int LPW = 32>
+// INFO: every step's counters go to ra.info (compile-time: a run-time null check slowed the headline instance by 0.7 %).
+template <int ET, int POLICY, bool TRACE = false, int KIND = ORLG_DEEPRMSA, int LPW = 32, bool INFO = false>
 __global__ void __launch_bounds__(RO_MAX_THREADS, 1)
 deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
     constexpr int KM = 5;
@@ -690,6 +692,19 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
         RPH_MARK(3);                 // rebuild
         if (live && t >= 0) {
             done = (ep_proc == p.episode_length);
+            if (INFO) {
+                // the counters as the reference builds `info` (rmsa_env.py:234-248, rwa_env.py:141-152): before _next_service,
+                // so RMSA / DeepRMSA take back the next request that phase B has already counted.  The running totals are
+                // the launch-entry values (unchanged in HBM until the exit below) plus this launch's deltas, re-read here
+                // rather than held in registers across the step loop.  One env = 64 contiguous bytes, a warp 2 KB.
+                const int nq = KIND == ORLG_RWA ? 0 : 1, nbr = KIND == ORLG_RWA ? 0 : br;
+                const long long *c = p.counters + env;
+                longlong2 *o = reinterpret_cast<longlong2 *>(ra.info + ((size_t)t * p.n + env) * 8);
+                o[0] = make_longlong2(c[0] + d_proc - nq, c[(size_t)p.n] + d_acc);
+                o[1] = make_longlong2(ep_proc - nq, ep_acc);
+                o[2] = make_longlong2(c[(size_t)4 * p.n] + d_req - nbr, c[(size_t)5 * p.n] + d_prov);
+                o[3] = make_longlong2(ep_req - nbr, ep_prov);
+            }
             if (done && p.auto_reset) {                          // rmsa_env.py:285-330, rwa_env.py:164-179
                 ep_acc = 0; ep_prov = 0;
                 if (KIND == ORLG_RWA) { ep_proc = 0; ep_req = 0; } else { ep_proc = 1; ep_req = br; }

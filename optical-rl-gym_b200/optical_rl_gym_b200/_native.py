@@ -39,6 +39,11 @@ class PolicyDraw(C.Structure):
                 ("row_id_base", C.c_int64)]
 
 
+class InfoOut(C.Structure):
+    """orlg_info_out: device pointers of the per-step info outputs of a rollout (None = not written)."""
+    _fields_ = [(n, C.c_void_p) for n in ("counters_dev", "stats_dev", "bit_rate_blocking_dev", "action_probability_dev")]
+
+
 class Tables(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("num_nodes", "num_links", "k_paths", "num_paths", "num_mods", "num_bit_rates")] + [
         (n, C.c_void_p) for n in ("pair_first", "pair_count", "path_hops", "path_se", "path_mod", "path_link_ptr",
@@ -102,6 +107,7 @@ def lib():
     L.orlg_action_hist_dim.argtypes = [vp]
     L.orlg_action_probability.argtypes = [vp, vp, vp]
     L.orlg_rollout.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp]
+    L.orlg_rollout_info.argtypes = [vp, i32, i32, vp, vp, vp, vp, C.POINTER(InfoOut), vp]
     L.orlg_state_save_bytes.argtypes = [vp]
     L.orlg_state_save_bytes.restype = i64
     L.orlg_state_save.argtypes = [vp, vp, vp]
@@ -111,6 +117,7 @@ def lib():
     L.orlg_policy_destroy.argtypes = [vp]
     L.orlg_policy_sample.argtypes = [vp, vp, i32, C.POINTER(PolicyDraw), vp, vp, vp, vp]
     L.orlg_rollout_policy.argtypes = [vp, i32, vp, vp, C.c_uint64, i32, vp, vp, vp, vp, vp, vp, vp]
+    L.orlg_rollout_policy_info.argtypes = [vp, i32, vp, vp, C.c_uint64, i32, vp, vp, vp, vp, vp, vp, C.POINTER(InfoOut), vp]
     L.orlg_request_index.argtypes = [vp]
     L.orlg_request_index.restype = i64
     L.orlg_rollout_packed.argtypes = [vp, i32, i32, vp, vp, vp]
@@ -131,4 +138,5 @@ EXPORTED = ["orlg_create", "orlg_destroy", "orlg_last_error", "orlg_version", "o
             "orlg_get_requests", "orlg_export_state", "orlg_error_flags", "orlg_reduce_counters", "orlg_enable_stats",
             "orlg_num_bit_rates", "orlg_bit_rate_blocking", "orlg_matrix_obs_dim", "orlg_matrix_observation",
             "orlg_path_only_first_fit", "orlg_rollout", "orlg_state_save_bytes", "orlg_state_save", "orlg_state_load", "orlg_policy_create", "orlg_policy_act", "orlg_policy_destroy", "orlg_rollout_packed", "orlg_expand_packed", "orlg_rollout_host", "orlg_action_hist_dim", "orlg_action_probability",
-            "orlg_enable_link_stats", "orlg_link_stats", "orlg_policy_sample", "orlg_rollout_policy", "orlg_request_index"]
+            "orlg_enable_link_stats", "orlg_link_stats", "orlg_policy_sample", "orlg_rollout_policy", "orlg_request_index",
+            "orlg_rollout_info", "orlg_rollout_policy_info"]

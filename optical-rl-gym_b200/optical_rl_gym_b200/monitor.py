@@ -7,7 +7,8 @@ examples/stable_baselines3/bkp/deeprmsa-ppo-trained/training.monitor.csv).
 File layout: ``#{"t_start": ..., "env_id": ...}`` then a CSV with header ``r,l,t,<info_keywords>``; one
 row per finished episode = sum of rewards, number of steps, seconds since ``t_start`` and the value of each
 info keyword at the terminal step.  Sums and lengths accumulate on the device; the host is only touched
-when an episode ends (one 1-byte read per step to learn whether any did).
+when an episode ends (one 1-byte read per step to learn whether any did).  ``rollout`` and ``rollout_policy``
+write the same rows as the equivalent ``step`` loop, from every step's reward, done and info of the rollout.
 """
 from __future__ import annotations
 
@@ -64,23 +65,76 @@ class VecMonitor(VecWrapper):
         self.total_steps += int(self._len.shape[0])
         if bool(done.any()):
             idx = torch.nonzero(done, as_tuple=False).flatten()
-            r = self._ret[idx].cpu().numpy()
-            l = self._len[idx].cpu().numpy()
-            t = round(time.time() - self.t_start, 6)
-            cols = [np.asarray(info[k][idx].cpu().numpy(), np.float64) for k in self.info_keywords]
-            self.episode_returns.extend(r.tolist())
-            self.episode_lengths.extend(l.tolist())
-            self.episode_times.extend([t] * len(r))
-            for k, c in zip(self.info_keywords, cols):
-                self.episode_infos[k].extend(c.tolist())
-            if self._fh is not None:
-                # every finished episode gets its row (SB3's Monitor writes one per episode): one buffered write per step
-                self._fh.write("".join(",".join([repr(float(r[i])), str(int(l[i])), repr(t)] + [repr(float(c[i])) for c in cols]) + "\n"
-                                       for i in range(len(r))))
-                self._fh.flush()
+            self._record(self._ret[idx], self._len[idx], [info[k][idx] for k in self.info_keywords])
             self._ret[idx] = 0.0
             self._len[idx] = 0
         return obs, reward, done, info
+
+    def _record(self, r, l, cols):
+        """Appends the rows of finished episodes: returns, lengths and info keyword values (device tensors, in row order)."""
+        r, l = r.cpu().numpy(), l.cpu().numpy()
+        t = round(time.time() - self.t_start, 6)
+        cols = [np.asarray(c.cpu().numpy(), np.float64) for c in cols]
+        self.episode_returns.extend(r.tolist())
+        self.episode_lengths.extend(l.tolist())
+        self.episode_times.extend([t] * len(r))
+        for k, c in zip(self.info_keywords, cols):
+            self.episode_infos[k].extend(c.tolist())
+        if self._fh is not None:
+            # every finished episode gets its row (SB3's Monitor writes one per episode): one buffered write per call
+            self._fh.write("".join(",".join([repr(float(r[i])), str(int(l[i])), repr(t)] + [repr(float(c[i])) for c in cols]) + "\n"
+                                   for i in range(len(r))))
+            self._fh.flush()
+
+    def _base(self, method):
+        from .vec_env import OpticalVecEnv
+
+        if not isinstance(self.venv, OpticalVecEnv):
+            # a wrapper in between (UseInfoReward, ...) would be bypassed by the native rollout: its rows would be wrong
+            raise TypeError("VecMonitor.%s needs the OpticalVecEnv itself as its venv, not %s" % (method, type(self.venv).__name__))
+        return self.venv
+
+    def _record_rollout(self, reward, done, info):
+        """The rows a ``step`` loop over the rollout's T steps would write, from reward / done ``[T, N]`` and ``info``."""
+        T, n = done.shape
+        self.total_steps += T * n
+        if T == 0:
+            return
+        d = done.bool()
+        csum = torch.cumsum(reward.to(torch.float64), 0)         # rewards are -1 / 0 / 1: exact in any order of addition
+        steps = torch.arange(T, device=d.device).unsqueeze(1).expand(T, n)
+        last = torch.where(d, steps, torch.full_like(steps, -1)).cummax(0).values      # last episode end at or before t
+        idx = torch.nonzero(d, as_tuple=False)                    # (t, env) in the step loop's row order
+        if idx.shape[0]:
+            t, e = idx[:, 0], idx[:, 1]
+            prev = torch.where(t > 0, last[(t - 1).clamp(min=0), e], torch.full_like(t, -1))   # the env's previous end
+            first = prev < 0                                      # the episode began before this call
+            before = torch.where(first, torch.zeros_like(csum[t, e]), csum[prev.clamp(min=0), e])
+            r = torch.where(first, self._ret[e], torch.zeros_like(before)) + (csum[t, e] - before)
+            l = torch.where(first, self._len[e], torch.zeros_like(t)) + (t - prev)
+            self._record(r, l, [info[k][t, e] for k in self.info_keywords])
+        end = last[T - 1]
+        ended = end >= 0
+        self._ret = torch.where(ended, csum[T - 1] - csum[end.clamp(min=0), torch.arange(n, device=d.device)], self._ret + csum[T - 1])
+        self._len = torch.where(ended, T - 1 - end, self._len + T)
+
+    def rollout(self, steps, policy="random", **kw):
+        """:meth:`OpticalVecEnv.rollout` that logs the episodes it finishes like the equivalent ``step`` loop; returns what
+        the env returns (with the info only when ``want_info=True`` is passed)."""
+        want = kw.pop("want_info", False)
+        with_info = want or bool(self.info_keywords)
+        res = self._base("rollout").rollout(steps, policy, want_info=with_info, **kw)
+        self._record_rollout(res[1], res[2], res[4] if with_info else None)
+        return res if want or not with_info else res[:4]
+
+    def rollout_policy(self, agent, steps, **kw):
+        """:meth:`OpticalVecEnv.rollout_policy` that logs the episodes it finishes like the equivalent ``step`` loop."""
+        want = kw.pop("want_info", False)
+        with_info = want or bool(self.info_keywords)
+        res = self._base("rollout_policy").rollout_policy(agent, steps, want_info=with_info, **kw)
+        out, info = res if with_info else (res, None)
+        self._record_rollout(out.reward, out.done, info)
+        return res if want or not with_info else out
 
     def get_episode_rewards(self):
         return self.episode_returns

@@ -54,7 +54,8 @@ COUNTER_NAMES = ("services_processed", "services_accepted", "episode_services_pr
 
 class StepInfo:
     """``info`` of a batched step: blocking rates as float64 ``[N]`` tensors, computed on demand from
-    the integer counters the kernel snapshots where the reference builds its dict (rmsa_env.py:234-248)."""
+    the integer counters the kernel snapshots where the reference builds its dict (rmsa_env.py:234-248).
+    The info of a rollout has a leading step axis: every array is ``[T, N, ...]`` and every value ``[T, N]``."""
 
     _COL = {"service_blocking_rate": (0, 1), "episode_service_blocking_rate": (2, 3),
             "bit_rate_blocking_rate": (4, 5), "episode_bit_rate_blocking_rate": (6, 7)}
@@ -62,7 +63,7 @@ class StepInfo:
     def __init__(self, counters: torch.Tensor, keys, stats: Optional[torch.Tensor] = None,
                  bit_rate_blocking: Optional[torch.Tensor] = None, bit_rates=(),
                  action_probability: Optional[torch.Tensor] = None, n_path_actions: int = 0):
-        self.counters = counters       # int64 [N, 8]
+        self.counters = counters       # int64 [N, 8] ([T, N, 8] for a rollout, likewise below)
         self.stats = stats             # float64 [N, 4] (rmsa_env.py:249-263) when link_stats=True
         self.bit_rate_blocking = bit_rate_blocking     # float64 [N, B + 1] (rmsa_env.py:217-227, 268-273), discrete mode
         self._br_keys = ["bit_rate_blocking_%d" % int(b) for b in bit_rates] + ["fairness"] if bit_rate_blocking is not None else []
@@ -84,16 +85,16 @@ class StepInfo:
         if key not in self._keys:
             raise KeyError(key)
         if key in STAT_KEYS:
-            return self.stats[:, STAT_KEYS.index(key)]
+            return self.stats[..., STAT_KEYS.index(key)]
         if key in self._br_keys:
-            return self.bit_rate_blocking[:, self._br_keys.index(key)]
+            return self.bit_rate_blocking[..., self._br_keys.index(key)]
         if key == "path_action_probability":
-            return self.action_probability[:, :self._n_path_actions]
+            return self.action_probability[..., :self._n_path_actions]
         if key == "wavelength_action_probability":
-            return self.action_probability[:, self._n_path_actions:]
+            return self.action_probability[..., self._n_path_actions:]
         a, b = self._COL[key]
         c = self.counters
-        return (c[:, a] - c[:, b]).to(torch.float64) / c[:, a].to(torch.float64)
+        return (c[..., a] - c[..., b]).to(torch.float64) / c[..., a].to(torch.float64)
 
     def items(self):
         return [(k, self[k]) for k in self._keys]
@@ -367,6 +368,16 @@ class OpticalVecEnv:
         return StepInfo(self._info, self.metadata["metrics"], self._stats, self._brb, self.bit_rates, self._ap,
                         self.k_paths + self.reject_action).keys()
 
+    def _rollout_info(self, steps: int):
+        """Device buffers for every step's info of a ``steps``-step rollout: ``(StepInfo, orlg_info_out)``."""
+        if self._info is None:
+            raise ValueError("want_info=True needs the env's info: construct it with collect_info=True")
+        bufs = [None if b is None else torch.empty((steps,) + tuple(b.shape), dtype=b.dtype, device=self.device)
+                for b in (self._info, self._stats, self._brb, self._ap)]
+        info = StepInfo(bufs[0], self.metadata["metrics"], bufs[1], bufs[2], self.bit_rates, bufs[3],
+                        self.k_paths + self.reject_action)
+        return info, nat.InfoOut(*(None if b is None else b.data_ptr() for b in bufs))
+
     def step_raw(self, actions_i32: torch.Tensor):
         """Hot-loop variant: ``actions_i32`` must already be a contiguous int32 CUDA tensor ``[N, action_dim]``."""
         rc = self._lib.orlg_step(self._h, C.c_void_p(actions_i32.data_ptr()), *self._out_ptrs, self._stream())
@@ -375,12 +386,15 @@ class OpticalVecEnv:
         return self._obs, self._reward, self._done
 
     def rollout(self, steps: int, policy="random", *, obs=None, reward=None, done=None, actions=None,
-                want_obs: bool = True, want_actions: bool = True):
+                want_obs: bool = True, want_actions: bool = True, want_info: bool = False):
         """``steps`` iterations of ``a = policy(env); env.step(a)`` in ONE native call (``orlg_rollout``), every step's
         results kept: returns ``(obs [T, N, obs_dim] | None, reward [T, N], done [T, N], actions [T, N, action_dim] | None)``.
         ``policy``: "random" (:meth:`sample_actions`) or a heuristic name (:meth:`heuristic`).  Identical to the
-        step-by-step loop; DeepRMSA-v0 with Philox traffic and float32 observations runs as one persistent kernel."""
+        step-by-step loop; DeepRMSA-v0 with Philox traffic and float32 observations runs as one persistent kernel.
+        ``want_info=True`` (needs ``collect_info=True``) appends every step's ``info``: a :class:`StepInfo` with the keys of
+        :attr:`info_keys` and ``[T, N]`` values (``orlg_rollout_info``; RWA-v0's action probabilities make it step by step)."""
         T, n, dev = int(steps), self.num_envs, self.device
+        info, info_out = self._rollout_info(T) if want_info else (None, None)
         if policy == "replay":          # the given `actions` [T, N, action_dim] are applied (with trace traffic: a recorded run)
             assert actions is not None, "policy='replay' needs the action sequence"
             actions = torch.as_tensor(actions, device=dev).to(torch.int32).reshape(T, n, self.action_dim).contiguous()
@@ -399,21 +413,27 @@ class OpticalVecEnv:
             if tns is not None:
                 assert tuple(tns.shape) == shape and tns.is_contiguous() and tns.device == dev, (tuple(tns.shape), shape)
         with torch.cuda.device(self._dev_index):
+            if want_info:
+                nat.check(self._lib.orlg_rollout_info(self._h, T, pol, _ptr(obs), _ptr(reward), _ptr(done), _ptr(actions),
+                                                      C.byref(info_out), self._stream()))
+                return obs, reward, done, actions, info
             nat.check(self._lib.orlg_rollout(self._h, T, pol, _ptr(obs), _ptr(reward), _ptr(done), _ptr(actions), self._stream()))
         return obs, reward, done, actions
 
     def rollout_policy(self, policy, steps: int, *, deterministic: bool = False, seed: Optional[int] = None,
-                       out: Optional[PolicyRollout] = None) -> PolicyRollout:
+                       out: Optional[PolicyRollout] = None, want_info: bool = False):
         """``steps`` iterations of ``a, log p(a), V(obs) = policy(obs); obs, r, done = env.step(a)`` in ONE native call
         (``orlg_rollout_policy``): a :class:`PolicyRollout` of device tensors, what SB3's ``collect_rollouts`` gathers.
         ``policy`` is an :class:`~optical_rl_gym_b200.policy.MlpPolicy` on this device (its current weights; the value comes
         from its critic trunk when it has one).  Actions are drawn from softmax(logits) (``deterministic=True``: argmax) with
         Philox stream 3 keyed by ``seed`` (default: the env's seed), the global env id and the env's request index, so the
         result does not depend on the number of GPUs, on how the rollout is split into calls or on a checkpoint in between.
-        ``out`` reuses the buffers of an earlier call.  DeepRMSA-v0 with float32 observations."""
+        ``out`` reuses the buffers of an earlier call.  DeepRMSA-v0 with float32 observations.  ``want_info=True`` (needs
+        ``collect_info=True``) returns ``(PolicyRollout, StepInfo)``, the latter every step's ``info`` with ``[T, N]`` values."""
         T, n, dev = int(steps), self.num_envs, self.device
         if T < 0:
             raise ValueError("steps must be >= 0")
+        info, info_out = self._rollout_info(T) if want_info else (None, None)
         if out is None:
             out = PolicyRollout(torch.empty((T + 1, n, self.obs_dim), dtype=torch.float32, device=dev),
                                 torch.empty((T, n), dtype=torch.int32, device=dev),
@@ -430,6 +450,10 @@ class OpticalVecEnv:
         actor, critic = policy._native_handles(self._dev_index)
         key = self.rand_seed if seed is None else int(seed)
         with torch.cuda.device(self._dev_index):
+            if want_info:
+                nat.check(self._lib.orlg_rollout_policy_info(self._h, T, actor, critic, key & (2 ** 64 - 1), int(bool(deterministic)),
+                                                             *[_ptr(t) for t in out], C.byref(info_out), self._stream()))
+                return out, info
             nat.check(self._lib.orlg_rollout_policy(self._h, T, actor, critic, key & (2 ** 64 - 1), int(bool(deterministic)),
                                                     *[_ptr(t) for t in out], self._stream()))
         return out
