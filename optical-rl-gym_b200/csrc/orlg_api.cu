@@ -246,7 +246,7 @@ void for_kind(int kind, F &&f) {
     }
 }
 
-// f(std::integral_constant<int, W>()) for the 128-slot mask words per (core, link) of the wide kernels
+// f(std::integral_constant<int, W>()) for the 128-slot mask words per (core, link): 1 on NSFNET-class handles
 template <typename F>
 void for_words(int nwv, F &&f) {
     switch (nwv) {
@@ -846,11 +846,8 @@ int orlg_heuristic(orlg_env *env, int which, int32_t *actions_dev, orlg_stream s
     const int threads = 128, blocks = (env->p.n + threads - 1) / threads;
     cudaStream_t s = (cudaStream_t)stream;
     if (const char *why = heuristic_refusal(env->p.kind, which)) return fail(ORLG_E_UNSUPPORTED, why);
-    for_kind(env->p.kind, [&](auto K) {
-        if (env->wide) for_words(env->p.nwv, [&](auto W) {
-            heuristic_wide_kernel<decltype(K)::value, decltype(W)::value><<<blocks, threads, 0, s>>>(env->p, which, actions_dev); });
-        else heuristic_kernel<decltype(K)::value><<<blocks, threads, 0, s>>>(env->p, which, actions_dev);
-    });
+    for_kind(env->p.kind, [&](auto K) { for_words(env->p.nwv, [&](auto W) {
+        heuristic_kernel<decltype(K)::value, decltype(W)::value><<<blocks, threads, 0, s>>>(env->p, which, actions_dev); }); });
     CUDA_OK(cudaGetLastError());
     return ORLG_OK;
 }

@@ -34,80 +34,6 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-// the same with the four shift amounts of n packed one per byte (table built by the host: orlg_api.cu)
-__device__ __forceinline__ Bits bits_runs_ge_sched(const Bits &a, unsigned sched) {
-    Bits b = a;
-#pragma unroll
-    for (int it = 0; it < 4; it++) {
-        b = bits_and(b, bits_shr_small(b, (int)((sched >> (8 * it)) & 0xffu)));
-    }
-    return b;
-}
-__device__ __forceinline__ Bits bits_runs_ge_flat(const Bits &a, int n) {
-    // shift-AND doubling without any branch; valid for 1 <= n <= 16 (the caller takes the generic path otherwise)
-    Bits b = a;
-    int len = 1;
-#pragma unroll
-    for (int it = 0; it < 4; it++) {
-        int s = max(min(len, n - len), 0);
-        Bits sh = bits_shr_small(b, s);       // s == 0: funnel shift by 0 returns b
-        b = bits_and(b, sh);
-        len += s;
-    }
-    return b;
-}
-
-// bits [start, start + n) for 1 <= n <= 32, 0 <= start, start + n <= 128: one 64-bit shift placed at word start / 32
-__device__ __forceinline__ Bits bits_range_short(int start, int n) {
-    const unsigned long long m = ((1ULL << n) - 1ULL) << (start & 31);
-    const unsigned lo = (unsigned)m, hi = (unsigned)(m >> 32);
-    const int ws = start >> 5;
-    Bits r;
-#pragma unroll
-    for (int i = 0; i < NW; i++) r.w[i] = (i == ws) ? lo : ((i == ws + 1) ? hi : 0u);
-    return r;
-}
-__device__ __forceinline__ Bits bits_range_auto(int start, int n) {
-    return (n <= 32) ? bits_range_short(start, n) : bits_range(start, start + n);
-}
-
-// mask of bits >= start (0 <= start <= 128)
-__device__ __forceinline__ Bits bits_from_pos(int start) {
-    Bits r;
-#pragma unroll
-    for (int i = 0; i < NW; i++) {
-        int a = min(max(start - 32 * i, 0), 32);
-        r.w[i] = a >= 32 ? 0u : (0xFFFFFFFFu << a);
-    }
-    return r;
-}
-
-__device__ __forceinline__ int bits_run_length_flat(const Bits &a, int start) {
-    Bits f = bits_from_pos(start);
-    Bits z;
-#pragma unroll
-    for (int i = 0; i < NW; i++) z.w[i] = ~a.w[i] & f.w[i];
-    int pos = bits_ffs(z);
-    return (pos < 0 ? MAX_SLOTS : pos) - start;
-}
-
-// index of the lowest set bit of a 128-bit mask, -1 if empty (select chain instead of 4 dependent branches)
-__device__ __forceinline__ int bits_ffs_flat(const Bits &a) {
-    const int p0 = __ffs(a.w[0]), p1 = __ffs(a.w[1]), p2 = __ffs(a.w[2]), p3 = __ffs(a.w[3]);
-    int r = p3 ? p3 + 95 : -1;
-    r = p2 ? p2 + 63 : r;
-    r = p1 ? p1 + 31 : r;
-    r = p0 ? p0 - 1 : r;
-    return r;
-}
-__device__ __forceinline__ Bits bits_shr1(const Bits &a) {
-    Bits r;
-#pragma unroll
-    for (int i = 0; i < NW; i++) r.w[i] = __funnelshift_r(a.w[i], i + 1 < NW ? a.w[i + 1] : 0u, 1);
-    return r;
-}
-
-
 // Optional per-phase cycle accounting (build with -DORLG_PHASE_TIMING; read with orlg_debug_phase_cycles):
 // sum over warps of the cycles between consecutive marks.  Not part of the product build.
 #ifdef ORLG_PHASE_TIMING
@@ -575,7 +501,7 @@ deeprmsa_fast_kernel(const Params p, const StepIO io_rt, const int mode_rt, cons
                 const int n = ns[q];
                 const Bits B = bits_runs_ge_sched(A[q], s_dbl[n]);
                 const int st = bits_ffs_flat(B);
-                const int fe = bits_ffs_flat(bits_andnot(B, bits_shr1(B)));
+                const int fe = bits_ffs_flat(bits_andnot(B, bits_shr_small(B, 1)));
                 const int len = fe - st + n;
                 const int total = bits_popc(A[q]);
                 const int runs = bits_popc(bits_andnot(A[q], bits_shl1(A[q])));
@@ -603,7 +529,7 @@ deeprmsa_fast_kernel(const Params p, const StepIO io_rt, const int mode_rt, cons
                 const int ob = 1 + 2 * p.N + q * W;
                 if (JT == 1) {
                     const int st = bits_ffs(starts);
-                    const int len = bits_run_length_flat(A[q], max(st, 0));
+                    const int len = bits_run_length(A[q], max(st, 0));
                     if (st >= 0) cand_out = (cand_out & ~(0xFFULL << (8 * q))) | ((unsigned long long)st << (8 * q));
                     if (want_obs && st >= 0) {
                         if (OBS64) {
@@ -629,7 +555,7 @@ deeprmsa_fast_kernel(const Params p, const StepIO io_rt, const int mode_rt, cons
                         int len = -1;
                         if (st >= 0) {
                             starts = bits_clear_lowest(starts);
-                            len = bits_run_length_flat(A[q], st);
+                            len = bits_run_length(A[q], st);
                             if (want_obs) {
                                 if (OBS64) {
                                     so64[ob + 2 * b] = __ddiv_rn(__dmul_rn(2.0, __dadd_rn((double)st, -__dmul_rn(0.5, (double)p.S))), (double)p.S);

@@ -14,10 +14,14 @@ constexpr int NW = 4;              // 32-bit words per (core, link): S <= 128
 constexpr int MAX_SLOTS = 32 * NW;
 constexpr uint32_t CAND_NONE = 0xFFu;
 
-// ---------------------------------------------------------------- 128-bit slot masks
-struct Bits {
-    uint32_t w[NW];
+// ---------------------------------------------------------------- slot masks of V x 128 bits
+// V = 1 (Bits) for the NSFNET-class kernels; the wide kernels take V = 1..4 word groups (S <= 512).  Each operation deduces V
+// from its argument; bits_ones and bits_range take no mask and default to V = 1.
+template <int V>
+struct WBits {
+    uint32_t w[4 * V];
 };
+using Bits = WBits<1>;
 
 __device__ __forceinline__ Bits bits_from(uint4 v) {
     Bits b;
@@ -25,85 +29,97 @@ __device__ __forceinline__ Bits bits_from(uint4 v) {
     return b;
 }
 __device__ __forceinline__ uint4 bits_to(const Bits &b) { return make_uint4(b.w[0], b.w[1], b.w[2], b.w[3]); }
-__device__ __forceinline__ Bits bits_ones() {
-    Bits b;
+template <int V = 1>
+__device__ __forceinline__ WBits<V> bits_ones() {
+    WBits<V> b;
 #pragma unroll
-    for (int i = 0; i < NW; i++) b.w[i] = 0xFFFFFFFFu;
+    for (int i = 0; i < 4 * V; i++) b.w[i] = 0xFFFFFFFFu;
     return b;
 }
-__device__ __forceinline__ Bits bits_and(const Bits &a, const Bits &b) {
-    Bits r;
+template <int V>
+__device__ __forceinline__ WBits<V> bits_and(const WBits<V> &a, const WBits<V> &b) {
+    WBits<V> r;
 #pragma unroll
-    for (int i = 0; i < NW; i++) r.w[i] = a.w[i] & b.w[i];
+    for (int i = 0; i < 4 * V; i++) r.w[i] = a.w[i] & b.w[i];
     return r;
 }
-__device__ __forceinline__ Bits bits_or(const Bits &a, const Bits &b) {
-    Bits r;
+template <int V>
+__device__ __forceinline__ WBits<V> bits_or(const WBits<V> &a, const WBits<V> &b) {
+    WBits<V> r;
 #pragma unroll
-    for (int i = 0; i < NW; i++) r.w[i] = a.w[i] | b.w[i];
+    for (int i = 0; i < 4 * V; i++) r.w[i] = a.w[i] | b.w[i];
     return r;
 }
-__device__ __forceinline__ Bits bits_andnot(const Bits &a, const Bits &b) {   // a & ~b
-    Bits r;
+template <int V>
+__device__ __forceinline__ WBits<V> bits_andnot(const WBits<V> &a, const WBits<V> &b) {   // a & ~b
+    WBits<V> r;
 #pragma unroll
-    for (int i = 0; i < NW; i++) r.w[i] = a.w[i] & ~b.w[i];
+    for (int i = 0; i < 4 * V; i++) r.w[i] = a.w[i] & ~b.w[i];
     return r;
 }
-__device__ __forceinline__ bool bits_contains(const Bits &a, const Bits &m) {   // (a & m) == m
+template <int V>
+__device__ __forceinline__ bool bits_contains(const WBits<V> &a, const WBits<V> &m) {   // (a & m) == m
     uint32_t miss = 0;
 #pragma unroll
-    for (int i = 0; i < NW; i++) miss |= (~a.w[i]) & m.w[i];
+    for (int i = 0; i < 4 * V; i++) miss |= (~a.w[i]) & m.w[i];
     return miss == 0;
 }
-// logical shift right by 0 < s < 32
-__device__ __forceinline__ Bits bits_shr_small(const Bits &a, int s) {
-    Bits r;
+// logical shift right by 0 <= s < 32
+template <int V>
+__device__ __forceinline__ WBits<V> bits_shr_small(const WBits<V> &a, int s) {
+    WBits<V> r;
 #pragma unroll
-    for (int i = 0; i < NW; i++) r.w[i] = __funnelshift_r(a.w[i], i + 1 < NW ? a.w[i + 1] : 0u, s);
+    for (int i = 0; i < 4 * V; i++) r.w[i] = __funnelshift_r(a.w[i], i + 1 < 4 * V ? a.w[i + 1] : 0u, s);
     return r;
 }
-__device__ __forceinline__ Bits bits_shl1(const Bits &a) {
-    Bits r;
+template <int V>
+__device__ __forceinline__ WBits<V> bits_shl1(const WBits<V> &a) {
+    WBits<V> r;
 #pragma unroll
-    for (int i = 0; i < NW; i++) r.w[i] = __funnelshift_l(i > 0 ? a.w[i - 1] : 0u, a.w[i], 1);
+    for (int i = 0; i < 4 * V; i++) r.w[i] = __funnelshift_l(i > 0 ? a.w[i - 1] : 0u, a.w[i], 1);
     return r;
 }
-__device__ __forceinline__ int bits_popc(const Bits &a) {
+template <int V>
+__device__ __forceinline__ int bits_popc(const WBits<V> &a) {
     int c = 0;
 #pragma unroll
-    for (int i = 0; i < NW; i++) c += __popc(a.w[i]);
+    for (int i = 0; i < 4 * V; i++) c += __popc(a.w[i]);
     return c;
 }
 // index of the lowest set bit, or -1
-__device__ __forceinline__ int bits_ffs(const Bits &a) {
+template <int V>
+__device__ __forceinline__ int bits_ffs(const WBits<V> &a) {
     int r = -1;
 #pragma unroll
-    for (int i = NW - 1; i >= 0; i--)
+    for (int i = 4 * V - 1; i >= 0; i--)
         if (a.w[i]) r = 32 * i + __ffs(a.w[i]) - 1;
     return r;
 }
 // index of the highest set bit, or -1
-__device__ __forceinline__ int bits_fls(const Bits &a) {
+template <int V>
+__device__ __forceinline__ int bits_fls(const WBits<V> &a) {
     int r = -1;
 #pragma unroll
-    for (int i = 0; i < NW; i++)
+    for (int i = 0; i < 4 * V; i++)
         if (a.w[i]) r = 32 * i + 31 - __clz(a.w[i]);
     return r;
 }
-__device__ __forceinline__ Bits bits_clear_lowest(const Bits &a) {
-    Bits r = a;
+template <int V>
+__device__ __forceinline__ WBits<V> bits_clear_lowest(const WBits<V> &a) {
+    WBits<V> r = a;
     bool done = false;
 #pragma unroll
-    for (int i = 0; i < NW; i++) {
+    for (int i = 0; i < 4 * V; i++) {
         if (!done && r.w[i]) { r.w[i] &= r.w[i] - 1; done = true; }
     }
     return r;
 }
-// bits [lo, hi) set, 0 <= lo <= hi <= 128
-__device__ __forceinline__ Bits bits_range(int lo, int hi) {
-    Bits r;
+// bits [lo, hi) set, 0 <= lo <= hi <= 128 * V
+template <int V = 1>
+__device__ __forceinline__ WBits<V> bits_range(int lo, int hi) {
+    WBits<V> r;
 #pragma unroll
-    for (int i = 0; i < NW; i++) {
+    for (int i = 0; i < 4 * V; i++) {
         int a = min(max(lo - 32 * i, 0), 32), b = min(max(hi - 32 * i, 0), 32);
         uint32_t ma = a >= 32 ? 0u : (0xFFFFFFFFu << a);     // bits >= a
         uint32_t mb = b >= 32 ? 0xFFFFFFFFu : ~(0xFFFFFFFFu << b);   // bits < b
@@ -111,29 +127,96 @@ __device__ __forceinline__ Bits bits_range(int lo, int hi) {
     }
     return r;
 }
-// B[i] = 1 iff A[i .. i+n-1] are all 1 (n >= 1): shift-AND doubling
-__device__ __forceinline__ Bits bits_runs_ge(const Bits &a, int n) {
-    Bits b = a;
+// B[i] = 1 iff A[i .. i+n-1] are all 1 (n >= 1): shift-AND doubling, shifts kept below 32
+template <int V>
+__device__ __forceinline__ WBits<V> bits_runs_ge(const WBits<V> &a, int n) {
+    WBits<V> b = a;
     int len = 1;
     while (len < n) {
-        int s = min(len, n - len);
-        if (s >= 32) {            // only reachable for n > 32 (never with the reference's bit rates)
-            for (int q = 0; q < s; q++) b = bits_and(b, bits_shr_small(b, 1));
-        } else {
-            b = bits_and(b, bits_shr_small(b, s));
-        }
+        const int s = min(min(len, n - len), 31);
+        const WBits<V> sh = bits_shr_small(b, s);
+#pragma unroll
+        for (int i = 0; i < 4 * V; i++) b.w[i] &= sh.w[i];
         len += s;
     }
     return b;
 }
-// length of the run of ones starting at bit `start` (A[start] must be 1; bit 128 counts as 0)
-__device__ __forceinline__ int bits_run_length(const Bits &a, int start) {
-    Bits z;
-    Bits below = bits_range(0, start);
+// length of the run of ones starting at bit `start` (A[start] must be 1; bit 128 * V counts as 0)
+template <int V>
+__device__ __forceinline__ int bits_run_length(const WBits<V> &a, int start) {
+    const WBits<V> from = bits_range<V>(start, 128 * V);
+    WBits<V> z;
 #pragma unroll
-    for (int i = 0; i < NW; i++) z.w[i] = ~a.w[i] & ~below.w[i];
-    int pos = bits_ffs(z);
-    return (pos < 0 ? MAX_SLOTS : pos) - start;
+    for (int i = 0; i < 4 * V; i++) z.w[i] = ~a.w[i] & from.w[i];
+    const int pos = bits_ffs(z);
+    return (pos < 0 ? 128 * V : pos) - start;
+}
+// the longest run of ones: one pass over the words, ctz / clz at every run boundary (no shift-AND pass per slot)
+template <int V>
+__device__ __forceinline__ int bits_longest_run(const WBits<V> &a) {
+    int best = 0, cur = 0;                             // cur: the run that reaches the top of the words seen so far
+#pragma unroll
+    for (int i = 0; i < 4 * V; i++) {
+        const uint32_t x = a.w[i];
+        if (x == 0xFFFFFFFFu) { cur += 32; continue; }
+        best = max(best, cur + __ffs(~x) - 1);         // the run coming from below ends at the lowest 0 of x
+        const int top = __clz(~x);                     // ones reaching bit 31 start the next carried run
+        uint32_t y = (x & (x + 1u)) & (0xFFFFFFFFu >> top);   // the runs strictly inside x (bit 0 of y is 0)
+        while (y) {
+            const int s = __ffs(y) - 1, len = __ffs(~(y >> s)) - 1;      // s >= 1, so len <= 31
+            best = max(best, len);
+            y &= ~(((1u << len) - 1u) << s);
+        }
+        cur = top;
+    }
+    return max(best, cur);
+}
+
+// 128-bit variants of the fast DeepRMSA and rollout kernels, each compiling to different code on purpose:
+// bits_runs_ge with the four shift amounts of n packed one per byte (table built by the host: orlg_api.cu): no loop control
+__device__ __forceinline__ Bits bits_runs_ge_sched(const Bits &a, unsigned sched) {
+    Bits b = a;
+#pragma unroll
+    for (int it = 0; it < 4; it++) {
+        b = bits_and(b, bits_shr_small(b, (int)((sched >> (8 * it)) & 0xffu)));
+    }
+    return b;
+}
+// bits_runs_ge without any branch; valid for 1 <= n <= 16 (the caller takes bits_runs_ge otherwise)
+__device__ __forceinline__ Bits bits_runs_ge_flat(const Bits &a, int n) {
+    Bits b = a;
+    int len = 1;
+#pragma unroll
+    for (int it = 0; it < 4; it++) {
+        int s = max(min(len, n - len), 0);
+        Bits sh = bits_shr_small(b, s);       // s == 0: funnel shift by 0 returns b
+        b = bits_and(b, sh);
+        len += s;
+    }
+    return b;
+}
+// bits [start, start + n) for 1 <= n <= 32, 0 <= start, start + n <= 128: one 64-bit shift placed at word start / 32
+__device__ __forceinline__ Bits bits_range_short(int start, int n) {
+    const unsigned long long m = ((1ULL << n) - 1ULL) << (start & 31);
+    const unsigned lo = (unsigned)m, hi = (unsigned)(m >> 32);
+    const int ws = start >> 5;
+    Bits r;
+#pragma unroll
+    for (int i = 0; i < NW; i++) r.w[i] = (i == ws) ? lo : ((i == ws + 1) ? hi : 0u);
+    return r;
+}
+// bits [start, start + n): bits_range_short where it applies (the common case), else bits_range
+__device__ __forceinline__ Bits bits_range_auto(int start, int n) {
+    return (n <= 32) ? bits_range_short(start, n) : bits_range(start, start + n);
+}
+// bits_ffs as a select chain instead of 4 dependent branches
+__device__ __forceinline__ int bits_ffs_flat(const Bits &a) {
+    const int p0 = __ffs(a.w[0]), p1 = __ffs(a.w[1]), p2 = __ffs(a.w[2]), p3 = __ffs(a.w[3]);
+    int r = p3 ? p3 + 95 : -1;
+    r = p2 ? p2 + 63 : r;
+    r = p1 ? p1 + 31 : r;
+    r = p0 ? p0 - 1 : r;
+    return r;
 }
 
 // ---------------------------------------------------------------- Philox4x32-10 (counter-based traffic)

@@ -203,31 +203,42 @@ __device__ __forceinline__ void philox_request(const Params &p, const unsigned *
     }
 }
 
-// ---------------------------------------------------------------- row f1: float statistics (generic kernel only)
+// ---------------------------------------------------------------- row f1: float statistics
 // Per link, from the packed mask (identities checked against the reference, SURVEY.md section 8f):
 // used = ~free; used blocks = popc(used & ~(used << 1)); lambda_min = ffs(used), lambda_max = fls(used) + 1;
-// free runs inside [lambda_min, lambda_max) = popc(F & ~(F << 1)) with F = free restricted to the window.
+// free runs inside [lambda_min, lambda_max) = popc(free & ~(free << 1)) less the free runs at slot 0 and at slot S - 1: with
+// two or more used runs those are exactly the free runs outside the window.
 struct LinkShape {
     int free_cnt, used_runs, span, free_runs_in;
     int free_runs, longest_free;       // number of free runs and the longest one (external fragmentation)
     bool free_at_both_ends;            // slot 0 and slot S - 1 are free
 };
-__device__ __forceinline__ LinkShape link_shape(const Bits &fr, int S) {
+template <int V>
+__device__ __forceinline__ LinkShape link_shape(const WBits<V> &fr, int S) {
+    const WBits<V> valid = bits_range<V>(0, S), last = bits_range<V>(S - 1, S);
+    WBits<V> used;
+#pragma unroll
+    for (int i = 0; i < 4 * V; i++) used.w[i] = valid.w[i] & ~fr.w[i];
+    const WBits<V> ul = bits_shl1(used), fl = bits_shl1(fr);
     LinkShape r;
-    const Bits valid = bits_range(0, S);
-    const Bits used = bits_andnot(valid, fr);
+    int ur = 0, frn = 0;
+    uint32_t at_end = 0;
+#pragma unroll
+    for (int i = 0; i < 4 * V; i++) {
+        ur += __popc(used.w[i] & ~ul.w[i]);
+        frn += __popc(fr.w[i] & ~fl.w[i]);
+        at_end |= fr.w[i] & last.w[i];
+    }
+    const int f0 = fr.w[0] & 1u, f1 = at_end != 0;
     r.free_cnt = bits_popc(fr);
-    r.used_runs = bits_popc(bits_andnot(used, bits_shl1(used)));
+    r.used_runs = ur;
+    r.free_runs = frn;
+    r.longest_free = bits_longest_run(fr);
+    r.free_at_both_ends = f0 && f1;
     r.span = 0; r.free_runs_in = 0;
-    r.free_runs = bits_popc(bits_andnot(fr, bits_shl1(fr)));
-    r.longest_free = 0;
-    for (Bits x = fr; bits_popc(x) != 0; x = bits_and(x, bits_shl1(x))) r.longest_free++;      // statistics path only: not hot
-    r.free_at_both_ends = bits_popc(bits_and(fr, bits_range(0, 1))) != 0 && bits_popc(bits_and(fr, bits_range(S - 1, S))) != 0;
-    if (r.used_runs > 1) {
-        const int lo = bits_ffs(used), hi = bits_fls(used) + 1;
-        r.span = hi - lo;
-        const Bits F = bits_and(fr, bits_range(lo, hi));
-        r.free_runs_in = bits_popc(bits_andnot(F, bits_shl1(F)));
+    if (ur > 1) {
+        r.span = bits_fls(used) + 1 - bits_ffs(used);
+        r.free_runs_in = frn - f0 - f1;
     }
     return r;
 }
@@ -748,96 +759,6 @@ __global__ void __launch_bounds__(STEP_THREADS) step_kernel(const Params p, cons
         p.ev_tail[env] = tailmin;
         p.errors[env] = err;
         if (mode == MODE_STEP && io.done) io.done[env] = done ? 1 : 0;
-    }
-}
-
-// ---------------------------------------------------------------- heuristic action sources
-// Thread per env; reads the masks of the candidate paths only.  NB the reference's first-fit loops
-// run over range(0, S - n): the last feasible start S - n is never tried (SURVEY.md App. B-5).
-template <int KIND>
-__global__ void heuristic_kernel(const Params p, const int which, int *actions) {
-    const int env = blockIdx.x * blockDim.x + threadIdx.x;
-    if (env >= p.n) return;
-    uint2 rq = p.cur_req[env];
-    const int src = rq.x & 0xff, dst = (rq.x >> 8) & 0xff, br = (int)(rq.x >> 16);
-    const int pair = src * p.N + dst;
-    const int first = p.pair_first[pair];
-    const int npaths = min((int)p.pair_count[pair], p.k);
-    if (KIND == ORLG_DEEPRMSA) {
-        // deeprmsa_env.py:135-155 on the cached block starts
-        int a = p.k * p.J;
-        if (which == ORLG_HEUR_SP_FF) {
-            a = (!p.allow_rejection || p.cand[(size_t)env * p.cand_stride] != CAND_NONE) ? 0 : p.k * p.J;
-        } else {
-            for (int q = 0; q < npaths; q++)
-                if (p.cand[(size_t)env * p.cand_stride + q * p.J] != CAND_NONE) { a = q * p.J; break; }
-        }
-        actions[env] = a;
-    } else if (KIND == ORLG_RMSA) {
-        // rmsa_env.py:747-803
-        int ap = p.k, as = p.S, max_free = 0;
-        const int np_ = (which == ORLG_HEUR_SP_FF) ? min(npaths, 1) : npaths;
-        for (int q = 0; q < np_; q++) {
-            unsigned meta = p.path_meta[first + q];
-            int n = p.nslots[meta_se(meta) * (p.br_max + 1) + br];
-            Bits A = path_free(p, env, p.path_linkmask[first + q], 0);
-            Bits B = bits_and(bits_runs_ge(A, n), bits_range(0, max(p.S - n, 0)));
-            int s = bits_ffs(B);
-            if (s >= 0) {
-                if (which == ORLG_HEUR_LLP_FF) {
-                    int fr = bits_popc(A);
-                    if (fr > max_free) { ap = q; as = s; max_free = fr; }
-                } else { ap = q; as = s; break; }
-            }
-        }
-        actions[2 * env] = ap; actions[2 * env + 1] = as;
-    } else if (KIND == ORLG_RWA) {
-        // rwa_env.py:425-502
-        int ap = p.k, as = p.S;
-        if (which == ORLG_HEUR_SP_FF) {
-            if (npaths > 0) {
-                int s = bits_ffs(path_free(p, env, p.path_linkmask[first], 0));
-                if (s >= 0) { ap = 0; as = s; }
-            }
-        } else if (which == ORLG_HEUR_SAP_FF || which == ORLG_HEUR_SAP_LF) {
-            int best_hops = 0x7fffffff;
-            for (int q = 0; q < npaths; q++) {
-                int hops = meta_hops(p.path_meta[first + q]);
-                if (hops < best_hops) {
-                    Bits A = path_free(p, env, p.path_linkmask[first + q], 0);
-                    int s;
-                    if (which == ORLG_HEUR_SAP_FF) s = bits_ffs(A);
-                    else { A.w[0] &= ~1u; s = bits_fls(A); }      // range(W-1, 0, -1): wavelength 0 is never tried
-                    if (s >= 0) { best_hops = hops; ap = q; as = s; }
-                }
-            }
-        } else {
-            int best = -1;
-            for (int q = 0; q < npaths; q++) {
-                Bits A = path_free(p, env, p.path_linkmask[first + q], 0);
-                int cap = bits_popc(A);
-                if (cap > best) {
-                    int s = bits_ffs(A);
-                    if (s >= 0) { best = cap; ap = q; as = s; }
-                }
-            }
-        }
-        actions[2 * env] = ap; actions[2 * env + 1] = as;
-    } else {
-        // rmcsa_env.py:882-911 (reject = 4-tuple (k, M, C, S))
-        int a0 = p.k, a1 = p.M, a2 = p.C, a3 = p.S;
-        bool found = false;
-        for (int q = 0; q < npaths && !found; q++) {
-            int mod = meta_mod(p.path_meta[first + q]);
-            int n = p.nslots[p.mod_se[mod] * (p.br_max + 1) + br];
-            Bits lim = bits_range(0, max(p.S - n, 0));
-            for (int c = 0; c < p.C && !found; c++) {
-                Bits B = bits_and(bits_runs_ge(path_free(p, env, p.path_linkmask[first + q], c), n), lim);
-                int s = bits_ffs(B);
-                if (s >= 0) { a0 = q; a1 = mod; a2 = c; a3 = s; found = true; }
-            }
-        }
-        actions[4 * env] = a0; actions[4 * env + 1] = a1; actions[4 * env + 2] = a2; actions[4 * env + 3] = a3;
     }
 }
 

@@ -749,7 +749,7 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
                     const int n = s_nslots[s_path_se[row] * 128 + br];
                     const Bits B = bits_runs_ge_sched(A, s_dbl[n]);
                     st = bits_ffs_flat(B);
-                    const int fe = bits_ffs_flat(bits_andnot(B, bits_shr1(B)));
+                    const int fe = bits_ffs_flat(bits_andnot(B, bits_shr_small(B, 1)));
                     const int total = bits_popc(A);
                     const int runs = bits_popc(bits_andnot(A, bits_shl1(A)));
                     f = feat_pack(st, fe - st + n, total, runs, n);

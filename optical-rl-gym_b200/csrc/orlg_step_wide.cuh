@@ -7,120 +7,18 @@
 //     masks[(env * C * E + core * E + link) * wstride + v]   (uint4; env-major: an entry's words share one DRAM burst,
 //     an env's entries one page -- every thread walks its OWN path, so the [link][env] layout of the NSFNET-class kernels
 //     would put each of its accesses on a different 2 MB page)
+// The hop lists and wide_path_free read both mask layouts (mask_index), so the heuristic kernel here serves every handle.
 #pragma once
 #include "orlg_kernels.cuh"
 
 namespace orlg {
-
-template <int NWV>
-struct WBits {
-    uint32_t w[4 * NWV];
-};
-
-template <int NWV>
-__device__ __forceinline__ WBits<NWV> wb_fill(uint32_t v) {
-    WBits<NWV> b;
-#pragma unroll
-    for (int i = 0; i < 4 * NWV; i++) b.w[i] = v;
-    return b;
-}
-// bits [lo, hi) set
-template <int NWV>
-__device__ __forceinline__ WBits<NWV> wb_range(int lo, int hi) {
-    WBits<NWV> r;
-#pragma unroll
-    for (int i = 0; i < 4 * NWV; i++) {
-        int a = min(max(lo - 32 * i, 0), 32), b = min(max(hi - 32 * i, 0), 32);
-        uint32_t ma = a >= 32 ? 0u : (0xFFFFFFFFu << a);
-        uint32_t mb = b >= 32 ? 0xFFFFFFFFu : ~(0xFFFFFFFFu << b);
-        r.w[i] = ma & mb;
-    }
-    return r;
-}
-template <int NWV>
-__device__ __forceinline__ bool wb_contains(const WBits<NWV> &a, const WBits<NWV> &m) {
-    uint32_t miss = 0;
-#pragma unroll
-    for (int i = 0; i < 4 * NWV; i++) miss |= (~a.w[i]) & m.w[i];
-    return miss == 0;
-}
-template <int NWV>
-__device__ __forceinline__ int wb_popc(const WBits<NWV> &a) {
-    int c = 0;
-#pragma unroll
-    for (int i = 0; i < 4 * NWV; i++) c += __popc(a.w[i]);
-    return c;
-}
-template <int NWV>
-__device__ __forceinline__ int wb_ffs(const WBits<NWV> &a) {
-    int r = -1;
-#pragma unroll
-    for (int i = 4 * NWV - 1; i >= 0; i--)
-        if (a.w[i]) r = 32 * i + __ffs(a.w[i]) - 1;
-    return r;
-}
-template <int NWV>
-__device__ __forceinline__ int wb_fls(const WBits<NWV> &a) {
-    int r = -1;
-#pragma unroll
-    for (int i = 0; i < 4 * NWV; i++)
-        if (a.w[i]) r = 32 * i + 31 - __clz(a.w[i]);
-    return r;
-}
-template <int NWV>
-__device__ __forceinline__ WBits<NWV> wb_shr_small(const WBits<NWV> &a, int s) {     // 0 <= s < 32
-    WBits<NWV> r;
-#pragma unroll
-    for (int i = 0; i < 4 * NWV; i++) r.w[i] = __funnelshift_r(a.w[i], i + 1 < 4 * NWV ? a.w[i + 1] : 0u, s);
-    return r;
-}
-template <int NWV>
-__device__ __forceinline__ WBits<NWV> wb_shl1(const WBits<NWV> &a) {
-    WBits<NWV> r;
-#pragma unroll
-    for (int i = 0; i < 4 * NWV; i++) r.w[i] = __funnelshift_l(i > 0 ? a.w[i - 1] : 0u, a.w[i], 1);
-    return r;
-}
-// B[i] = 1 iff A[i .. i+n-1] are all 1 (shift-AND doubling, shifts kept below 32)
-template <int NWV>
-__device__ __forceinline__ WBits<NWV> wb_runs_ge(const WBits<NWV> &a, int n) {
-    WBits<NWV> b = a;
-    int len = 1;
-    while (len < n) {
-        const int s = min(min(len, n - len), 31);
-        const WBits<NWV> sh = wb_shr_small(b, s);
-#pragma unroll
-        for (int i = 0; i < 4 * NWV; i++) b.w[i] &= sh.w[i];
-        len += s;
-    }
-    return b;
-}
-template <int NWV>
-__device__ __forceinline__ WBits<NWV> wb_clear_lowest(const WBits<NWV> &a) {
-    WBits<NWV> r = a;
-    bool done = false;
-#pragma unroll
-    for (int i = 0; i < 4 * NWV; i++)
-        if (!done && r.w[i]) { r.w[i] &= r.w[i] - 1; done = true; }
-    return r;
-}
-// length of the run of ones starting at bit `start`
-template <int NWV>
-__device__ __forceinline__ int wb_run_length(const WBits<NWV> &a, int start) {
-    const WBits<NWV> from = wb_range<NWV>(start, 128 * NWV);
-    WBits<NWV> z;
-#pragma unroll
-    for (int i = 0; i < 4 * NWV; i++) z.w[i] = ~a.w[i] & from.w[i];
-    const int pos = wb_ffs(z);
-    return (pos < 0 ? 128 * NWV : pos) - start;
-}
 
 // get_available_slots (rmsa_env.py:638-649): AND of the path's link masks.  Four hops at a time: the four link indices are
 // fetched together, then all 4 x NWV mask words are requested before any is used (2 dependent round trips per 4 hops instead
 // of 2 per hop: the kernel is latency-bound, every lane walks its own path).
 template <int NWV>
 __device__ __forceinline__ WBits<NWV> wide_path_free(const Params &p, int env, int row, int core) {
-    WBits<NWV> a = wb_fill<NWV>(0xFFFFFFFFu);
+    WBits<NWV> a = bits_ones<NWV>();
     const int h0 = p.path_link_ptr[row], h1 = p.path_link_ptr[row + 1];
     const size_t vs = p.wstride ? 1 : (size_t)p.n;          // distance between the word groups of one entry (mask_index)
     const uint4 ones = make_uint4(0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu);
@@ -176,59 +74,6 @@ __device__ __forceinline__ void wide_path_update(const Params &p, int env, int r
 __device__ __forceinline__ int wide_nslots(const Params &p, int se, int br) { return p.nslots[se * (p.br_max + 1) + br]; }
 
 // ---------------------------------------------------------------- row f1 (float statistics) on the wide layout
-// longest run of ones: one pass over the words, ctz / clz at every run boundary (no shift-AND pass per slot)
-template <int NWV>
-__device__ __forceinline__ int wb_longest_run(const WBits<NWV> &a) {
-    int best = 0, cur = 0;                             // cur: the run that reaches the top of the words seen so far
-#pragma unroll
-    for (int i = 0; i < 4 * NWV; i++) {
-        const uint32_t x = a.w[i];
-        if (x == 0xFFFFFFFFu) { cur += 32; continue; }
-        best = max(best, cur + __ffs(~x) - 1);         // the run coming from below ends at the lowest 0 of x
-        const int top = __clz(~x);                     // ones reaching bit 31 start the next carried run
-        uint32_t y = (x & (x + 1u)) & (0xFFFFFFFFu >> top);   // the runs strictly inside x (bit 0 of y is 0)
-        while (y) {
-            const int s = __ffs(y) - 1, len = __ffs(~(y >> s)) - 1;      // s >= 1, so len <= 31
-            best = max(best, len);
-            y &= ~(((1u << len) - 1u) << s);
-        }
-        cur = top;
-    }
-    return max(best, cur);
-}
-
-// link_shape (orlg_kernels.cuh) of a multi-word mask: the same integers.  With two or more used runs the free runs outside
-// [ffs(used), fls(used) + 1) are exactly the one at slot 0 and the one at slot S - 1 (when those slots are free).
-template <int NWV>
-__device__ __forceinline__ LinkShape wb_link_shape(const WBits<NWV> &fr, int S) {
-    const WBits<NWV> valid = wb_range<NWV>(0, S), last = wb_range<NWV>(S - 1, S);
-    WBits<NWV> used;
-#pragma unroll
-    for (int i = 0; i < 4 * NWV; i++) used.w[i] = valid.w[i] & ~fr.w[i];
-    const WBits<NWV> ul = wb_shl1(used), fl = wb_shl1(fr);
-    LinkShape r;
-    int ur = 0, frn = 0;
-    uint32_t at_end = 0;
-#pragma unroll
-    for (int i = 0; i < 4 * NWV; i++) {
-        ur += __popc(used.w[i] & ~ul.w[i]);
-        frn += __popc(fr.w[i] & ~fl.w[i]);
-        at_end |= fr.w[i] & last.w[i];
-    }
-    const int f0 = fr.w[0] & 1u, f1 = at_end != 0;
-    r.free_cnt = wb_popc(fr);
-    r.used_runs = ur;
-    r.free_runs = frn;
-    r.longest_free = wb_longest_run(fr);
-    r.free_at_both_ends = f0 && f1;
-    r.span = 0; r.free_runs_in = 0;
-    if (ur > 1) {
-        r.span = wb_fls(used) + 1 - wb_ffs(used);
-        r.free_runs_in = frn - f0 - f1;
-    }
-    return r;
-}
-
 __device__ __forceinline__ int wide_hops(const Params &p, int row) { return p.path_link_ptr[row + 1] - p.path_link_ptr[row]; }
 
 // The integer terms of _get_network_compactness (rmsa_env.py:699-744), kept current so that the compactness needs no pass over
@@ -250,7 +95,7 @@ __device__ __forceinline__ double wide_compactness(const Params &p, int env, int
 // (span, free runs inside it) are refreshed from the same shape and the core's sums adjusted by the difference.
 template <int KIND, int NWV>
 __device__ __forceinline__ void wide_path_update_stats(const Params &p, int env, int row, int core, int start, int n, bool set, double now) {
-    const WBits<NWV> rm = wb_range<NWV>(start, start + n);
+    const WBits<NWV> rm = bits_range<NWV>(start, start + n);
     const size_t vs = p.wstride ? 1 : (size_t)p.n;
     int d_occ = 0, d_unused = 0;
     for (int h = p.path_link_ptr[row]; h < p.path_link_ptr[row + 1]; h++) {
@@ -268,9 +113,9 @@ __device__ __forceinline__ void wide_path_update_stats(const Params &p, int env,
         for (int v = 0; v < NWV; v++) m[v * vs] = make_uint4(b.w[4 * v], b.w[4 * v + 1], b.w[4 * v + 2], b.w[4 * v + 3]);
         LinkShape s{};
         if (KIND == ORLG_RWA) {
-            s.free_cnt = wb_popc(b);                   // rwa_env.py:365-383: utilisation only
+            s.free_cnt = bits_popc(b);                   // rwa_env.py:365-383: utilisation only
         } else {
-            s = wb_link_shape(b, p.S);
+            s = link_shape(b, p.S);
             unsigned *t = nc_links(p) + ((size_t)env * p.C + core) * p.E + l;
             const unsigned old = *t;
             d_occ += s.span - (int)(old & 0xFFFFu);
@@ -287,7 +132,15 @@ __device__ __forceinline__ void wide_path_update_stats(const Params &p, int env,
     }
 }
 
-// heuristic action sources (SURVEY a21) for the wide layout: the action of env's pending request (src, dst, br) into a[0..3]
+// DeepRMSA's cached block start i of env's pending request exists: 16-bit entries on wide handles, 8-bit otherwise
+__device__ __forceinline__ bool cand_found(const Params &p, int env, int i) {
+    const size_t at = (size_t)env * p.cand_stride + i;
+    return p.cand16 ? p.cand16[at] != 0xFFFFu : p.cand[at] != CAND_NONE;
+}
+
+// ---------------------------------------------------------------- heuristic action sources (SURVEY a21), every handle
+// The action of env's pending request (src, dst, br) into a[0..3], from the masks of its candidate paths only.  NB the
+// reference's first-fit loops run over range(0, S - n): the last feasible start S - n is never tried (SURVEY.md App. B-5).
 // Returns true when the action is KNOWN to fit (it was derived from the path's free mask just now), so that the fused step
 // does not have to read the masks a second time for is_path_free.
 template <int KIND, int NWV>
@@ -296,27 +149,29 @@ __device__ __forceinline__ bool wide_heuristic(const Params &p, const int env, c
     const int first = p.pair_first[pair];
     const int npaths = min((int)p.pair_count[pair], p.k);
     if (KIND == ORLG_DEEPRMSA) {
+        // deeprmsa_env.py:135-155 on the cached block starts
         int act = p.k * p.J;
-        if (which == ORLG_HEUR_SP_FF) act = (!p.allow_rejection || p.cand16[(size_t)env * p.cand_stride] != 0xFFFFu) ? 0 : p.k * p.J;
+        if (which == ORLG_HEUR_SP_FF) act = (!p.allow_rejection || cand_found(p, env, 0)) ? 0 : p.k * p.J;
         else
             for (int q = 0; q < npaths; q++)
-                if (p.cand16[(size_t)env * p.cand_stride + q * p.J] != 0xFFFFu) { act = q * p.J; break; }
+                if (cand_found(p, env, q * p.J)) { act = q * p.J; break; }
         a[0] = act;
         return false;
     } else if (KIND == ORLG_RMSA) {
+        // rmsa_env.py:747-803
         int ap = p.k, as = p.S, max_free = 0;
         const int np_ = (which == ORLG_HEUR_SP_FF) ? min(npaths, 1) : npaths;
         for (int q = 0; q < np_; q++) {
             const int n = wide_nslots(p, meta_se(p.path_meta[first + q]), br);
             const WBits<NWV> A = wide_path_free<NWV>(p, env, first + q, 0);
-            WBits<NWV> B = wb_runs_ge(A, n);
-            const WBits<NWV> lim = wb_range<NWV>(0, max(p.S - n, 0));          // range(0, S - n): App. B-5
+            WBits<NWV> B = bits_runs_ge(A, n);
+            const WBits<NWV> lim = bits_range<NWV>(0, max(p.S - n, 0));
 #pragma unroll
             for (int i = 0; i < 4 * NWV; i++) B.w[i] &= lim.w[i];
-            const int s = wb_ffs(B);
+            const int s = bits_ffs(B);
             if (s >= 0) {
                 if (which == ORLG_HEUR_LLP_FF) {
-                    const int fr = wb_popc(A);
+                    const int fr = bits_popc(A);
                     if (fr > max_free) { ap = q; as = s; max_free = fr; }
                 } else { ap = q; as = s; break; }
             }
@@ -324,21 +179,22 @@ __device__ __forceinline__ bool wide_heuristic(const Params &p, const int env, c
         a[0] = ap; a[1] = as;
         return ap < p.k;
     } else if (KIND == ORLG_RWA) {
+        // rwa_env.py:425-502
         int ap = p.k, as = p.S;
         if (which == ORLG_HEUR_SP_FF) {
             if (npaths > 0) {
-                const int s = wb_ffs(wide_path_free<NWV>(p, env, first, 0));
+                const int s = bits_ffs(wide_path_free<NWV>(p, env, first, 0));
                 if (s >= 0) { ap = 0; as = s; }
             }
         } else if (which == ORLG_HEUR_SAP_FF || which == ORLG_HEUR_SAP_LF) {
             int best_hops = 0x7fffffff;
             for (int q = 0; q < npaths; q++) {
-                const int hops = p.path_link_ptr[first + q + 1] - p.path_link_ptr[first + q];
+                const int hops = wide_hops(p, first + q);        // = the table's hop count (orlg_create checks them)
                 if (hops < best_hops) {
                     WBits<NWV> A = wide_path_free<NWV>(p, env, first + q, 0);
                     int s;
-                    if (which == ORLG_HEUR_SAP_FF) s = wb_ffs(A);
-                    else { A.w[0] &= ~1u; s = wb_fls(A); }
+                    if (which == ORLG_HEUR_SAP_FF) s = bits_ffs(A);
+                    else { A.w[0] &= ~1u; s = bits_fls(A); }      // range(W-1, 0, -1): wavelength 0 is never tried
                     if (s >= 0) { best_hops = hops; ap = q; as = s; }
                 }
             }
@@ -346,9 +202,9 @@ __device__ __forceinline__ bool wide_heuristic(const Params &p, const int env, c
             int best = -1;
             for (int q = 0; q < npaths; q++) {
                 const WBits<NWV> A = wide_path_free<NWV>(p, env, first + q, 0);
-                const int cap = wb_popc(A);
+                const int cap = bits_popc(A);
                 if (cap > best) {
-                    const int s = wb_ffs(A);
+                    const int s = bits_ffs(A);
                     if (s >= 0) { best = cap; ap = q; as = s; }
                 }
             }
@@ -356,17 +212,18 @@ __device__ __forceinline__ bool wide_heuristic(const Params &p, const int env, c
         a[0] = ap; a[1] = as;
         return ap < p.k;
     } else {
+        // rmcsa_env.py:882-911 (reject = 4-tuple (k, M, C, S))
         int a0 = p.k, a1 = p.M, a2 = p.C, a3 = p.S;
         bool found = false;
         for (int q = 0; q < npaths && !found; q++) {
             const int mod = meta_mod(p.path_meta[first + q]);
             const int n = wide_nslots(p, p.mod_se[mod], br);
-            const WBits<NWV> lim = wb_range<NWV>(0, max(p.S - n, 0));
+            const WBits<NWV> lim = bits_range<NWV>(0, max(p.S - n, 0));
             for (int c = 0; c < p.C && !found; c++) {
-                WBits<NWV> B = wb_runs_ge(wide_path_free<NWV>(p, env, first + q, c), n);
+                WBits<NWV> B = bits_runs_ge(wide_path_free<NWV>(p, env, first + q, c), n);
 #pragma unroll
                 for (int i = 0; i < 4 * NWV; i++) B.w[i] &= lim.w[i];
-                const int s = wb_ffs(B);
+                const int s = bits_ffs(B);
                 if (s >= 0) { a0 = q; a1 = mod; a2 = c; a3 = s; found = true; }
             }
         }
@@ -375,8 +232,9 @@ __device__ __forceinline__ bool wide_heuristic(const Params &p, const int env, c
     }
 }
 
+// thread per env; NSFNET-class handles take NWV = 1
 template <int KIND, int NWV>
-__global__ void heuristic_wide_kernel(const Params p, const int which, int *actions) {
+__global__ void heuristic_kernel(const Params p, const int which, int *actions) {
     const int env = blockIdx.x * blockDim.x + threadIdx.x;
     if (env >= p.n) return;
     const uint2 rq = p.cur_req[env];
@@ -422,7 +280,7 @@ __global__ void __launch_bounds__(ORLG_WIDE_THREADS, STATS ? ORLG_WIDE_STATS_MIN
     bool accepted = false, done = false;
 
     if (mode == MODE_FULL_RESET) {
-        const WBits<NWV> full = wb_range<NWV>(0, p.S);
+        const WBits<NWV> full = bits_range<NWV>(0, p.S);
         for (int l = 0; l < p.C * p.E; l++)
 #pragma unroll
             for (int v = 0; v < NWV; v++)
@@ -475,7 +333,7 @@ __global__ void __launch_bounds__(ORLG_WIDE_THREADS, STATS ? ORLG_WIDE_STATS_MIN
                     n = (KIND == ORLG_RWA) ? 1 : wide_nslots(p, meta_se(p.path_meta[row]), br);
                     start = slot;
                     if (known_free) accepted = true;
-                    else if (start + n <= p.S) accepted = wb_contains(wide_path_free<NWV>(p, env, row, 0), wb_range<NWV>(start, start + n));
+                    else if (start + n <= p.S) accepted = bits_contains(wide_path_free<NWV>(p, env, row, 0), bits_range<NWV>(start, start + n));
                 } else err |= ORLG_ERR_NO_SUCH_PATH;
             }
         } else {
@@ -486,7 +344,7 @@ __global__ void __launch_bounds__(ORLG_WIDE_THREADS, STATS ? ORLG_WIDE_STATS_MIN
                     n = wide_nslots(p, p.mod_se[am], br);
                     start = slot; core = ac; mod = am;
                     if (start + n <= p.S)
-                        accepted = (known_free || wb_contains(wide_path_free<NWV>(p, env, row, core), wb_range<NWV>(start, start + n))) &&
+                        accepted = (known_free || bits_contains(wide_path_free<NWV>(p, env, row, core), bits_range<NWV>(start, start + n))) &&
                                    (p.path_length[row] < p.reach[am * (p.br_max + 1) + br]);
                 } else err |= ORLG_ERR_NO_SUCH_PATH;
             }
@@ -644,20 +502,20 @@ __global__ void __launch_bounds__(ORLG_WIDE_THREADS, STATS ? ORLG_WIDE_STATS_MIN
             const int row = first + q;
             const int n = wide_nslots(p, meta_se(p.path_meta[row]), br);
             const WBits<NWV> A = wide_path_free<NWV>(p, env, row, 0);
-            const WBits<NWV> B = wb_runs_ge(A, n);
-            const WBits<NWV> Bl = wb_shl1(B), Al = wb_shl1(A);
+            const WBits<NWV> B = bits_runs_ge(A, n);
+            const WBits<NWV> Bl = bits_shl1(B), Al = bits_shl1(A);
             WBits<NWV> starts, arun;
 #pragma unroll
             for (int i = 0; i < 4 * NWV; i++) { starts.w[i] = B.w[i] & ~Bl.w[i]; arun.w[i] = A.w[i] & ~Al.w[i]; }
-            const int total = wb_popc(A), runs = wb_popc(arun);
+            const int total = bits_popc(A), runs = bits_popc(arun);
             const int ob = head + q * W;
             for (int b = 0; b < p.J; b++) {
-                const int st = wb_ffs(starts);
+                const int st = bits_ffs(starts);
                 p.cand16[(size_t)env * p.cand_stride + q * p.J + b] = (unsigned short)(st < 0 ? 0xFFFF : st);
                 int len = -1;
                 if (st >= 0) {
-                    starts = wb_clear_lowest(starts);
-                    len = wb_run_length(A, st);
+                    starts = bits_clear_lowest(starts);
+                    len = bits_run_length(A, st);
                     if (io.obs) {
                         if (p.obs_f64) {
                             o64[ob + 2 * b] = __ddiv_rn(__dmul_rn(2.0, __dadd_rn((double)st, -__dmul_rn(0.5, (double)p.S))), (double)p.S);

@@ -24,14 +24,14 @@ __global__ void path_only_first_fit_kernel(const Params p, const int *path_actio
             const WBits<NWV> A = wide_path_free<NWV>(p, env, row, 0);
             int s;
             if (p.kind == ORLG_RWA) {
-                s = wb_ffs(A);
+                s = bits_ffs(A);
             } else {
                 const int n = wide_nslots(p, meta_se(p.path_meta[row]), br);
-                WBits<NWV> B = wb_runs_ge(A, n);
-                const WBits<NWV> lim = wb_range<NWV>(0, max(p.S - n, 0));
+                WBits<NWV> B = bits_runs_ge(A, n);
+                const WBits<NWV> lim = bits_range<NWV>(0, max(p.S - n, 0));
 #pragma unroll
                 for (int i = 0; i < 4 * NWV; i++) B.w[i] &= lim.w[i];
-                s = wb_ffs(B);
+                s = bits_ffs(B);
             }
             if (s >= 0) { ap = a; as = s; }
         }
