@@ -258,6 +258,30 @@ int orlg_rollout_policy_info(orlg_env *env, int steps, orlg_policy *actor, orlg_
  * makes at its next step.  Host state, no device access. */
 int64_t orlg_request_index(const orlg_env *env);
 
+/* ---- invalid-action masks (DeepRMSA-v0), as sb3-contrib's MaskablePPO uses them ------------------------------------ */
+/* A = k * j + allow_rejection (= action_space.n) for DeepRMSA-v0, 0 for the other kinds (their MultiDiscrete spaces have no
+ * joint mask that per-dimension masks could express). */
+int orlg_action_mask_dim(const orlg_env *env);
+/* env.action_masks() of every env's pending request: mask_dev uint8 [num_envs, A], 1 = valid.  Action p * j + b is valid iff
+ * path p is a candidate of the request's pair and its block b exists, i.e. exactly when env.step(p * j + b) provisions
+ * (deeprmsa_env.py:48-58); the reject action k * j is valid when allow_rejection.  A row may be all zeros.  Any DeepRMSA-v0
+ * handle; other kinds are ORLG_E_UNSUPPORTED. */
+int orlg_action_masks(orlg_env *env, uint8_t *mask_dev, orlg_stream stream);
+/* orlg_policy_sample from the masked distribution of MaskableCategorical: logits l_a = -1e8 where mask_dev[row, a] == 0
+ * (mask_dev uint8 [n, n_actions], required), then the same draw; the rounding fallback is the last action with e_a > 0, so a
+ * masked action is never returned while the row has a valid one.  An all-zero row is the uniform distribution (action 0 when
+ * deterministic); an all-ones row gives exactly orlg_policy_sample's results. */
+int orlg_policy_sample_masked(orlg_policy *pol, const float *obs_dev, int n, const orlg_policy_draw *draw, const uint8_t *mask_dev,
+                              int32_t *actions_dev, float *log_prob_dev, float *value_dev, orlg_stream stream);
+/* orlg_rollout_policy_info with the actions drawn under the invalid-action masks: per step orlg_action_masks, the masked actor
+ * launch, the (unmasked) critic launch, the step.  masks_dev uint8 [steps, N, A], required when steps > 0: row t is the mask of obs[t]'s
+ * request, the mask step t's action was drawn under (what MaskablePPO keeps in its rollout buffer).  The refusals of
+ * orlg_rollout_policy_info, and the actor's n_actions must be A. */
+int orlg_rollout_policy_masked(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
+                               float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
+                               float *reward_dev, uint8_t *done_dev, uint8_t *masks_dev, const orlg_info_out *info,
+                               orlg_stream stream);
+
 /* Float statistics of `info` (rmsa_env.py:229-264, 439-543, 699-744; RMSA-v0 / DeepRMSA-v0, any topology the handle
  * takes: any link count, up to 512 slots): after this call every orlg_step also writes, per env, float64
  *   stats_dev[env][0..3] = network_compactness, network_compactness_difference,

@@ -332,6 +332,17 @@ int launch_step(const orlg_env *env, const StepIO &io, int mode, cudaStream_t s)
     return ORLG_OK;
 }
 
+// DeepRMSA-v0's invalid-action masks of the pending requests, uint8 [n, k * j + rej], as a programmatic dependent launch that
+// waits in every thread (action_mask_kernel): it may sit between a step kernel and the policy kernel that reads the step's
+// observation
+int launch_action_masks(const orlg_env *env, uint8_t *mask_dev, cudaStream_t s) {
+    const int threads = 128;
+    cudaLaunchConfig_t cfg = pdl_config((env->p.n + threads - 1) / threads, threads, 0, s);
+    unsigned char *mask = mask_dev;
+    CUDA_OK(cudaLaunchKernelEx(&cfg, action_mask_kernel, env->p, mask));
+    return ORLG_OK;
+}
+
 // envs per warp of the rollout kernel: a batch that would leave most SMs with one or two warps is spread over more warps
 // with fewer lanes in use (less divergence per warp, more warps to hide latency).  Chosen by orlg_create (ORLG_RO_LPW = 8 or
 // 32 overrides it for the handles created while it is set) and fixed per handle: the event slabs follow it.
@@ -852,6 +863,20 @@ int orlg_heuristic(orlg_env *env, int which, int32_t *actions_dev, orlg_stream s
     return ORLG_OK;
 }
 
+int orlg_action_mask_dim(const orlg_env *env) {
+    return env && env->p.kind == ORLG_DEEPRMSA ? env->p.k * env->p.J + env->p.allow_rejection : 0;
+}
+
+int orlg_action_masks(orlg_env *env, uint8_t *mask_dev, orlg_stream stream) {
+    if (!env) return fail(ORLG_E_INVALID, "null handle");
+    if (env->p.kind != ORLG_DEEPRMSA)
+        return fail(ORLG_E_UNSUPPORTED, "action masks exist for DeepRMSA-v0 (a Discrete action space); a MultiDiscrete space has no "
+                                        "joint mask that per-dimension masks could express");
+    if (!mask_dev) return fail(ORLG_E_INVALID, "null mask buffer");
+    DeviceGuard guard(env->device);
+    return launch_action_masks(env, mask_dev, (cudaStream_t)stream);
+}
+
 int orlg_random_actions(orlg_env *env, int32_t *actions_dev, orlg_stream stream) {
     if (!env || !actions_dev) return fail(ORLG_E_INVALID, "null handle or buffer");
     DeviceGuard guard(env->device);
@@ -1366,10 +1391,10 @@ struct orlg_policy {
 
 // The one place that picks the kernel instance of a handle: the shipped agent's 5 x 128 has one compiled for it, every other
 // architecture runs the instance that reads H and L from PolicyParams.
-template <bool SAMPLE>
+template <bool SAMPLE, bool MASKED = false>
 static decltype(&mlp_policy_kernel<SAMPLE, 0, 0>) policy_kernel(const orlg_policy *pol) {
-    if (pol->pp.H == 128 && pol->pp.L == 5 && !pol->general) return mlp_policy_kernel<SAMPLE, 128, 5>;
-    return mlp_policy_kernel<SAMPLE, 0, 0>;
+    if (pol->pp.H == 128 && pol->pp.L == 5 && !pol->general) return mlp_policy_kernel<SAMPLE, 128, 5, MASKED>;
+    return mlp_policy_kernel<SAMPLE, 0, 0, MASKED>;
 }
 
 extern "C" {
@@ -1433,15 +1458,12 @@ int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers,
     pol->pp.H = H; pol->pp.L = L;
     pol->smem = smem;
     // the attribute only raises a kernel's limit: a larger policy made earlier on this device keeps its launches valid
-    int have_act = 0, have_sample = 0;
-    cudaFuncAttributes fa;
-    if (cudaFuncGetAttributes(&fa, policy_kernel<false>(pol.get())) == cudaSuccess) have_act = fa.maxDynamicSharedSizeBytes;
-    if (cudaFuncGetAttributes(&fa, policy_kernel<true>(pol.get())) == cudaSuccess) have_sample = fa.maxDynamicSharedSizeBytes;
-    if ((have_act < (int)smem &&
-         cudaFuncSetAttribute(policy_kernel<false>(pol.get()), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) ||
-        (have_sample < (int)smem &&
-         cudaFuncSetAttribute(policy_kernel<true>(pol.get()), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess))
-        return fail(ORLG_E_CUDA, "cudaFuncSetAttribute(policy kernel shared memory) failed");
+    for (auto kernel : {policy_kernel<false>(pol.get()), policy_kernel<true>(pol.get()), policy_kernel<true, true>(pol.get())}) {
+        cudaFuncAttributes fa;
+        const int have = cudaFuncGetAttributes(&fa, kernel) == cudaSuccess ? fa.maxDynamicSharedSizeBytes : 0;
+        if (have < (int)smem && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+            return fail(ORLG_E_CUDA, "cudaFuncSetAttribute(policy kernel shared memory) failed");
+    }
     *out = pol.release();
     return ORLG_OK;
 }
@@ -1449,7 +1471,7 @@ int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers,
 }  // extern "C"
 
 // one launch of the fused policy kernel over n rows: a persistent CTA per SM (each walks PL_GROUPS tile streams)
-template <bool SAMPLE>
+template <bool SAMPLE, bool MASKED = false>
 static int launch_policy(const orlg_policy *pol, const float *obs_dev, int n, int32_t *actions_dev, float *logits_dev,
                          const PolicyDraw &dr, cudaStream_t s) {
     int sms = 148;
@@ -1457,7 +1479,7 @@ static int launch_policy(const orlg_policy *pol, const float *obs_dev, int n, in
     const int pairs = ((n + PL_TILE - 1) / PL_TILE + PL_GROUPS - 1) / PL_GROUPS;
     cudaLaunchConfig_t cfg = pdl_config(pairs < sms ? pairs : sms, PL_WG * PL_GROUPS, pol->smem, s);
     int *actions = actions_dev;
-    CUDA_OK(cudaLaunchKernelEx(&cfg, policy_kernel<SAMPLE>(pol), pol->pp, obs_dev, n, actions, logits_dev, dr));
+    CUDA_OK(cudaLaunchKernelEx(&cfg, policy_kernel<SAMPLE, MASKED>(pol), pol->pp, obs_dev, n, actions, logits_dev, dr));
     return ORLG_OK;
 }
 
@@ -1493,16 +1515,23 @@ int orlg_policy_sample(orlg_policy *pol, const float *obs_dev, int n, const orlg
     return launch_policy<true>(pol, obs_dev, n, actions_dev, nullptr, policy_draw(*draw, log_prob_dev, value_dev), (cudaStream_t)stream);
 }
 
-int orlg_rollout_policy(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
-                        float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
-                        float *reward_dev, uint8_t *done_dev, orlg_stream stream) {
-    return orlg_rollout_policy_info(env, steps, actor, critic, seed, deterministic, obs_dev, actions_dev, log_prob_dev, value_dev,
-                                    reward_dev, done_dev, nullptr, stream);
+int orlg_policy_sample_masked(orlg_policy *pol, const float *obs_dev, int n, const orlg_policy_draw *draw, const uint8_t *mask_dev,
+                              int32_t *actions_dev, float *log_prob_dev, float *value_dev, orlg_stream stream) {
+    if (!pol || !obs_dev || !draw || n < 0) return fail(ORLG_E_INVALID, "null policy, observation buffer or draw");
+    if (!mask_dev) return fail(ORLG_E_INVALID, "orlg_policy_sample_masked needs mask_dev (uint8 [n, n_actions])");
+    if (n == 0) return ORLG_OK;
+    DeviceGuard guard(pol->device);
+    PolicyDraw dr = policy_draw(*draw, log_prob_dev, value_dev);
+    dr.mask = mask_dev;
+    return launch_policy<true, true>(pol, obs_dev, n, actions_dev, nullptr, dr, (cudaStream_t)stream);
 }
 
-int orlg_rollout_policy_info(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
-                             float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
-                             float *reward_dev, uint8_t *done_dev, const orlg_info_out *info, orlg_stream stream) {
+}  // extern "C"
+
+// orlg_rollout_policy_info (masked = false) and orlg_rollout_policy_masked: the one loop of both
+static int rollout_policy_impl(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
+                               float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev, float *reward_dev,
+                               uint8_t *done_dev, bool masked, uint8_t *masks_dev, const orlg_info_out *info, orlg_stream stream) {
     if (!env || !actor) return fail(ORLG_E_INVALID, "null env or actor handle");
     const Params &p = env->p;
     if (p.kind != ORLG_DEEPRMSA) return fail(ORLG_E_UNSUPPORTED, "orlg_rollout_policy drives DeepRMSA-v0 (the env kind with a tensor observation)");
@@ -1518,6 +1547,7 @@ int orlg_rollout_policy_info(orlg_env *env, int steps, orlg_policy *actor, orlg_
         return fail(ORLG_E_INVALID, "policy and env handles live on different devices");
     if (!obs_dev) return fail(ORLG_E_INVALID, "orlg_rollout_policy needs obs_dev (the policy reads it)");
     if (steps < 0) return fail(ORLG_E_INVALID, "steps must be >= 0");
+    if (masked && steps > 0 && !masks_dev) return fail(ORLG_E_INVALID, "orlg_rollout_policy_masked needs masks_dev (uint8 [steps, N, A])");
     if (p.traffic == ORLG_TRAFFIC_TRACE && p.trace == nullptr) return fail(ORLG_E_INVALID, "trace traffic selected but orlg_set_trace was not called");
     if (const char *why = info_refusal(p, info)) return fail(ORLG_E_UNSUPPORTED, why);
     DeviceGuard guard(env->device);
@@ -1536,8 +1566,14 @@ int orlg_rollout_policy_info(orlg_env *env, int steps, orlg_policy *actor, orlg_
         const float *o = obs_dev + (size_t)t * row;
         int32_t *a = actions_dev ? actions_dev + (size_t)t * n : env->ro_actions;
         float *v = value_dev ? value_dev + (size_t)t * n : nullptr;
-        rc = launch_policy<true>(actor, o, p.n, a, nullptr, policy_draw(d, log_prob_dev ? log_prob_dev + (size_t)t * n : nullptr,
-                                                                       critic ? nullptr : v), s);
+        PolicyDraw dr = policy_draw(d, log_prob_dev ? log_prob_dev + (size_t)t * n : nullptr, critic ? nullptr : v);
+        if (masked) {
+            dr.mask = masks_dev + (size_t)t * n * n_act;
+            rc = launch_action_masks(env, masks_dev + (size_t)t * n * n_act, s);
+            if (!rc) rc = launch_policy<true, true>(actor, o, p.n, a, nullptr, dr, s);
+        } else {
+            rc = launch_policy<true>(actor, o, p.n, a, nullptr, dr, s);
+        }
         if (!rc && critic && v) rc = launch_policy<true>(critic, o, p.n, nullptr, nullptr, policy_draw(d, nullptr, v), s);
         if (!rc) rc = step_impl(env, a, -1, nullptr, obs_dev + (size_t)(t + 1) * row, reward_dev ? reward_dev + (size_t)t * n : nullptr,
                                 done_dev ? done_dev + (size_t)t * n : nullptr, nullptr,
@@ -1549,6 +1585,29 @@ int orlg_rollout_policy_info(orlg_env *env, int steps, orlg_policy *actor, orlg_
         rc = launch_policy<true>(critic ? critic : actor, obs_dev + (size_t)steps * row, p.n, nullptr, nullptr,
                                  policy_draw(d, nullptr, value_dev + (size_t)steps * n), s);
     return rc;
+}
+
+extern "C" {
+
+int orlg_rollout_policy(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
+                        float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
+                        float *reward_dev, uint8_t *done_dev, orlg_stream stream) {
+    return orlg_rollout_policy_info(env, steps, actor, critic, seed, deterministic, obs_dev, actions_dev, log_prob_dev, value_dev,
+                                    reward_dev, done_dev, nullptr, stream);
+}
+
+int orlg_rollout_policy_info(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
+                             float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
+                             float *reward_dev, uint8_t *done_dev, const orlg_info_out *info, orlg_stream stream) {
+    return rollout_policy_impl(env, steps, actor, critic, seed, deterministic, obs_dev, actions_dev, log_prob_dev, value_dev,
+                               reward_dev, done_dev, false, nullptr, info, stream);
+}
+
+int orlg_rollout_policy_masked(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
+                               float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
+                               float *reward_dev, uint8_t *done_dev, uint8_t *masks_dev, const orlg_info_out *info, orlg_stream stream) {
+    return rollout_policy_impl(env, steps, actor, critic, seed, deterministic, obs_dev, actions_dev, log_prob_dev, value_dev,
+                               reward_dev, done_dev, true, masks_dev, info, stream);
 }
 
 int64_t orlg_request_index(const orlg_env *env) { return env ? (int64_t)env->p.lockstep_ridx : -1; }

@@ -12,7 +12,8 @@
 // B = the layer's weights, D = fp32 accumulators in TMEM; the warps then read their 32 TMEM lanes back with
 // tcgen05.ld, add the bias, apply tanh and write the next layer's A operand.  Nothing but the observation rows and
 // the actions touches HBM.  A second instance (mlp_policy_kernel<true>) ends in a sampling epilogue: the action drawn from
-// softmax(logits) with Philox stream 3, its log-probability and the value (PPO's rollout collection, orlg_policy_sample).
+// softmax(logits) with Philox stream 3, its log-probability and the value (PPO's rollout collection, orlg_policy_sample), and
+// its MASKED variant draws under an invalid-action mask (orlg_policy_sample_masked).
 #pragma once
 #include <cuda_bf16.h>
 #include "orlg_deeprmsa_fast.cuh"
@@ -51,6 +52,7 @@ struct PolicyDraw {
     long long row_id_base;
     float *log_prob;                  // [n] log softmax(logits)[action]
     float *value;                     // [n] the value head
+    const unsigned char *mask;        // [n, n_actions] invalid-action mask, 0 = invalid (read by the MASKED instances only)
 };
 
 // Shared-memory operand layout (no swizzle): 8 x 8 bf16 core matrices of 128 contiguous bytes (row r of the core matrix at
@@ -127,14 +129,28 @@ __device__ __forceinline__ void pl_tmem_ld16(unsigned taddr, float (&v)[16]) {
 // l_a = acc_a + bias_a, m = max l, e_a = expf(l_a - m), S = e_0 + ... in index order; the action is the argmax (deterministic)
 // or the smallest a with u S < e_0 + ... + e_a for u = (Philox word 0 >> 8) 2^-24 (the last action if rounding leaves none);
 // log_prob = l_a - m - logf(S).  expf / logf, not the intrinsics: 15 values per row.
+// MASKED (sb3-contrib's MaskableCategorical): l_a = -1e8 where the row's mask byte is 0, before all of the above, and the
+// rounding fallback is the last action with e_a > 0, so a masked action is never drawn while any action is valid.  An all-zero
+// row gives the uniform distribution (action 0 when deterministic).  The unmasked instances compile as before: every MASKED
+// statement is a constant-false branch there.
+template <bool MASKED>
 __device__ __forceinline__ void pl_sample_epilogue(const PolicyParams &pp, const PolicyDraw &dr, const float (&v)[16], const float *b,
                                                    int env, int *actions) {
     constexpr int NA = PL_NOUT - 1;
     const int na = pp.n_actions;
+    unsigned valid = 0;               // bit a = action a is valid
+    if (MASKED) {
+        const unsigned char *mrow = dr.mask + (size_t)env * na;
+#pragma unroll
+        for (int a = 0; a < NA; a++)
+            if (a < na && mrow[a]) valid |= 1u << a;
+    }
     float l[NA], m = v[0] + b[0];
+    if (MASKED && !(valid & 1u)) m = -1e8f;
 #pragma unroll
     for (int a = 0; a < NA; a++) {
         l[a] = v[a] + b[a];
+        if (MASKED && !((valid >> a) & 1u)) l[a] = -1e8f;
         if (a < na && l[a] > m) m = l[a];
     }
     float value = 0.0f;
@@ -162,6 +178,12 @@ __device__ __forceinline__ void pl_sample_epilogue(const PolicyParams &pp, const
         float acc = 0.0f;
         bool found = false;
         pick = na - 1;
+        if (MASKED) {
+            pick = 0;
+#pragma unroll
+            for (int a = 0; a < NA; a++)
+                if (a < na && e[a] > 0.0f) pick = a;
+        }
 #pragma unroll
         for (int a = 0; a < NA; a++) {
             if (a < na) {
@@ -191,8 +213,9 @@ __device__ __forceinline__ void pl_group_sync(int group) {          // named bar
 
 // SAMPLE = false: orlg_policy_act (argmax, optional logits; `dr` unused).  SAMPLE = true: orlg_policy_sample (the epilogue
 // of PolicyDraw; `actions` may be NULL, `logits_out` is unused).  HC, LC: the hidden width and depth fixed at compile time
-// (they must equal pp.H, pp.L), or 0: read from pp at run time.
-template <bool SAMPLE, int HC, int LC>
+// (they must equal pp.H, pp.L), or 0: read from pp at run time.  MASKED (with SAMPLE only): the epilogue draws under the
+// invalid-action mask dr.mask (orlg_policy_sample_masked); a template flag, so that the unmasked instances keep their code.
+template <bool SAMPLE, int HC, int LC, bool MASKED = false>
 __global__ void __launch_bounds__(PL_WG * PL_GROUPS, 1)
 mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const int n, int *__restrict__ actions,
                   float *__restrict__ logits_out /* [n, n_actions + 1] = logits + value, or NULL */, const PolicyDraw dr) {
@@ -353,7 +376,7 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
                     float v[16];
                     pl_tmem_ld16(t_lane, v);
                     if (SAMPLE) {
-                        if (env < n) pl_sample_epilogue(pp, dr, v, b, env, actions);
+                        if (env < n) pl_sample_epilogue<MASKED>(pp, dr, v, b, env, actions);
                     } else if (env < n) {
                         int best = 0;
                         float bv = v[0] + b[0];

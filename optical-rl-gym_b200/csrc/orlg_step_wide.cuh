@@ -245,6 +245,24 @@ __global__ void heuristic_kernel(const Params p, const int which, int *actions) 
     for (int i = 0; i < AD; i++) actions[AD * env + i] = a[i];
 }
 
+// DeepRMSA-v0 invalid-action mask of env's pending request, thread per env: row [k * j + rej] of uint8, action q * j + b valid
+// iff path q is a candidate of the pair and its block b exists (exactly when env.step(q * j + b) provisions, deeprmsa_env.py:48-58),
+// the reject action always valid.  Any DeepRMSA handle: every step kernel and the persistent rollout kernel keep the block cache.
+// Launched with programmatic dependent launch, and every thread waits before it reads or exits: the policy kernel that follows
+// waits on this grid only, then reads the observation the step kernel before it wrote.
+__global__ void action_mask_kernel(const Params p, unsigned char *mask) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const int env = blockIdx.x * blockDim.x + threadIdx.x;
+    if (env >= p.n) return;
+    const unsigned rq = p.cur_req[env].x;
+    const int npaths = min((int)p.pair_count[(rq & 0xff) * p.N + ((rq >> 8) & 0xff)], p.k);
+    const int kj = p.k * p.J;
+    unsigned char *row = mask + (size_t)env * (kj + p.allow_rejection);
+    for (int i = 0; i < kj; i++) row[i] = i < npaths * p.J && cand_found(p, env, i) ? 1 : 0;
+    if (p.allow_rejection) row[kj] = 1;
+}
+
 // Launch shape, A/B-ed on the B200 (profiles/r2_experiments.md): 64-thread CTAs, 8 per SM (128 registers per thread, 16 warps per
 // SM); 128 x 3, 128 x 4 and 64 x 6 are within 3 % of it -- the kernel is bound by its dependent loads, not by occupancy.
 #ifndef ORLG_WIDE_THREADS

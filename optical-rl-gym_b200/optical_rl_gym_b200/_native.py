@@ -118,6 +118,10 @@ def lib():
     L.orlg_policy_sample.argtypes = [vp, vp, i32, C.POINTER(PolicyDraw), vp, vp, vp, vp]
     L.orlg_rollout_policy.argtypes = [vp, i32, vp, vp, C.c_uint64, i32, vp, vp, vp, vp, vp, vp, vp]
     L.orlg_rollout_policy_info.argtypes = [vp, i32, vp, vp, C.c_uint64, i32, vp, vp, vp, vp, vp, vp, C.POINTER(InfoOut), vp]
+    L.orlg_action_mask_dim.argtypes = [vp]
+    L.orlg_action_masks.argtypes = [vp, vp, vp]
+    L.orlg_policy_sample_masked.argtypes = [vp, vp, i32, C.POINTER(PolicyDraw), vp, vp, vp, vp, vp]
+    L.orlg_rollout_policy_masked.argtypes = [vp, i32, vp, vp, C.c_uint64, i32, vp, vp, vp, vp, vp, vp, vp, C.POINTER(InfoOut), vp]
     L.orlg_request_index.argtypes = [vp]
     L.orlg_request_index.restype = i64
     L.orlg_rollout_packed.argtypes = [vp, i32, i32, vp, vp, vp]
@@ -139,4 +143,5 @@ EXPORTED = ["orlg_create", "orlg_destroy", "orlg_last_error", "orlg_version", "o
             "orlg_num_bit_rates", "orlg_bit_rate_blocking", "orlg_matrix_obs_dim", "orlg_matrix_observation",
             "orlg_path_only_first_fit", "orlg_rollout", "orlg_state_save_bytes", "orlg_state_save", "orlg_state_load", "orlg_policy_create", "orlg_policy_act", "orlg_policy_destroy", "orlg_rollout_packed", "orlg_expand_packed", "orlg_rollout_host", "orlg_action_hist_dim", "orlg_action_probability",
             "orlg_enable_link_stats", "orlg_link_stats", "orlg_policy_sample", "orlg_rollout_policy", "orlg_request_index",
-            "orlg_rollout_info", "orlg_rollout_policy_info"]
+            "orlg_rollout_info", "orlg_rollout_policy_info", "orlg_action_mask_dim", "orlg_action_masks",
+            "orlg_policy_sample_masked", "orlg_rollout_policy_masked"]

@@ -128,13 +128,18 @@ class VecMonitor(VecWrapper):
         return res if want or not with_info else res[:4]
 
     def rollout_policy(self, agent, steps, **kw):
-        """:meth:`OpticalVecEnv.rollout_policy` that logs the episodes it finishes like the equivalent ``step`` loop."""
+        """:meth:`OpticalVecEnv.rollout_policy` that logs the episodes it finishes like the equivalent ``step`` loop; returns
+        what the env returns (``action_masks=True`` appends the masks, the info only comes with ``want_info=True``)."""
         want = kw.pop("want_info", False)
         with_info = want or bool(self.info_keywords)
         res = self._base("rollout_policy").rollout_policy(agent, steps, want_info=with_info, **kw)
-        out, info = res if with_info else (res, None)
+        parts = list(res) if with_info or kw.get("action_masks", False) else [res]     # [PolicyRollout, StepInfo?, masks?]
+        out, info = parts[0], (parts[1] if with_info else None)
         self._record_rollout(out.reward, out.done, info)
-        return res if want or not with_info else out
+        if want or not with_info:
+            return res
+        rest = parts[2:]                  # the masks, after the info this call added for its own rows
+        return (out, *rest) if rest else out
 
     def get_episode_rewards(self):
         return self.episode_returns

@@ -226,12 +226,14 @@ class MlpPolicy(torch.nn.Module):
 
     @torch.no_grad()
     def sample_native(self, obs: torch.Tensor, *, seed: int, counter: int, row_id_base: int = 0, deterministic: bool = False,
-                      out=None):
+                      out=None, action_masks: torch.Tensor = None):
         """What PPO collects per observation, from the fused kernel: ``(actions int32 [N, 1], log_prob f32 [N], value f32 [N])``.
         Sampled actions come from softmax(logits) with one Philox4x32-10 draw per row (key ``seed``, counter
         ``(counter, 0, row_id_base + row, 3)``); ``deterministic=True`` gives the argmax of :meth:`act_native`.  ``log_prob`` is
         log softmax(logits)[action]; ``value`` is the critic's (``critic_net``) when the policy has a separate one.
-        ``out`` = the three tensors to fill."""
+        ``out`` = the three tensors to fill.  ``action_masks`` (a contiguous bool or uint8 CUDA tensor ``[N, n_actions]``, 0 =
+        invalid, e.g. ``OpticalVecEnv.action_masks()``) draws from the masked distribution of sb3-contrib's ``MaskablePPO``
+        (``orlg_policy_sample_masked``): ``deterministic=True`` with it is the masked ``predict``."""
         import ctypes as C
 
         from . import _native as nat
@@ -244,13 +246,20 @@ class MlpPolicy(torch.nn.Module):
         self._check_out("actions", actions, (n, 1), torch.int32, obs.device)
         self._check_out("log_prob", log_prob, (n,), torch.float32, obs.device)
         self._check_out("value", value, (n,), torch.float32, obs.device)
+        mask_dtype = torch.uint8 if action_masks is not None and action_masks.dtype == torch.uint8 else torch.bool
+        self._check_out("action_masks", action_masks, (n, self.action_net.out_features), mask_dtype, obs.device)
         actor, critic = self._native_handles(obs.device.index)
         stream = C.c_void_p(torch.cuda.current_stream(obs.device).cuda_stream)
         draw = nat.PolicyDraw(seed=int(seed) & (2 ** 64 - 1), counter_dev=None, counter=int(counter) & 0xFFFFFFFF,
                               deterministic=int(bool(deterministic)), row_id_base=int(row_id_base))
         L, o = nat.lib(), C.c_void_p(obs.data_ptr())
-        nat.check(L.orlg_policy_sample(actor, o, n, C.byref(draw), C.c_void_p(actions.data_ptr()), C.c_void_p(log_prob.data_ptr()),
-                                       None if critic is not None else C.c_void_p(value.data_ptr()), stream))
+        own_value = None if critic is not None else C.c_void_p(value.data_ptr())
+        if action_masks is None:
+            nat.check(L.orlg_policy_sample(actor, o, n, C.byref(draw), C.c_void_p(actions.data_ptr()),
+                                           C.c_void_p(log_prob.data_ptr()), own_value, stream))
+        else:
+            nat.check(L.orlg_policy_sample_masked(actor, o, n, C.byref(draw), C.c_void_p(action_masks.data_ptr()),
+                                                  C.c_void_p(actions.data_ptr()), C.c_void_p(log_prob.data_ptr()), own_value, stream))
         if critic is not None:
             nat.check(L.orlg_policy_sample(critic, o, n, C.byref(draw), None, None, C.c_void_p(value.data_ptr()), stream))
         return actions, log_prob, value

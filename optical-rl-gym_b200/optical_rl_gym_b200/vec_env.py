@@ -421,7 +421,7 @@ class OpticalVecEnv:
         return obs, reward, done, actions
 
     def rollout_policy(self, policy, steps: int, *, deterministic: bool = False, seed: Optional[int] = None,
-                       out: Optional[PolicyRollout] = None, want_info: bool = False):
+                       out: Optional[PolicyRollout] = None, want_info: bool = False, action_masks: bool = False):
         """``steps`` iterations of ``a, log p(a), V(obs) = policy(obs); obs, r, done = env.step(a)`` in ONE native call
         (``orlg_rollout_policy``): a :class:`PolicyRollout` of device tensors, what SB3's ``collect_rollouts`` gathers.
         ``policy`` is an :class:`~optical_rl_gym_b200.policy.MlpPolicy` on this device (its current weights; the value comes
@@ -429,7 +429,11 @@ class OpticalVecEnv:
         Philox stream 3 keyed by ``seed`` (default: the env's seed), the global env id and the env's request index, so the
         result does not depend on the number of GPUs, on how the rollout is split into calls or on a checkpoint in between.
         ``out`` reuses the buffers of an earlier call.  DeepRMSA-v0 with float32 observations.  ``want_info=True`` (needs
-        ``collect_info=True``) returns ``(PolicyRollout, StepInfo)``, the latter every step's ``info`` with ``[T, N]`` values."""
+        ``collect_info=True``) returns ``(PolicyRollout, StepInfo)``, the latter every step's ``info`` with ``[T, N]`` values.
+        ``action_masks=True`` draws every action from the masked distribution of sb3-contrib's ``MaskablePPO`` and appends
+        the masks they were drawn under, ``torch.bool [T, N, A]`` (row t = :meth:`action_masks` of ``obs[t]``'s request):
+        ``(PolicyRollout, masks)``, or ``(PolicyRollout, StepInfo, masks)`` with ``want_info=True``
+        (``orlg_rollout_policy_masked``)."""
         T, n, dev = int(steps), self.num_envs, self.device
         if T < 0:
             raise ValueError("steps must be >= 0")
@@ -450,6 +454,12 @@ class OpticalVecEnv:
         actor, critic = policy._native_handles(self._dev_index)
         key = self.rand_seed if seed is None else int(seed)
         with torch.cuda.device(self._dev_index):
+            if action_masks:
+                masks = torch.empty((T, n, self._lib.orlg_action_mask_dim(self._h)), dtype=torch.bool, device=dev)
+                nat.check(self._lib.orlg_rollout_policy_masked(self._h, T, actor, critic, key & (2 ** 64 - 1), int(bool(deterministic)),
+                                                               *[_ptr(t) for t in out], _ptr(masks),
+                                                               C.byref(info_out) if want_info else None, self._stream()))
+                return (out, info, masks) if want_info else (out, masks)
             if want_info:
                 nat.check(self._lib.orlg_rollout_policy_info(self._h, T, actor, critic, key & (2 ** 64 - 1), int(bool(deterministic)),
                                                              *[_ptr(t) for t in out], C.byref(info_out), self._stream()))
@@ -463,6 +473,22 @@ class OpticalVecEnv:
         """Requests drawn so far by every env (they step together): counter word 0 of the action draws of the next
         :meth:`rollout_policy` step, for a Python loop that wants the same keying (``MlpPolicy.sample_native(counter=...)``)."""
         return int(self._lib.orlg_request_index(self._h))
+
+    def action_masks(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The invalid-action mask of every env's pending request, ``torch.bool [N, A]`` on the device (``A`` =
+        ``action_space.n``), the method sb3-contrib's ``MaskablePPO`` calls: action ``p * j + b`` is valid iff path ``p`` is a
+        candidate of the request's pair and its block ``b`` exists, i.e. exactly when ``step`` provisions it; the reject
+        action is always valid.  DeepRMSA-v0 only (``NativeError`` for the other kinds).  ``out``: a bool or uint8 tensor
+        ``[N, A]`` to fill."""
+        A = self._lib.orlg_action_mask_dim(self._h)
+        if out is None:
+            out = torch.empty((self.num_envs, A), dtype=torch.bool, device=self.device)
+        elif (tuple(out.shape) != (self.num_envs, A) or out.dtype not in (torch.bool, torch.uint8) or out.device != self.device
+              or not out.is_contiguous()):
+            raise ValueError("out must be a contiguous bool or uint8 tensor %s on %s, got %s %s %s" % (
+                (self.num_envs, A), self.device, tuple(out.shape), out.dtype, out.device))
+        nat.check(self._lib.orlg_action_masks(self._h, _ptr(out), self._stream()))
+        return out
 
     def rollout_packed(self, steps: int, policy="random", out=None):
         """Like :meth:`rollout`, but ONE 32-byte record per env-step (int32 ``[T, N, 8]`` on the device): the integer
