@@ -216,6 +216,16 @@ int orlg_rollout_host(orlg_env *env, int steps, int policy, float *obs_host, flo
 typedef struct orlg_policy orlg_policy;
 int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers, int n_actions, const float *weights,
                        const float *biases, orlg_policy **out);
+/* The same policy for observations up to 256 wide (germany50's 126, a 100-node topology's 251), any parity: same weights and
+ * biases, same hidden rules, obs_dim 1..256, n_actions 1..15.  Layer 0 has K0 = obs_dim rounded up to 16 inputs and runs in
+ * chunks of 64.  Shared memory is hidden * K0 * 2 + (n_hidden_layers - 1) * hidden^2 * 2 + 16 * hidden * 2 + G * 32768 +
+ * (n_hidden_layers * hidden + 16) * 4 + 64 bytes with G = 2 tile groups per CTA when that fits in 232448, else G = 1, else
+ * ORLG_E_UNSUPPORTED (e.g. 5 x 128 at obs_dim 251).  Every call that takes an orlg_policy accepts the handle; at obs_dim <= 64
+ * its results equal those of an orlg_policy_create handle bit for bit. */
+int orlg_policy_create_wide(int device, int obs_dim, int hidden, int n_hidden_layers, int n_actions, const float *weights,
+                            const float *biases, orlg_policy **out);
+/* tile groups per CTA of the handle's launches: 2 (every orlg_policy_create handle), or 1; 0 for NULL */
+int orlg_policy_tile_groups(const orlg_policy *pol);
 /* actions_dev int32 [n]; logits_dev float32 [n, n_actions + 1] = logits then value (NULL: skip) */
 int orlg_policy_act(orlg_policy *pol, const float *obs_dev, int n, int32_t *actions_dev, float *logits_dev, orlg_stream stream);
 int orlg_policy_destroy(orlg_policy *pol);

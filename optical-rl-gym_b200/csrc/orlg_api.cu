@@ -1382,6 +1382,8 @@ struct orlg_policy {
     int device;
     size_t smem;
     bool general;                     // ORLG_POLICY_GENERAL at orlg_policy_create: the run-time (H, L) instance also for 5 x 128
+    bool wide = false;                // orlg_policy_create_wide: the WIDE instances (layer 0 in chunks of 64 inputs, up to 256)
+    int groups = PL_GROUPS;           // tile groups per CTA (PL_WG threads each): 2, or 1 for a wide handle whose weights leave room for one
     void *w_dev = nullptr, *b_dev = nullptr;
 
     ~orlg_policy() { cudaFree(w_dev); cudaFree(b_dev); }
@@ -1389,10 +1391,11 @@ struct orlg_policy {
 
 }  // extern "C"
 
-// The one place that picks the kernel instance of a handle: the shipped agent's 5 x 128 has one compiled for it, every other
-// architecture runs the instance that reads H and L from PolicyParams.
+// The one place that picks the kernel instance of a handle: a wide handle runs the WIDE instance, the shipped agent's 5 x 128
+// has one compiled for it, every other architecture runs the instance that reads H and L from PolicyParams.
 template <bool SAMPLE, bool MASKED = false>
 static decltype(&mlp_policy_kernel<SAMPLE, 0, 0>) policy_kernel(const orlg_policy *pol) {
+    if (pol->wide) return mlp_policy_kernel<SAMPLE, 0, 0, MASKED, true>;
     if (pol->pp.H == 128 && pol->pp.L == 5 && !pol->general) return mlp_policy_kernel<SAMPLE, 128, 5, MASKED>;
     return mlp_policy_kernel<SAMPLE, 0, 0, MASKED>;
 }
@@ -1406,36 +1409,23 @@ static unsigned short f32_to_bf16(float f) {          // round to nearest even
     return (unsigned short)((u + 0x7fffu + ((u >> 16) & 1u)) >> 16);
 }
 
-int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers, int n_actions, const float *weights,
-                       const float *biases, orlg_policy **out) {
-    if (!weights || !biases || !out) return fail(ORLG_E_INVALID, "null argument");
-    *out = nullptr;
-    if (obs_dim < 2 || obs_dim > PL_K0 || (obs_dim & 1) || n_actions < 1 || n_actions + 1 > PL_NOUT)
-        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel is built for obs_dim <= 64 (even), <= 15 actions; got obs_dim " +
-                                            std::to_string(obs_dim) + ", " + std::to_string(n_actions) + " actions");
-    if (hidden < 16 || hidden > PL_HMAX || hidden % 16)
-        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs a hidden width that is a multiple of 16 in 16..128; got " +
-                                            std::to_string(hidden));
-    if (n_hidden_layers < 1)
-        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs at least one hidden layer; got " + std::to_string(n_hidden_layers));
-    const int H = hidden, L = n_hidden_layers;
-    const size_t smem = pl_smem_bytes(H, L);
-    if (smem > (size_t)PL_SMEM_MAX)         // all weights stay resident in shared memory
-        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs " + std::to_string(smem) + " bytes of shared memory, " +
-                                            std::to_string(PL_SMEM_MAX) + " available, for " + std::to_string(L) +
-                                            " hidden layers of " + std::to_string(H));
+// the shape checks of both create calls have passed: pack and upload the weights, make the handle
+static int policy_build(int device, int obs_dim, int H, int L, int n_actions, const float *weights, const float *biases, bool wide,
+                        int groups, orlg_policy **out) {
     int n_dev = 0;
     if (cudaGetDeviceCount(&n_dev) != cudaSuccess || device < 0 || device >= n_dev) return fail(ORLG_E_CUDA, "no such CUDA device");
     DeviceGuard guard(device);
-    // bf16 weights in the shared-memory operand layout of the kernel: layer l is an [N x K] K-major operand, K = 64 (the
-    // padded observation) for layer 0, H after it
-    const size_t bytes = pl_weight_bytes(H, L);
+    // bf16 weights in the shared-memory operand layout of the kernel: layer l is an [N x K] K-major operand, K = K0 (the
+    // padded observation: 64, or obs_dim rounded up to 16 on a wide handle) for layer 0, H after it
+    const int K0 = wide ? (obs_dim + 15) & ~15 : PL_K0;
+    const size_t bytes = pl_weight_bytes(H, L, K0);
+    const size_t smem = pl_smem_bytes(H, L, K0, groups);
     std::vector<unsigned short> blob(bytes / 2, 0);
     std::vector<float> bias((size_t)L * H + PL_NOUT, 0.0f);
     const float *w = weights, *b = biases;
     size_t off = 0;
     for (int l = 0; l < L; l++) {
-        const int K = l == 0 ? obs_dim : H, Kp = l == 0 ? PL_K0 : H;
+        const int K = l == 0 ? obs_dim : H, Kp = l == 0 ? K0 : H;
         for (int r = 0; r < H; r++)
             for (int k = 0; k < K; k++) blob[(off + pl_operand_offset(H, r, k)) / 2] = f32_to_bf16(w[(size_t)r * K + k]);
         for (int r = 0; r < H; r++) bias[(size_t)l * H + r] = b[r];
@@ -1447,6 +1437,8 @@ int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers,
     std::unique_ptr<orlg_policy, int (*)(orlg_policy *)> pol(new orlg_policy(), orlg_policy_destroy);
     pol->device = device;
     pol->general = std::getenv("ORLG_POLICY_GENERAL") != nullptr;
+    pol->wide = wide;
+    pol->groups = groups;
     if (cudaMalloc(&pol->w_dev, bytes) != cudaSuccess || cudaMalloc(&pol->b_dev, bias.size() * 4) != cudaSuccess ||
         cudaMemcpy(pol->w_dev, blob.data(), bytes, cudaMemcpyHostToDevice) != cudaSuccess ||
         cudaMemcpy(pol->b_dev, bias.data(), bias.size() * 4, cudaMemcpyHostToDevice) != cudaSuccess)
@@ -1468,16 +1460,63 @@ int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers,
     return ORLG_OK;
 }
 
+int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers, int n_actions, const float *weights,
+                       const float *biases, orlg_policy **out) {
+    if (!weights || !biases || !out) return fail(ORLG_E_INVALID, "null argument");
+    *out = nullptr;
+    if (obs_dim < 2 || obs_dim > PL_K0 || (obs_dim & 1) || n_actions < 1 || n_actions + 1 > PL_NOUT)
+        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel is built for obs_dim <= 64 (even), <= 15 actions; got obs_dim " +
+                                            std::to_string(obs_dim) + ", " + std::to_string(n_actions) + " actions");
+    if (hidden < 16 || hidden > PL_HMAX || hidden % 16)
+        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs a hidden width that is a multiple of 16 in 16..128; got " +
+                                            std::to_string(hidden));
+    if (n_hidden_layers < 1)
+        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs at least one hidden layer; got " + std::to_string(n_hidden_layers));
+    const int H = hidden, L = n_hidden_layers;
+    const size_t smem = pl_smem_bytes(H, L);
+    if (smem > (size_t)PL_SMEM_MAX)         // all weights stay resident in shared memory
+        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs " + std::to_string(smem) + " bytes of shared memory, " +
+                                            std::to_string(PL_SMEM_MAX) + " available, for " + std::to_string(L) +
+                                            " hidden layers of " + std::to_string(H));
+    return policy_build(device, obs_dim, H, L, n_actions, weights, biases, false, PL_GROUPS, out);
+}
+
+int orlg_policy_create_wide(int device, int obs_dim, int hidden, int n_hidden_layers, int n_actions, const float *weights,
+                            const float *biases, orlg_policy **out) {
+    if (!weights || !biases || !out) return fail(ORLG_E_INVALID, "null argument");
+    *out = nullptr;
+    if (obs_dim < 1 || obs_dim > PL_K0_WIDE || n_actions < 1 || n_actions + 1 > PL_NOUT)
+        return fail(ORLG_E_UNSUPPORTED, "the wide fused policy kernel is built for obs_dim 1..256, <= 15 actions; got obs_dim " +
+                                            std::to_string(obs_dim) + ", " + std::to_string(n_actions) + " actions");
+    if (hidden < 16 || hidden > PL_HMAX || hidden % 16)
+        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs a hidden width that is a multiple of 16 in 16..128; got " +
+                                            std::to_string(hidden));
+    if (n_hidden_layers < 1)
+        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs at least one hidden layer; got " + std::to_string(n_hidden_layers));
+    const int H = hidden, L = n_hidden_layers, K0 = (obs_dim + 15) & ~15;
+    // two tile groups when their A buffers fit next to the weights, else one (half the threads, the same per-tile work)
+    const int groups = pl_smem_bytes(H, L, K0, 2) <= (size_t)PL_SMEM_MAX ? 2 : 1;
+    const size_t smem = pl_smem_bytes(H, L, K0, groups);
+    if (smem > (size_t)PL_SMEM_MAX)
+        return fail(ORLG_E_UNSUPPORTED, "the wide fused policy kernel needs " + std::to_string(smem) + " bytes of shared memory with " +
+                                            "one tile group, " + std::to_string(PL_SMEM_MAX) + " available, for obs_dim " +
+                                            std::to_string(obs_dim) + " (K0 " + std::to_string(K0) + ") and " + std::to_string(L) +
+                                            " hidden layers of " + std::to_string(H));
+    return policy_build(device, obs_dim, H, L, n_actions, weights, biases, true, groups, out);
+}
+
+int orlg_policy_tile_groups(const orlg_policy *pol) { return pol ? pol->groups : 0; }
+
 }  // extern "C"
 
-// one launch of the fused policy kernel over n rows: a persistent CTA per SM (each walks PL_GROUPS tile streams)
+// one launch of the fused policy kernel over n rows: a persistent CTA per SM (each walks pol->groups tile streams)
 template <bool SAMPLE, bool MASKED = false>
 static int launch_policy(const orlg_policy *pol, const float *obs_dev, int n, int32_t *actions_dev, float *logits_dev,
                          const PolicyDraw &dr, cudaStream_t s) {
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, pol->device);
-    const int pairs = ((n + PL_TILE - 1) / PL_TILE + PL_GROUPS - 1) / PL_GROUPS;
-    cudaLaunchConfig_t cfg = pdl_config(pairs < sms ? pairs : sms, PL_WG * PL_GROUPS, pol->smem, s);
+    const int pairs = ((n + PL_TILE - 1) / PL_TILE + pol->groups - 1) / pol->groups;
+    cudaLaunchConfig_t cfg = pdl_config(pairs < sms ? pairs : sms, PL_WG * pol->groups, pol->smem, s);
     int *actions = actions_dev;
     CUDA_OK(cudaLaunchKernelEx(&cfg, policy_kernel<SAMPLE, MASKED>(pol), pol->pp, obs_dev, n, actions, logits_dev, dr));
     return ORLG_OK;

@@ -13,7 +13,8 @@
 // tcgen05.ld, add the bias, apply tanh and write the next layer's A operand.  Nothing but the observation rows and
 // the actions touches HBM.  A second instance (mlp_policy_kernel<true>) ends in a sampling epilogue: the action drawn from
 // softmax(logits) with Philox stream 3, its log-probability and the value (PPO's rollout collection, orlg_policy_sample), and
-// its MASKED variant draws under an invalid-action mask (orlg_policy_sample_masked).
+// its MASKED variant draws under an invalid-action mask (orlg_policy_sample_masked).  The WIDE instances
+// (orlg_policy_create_wide) take observations up to 256 wide, layer 0 in chunks of 64 inputs.
 #pragma once
 #include <cuda_bf16.h>
 #include "orlg_deeprmsa_fast.cuh"
@@ -23,23 +24,29 @@ namespace orlg {
 constexpr int PL_TILE = 128;          // environments per tile = UMMA M
 constexpr int PL_HMAX = 128;          // widest hidden layer: the TMEM columns and the A buffer of a tile group
 constexpr int PL_K0 = 64;             // observation width padded to a multiple of 16 (54 -> 64)
+constexpr int PL_K0_WIDE = 256;       // widest observation of the WIDE instances (orlg_policy_create_wide), K0 = obs_dim rounded up to 16
 constexpr int PL_NOUT = 16;           // output layer padded: 5 logits + 1 value
 constexpr int PL_SMEM_MAX = 232448;   // dynamic shared memory a block may opt in to on sm_100 (227 KB)
 
 struct PolicyParams {
     const uint4 *w_blob;              // all weights, bf16, already in the shared-memory operand layout (orlg_policy_create)
-    int w_bytes;                      // H * 64 * 2 + (L - 1) * H * H * 2 + 16 * H * 2
+    int w_bytes;                      // H * K0 * 2 + (L - 1) * H * H * 2 + 16 * H * 2 (K0 = 64; WIDE: obs_dim rounded up to 16)
     const float *bias;                // [L * H + 16]
     int obs_dim, n_actions;           // 54, 5
     int H, L;                         // hidden width (multiple of 16, 16..128) and number of hidden layers (>= 1)
 };
 
-// bytes of weights and of dynamic shared memory of a policy with hidden width H and L hidden layers
-inline size_t pl_weight_bytes(int H, int L) { return (size_t)H * PL_K0 * 2 + (size_t)(L - 1) * H * H * 2 + (size_t)PL_NOUT * H * 2; }
-constexpr int PL_GROUPS = 2;          // tile groups per CTA
-inline size_t pl_smem_bytes(int H, int L) {
-    return pl_weight_bytes(H, L) + (size_t)PL_GROUPS * PL_TILE * PL_HMAX * 2 + ((size_t)L * H + PL_NOUT) * 4 + 64;
+// bytes of weights and of dynamic shared memory of a policy with hidden width H, L hidden layers, layer 0 padded to K0 inputs
+// and G tile groups per CTA (the 2-argument forms: K0 = 64, G = 2, the instances of orlg_policy_create)
+inline size_t pl_weight_bytes(int H, int L, int K0) {
+    return (size_t)H * K0 * 2 + (size_t)(L - 1) * H * H * 2 + (size_t)PL_NOUT * H * 2;
 }
+inline size_t pl_weight_bytes(int H, int L) { return pl_weight_bytes(H, L, PL_K0); }
+constexpr int PL_GROUPS = 2;          // tile groups per CTA
+inline size_t pl_smem_bytes(int H, int L, int K0, int G) {
+    return pl_weight_bytes(H, L, K0) + (size_t)G * PL_TILE * PL_HMAX * 2 + ((size_t)L * H + PL_NOUT) * 4 + 64;
+}
+inline size_t pl_smem_bytes(int H, int L) { return pl_smem_bytes(H, L, PL_K0, PL_GROUPS); }
 
 // The sampling epilogue (mlp_policy_kernel<true>, orlg_policy_sample): one Philox4x32-10 block per row, key = seed,
 // counter = (c0, 0, row_id_base + row, 3) -- stream 3 of DESIGN.md section 5 -- where c0 = counter_dev[row] (the env's
@@ -205,7 +212,8 @@ __device__ __forceinline__ void pl_sample_epilogue(const PolicyParams &pp, const
 // Inside a group warp w reads TMEM lanes 32 (w % 4) .. + 31 (the hardware's lane quarter of a warp) and takes columns
 // (H / 2) (w / 4) .. + H / 2 - 1: thread t owns row t % 128 and one half of its columns, so the epilogue of a layer (128 x H
 // tanh, the chain that bounds this kernel) is spread over 8 warps with all of a thread's TMEM loads in flight before the first use.
-// smem: [weights w_bytes][2 x A tile 128 x 128 bf16 = 64 KB][bias floats][mbarriers][tmem base]  (pl_smem_bytes)
+// smem: [weights w_bytes][G x A tile 128 x 128 bf16 = G x 32 KB][bias floats][mbarriers][tmem base]  (pl_smem_bytes; G = 2, or
+// 1 on a WIDE handle whose layer-0 weights leave room for one group only)
 constexpr int PL_WG = 256;            // threads per group
 __device__ __forceinline__ void pl_group_sync(int group) {          // named barrier of one group (ids 1, 2; 0 = __syncthreads)
     asm volatile("bar.sync %0, %1;" ::"r"(group + 1), "n"(PL_WG) : "memory");
@@ -215,24 +223,30 @@ __device__ __forceinline__ void pl_group_sync(int group) {          // named bar
 // of PolicyDraw; `actions` may be NULL, `logits_out` is unused).  HC, LC: the hidden width and depth fixed at compile time
 // (they must equal pp.H, pp.L), or 0: read from pp at run time.  MASKED (with SAMPLE only): the epilogue draws under the
 // invalid-action mask dr.mask (orlg_policy_sample_masked); a template flag, so that the unmasked instances keep their code.
-template <bool SAMPLE, int HC, int LC, bool MASKED = false>
+// WIDE (run-time H, L only; orlg_policy_create_wide): observations up to 256 wide, any parity.  Layer 0 has K0 = obs_dim
+// rounded up to 16 inputs and runs in chunks of 64 columns through the A buffer (see the staging block), and the CTA has
+// G = blockDim.x / PL_WG tile groups (1 or 2: what fits in shared memory next to the larger layer-0 weights).
+template <bool SAMPLE, int HC, int LC, bool MASKED = false, bool WIDE = false>
 __global__ void __launch_bounds__(PL_WG * PL_GROUPS, 1)
 mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const int n, int *__restrict__ actions,
                   float *__restrict__ logits_out /* [n, n_actions + 1] = logits + value, or NULL */, const PolicyDraw dr) {
     extern __shared__ __align__(128) unsigned char psm[];
     const int H = HC ? HC : pp.H, L = LC ? LC : pp.L;
+    const int G = WIDE ? (int)(blockDim.x / PL_WG) : PL_GROUPS;                   // tile groups of this CTA
+    const int K0 = WIDE ? (pp.obs_dim + 15) & ~15 : PL_K0;                        // layer-0 inputs
+    const int nch = WIDE ? (K0 + 63) >> 6 : 1;                                    // layer-0 chunks of 64 columns
     const int group = threadIdx.x / PL_WG, tid = threadIdx.x % PL_WG, warp = (tid >> 5) & 3;     // warp = TMEM lane quarter of this warp
     const int half = tid >> 7;        // which half of the H columns (K elements of the next layer) this thread produces
     unsigned char *s_w = psm;
     unsigned char *s_a = psm + pp.w_bytes + (size_t)group * PL_TILE * PL_HMAX * 2;
-    float *s_bias = reinterpret_cast<float *>(psm + pp.w_bytes + (size_t)PL_GROUPS * PL_TILE * PL_HMAX * 2);
+    float *s_bias = reinterpret_cast<float *>(psm + pp.w_bytes + (size_t)G * PL_TILE * PL_HMAX * 2);
     unsigned long long *bars = reinterpret_cast<unsigned long long *>(s_bias + L * H + PL_NOUT);   // [0] weights, [1 + g] mma of group g
-    unsigned *s_tmem = reinterpret_cast<unsigned *>(bars + 1 + PL_GROUPS);
+    unsigned *s_tmem = reinterpret_cast<unsigned *>(bars + 1 + G);
 
     pdl_launch_dependents();
     if (threadIdx.x == 0) {
         mbar_init(&bars[0], 1);
-        for (int g = 0; g < PL_GROUPS; g++) mbar_init(&bars[1 + g], 1);
+        for (int g = 0; g < G; g++) mbar_init(&bars[1 + g], 1);
         mbar_expect_tx(&bars[0], (unsigned)pp.w_bytes);
         // the weights do not depend on the previous kernel of the stream: requested before the dependency wait
         const unsigned chunk = 32768u;
@@ -243,10 +257,10 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
                            "r"(bytes), "r"((unsigned)__cvta_generic_to_shared(&bars[0])) : "memory");
         }
     }
-    for (int i = threadIdx.x; i < L * H + PL_NOUT; i += PL_WG * PL_GROUPS) s_bias[i] = pp.bias[i];
+    for (int i = threadIdx.x; i < L * H + PL_NOUT; i += PL_WG * G) s_bias[i] = pp.bias[i];
     if (threadIdx.x < 32) {     // TMEM: 128 columns (one 128 x 128 fp32 accumulator tile, of which H are used) per tile group
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                     ::"r"((unsigned)__cvta_generic_to_shared(s_tmem)), "r"(128u * PL_GROUPS) : "memory");
+                     ::"r"((unsigned)__cvta_generic_to_shared(s_tmem)), "r"(128u * G) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -264,14 +278,82 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
     unsigned char *a_row = s_a + (row >> 3) * 128 + (row & 7) * 16;        // + (k >> 3) * 2048 + (k & 7) * 2
 
     unsigned long long *bar = &bars[1 + group];
-    for (int tile = blockIdx.x * PL_GROUPS + group; tile * PL_TILE < n; tile += gridDim.x * PL_GROUPS) {
+    for (int tile = blockIdx.x * G + group; tile * PL_TILE < n; tile += gridDim.x * G) {
         const int env = tile * PL_TILE + row;
+        if (WIDE) {
+            // ---- layer-0 input of the WIDE instance, in chunks of 64 columns.  Chunk c (columns 64 c .. + 63) goes to half c & 1
+            // of the A buffer (k blocks 8 (c & 1) .. + 7) as bf16; its fp32 rows are staged, 64 at a time, in the other half.  That
+            // half is what chunk c - 1's MMAs read, so chunk c waits for them (their commit, on the group's mbarrier) before its
+            // first stage store; its global loads are issued before that wait.  Every chunk but the last is multiplied here,
+            // accumulating into the tile's TMEM columns from the second chunk on; the last one is layer 0 of the layer loop.  With
+            // K0 <= 64 this is the narrow instance's single pass on the same bf16 operands.
+            // Loads: thread tid reads elements tid + 256 i (i < 16) of the 64 x 64 block, so a warp reads 32 consecutive floats of
+            // one row, coalesced whatever the row's alignment (rows are obs_dim * 4 bytes, only 4-byte aligned when obs_dim is
+            // odd); columns >= obs_dim and rows >= n are zeros.  Stage: row r at r * 256, its 16-byte word q at word q ^ (r & 15),
+            // so the float4 reads of one word by a warp's 32 rows take 4 wavefronts instead of the 32 of a plain 256-byte stride.
+            for (int c = 0; c < nch; c++) {
+                const int h = c & 1;
+                unsigned char *stage = s_a + (1 - h) * 8 * 2048;              // 16 KB: 64 rows x 64 floats
+                for (int hseg = 0; hseg < 2; hseg++) {
+                    const int r0 = tile * PL_TILE + hseg * 64;                  // first env of this half tile
+                    float v[16];
+#pragma unroll
+                    for (int i = 0; i < 16; i++) {
+                        const int e = tid + i * PL_WG, rr = e >> 6, col = 64 * c + (e & 63);
+                        v[i] = col < pp.obs_dim && r0 + rr < n ? obs[(size_t)(r0 + rr) * pp.obs_dim + col] : 0.0f;
+                    }
+                    if (c > 0 && hseg == 0) {                                   // chunk c - 1's MMAs have read the stage half
+                        mbar_wait(bar, phase);
+                        phase ^= 1u;
+                    }
+#pragma unroll
+                    for (int i = 0; i < 16; i++) {
+                        const int e = tid + i * PL_WG, rr = e >> 6, k = e & 63;
+                        *reinterpret_cast<float *>(stage + rr * 256 + (((k >> 2) ^ (rr & 15)) << 4) + (k & 3) * 4) = v[i];
+                    }
+                    pl_group_sync(group);
+                    if ((row >> 6) == hseg) {
+                        const int rr = row & 63;
+                        const unsigned char *src = stage + rr * 256;
+#pragma unroll
+                        for (int j = 0; j < 4; j++) {                           // this thread's columns half * 32 + 8 j .. + 7
+                            const int q = half * 8 + 2 * j;
+                            const float4 x0 = *reinterpret_cast<const float4 *>(src + ((q ^ (rr & 15)) << 4));
+                            const float4 x1 = *reinterpret_cast<const float4 *>(src + (((q + 1) ^ (rr & 15)) << 4));
+                            uint4 pk;
+                            __nv_bfloat162 h0 = __floats2bfloat162_rn(x0.x, x0.y), h1 = __floats2bfloat162_rn(x0.z, x0.w);
+                            __nv_bfloat162 h2 = __floats2bfloat162_rn(x1.x, x1.y), h3 = __floats2bfloat162_rn(x1.z, x1.w);
+                            pk.x = *reinterpret_cast<unsigned *>(&h0); pk.y = *reinterpret_cast<unsigned *>(&h1);
+                            pk.z = *reinterpret_cast<unsigned *>(&h2); pk.w = *reinterpret_cast<unsigned *>(&h3);
+                            *reinterpret_cast<uint4 *>(a_row + (h * 8 + half * 4 + j) * 2048) = pk;
+                        }
+                    }
+                    pl_group_sync(group);                                       // the stage is refilled next
+                }
+                if (c + 1 < nch) {
+                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                    pl_group_sync(group);
+                    if (tid == 0) {
+                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                        const unsigned idesc = pl_instr_desc(PL_TILE, H);
+                        const unsigned a_lbo = (PL_TILE / 8) * 128, b_lbo = (unsigned)(H / 8) * 128;
+#pragma unroll 1
+                        for (int kk = 0; kk < 4; kk++) {
+                            const unsigned long long ad = pl_smem_desc(a_addr + (unsigned)(h * 8 + 2 * kk) * a_lbo, a_lbo, 128u);
+                            const unsigned long long bd = pl_smem_desc(w_addr + (unsigned)(8 * c + 2 * kk) * b_lbo, b_lbo, 128u);
+                            pl_mma(tmem, ad, bd, idesc, c > 0 || kk > 0 ? 1u : 0u);
+                        }
+                        pl_commit(bar);
+                    }
+                }
+            }
+        } else {
         // ---- layer-0 input: the tile's observation rows as bf16, K padded to 64 with zeros.  The 128 rows are one contiguous
         // 27 KB run of obs: they are fetched with coalesced 16-byte loads, 64 rows at a time, into the upper half of the A
         // buffer (k blocks 8..15: unused by layer 0), and each thread then converts its 32 of a row's 64 elements from there.
         // (A thread reading its own 216-byte row from global memory cost 32 sectors per load instruction: 42 % of the kernel's
         // stall samples were lg_throttle / long scoreboard on those loads.)
-        {
             constexpr int KH = PL_K0 / 2;
             unsigned char *stage = s_a + 8 * 2048;                          // 16 KB
             const bool fast = (pp.obs_dim * 4 * 64) % 16 == 0 && (reinterpret_cast<size_t>(obs) & 15) == 0 && pp.obs_dim * 4 * 64 <= 16384;
@@ -320,8 +402,9 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
         }
         int w_off = 0;                 // byte offset of the current layer's weights in s_w
         for (int layer = 0; layer <= L; layer++) {
-            const int K = layer == 0 ? PL_K0 : H;
+            const int K = layer == 0 ? (WIDE ? K0 - 64 * (nch - 1) : PL_K0) : H;     // WIDE layer 0: its last chunk
             const int N = layer == L ? PL_NOUT : H;
+            const bool chunked = WIDE && layer == 0 && nch > 1;
             // activations written by the generic proxy -> visible to the tensor core (async proxy); previous TMEM reads done
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -332,9 +415,14 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
                 const unsigned a_lbo = (PL_TILE / 8) * 128, b_lbo = (unsigned)(N / 8) * 128;
 #pragma unroll 1
                 for (int kk = 0; kk < K / 16; kk++) {            // one instruction per 16 elements of K (two core matrices)
-                    const unsigned long long ad = pl_smem_desc(a_addr + (unsigned)kk * 2u * a_lbo, a_lbo, 128u);
-                    const unsigned long long bd = pl_smem_desc(w_addr + (unsigned)w_off + (unsigned)kk * 2u * b_lbo, b_lbo, 128u);
-                    pl_mma(tmem, ad, bd, idesc, kk > 0 ? 1u : 0u);
+                    unsigned a_k = a_addr + (unsigned)kk * 2u * a_lbo, w_k = w_addr + (unsigned)w_off + (unsigned)kk * 2u * b_lbo;
+                    if (chunked) {                                // the last chunk: A half (nch - 1) & 1, weight columns 64 (nch - 1) ..
+                        a_k += (unsigned)((nch - 1) & 1) * 8u * a_lbo;
+                        w_k += (unsigned)(nch - 1) * 8u * b_lbo;
+                    }
+                    const unsigned long long ad = pl_smem_desc(a_k, a_lbo, 128u);
+                    const unsigned long long bd = pl_smem_desc(w_k, b_lbo, 128u);
+                    pl_mma(tmem, ad, bd, idesc, kk > 0 || chunked ? 1u : 0u);
                 }
                 pl_commit(bar);
             }
@@ -394,12 +482,12 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
                     }
                 }
             }
-            w_off += N * K * 2;
+            w_off += N * (WIDE && layer == 0 ? K0 : K) * 2;
         }
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (threadIdx.x < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*s_tmem), "r"(128u * PL_GROUPS) : "memory");
+    if (threadIdx.x < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*s_tmem), "r"(128u * G) : "memory");
 }
 
 }  // namespace orlg

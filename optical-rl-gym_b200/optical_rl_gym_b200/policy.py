@@ -11,7 +11,11 @@ Two forward paths: :meth:`forward` (plain torch float32, the numerics reference)
 ``model.predict(obs, deterministic=True)`` as ONE fused sm_100a kernel of liborlg.so (``orlg_policy_act``: bf16
 ``tcgen05.mma`` with TMEM accumulators, weights resident in shared memory, tanh + argmax epilogue, int32 actions out).
 The kernel takes any trunk of one width H (a multiple of 16 in 16..128) and any depth whose weights fit in shared memory
-(5 x 128 and 6 x 112 do, 6 x 128 does not), observations up to 64 wide and up to 15 actions.
+(5 x 128 and 6 x 112 do, 6 x 128 does not), observations up to 64 wide (even) and up to 15 actions.
+``wide_observations=True`` builds the handles with ``orlg_policy_create_wide`` instead: observations 1..256 wide, any parity
+(DeepRMSA on germany50 is 126 wide, on a 100-node topology with k = 10 251), the first layer in chunks of 64 inputs; its
+weights take more shared memory, so 5 x 128 fits up to 240 inputs.  At 64 inputs or fewer it gives the same results bit for
+bit.  It is opt-in: the default handles keep the kernel instances and the timing they have.
 :meth:`sample_native` is the same kernel with a sampling epilogue (``orlg_policy_sample``): sampled or argmax actions, their
 log-probabilities and the value estimate, as PPO's rollout collection needs them.  The native weights follow the module:
 an in-place update (``optimizer.step()``, ``load_state_dict``) rebuilds them at the next call.
@@ -26,8 +30,10 @@ import torch
 
 
 class MlpPolicy(torch.nn.Module):
-    def __init__(self, obs_dim: int = 54, n_actions: int = 5, net_arch: Sequence[int] = (128,) * 5):
+    def __init__(self, obs_dim: int = 54, n_actions: int = 5, net_arch: Sequence[int] = (128,) * 5,
+                 wide_observations: bool = False):
         super().__init__()
+        self.wide_observations = wide_observations      # native handles from orlg_policy_create_wide (see the module docstring)
         layers, d = [], obs_dim
         for width in net_arch:
             layers += [torch.nn.Linear(d, width), torch.nn.Tanh()]
@@ -38,19 +44,20 @@ class MlpPolicy(torch.nn.Module):
         self.critic_net = None          # the critic's own trunk when the checkpoint has separate ones (SB3 >= 1.8)
 
     @classmethod
-    def from_state_dict(cls, sd) -> "MlpPolicy":
+    def from_state_dict(cls, sd, wide_observations: bool = False) -> "MlpPolicy":
         """``policy.pth`` of an SB3 ``ActorCriticPolicy`` with a shared trunk (keys ``mlp_extractor.shared_net.<2i>``)
         or with separate actor/critic trunks (``mlp_extractor.policy_net`` / ``mlp_extractor.value_net``, SB3 >= 1.8: the
         actor's trunk becomes ``shared_net``, the critic's is kept as ``critic_net``: ``forward``, :meth:`sample_native` and
         ``OpticalVecEnv.rollout_policy`` return its value (a second native handle evaluates it); the value column of
         :meth:`act_native`'s ``logits`` is the actor trunk's, or NaN when ``value_net`` does not fit the actor's trunk).
-        ``value_net`` is sized from the checkpoint: with separate trunks it takes the critic's last width."""
+        ``value_net`` is sized from the checkpoint: with separate trunks it takes the critic's last width.
+        ``wide_observations``: as in the constructor, for the actor's and the critic's handle."""
         shared = any(k.startswith("mlp_extractor.shared_net.") for k in sd)
         trunk = "mlp_extractor.shared_net." if shared else "mlp_extractor.policy_net."
         idx = sorted({int(k[len(trunk):].split(".")[0]) for k in sd if k.startswith(trunk)})
         widths = [sd["%s%d.weight" % (trunk, i)].shape[0] for i in idx]
         obs_dim = sd["%s%d.weight" % (trunk, idx[0])].shape[1]
-        pol = cls(obs_dim, sd["action_net.weight"].shape[0], widths)
+        pol = cls(obs_dim, sd["action_net.weight"].shape[0], widths, wide_observations=wide_observations)
         if sd["value_net.weight"].shape[1] != pol.value_net.in_features:
             pol.value_net = torch.nn.Linear(sd["value_net.weight"].shape[1], 1)
         mine = {}
@@ -73,10 +80,10 @@ class MlpPolicy(torch.nn.Module):
         return pol
 
     @classmethod
-    def from_sb3_zip(cls, path, device=None) -> "MlpPolicy":
+    def from_sb3_zip(cls, path, device=None, wide_observations: bool = False) -> "MlpPolicy":
         with zipfile.ZipFile(path) as z:
             sd = torch.load(io.BytesIO(z.read("policy.pth")), map_location="cpu", weights_only=True)
-        pol = cls.from_state_dict(sd)
+        pol = cls.from_state_dict(sd, wide_observations=wide_observations)
         return pol.to(device) if device is not None else pol
 
     # ------------------------------------------------------------------ fused native kernel (csrc/orlg_policy.cuh)
@@ -102,7 +109,7 @@ class MlpPolicy(torch.nn.Module):
         return specs
 
     @staticmethod
-    def _create_handle(device_index: int, spec):
+    def _create_handle(device_index: int, spec, wide: bool = False):
         import ctypes as C
 
         import numpy as np
@@ -123,8 +130,9 @@ class MlpPolicy(torch.nn.Module):
         w = np.concatenate([m.weight.detach().float().cpu().numpy().reshape(-1) for m in mats]).astype(np.float32)
         b = np.concatenate([m.bias.detach().float().cpu().numpy().reshape(-1) for m in mats]).astype(np.float32)
         h = C.c_void_p()
-        nat.check(nat.lib().orlg_policy_create(device_index, obs_dim, H, len(lins), heads[0].out_features,
-                                               w.ctypes.data_as(C.c_void_p), b.ctypes.data_as(C.c_void_p), C.byref(h)))
+        create = nat.lib().orlg_policy_create_wide if wide else nat.lib().orlg_policy_create
+        nat.check(create(device_index, obs_dim, H, len(lins), heads[0].out_features,
+                         w.ctypes.data_as(C.c_void_p), b.ctypes.data_as(C.c_void_p), C.byref(h)))
         return h
 
     def _weights_key(self):
@@ -156,9 +164,10 @@ class MlpPolicy(torch.nn.Module):
 
     def _native_handles(self, device_index: int):
         """(actor handle, critic handle | None) holding the CURRENT weights: rebuilt when a parameter was changed in place
-        (optimizer step, load_state_dict) or moved since the handles were made."""
+        (optimizer step, load_state_dict) or moved since the handles were made, or ``wide_observations`` was flipped."""
         cache = self.__dict__.setdefault("_native_cache", {})
-        key = self._weights_key()
+        wide = bool(self.wide_observations)
+        key = (wide,) + self._weights_key()
         entry = cache.get(device_index)
         if entry is not None and entry[0] == key:
             return entry[1], entry[2]
@@ -166,9 +175,9 @@ class MlpPolicy(torch.nn.Module):
             del cache[device_index]
             self._destroy_handles(entry[1:], device_index)
         specs = self._native_specs()
-        actor = self._create_handle(device_index, specs["actor"])
+        actor = self._create_handle(device_index, specs["actor"], wide)
         try:
-            critic = None if specs["critic"] is None else self._create_handle(device_index, specs["critic"])
+            critic = None if specs["critic"] is None else self._create_handle(device_index, specs["critic"], wide)
         except Exception:
             self._destroy_handles((actor,), device_index)
             raise
@@ -207,8 +216,9 @@ class MlpPolicy(torch.nn.Module):
         """Deterministic actions int32 ``[N, 1]`` from float32 CUDA observations ``[N, obs_dim]`` through the fused tensor-core
         kernel; ``logits`` (optional float32 ``[N, n_actions + 1]``) receives the logits and the value estimate of the actor's
         trunk (NaN when the critic's separate trunk has another width: :meth:`sample_native` gives the critic's value).  Any
-        trunk of one width H, a multiple of 16 in 16..128, whose weights fit in shared memory (see the module docstring);
-        other architectures raise ``ValueError`` (widths) or ``NativeError`` (shapes outside the kernel)."""
+        trunk of one width H, a multiple of 16 in 16..128, whose weights fit in shared memory, and observations up to 64 wide
+        (even), or 1..256 wide with ``wide_observations=True`` (see the module docstring); other architectures raise
+        ``ValueError`` (widths) or ``NativeError`` (shapes outside the kernel)."""
         import ctypes as C
 
         from . import _native as nat
