@@ -164,8 +164,8 @@ deeprmsa_fast_kernel(const Params p, const StepIO io_rt, const int mode_rt, cons
         rd_[0] = r0; rd_[2] = (uint32_t)gid; rd_[3] = 1u;
         philox4x32_10(rc_, (uint32_t)p.seed, (uint32_t)(p.seed >> 32));
         philox4x32_10(rd_, (uint32_t)p.seed, (uint32_t)(p.seed >> 32));
-        e_iat = __dmul_rn(neg_log_u32(rc_[0]), p.mean_iat);
-        e_hold = __dmul_rn(neg_log_u32(rc_[1]), p.mean_holding);
+        e_iat = request_iat(p, rc_);
+        e_hold = request_holding(p, rc_);
     }
     // HOT: the rest of the draw (source, destination, bit rate) and the candidate-path tables of the NEXT request
     // also depend on nothing but the tables and the Philox words: done here, ahead of the dependency wait.
@@ -177,16 +177,8 @@ deeprmsa_fast_kernel(const Params p, const StepIO io_rt, const int mode_rt, cons
     if (HOT) {
         __syncthreads();             // the table barrier initialised by thread 0 is visible ...
         mbar_wait(tab_bar, 0);       // ... and the tables have landed
-        const int n = p.N;
-        p_src = pick_thr_bsearch(s_node_thr, n, p.node_top_step, rc_[2]);
-        const unsigned lo = p_src ? s_node_thr[p_src - 1] : 0u;
-        const unsigned long long hi = (p_src == n - 1) ? 4294967296ULL : (unsigned long long)s_node_thr[p_src];
-        const unsigned long long mass = hi - lo;
-        unsigned long long tt = ((unsigned long long)rc_[3] * (4294967296ULL - mass)) >> 32;
-        if (tt >= lo) tt += mass;
-        p_dst = pick_thr_bsearch(s_node_thr, n, p.node_top_step, (unsigned)tt);
-        if (p_dst == p_src) p_dst = (p_src + 1) % n;
-        p_br = p.br_lo + (int)__umulhi(rd_[0], (unsigned)p.br_span);
+        request_nodes(p, s_node_thr, rc_, p_src, p_dst);
+        p_br = request_bit_rate<false>(p, rd_[0]);
         const int pair = p_src * p.N + p_dst;
         p_first = s_pair_first[pair];
         p_npaths = min((int)s_pair_count[pair], KM);
@@ -273,7 +265,7 @@ deeprmsa_fast_kernel(const Params p, const StepIO io_rt, const int mode_rt, cons
                             a_start = (int)st;
                             const double rel = __dadd_rn(now, hold);
                             events_push(ev, nheap, hmin, tailmin, rel, pack_service(a_row, a_start, a_n, 0, sid));
-                            cnt[1] += 1; cnt[3] += 1; cnt[5] += br; cnt[7] += br;
+                            count_decision<ORLG_DEEPRMSA>(cnt, true, br);
                             accepted = true;
                             d_row = a_row; d_start = a_start; d_n = a_n;
                         }
@@ -304,33 +296,19 @@ deeprmsa_fast_kernel(const Params p, const StepIO io_rt, const int mode_rt, cons
                 holding = e_hold;
                 nsrc = p_src; ndst = p_dst; nbr = p_br;
             } else if (philox) {
-                const uint32_t *c = rc_, *d = rd_;
                 if (ridx != (mode == MODE_FULL_RESET ? 0u : p.lockstep_ridx)) err |= ORLG_ERR_LOCKSTEP;
                 arrival = __dadd_rn(now, e_iat);
                 holding = e_hold;
-                const int n = p.N;
-                nsrc = pick_thr_bsearch(s_node_thr, n, p.node_top_step, c[2]);
-                const unsigned lo = nsrc ? s_node_thr[nsrc - 1] : 0u;
-                const unsigned long long hi = (nsrc == n - 1) ? 4294967296ULL : (unsigned long long)s_node_thr[nsrc];
-                const unsigned long long mass = hi - lo;
-                unsigned long long tt = ((unsigned long long)c[3] * (4294967296ULL - mass)) >> 32;
-                if (tt >= lo) tt += mass;
-                ndst = pick_thr_bsearch(s_node_thr, n, p.node_top_step, (unsigned)tt);
-                if (ndst == nsrc) ndst = (nsrc + 1) % n;
-                if (!HOT && p.n_bit_rates > 0) nbr = p.bit_rates[pick_thr(p.br_thr, p.n_bit_rates, d[0])];
-                else nbr = p.br_lo + (int)__umulhi(d[0], (unsigned)p.br_span);
-            } else if ((long long)ridx < p.trace_len) {
-                const orlg_request r = p.trace[(size_t)e * p.trace_len + ridx];
-                arrival = r.arrival; holding = r.holding; nsrc = r.src; ndst = r.dst;
-                nbr = min(max(r.bit_rate, 0), p.br_max);
+                request_nodes(p, s_node_thr, rc_, nsrc, ndst);
+                nbr = request_bit_rate<!HOT>(p, rd_[0]);
             } else {
-                err |= ORLG_ERR_TRACE_EXHAUSTED;
-                arrival = now; holding = 0.0; nsrc = 0; ndst = 1; nbr = p.br_lo;
+                const orlg_request r = trace_request(p, e, ridx, now, p.br_max, p.br_lo, false, err);
+                arrival = r.arrival; holding = r.holding; nsrc = r.src; ndst = r.dst; nbr = r.bit_rate;
             }
             ridx++;
             now = arrival; hold = holding; src = nsrc; dst = ndst; br = nbr;
             sid = (int)cnt[2];
-            cnt[0] += 1; cnt[2] += 1; cnt[4] += br; cnt[6] += br;
+            count_request<ORLG_DEEPRMSA>(cnt, br);
         }
 
         PHASE_MARK(3);               // phase B: traffic draw
@@ -369,9 +347,7 @@ deeprmsa_fast_kernel(const Params p, const StepIO io_rt, const int mode_rt, cons
             }));
             done = (cnt[2] == (long long)p.episode_length);
         }
-        if (mode == MODE_EPISODE_RESET || (mode == MODE_STEP && done && p.auto_reset)) {
-            cnt[2] = 1; cnt[3] = 0; cnt[6] = br; cnt[7] = 0;      // rmsa_env.py:285-330
-        }
+        if (mode == MODE_EPISODE_RESET || (mode == MODE_STEP && done && p.auto_reset)) reset_episode_counters<ORLG_DEEPRMSA>(cnt, br);
         if (mode != MODE_OBSERVE) {      // ---- store the scalar block (final from here on: frees its registers for phase C)
             p.now[env] = now;
             p.cur_hold[env] = hold;

@@ -177,30 +177,101 @@ __device__ __forceinline__ int pick_thr_bsearch(const unsigned *thr, int n, int 
     return i;
 }
 
-// _next_service's draws (rmsa_env.py:548-561) from the counter-based generator
+// ---------------------------------------------------------------- the request stream (DESIGN.md section 5)
+// _next_service's draws (rmsa_env.py:548-561) from the counter-based generator, in pieces: the persistent and the fast kernels
+// draw the times before their tables have landed and the nodes from the tables in shared memory.  The Philox blocks themselves
+// stay at the call sites: behind a function boundary the compiler orders the XORs of the rounds differently and the code of
+// the persistent and fast kernels changes.
+
+// inter-arrival and holding time from stream 0 (the arrival is now + the inter-arrival time)
+__device__ __forceinline__ double request_iat(const Params &p, const uint32_t c[4]) { return __dmul_rn(neg_log_u32(c[0]), p.mean_iat); }
+__device__ __forceinline__ double request_holding(const Params &p, const uint32_t c[4]) { return __dmul_rn(neg_log_u32(c[1]), p.mean_holding); }
+
+// source and destination from stream 0: node_thr is the node CDF in global or in shared memory
+__device__ __forceinline__ void request_nodes(const Params &p, const unsigned *node_thr, const uint32_t c[4], int &src, int &dst) {
+    const int n = p.N;
+    src = pick_thr_bsearch(node_thr, n, p.node_top_step, c[2]);        // binary search: up to 255 nodes, every lane its own draw
+    const unsigned lo = src ? node_thr[src - 1] : 0u;
+    const unsigned long long hi = (src == n - 1) ? 4294967296ULL : (unsigned long long)node_thr[src];
+    const unsigned long long mass = hi - lo;
+    unsigned long long tt = ((unsigned long long)c[3] * (4294967296ULL - mass)) >> 32;
+    if (tt >= lo) tt += mass;
+    dst = pick_thr_bsearch(node_thr, n, p.node_top_step, (unsigned)tt);
+    if (dst == src) dst = (src + 1) % n;
+}
+
+// bit rate from word 0 of stream 1: the discrete CDF when the handle has one (only compiled in with DISCRETE), else uniform
+template <bool DISCRETE>
+__device__ __forceinline__ int request_bit_rate(const Params &p, uint32_t d0) {
+    if (DISCRETE && p.n_bit_rates > 0) return p.bit_rates[pick_thr(p.br_thr, p.n_bit_rates, d0)];
+    return p.br_lo + (int)__umulhi(d0, (unsigned)p.br_span);
+}
+
 __device__ __forceinline__ void philox_request(const Params &p, const unsigned *node_thr, int env, unsigned ridx, double now,
                                                double &arrival, double &holding, int &src, int &dst, int &br) {
     unsigned long long gid = (unsigned long long)(p.env_id_base + env);
     uint32_t c[4] = {ridx, 0u, (uint32_t)gid, 0u};
     philox4x32_10(c, (uint32_t)p.seed, (uint32_t)(p.seed >> 32));
-    arrival = __dadd_rn(now, __dmul_rn(neg_log_u32(c[0]), p.mean_iat));
-    holding = __dmul_rn(neg_log_u32(c[1]), p.mean_holding);
-    int n = p.N;
-    src = pick_thr_bsearch(node_thr, n, p.node_top_step, c[2]);        // binary search: up to 255 nodes, every lane its own draw
-    unsigned long long lo = src ? node_thr[src - 1] : 0u;
-    unsigned long long hi = (src == n - 1) ? 4294967296ULL : (unsigned long long)node_thr[src];
-    unsigned long long mass = hi - lo;
-    unsigned long long tt = ((unsigned long long)c[3] * (4294967296ULL - mass)) >> 32;
-    if (tt >= lo) tt += mass;
-    dst = pick_thr_bsearch(node_thr, n, p.node_top_step, (unsigned)tt);
-    if (dst == src) dst = (src + 1) % n;
+    arrival = __dadd_rn(now, request_iat(p, c));
+    holding = request_holding(p, c);
+    request_nodes(p, node_thr, c, src, dst);
     br = 0;
     if (p.kind != ORLG_RWA) {
         uint32_t d[4] = {ridx, 0u, (uint32_t)gid, 1u};
         philox4x32_10(d, (uint32_t)p.seed, (uint32_t)(p.seed >> 32));
-        if (p.n_bit_rates > 0) br = p.bit_rates[pick_thr(p.br_thr, p.n_bit_rates, d[0])];
-        else br = p.br_lo + (int)__umulhi(d[0], (unsigned)p.br_span);
+        br = request_bit_rate<true>(p, d[0]);
     }
+}
+
+// request ridx of env e from the recorded trace, its bit rate clamped to [0, br_cap]; above br_cap it sets
+// ORLG_ERR_TRACE_RANGE when flag_range.  Past the end of the trace: ORLG_ERR_TRACE_EXHAUSTED and the request
+// (now, holding 0, node 0 -> 1, br_past_end).
+__device__ __forceinline__ orlg_request trace_request(const Params &p, int e, unsigned ridx, double now, int br_cap, int br_past_end,
+                                                      bool flag_range, unsigned &err) {
+    orlg_request r;
+    if ((long long)ridx < p.trace_len) {
+        r = p.trace[(size_t)e * p.trace_len + ridx];
+        if (flag_range && r.bit_rate > br_cap) err |= ORLG_ERR_TRACE_RANGE;
+        r.bit_rate = min(max(r.bit_rate, 0), br_cap);
+    } else {
+        err |= ORLG_ERR_TRACE_EXHAUSTED;
+        r.arrival = now; r.holding = 0.0; r.src = 0; r.dst = 1; r.bit_rate = br_past_end;
+    }
+    return r;
+}
+
+// ---------------------------------------------------------------- the counters
+// cnt = services_processed, services_accepted, episode_services_processed, episode_services_accepted, bit_rate_requested,
+// bit_rate_provisioned, episode_bit_rate_requested, episode_bit_rate_provisioned.  The persistent rollout kernel keeps the
+// same updates in its register form (orlg_rollout.cuh).
+
+// the decision on the pending request (rmsa_env.py:163-209, rwa_env.py:135-136, rmcsa_env.py:292-295): RWA and RMCSA count
+// the request here, RMCSA its bit rate as well (it is counted again when the request is drawn)
+template <int KIND>
+__device__ __forceinline__ void count_decision(long long cnt[8], bool accepted, int br) {
+    if (accepted) {
+        cnt[1] += 1; cnt[3] += 1;                                // services_accepted (+episode)
+        if (KIND != ORLG_RWA) { cnt[5] += br; cnt[7] += br; }   // bit_rate_provisioned (+episode)
+    }
+    if (KIND == ORLG_RWA || KIND == ORLG_RMCSA) {
+        cnt[0] += 1; cnt[2] += 1;
+        if (KIND == ORLG_RMCSA) { cnt[4] += br; cnt[6] += br; }
+    }
+}
+
+// a new request (_next_service, rmsa_env.py:570-573, rmcsa_env.py:730-731)
+template <int KIND>
+__device__ __forceinline__ void count_request(long long cnt[8], int br) {
+    if (KIND == ORLG_RMSA || KIND == ORLG_DEEPRMSA) { cnt[0] += 1; cnt[2] += 1; cnt[4] += br; cnt[6] += br; }
+    else if (KIND == ORLG_RMCSA) { cnt[4] += br; cnt[6] += br; }
+}
+
+// reset(only_episode_counters=True) (rmsa_env.py:285-330, rwa_env.py:164-179, rmcsa_env.py:387-430): the pending request
+// (bit rate br) stays counted in the new episode, except on RWA
+template <int KIND>
+__device__ __forceinline__ void reset_episode_counters(long long cnt[8], int br) {
+    cnt[2] = 0; cnt[3] = 0; cnt[6] = 0; cnt[7] = 0;
+    if (KIND != ORLG_RWA) { cnt[2] = 1; cnt[6] = br; }
 }
 
 // ---------------------------------------------------------------- row f1: float statistics
@@ -367,6 +438,47 @@ __device__ __forceinline__ void path_update_stats(const Params &p, int env, int 
     }
 }
 
+// Release every service due at `now` on a handle with statistics (rmsa_env.py:591-597).  The reference releases in heap order
+// (by time) and every release updates the statistics of its links, so the due services are collected, sorted by release time
+// and applied in that order.  Beyond 24 of them in one step the rest are applied as they come (the masks stay exact, the order
+// of the statistics does not) and ORLG_ERR_STATS_ORDER is set.  release(payload) provisions the service's slots back with the
+// link statistics and returns its number_slots * hops, which leaves sum_nh; its bit rate leaves run_br.
+template <typename ReleaseFn>
+__device__ __forceinline__ void release_due_in_order(const Params &p, int env, const Events &ev, unsigned &nheap, double &hmin,
+                                                     double &tailmin, double now, unsigned &err, ReleaseFn release) {
+    constexpr int MAXR = 24;
+    double rt[MAXR];
+    unsigned long long rp[MAXR];
+    int nr = 0;
+    long long rel_br = 0;                                // bit rates leaving graph["running_services"]
+    events_release(ev, nheap, hmin, tailmin, now, apply_timed([&](unsigned long long pl, double t, unsigned sbr) {
+        rel_br += sbr;
+        if (nr < MAXR) { rt[nr] = t; rp[nr] = pl; nr++; }
+        else { err |= ORLG_ERR_STATS_ORDER; p.sum_nh[env] -= release(pl); }
+    }));
+    if (rel_br) p.run_br[env] -= rel_br;
+    for (int a = 1; a < nr; a++) {                       // insertion sort by release time
+        const double t = rt[a];
+        const unsigned long long q = rp[a];
+        int b = a - 1;
+        while (b >= 0 && rt[b] > t) { rt[b + 1] = rt[b]; rp[b + 1] = rp[b]; b--; }
+        rt[b + 1] = t; rp[b + 1] = q;
+    }
+    long long snh = p.sum_nh[env];
+    for (int a = 0; a < nr; a++) snh -= release(rp[a]);
+    p.sum_nh[env] = snh;
+}
+
+// the float statistics at a full reset (optical_network_env.py:181-203, rmsa_env.py:332-359)
+__device__ __forceinline__ void clear_stats(const Params &p, int env) {
+    for (int l = 0; l < p.E; l++) {
+        const size_t i = (size_t)l * p.n + env;
+        p.link_util[i] = 0.0; p.link_comp[i] = 0.0; p.link_last[i] = 0.0; p.link_frag[i] = 0.0;
+    }
+    p.sum_nh[env] = 0; p.run_br[env] = 0;
+    for (int q = 0; q < 3; q++) p.graph_stats[(size_t)q * p.n + env] = 0.0;
+}
+
 template <typename T>
 __device__ __forceinline__ T obs_ratio(int num, int den);
 // float32 observations: one correctly rounded division of the exact rational (<= 1 ulp of the
@@ -508,15 +620,10 @@ __global__ void __launch_bounds__(STEP_THREADS) step_kernel(const Params p, cons
                 double rel = __dadd_rn(now, hold);          // arrival_time + holding_time (now == arrival)
                 events_push(ev, nheap, hmin, tailmin, rel, pack_service(row, start, n, core, sid), (unsigned)br);
             }
-            cnt[1] += 1; cnt[3] += 1;                        // services_accepted (+episode)
-            if (KIND != ORLG_RWA) { cnt[5] += br; cnt[7] += br; }   // bit_rate_provisioned (+episode)
             if (KIND == ORLG_RMSA) br_hist_bump(p, env, 1, br);     // rmsa_env.py:408-415
             d_row = row; d_start = start; d_n = n; d_core = core; d_mod = mod;
         }
-        if (KIND == ORLG_RWA || KIND == ORLG_RMCSA) {         // rwa_env.py:135-136, rmcsa_env.py:292-295
-            cnt[0] += 1; cnt[2] += 1;
-            if (KIND == ORLG_RMCSA) { cnt[4] += br; cnt[6] += br; }
-        }
+        count_decision<KIND>(cnt, accepted, br);
         if (live) {
             if (io.reward) io.reward[env] = accepted ? 1.0f : (KIND == ORLG_DEEPRMSA ? -1.0f : 0.0f);
             if (io.decision) {
@@ -540,14 +647,7 @@ __global__ void __launch_bounds__(STEP_THREADS) step_kernel(const Params p, cons
         }
     }
 
-    if (mode == MODE_FULL_RESET && p.stats) {
-        for (int l = 0; l < p.E; l++) {
-            const size_t i = (size_t)l * p.n + env;
-            p.link_util[i] = 0.0; p.link_comp[i] = 0.0; p.link_last[i] = 0.0; p.link_frag[i] = 0.0;
-        }
-        p.sum_nh[env] = 0; p.run_br[env] = 0;
-        for (int q = 0; q < 3; q++) p.graph_stats[(size_t)q * p.n + env] = 0.0;
-    }
+    if (mode == MODE_FULL_RESET && p.stats) clear_stats(p, env);
 
     if (mode == MODE_STEP || mode == MODE_FULL_RESET) {
         // ================= Phase B: _next_service (rmsa_env.py:545-597) ==================
@@ -556,60 +656,22 @@ __global__ void __launch_bounds__(STEP_THREADS) step_kernel(const Params p, cons
         if (p.traffic == ORLG_TRAFFIC_PHILOX) {
             philox_request(p, p.node_thr, e, ridx, now, arrival, holding, nsrc, ndst, nbr);
         } else {
-            if ((long long)ridx < p.trace_len) {
-                const orlg_request r = p.trace[(size_t)e * p.trace_len + ridx];
-                arrival = r.arrival; holding = r.holding; nsrc = r.src; ndst = r.dst;
-                nbr = min(max(r.bit_rate, 0), p.br_max);
-            } else {
-                err |= ORLG_ERR_TRACE_EXHAUSTED;
-                arrival = now; holding = 0.0; nsrc = 0; ndst = 1; nbr = p.br_lo;
-            }
+            const orlg_request r = trace_request(p, e, ridx, now, p.br_max, p.br_lo, false, err);
+            arrival = r.arrival; holding = r.holding; nsrc = r.src; ndst = r.dst; nbr = r.bit_rate;
         }
         ridx++;
         now = arrival; hold = holding; src = nsrc; dst = ndst; br = nbr;
         sid = (int)cnt[2];                                    // Service(self.episode_services_processed, ...)
-        if (KIND == ORLG_RMSA || KIND == ORLG_DEEPRMSA) {
-            cnt[0] += 1; cnt[2] += 1; cnt[4] += br; cnt[6] += br;
-            if (KIND == ORLG_RMSA) br_hist_bump(p, env, 0, br);     // rmsa_env.py:579-581
-        } else if (KIND == ORLG_RMCSA) {
-            cnt[4] += br; cnt[6] += br;                       // rmcsa_env.py:730-731
-        }
+        count_request<KIND>(cnt, br);
+        if (KIND == ORLG_RMSA) br_hist_bump(p, env, 0, br);     // rmsa_env.py:579-581
         // release every service whose time has come (rmsa_env.py:591-597)
-        if (p.stats) {
-            // the reference releases in heap order (by time) and every release updates the float statistics of
-            // its links, so the due services are collected, sorted by release time and applied in that order
-            constexpr int MAXR = 24;
-            double rt[MAXR];
-            unsigned long long rp[MAXR];
-            int nr = 0;
-            long long rel_br = 0;                                // bit rates leaving graph["running_services"]
-            events_release(ev, nheap, hmin, tailmin, now, apply_timed([&](unsigned long long pl, double t, unsigned sbr) {
-                rel_br += sbr;
-                if (nr < MAXR) { rt[nr] = t; rp[nr] = pl; nr++; }
-                else {                                           // overflow: masks stay exact, statistics order is not
-                    err |= ORLG_ERR_STATS_ORDER;
-                    const int rs = svc_start(pl);
-                    path_update_stats(p, env, svc_row(pl), svc_core(pl), bits_range(rs, rs + svc_slots(pl)), true, now);
-                    p.sum_nh[env] -= (long long)svc_slots(pl) * meta_hops(p.path_meta[svc_row(pl)]);
-                }
-            }));
-            if (rel_br) p.run_br[env] -= rel_br;
-            for (int a = 1; a < nr; a++) {                       // insertion sort by release time
-                const double t = rt[a];
-                const unsigned long long q = rp[a];
-                int b = a - 1;
-                while (b >= 0 && rt[b] > t) { rt[b + 1] = rt[b]; rp[b + 1] = rp[b]; b--; }
-                rt[b + 1] = t; rp[b + 1] = q;
-            }
-            long long snh = p.sum_nh[env];
-            for (int a = 0; a < nr; a++) {
-                const unsigned long long pl = rp[a];
+        if (p.stats)
+            release_due_in_order(p, env, ev, nheap, hmin, tailmin, now, err, [&](unsigned long long pl) {
                 const int rs = svc_start(pl);
                 path_update_stats(p, env, svc_row(pl), svc_core(pl), bits_range(rs, rs + svc_slots(pl)), true, now);
-                snh -= (long long)svc_slots(pl) * meta_hops(p.path_meta[svc_row(pl)]);
-            }
-            p.sum_nh[env] = snh;
-        } else
+                return (long long)svc_slots(pl) * meta_hops(p.path_meta[svc_row(pl)]);
+            });
+        else
         events_release(ev, nheap, hmin, tailmin, now, apply_payload([&](unsigned long long pl) {
             const int rs = svc_start(pl);
             path_update(p, env, p.path_linkmask[svc_row(pl)], svc_core(pl), bits_range(rs, rs + svc_slots(pl)), true);
@@ -617,11 +679,7 @@ __global__ void __launch_bounds__(STEP_THREADS) step_kernel(const Params p, cons
         done = (cnt[2] == (long long)p.episode_length);
     }
 
-    if (mode == MODE_EPISODE_RESET || (mode == MODE_STEP && done && p.auto_reset)) {
-        // reset(only_episode_counters=True): rmsa_env.py:285-330, rwa_env.py:164-179, rmcsa_env.py:387-430
-        cnt[2] = 0; cnt[3] = 0; cnt[6] = 0; cnt[7] = 0;
-        if (KIND != ORLG_RWA) { cnt[2] = 1; cnt[6] = br; }
-    }
+    if (mode == MODE_EPISODE_RESET || (mode == MODE_STEP && done && p.auto_reset)) reset_episode_counters<KIND>(cnt, br);
 
     // ================= Phase C: observation of the pending request (deeprmsa_env.py:60-121) =========
     if (KIND == ORLG_DEEPRMSA) {

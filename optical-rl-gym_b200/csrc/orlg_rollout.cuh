@@ -397,6 +397,8 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
     int ep_proc = (int)p.counters[(size_t)2 * p.n + e], ep_acc = (int)p.counters[(size_t)3 * p.n + e];
     int ep_req = (int)p.counters[(size_t)6 * p.n + e], ep_prov = (int)p.counters[(size_t)7 * p.n + e];
     int d_proc = 0, d_acc = 0, d_req = 0, d_prov = 0;        // deltas of the four running totals over this launch
+    // (the updates below are those of count_decision, count_request and reset_episode_counters in orlg_kernels.cuh, on this
+    // register form of the counters; RMCSA does not run here)
     unsigned ridx = p.req_index[e];
     unsigned nlive = live ? p.nheap[e] : 0u;                  // live services = table + window + side (a lane without an env: none)
     unsigned n_tab = nlive;
@@ -492,34 +494,22 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
         } else if (live) {
             // ---- the next request (rmsa_env.py:545-561): a pure function of (seed, global env id, request index)
             double e_iat = 0.0, e_hold = 0.0, t_arrival = now;
-            int p_src = 0, p_dst = 1, p_br = KIND == ORLG_RWA ? 0 : p.br_lo;
-            if (TRACE) {
-                if ((long long)ridx < p.trace_len) {
-                    const orlg_request r = p.trace[(size_t)e * p.trace_len + ridx];
-                    t_arrival = r.arrival; e_hold = r.holding; p_src = r.src; p_dst = r.dst;
-                    p_br = KIND == ORLG_RWA ? 0 : min(max(r.bit_rate, 0), 127);
-                    if (KIND != ORLG_RWA && r.bit_rate > 127) err |= ORLG_ERR_TRACE_RANGE;       // beyond the slot-count table of this kernel
-                } else {
-                    err |= ORLG_ERR_TRACE_EXHAUSTED;
-                }
+            int p_src = 0, p_dst = 1, p_br = 0;
+            if constexpr (TRACE) {
+                // bit rates beyond the slot-count table of this kernel (127) are flagged; RWA requests carry none
+                const orlg_request r = trace_request(p, e, ridx, now, 127, p.br_lo, KIND != ORLG_RWA, err);
+                t_arrival = r.arrival; e_hold = r.holding; p_src = r.src; p_dst = r.dst;
+                if (KIND != ORLG_RWA) p_br = r.bit_rate;
             } else {
                 uint32_t rc_[4] = {ridx, 0u, (uint32_t)gid, 0u};
                 philox4x32_10(rc_, k0, k1);
-                e_iat = __dmul_rn(neg_log_u32(rc_[0]), p.mean_iat);
-                e_hold = __dmul_rn(neg_log_u32(rc_[1]), p.mean_holding);
-                const int nn = p.N;
-                p_src = pick_thr_bsearch(s_node_thr, nn, p.node_top_step, rc_[2]);
-                const unsigned lo = p_src ? s_node_thr[p_src - 1] : 0u;
-                const unsigned long long hi = (p_src == nn - 1) ? 4294967296ULL : (unsigned long long)s_node_thr[p_src];
-                const unsigned long long mass = hi - lo;
-                unsigned long long tt = ((unsigned long long)rc_[3] * (4294967296ULL - mass)) >> 32;
-                if (tt >= lo) tt += mass;
-                p_dst = pick_thr_bsearch(s_node_thr, nn, p.node_top_step, (unsigned)tt);
-                if (p_dst == p_src) p_dst = (p_src + 1) % nn;
+                e_iat = request_iat(p, rc_);
+                e_hold = request_holding(p, rc_);
+                request_nodes(p, s_node_thr, rc_, p_src, p_dst);
                 if (KIND != ORLG_RWA) {
                     uint32_t rd_[4] = {ridx, 0u, (uint32_t)gid, 1u};
                     philox4x32_10(rd_, k0, k1);
-                    p_br = p.br_lo + (int)__umulhi(rd_[0], (unsigned)p.br_span);
+                    p_br = request_bit_rate<false>(p, rd_[0]);
                 }
             }
             npaths = min((int)s_pair_count[p_src * p.N + p_dst], KM);

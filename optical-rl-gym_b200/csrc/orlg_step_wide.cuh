@@ -391,14 +391,9 @@ __global__ void __launch_bounds__(ORLG_WIDE_THREADS, STATS ? ORLG_WIDE_STATS_MIN
                 wide_path_update<NWV>(p, env, row, core, start, n, false);
                 events_push(ev, nheap, hmin, tailmin, __dadd_rn(now, hold), pack_service(row, start, n, core, sid));
             }
-            cnt[1] += 1; cnt[3] += 1;
-            if (KIND != ORLG_RWA) { cnt[5] += br; cnt[7] += br; }
-            if (KIND == ORLG_RMSA) br_hist_bump(p, env, 1, br);
         }
-        if (KIND == ORLG_RWA || KIND == ORLG_RMCSA) {
-            cnt[0] += 1; cnt[2] += 1;
-            if (KIND == ORLG_RMCSA) { cnt[4] += br; cnt[6] += br; }
-        }
+        count_decision<KIND>(cnt, accepted, br);
+        if (KIND == ORLG_RMSA && accepted) br_hist_bump(p, env, 1, br);
         if (io.reward) io.reward[env] = accepted ? 1.0f : (KIND == ORLG_DEEPRMSA ? -1.0f : 0.0f);
         if (io.decision) {
             int *d = io.decision + (size_t)env * 6;
@@ -420,12 +415,7 @@ __global__ void __launch_bounds__(ORLG_WIDE_THREADS, STATS ? ORLG_WIDE_STATS_MIN
     }
 
     if constexpr (STATS) if (mode == MODE_FULL_RESET) {
-        for (int l = 0; l < p.E; l++) {
-            const size_t i = (size_t)l * p.n + env;
-            p.link_util[i] = 0.0; p.link_comp[i] = 0.0; p.link_last[i] = 0.0; p.link_frag[i] = 0.0;
-        }
-        p.sum_nh[env] = 0; p.run_br[env] = 0;
-        for (int q = 0; q < 3; q++) p.graph_stats[(size_t)q * p.n + env] = 0.0;
+        clear_stats(p, env);
         if (KIND != ORLG_RWA) {
             for (int l = 0; l < p.C * p.E; l++) nc_links(p)[(size_t)env * p.C * p.E + l] = 0u;
             for (int c = 0; c < p.C; c++) nc_totals(p)[(size_t)env * p.C + c] = make_int2(0, 0);
@@ -437,63 +427,28 @@ __global__ void __launch_bounds__(ORLG_WIDE_THREADS, STATS ? ORLG_WIDE_STATS_MIN
         int nsrc, ndst, nbr;
         if (p.traffic == ORLG_TRAFFIC_PHILOX) {
             philox_request(p, p.node_thr, env, ridx, now, arrival, holding, nsrc, ndst, nbr);
-        } else if ((long long)ridx < p.trace_len) {
-            const orlg_request r = p.trace[(size_t)env * p.trace_len + ridx];
-            arrival = r.arrival; holding = r.holding; nsrc = r.src; ndst = r.dst;
-            nbr = min(max(r.bit_rate, 0), p.br_max);
         } else {
-            err |= ORLG_ERR_TRACE_EXHAUSTED;
-            arrival = now; holding = 0.0; nsrc = 0; ndst = 1; nbr = p.br_lo;
+            const orlg_request r = trace_request(p, env, ridx, now, p.br_max, p.br_lo, false, err);
+            arrival = r.arrival; holding = r.holding; nsrc = r.src; ndst = r.dst; nbr = r.bit_rate;
         }
         ridx++;
         now = arrival; hold = holding; src = nsrc; dst = ndst; br = nbr;
         sid = (int)cnt[2];
-        if (KIND == ORLG_RMSA || KIND == ORLG_DEEPRMSA) { cnt[0] += 1; cnt[2] += 1; cnt[4] += br; cnt[6] += br; }
+        count_request<KIND>(cnt, br);
         if (KIND == ORLG_RMSA) br_hist_bump(p, env, 0, br);
-        else if (KIND == ORLG_RMCSA) { cnt[4] += br; cnt[6] += br; }
-        if constexpr (STATS) {
-            // the reference releases in heap order (by time) and every release updates the statistics of its links: the due
-            // services are collected, sorted by release time and applied in that order (as in step_kernel)
-            constexpr int MAXR = 24;
-            double rt[MAXR];
-            unsigned long long rp[MAXR];
-            int nr = 0;
-            long long rel_br = 0;                                // bit rates leaving graph["running_services"]
-            long long snh = p.sum_nh[env];
-            events_release(ev, nheap, hmin, tailmin, now, apply_timed([&](unsigned long long pl, double t, unsigned sbr) {
-                rel_br += sbr;
-                if (nr < MAXR) { rt[nr] = t; rp[nr] = pl; nr++; }
-                else {                                           // overflow: masks stay exact, statistics order is not
-                    err |= ORLG_ERR_STATS_ORDER;
-                    wide_path_update_stats<KIND, NWV>(p, env, svc_row(pl), svc_core(pl), svc_start(pl), svc_slots(pl), true, now);
-                    snh -= (long long)svc_slots(pl) * wide_hops(p, svc_row(pl));
-                }
-            }));
-            if (rel_br) p.run_br[env] -= rel_br;
-            for (int a = 1; a < nr; a++) {                       // insertion sort by release time
-                const double t = rt[a];
-                const unsigned long long q = rp[a];
-                int b = a - 1;
-                while (b >= 0 && rt[b] > t) { rt[b + 1] = rt[b]; rp[b + 1] = rp[b]; b--; }
-                rt[b + 1] = t; rp[b + 1] = q;
-            }
-            for (int a = 0; a < nr; a++) {
-                const unsigned long long pl = rp[a];
+        if constexpr (STATS)
+            release_due_in_order(p, env, ev, nheap, hmin, tailmin, now, err, [&](unsigned long long pl) {
                 wide_path_update_stats<KIND, NWV>(p, env, svc_row(pl), svc_core(pl), svc_start(pl), svc_slots(pl), true, now);
-                snh -= (long long)svc_slots(pl) * wide_hops(p, svc_row(pl));
-            }
-            p.sum_nh[env] = snh;
-        } else
+                return (long long)svc_slots(pl) * wide_hops(p, svc_row(pl));
+            });
+        else
         events_release(ev, nheap, hmin, tailmin, now, apply_payload([&](unsigned long long pl) {
             wide_path_update<NWV>(p, env, svc_row(pl), svc_core(pl), svc_start(pl), svc_slots(pl), true);
         }));
         done = (cnt[2] == (long long)p.episode_length);
     }
 
-    if (mode == MODE_EPISODE_RESET || (mode == MODE_STEP && done && p.auto_reset)) {
-        cnt[2] = 0; cnt[3] = 0; cnt[6] = 0; cnt[7] = 0;
-        if (KIND != ORLG_RWA) { cnt[2] = 1; cnt[6] = br; }
-    }
+    if (mode == MODE_EPISODE_RESET || (mode == MODE_STEP && done && p.auto_reset)) reset_episode_counters<KIND>(cnt, br);
 
     if (KIND == ORLG_DEEPRMSA) {
         // observation of the pending request (deeprmsa_env.py:60-121), path by path, written in place

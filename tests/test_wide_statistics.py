@@ -265,34 +265,41 @@ def test_checkpoint_resumes_wide_statistics():
 
 @pytest.mark.gpu
 def test_more_than_24_releases_in_one_step_set_the_order_flag():
-    """One arrival that releases 30 services at once: ORLG_ERR_STATS_ORDER is set, the masks stay equal to the oracle's."""
+    """One arrival that releases 30 services at once: ORLG_ERR_STATS_ORDER is set, the masks stay equal to the oracle's.
+    Once per slot count: 160 slots on a 42-link ring run the wide kernel, 100 slots on NSFNET the generic step_kernel."""
+    for slots in (160, 100):
+        _more_than_24_releases(slots)
+
+
+def _more_than_24_releases(slots):
     from optical_rl_gym_b200 import OpticalVecEnv
     from oracle import oracle
 
-    tabs = tables("ring20")
+    tabs = tables("ring20" if slots == 160 else "nsfnet")
     n, R, T = 2, 30, 34
-    env_args = dict(episode_length=1000, load=100, mean_service_holding_time=25, num_spectrum_resources=160)
+    env_args = dict(episode_length=1000, load=100, mean_service_holding_time=25, num_spectrum_resources=slots)
     arrival = np.concatenate([0.01 * np.arange(1, R + 1), 5.0 + 0.01 * np.arange(T + 2 - R)])
     holding = np.concatenate([np.full(R, 1.0), np.full(T + 2 - R, 100.0)])
     src, dst = np.zeros(T + 2, np.int32), np.ones(T + 2, np.int32)
     env = OpticalVecEnv("RWA-v0", n, tabs, traffic="trace", record_decisions=True, link_stats=True, **env_args)
     env.set_trace(*[np.tile(x, (n, 1)) for x in (arrival, holding, src, dst)])
     env.reset(full=True)
+    assert env.kernel_info()["wide"] == (slots == 160), slots
     o = oracle.OracleEnv("RWA-v0", tabs, **helpers.sim_kwargs(dict(kind="RWA-v0", env_args=env_args)))
     o.set_trace(arrival, holding, src, dst)
     o.reset(full=True)
     for t in range(T):
-        act = np.array([0, t % 160], np.int32)
+        act = np.array([0, t % slots], np.int32)
         _, _, _, _ = env.step(torch.as_tensor(np.tile(act, (n, 1)), device="cuda"))
         out = oracle_step(o, act)
-        assert np.array_equal(env.decisions.cpu().numpy()[:, 0], [out.accepted] * n), t
+        assert np.array_equal(env.decisions.cpu().numpy()[:, 0], [out.accepted] * n), (slots, t)
     flags = env.error_flags().cpu().numpy()
-    assert np.all(flags == ERR_STATS_ORDER), flags
+    assert np.all(flags == ERR_STATS_ORDER), (slots, flags)
     oa = o.state()[0]
     avail = env.available_slots().cpu().numpy()
     for i in range(n):
-        assert np.array_equal(avail[i].reshape(oa.shape), oa), i
-    assert np.array_equal(env.export_state()[3].cpu().numpy(), [o.state()[3]] * n)
+        assert np.array_equal(avail[i].reshape(oa.shape), oa), (slots, i)
+    assert np.array_equal(env.export_state()[3].cpu().numpy(), [o.state()[3]] * n), slots
     env.close()
 
 
