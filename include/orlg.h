@@ -224,6 +224,20 @@ int orlg_policy_create(int device, int obs_dim, int hidden, int n_hidden_layers,
  * its results equal those of an orlg_policy_create handle bit for bit. */
 int orlg_policy_create_wide(int device, int obs_dim, int hidden, int n_hidden_layers, int n_actions, const float *weights,
                             const float *biases, orlg_policy **out);
+/* The same policy for an agent that sees SimpleMatrixObservation (rmsa_env.py:806-837) and acts through
+ * PathOnlyFirstFitAction, on RMSA-v0 / RWA-v0: weights and biases as orlg_policy_create with layer 0 SB3's [hidden,
+ * 2 num_nodes + num_links num_slots] matrix (an SB3 checkpoint loads unchanged).  Its calls read PACKED rows
+ * (orlg_matrix_observation_packed): orlg_policy_act / orlg_policy_sample take obs_dev = uint32 [n, W] (16-byte aligned, W =
+ * orlg_matrix_obs_words of the env) through the `const float *` argument.  Layer 0 is repacked to K0 = 64 ceil(2 N / 64) +
+ * 128 NWV E bf16 columns (NWV = ceil(S / 128); link l's slots at 64 ceil(2 N / 64) + 128 NWV l + s, padding zero), kept in a
+ * device buffer and streamed 64 columns at a time through a ring of shared-memory stages by every tile.  Shared memory is
+ * (n_hidden_layers - 1) hidden^2 2 + 16 hidden 2 + G (32768 + stages hidden 128 + seg 2048 + 64) + (n_hidden_layers hidden
+ * + 16) 4 + 64 bytes: G = 2 tile groups with the deepest ring (stages 6, 4 or 3; seg 8, 4, 2 or 1) that fits in 232448, else
+ * G = 1, else ORLG_E_UNSUPPORTED with the byte count.  Refused before any device access: the hidden rules of
+ * orlg_policy_create, n_actions outside 1..15, num_nodes outside 2..255, num_slots outside 1..512, num_links outside
+ * 1..4096.  orlg_policy_sample_masked refuses these handles. */
+int orlg_policy_create_matrix(int device, int num_nodes, int num_links, int num_slots, int hidden, int n_hidden_layers, int n_actions,
+                              const float *weights, const float *biases, orlg_policy **out);
 /* tile groups per CTA of the handle's launches: 2 (every orlg_policy_create handle), or 1; 0 for NULL */
 int orlg_policy_tile_groups(const orlg_policy *pol);
 /* actions_dev int32 [n]; logits_dev float32 [n, n_actions + 1] = logits then value (NULL: skip) */
@@ -259,8 +273,15 @@ int orlg_policy_sample(orlg_policy *pol, const float *obs_dev, int n, const orlg
 int orlg_rollout_policy(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
                         float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
                         float *reward_dev, uint8_t *done_dev, orlg_stream stream);
+/* RMSA-v0 / RWA-v0 (PathOnlyFirstFitAction(SimpleMatrixObservation(env)) with an SB3 agent): actor and optional critic from
+ * orlg_policy_create_matrix with the env's (nodes, links, slots) and the actor's n_actions = k + allow_rejection.  obs_dev
+ * then holds packed rows uint32 [steps + 1, N, orlg_matrix_obs_words] and actions_dev the agent's path actions [steps, N];
+ * per step the actor, the critic, PathOnlyFirstFitAction (into a handle-owned [N, 2] buffer), the step and the packed rows of
+ * obs[t + 1].  A matrix policy on DeepRMSA-v0 or RMCSA-v0, a DeepRMSA policy on RMSA-v0 / RWA-v0 and a layout that differs
+ * from the env's are refused. */
 /* orlg_rollout_policy (= this call with info NULL) that also keeps every step's info: counters_dev and stats_dev as in
- * orlg_rollout_info (DeepRMSA-v0 has neither discrete bit rates nor action probabilities). */
+ * orlg_rollout_info (DeepRMSA-v0 has neither discrete bit rates nor action probabilities; RMSA-v0 adds the per-bit-rate
+ * blocking, RWA-v0 the action probabilities of the mapped actions, as orlg_step counts them). */
 int orlg_rollout_policy_info(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
                              float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev,
                              float *reward_dev, uint8_t *done_dev, const orlg_info_out *info, orlg_stream stream);
@@ -345,6 +366,13 @@ int orlg_action_probability(orlg_env *env, double *out_dev, orlg_stream stream);
  * [nodes], available_slots flattened as (core, link, slot), 1 = free */
 int orlg_matrix_obs_dim(const orlg_env *env);   /* 2*nodes + cores*links*slots */
 int orlg_matrix_observation(orlg_env *env, uint8_t *out_dev, orlg_stream stream);
+/* The same rows packed as bits, for orlg_policy_create_matrix handles (RMSA-v0 / RWA-v0; other kinds ORLG_E_UNSUPPORTED):
+ * uint32 [num_envs, W], W = orlg_matrix_obs_words = 4 + 4 NWV links (NWV = ceil(slots / 128); 0 for other kinds), a multiple
+ * of 16 bytes.  Word 0 = min(src, dst) | max(src, dst) << 8, words 1..3 = 0; then per link, in link-index order, NWV groups of 4
+ * words: bit b of word w of group v = available_slots[link, 128 v + 32 w + b]; bits at and above slots are 0.  A programmatic
+ * dependent launch whose threads wait before they read. */
+int orlg_matrix_obs_words(const orlg_env *env);
+int orlg_matrix_observation_packed(orlg_env *env, uint32_t *out_dev, orlg_stream stream);
 /* PathOnlyFirstFitAction.action (rmsa_env.py:840-874, rwa_env.py:505-536): path_actions_dev int32 [num_envs]
  * (path index, anything else = reject) -> actions_dev int32 [num_envs, 2] = (path, first-fit slot) or (k, S).
  * RMSA-v0 scans range(0, S - n) like the reference (never the last feasible start), RWA-v0 range(W). */

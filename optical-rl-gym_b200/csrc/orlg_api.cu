@@ -115,6 +115,7 @@ struct orlg_env {
     bool ro_valid = false;                     // the events live in the rollout-private storage (canonical tables are stale)
     HostPipeline host_pipe;
     int *ro_actions = nullptr;    // [n, action_dim] scratch of the generic (kernel-per-step) rollout
+    int *ro_mapped = nullptr;     // [n, 2] the PathOnlyFirstFitAction actions of orlg_rollout_policy on RMSA-v0 / RWA-v0
 
     ~orlg_env() { for (void *ptr : allocs) cudaFree(ptr); }
 };
@@ -1049,6 +1050,29 @@ int orlg_matrix_observation(orlg_env *env, uint8_t *out_dev, orlg_stream stream)
     return ORLG_OK;
 }
 
+int orlg_matrix_obs_words(const orlg_env *env) {
+    return env && (env->p.kind == ORLG_RMSA || env->p.kind == ORLG_RWA) ? 4 + 4 * ((env->p.S + 127) / 128) * env->p.E : 0;
+}
+
+// the packed rows, a programmatic dependent launch (matrix_observation_packed_kernel waits in every thread)
+static int launch_matrix_packed(const orlg_env *env, uint32_t *out_dev, cudaStream_t s) {
+    const long long total = (long long)orlg_matrix_obs_words(env) * env->p.n;
+    long long blocks = (total + 255) / 256;
+    if (blocks > 148LL * 32) blocks = 148LL * 32;
+    cudaLaunchConfig_t cfg = pdl_config((int)blocks, 256, 0, s);
+    unsigned *out = out_dev;
+    CUDA_OK(cudaLaunchKernelEx(&cfg, matrix_observation_packed_kernel, env->p, out));
+    return ORLG_OK;
+}
+
+int orlg_matrix_observation_packed(orlg_env *env, uint32_t *out_dev, orlg_stream stream) {
+    if (!env || !out_dev) return fail(ORLG_E_INVALID, "null handle or buffer");
+    if (env->p.kind != ORLG_RMSA && env->p.kind != ORLG_RWA)
+        return fail(ORLG_E_UNSUPPORTED, "packed matrix observations exist for RMSA-v0 and RWA-v0 (one core, the agents of PathOnlyFirstFitAction)");
+    DeviceGuard guard(env->device);
+    return launch_matrix_packed(env, out_dev, (cudaStream_t)stream);
+}
+
 int orlg_path_only_first_fit(orlg_env *env, const int32_t *path_actions_dev, int32_t *actions_dev, orlg_stream stream) {
     if (!env || !path_actions_dev || !actions_dev) return fail(ORLG_E_INVALID, "null handle or buffer");
     DeviceGuard guard(env->device);
@@ -1384,17 +1408,24 @@ struct orlg_policy {
     bool general;                     // ORLG_POLICY_GENERAL at orlg_policy_create: the run-time (H, L) instance also for 5 x 128
     bool wide = false;                // orlg_policy_create_wide: the WIDE instances (layer 0 in chunks of 64 inputs, up to 256)
     int groups = PL_GROUPS;           // tile groups per CTA (PL_WG threads each): 2, or 1 for a wide handle whose weights leave room for one
-    void *w_dev = nullptr, *b_dev = nullptr;
+    bool matrix = false;              // orlg_policy_create_matrix: the MATRIX instances, packed matrix rows, layer 0 streamed from w0_dev
+    PolicyMatrix mx = {};             // their layout and ring (all zero on other handles)
+    void *w_dev = nullptr, *b_dev = nullptr, *w0_dev = nullptr;
 
-    ~orlg_policy() { cudaFree(w_dev); cudaFree(b_dev); }
+    ~orlg_policy() { cudaFree(w_dev); cudaFree(b_dev); cudaFree(w0_dev); }
 };
 
 }  // extern "C"
 
-// The one place that picks the kernel instance of a handle: a wide handle runs the WIDE instance, the shipped agent's 5 x 128
-// has one compiled for it, every other architecture runs the instance that reads H and L from PolicyParams.
+// The one place that picks the kernel instance of a handle: a matrix handle runs the MATRIX instance (none masked: NULL), a wide
+// handle the WIDE instance, the shipped agent's 5 x 128 has one compiled for it, every other architecture runs the instance that
+// reads H and L from PolicyParams.
 template <bool SAMPLE, bool MASKED = false>
 static decltype(&mlp_policy_kernel<SAMPLE, 0, 0>) policy_kernel(const orlg_policy *pol) {
+    if (pol->matrix) {
+        if constexpr (MASKED) return nullptr;
+        else return mlp_policy_kernel<SAMPLE, 0, 0, false, false, true>;
+    }
     if (pol->wide) return mlp_policy_kernel<SAMPLE, 0, 0, MASKED, true>;
     if (pol->pp.H == 128 && pol->pp.L == 5 && !pol->general) return mlp_policy_kernel<SAMPLE, 128, 5, MASKED>;
     return mlp_policy_kernel<SAMPLE, 0, 0, MASKED>;
@@ -1409,25 +1440,39 @@ static unsigned short f32_to_bf16(float f) {          // round to nearest even
     return (unsigned short)((u + 0x7fffu + ((u >> 16) & 1u)) >> 16);
 }
 
-// the shape checks of both create calls have passed: pack and upload the weights, make the handle
+// the shape checks of the create calls have passed: pack and upload the weights, make the handle.  mx: a matrix handle (its
+// layout, ring and row stage; w0 is filled in here)
 static int policy_build(int device, int obs_dim, int H, int L, int n_actions, const float *weights, const float *biases, bool wide,
-                        int groups, orlg_policy **out) {
+                        int groups, orlg_policy **out, const PolicyMatrix *mx = nullptr) {
     int n_dev = 0;
     if (cudaGetDeviceCount(&n_dev) != cudaSuccess || device < 0 || device >= n_dev) return fail(ORLG_E_CUDA, "no such CUDA device");
     DeviceGuard guard(device);
     // bf16 weights in the shared-memory operand layout of the kernel: layer l is an [N x K] K-major operand, K = K0 (the
-    // padded observation: 64, or obs_dim rounded up to 16 on a wide handle) for layer 0, H after it
-    const int K0 = wide ? (obs_dim + 15) & ~15 : PL_K0;
+    // padded observation: 64, or obs_dim rounded up to 16 on a wide handle) for layer 0, H after it.  A matrix handle keeps
+    // layer 0 apart ([H x K0m] in the same layout, K0m = 64 hdr_chunks + 128 nwv links, streamed by the kernel): the resident
+    // blob starts at layer 1.
+    const int K0 = mx ? 0 : wide ? (obs_dim + 15) & ~15 : PL_K0;
     const size_t bytes = pl_weight_bytes(H, L, K0);
-    const size_t smem = pl_smem_bytes(H, L, K0, groups);
-    std::vector<unsigned short> blob(bytes / 2, 0);
+    const size_t smem = mx ? pl_matrix_smem_bytes(H, L, groups, mx->stages, mx->seg_q) : pl_smem_bytes(H, L, K0, groups);
+    std::vector<unsigned short> blob(bytes / 2, 0), blob0;
     std::vector<float> bias((size_t)L * H + PL_NOUT, 0.0f);
     const float *w = weights, *b = biases;
     size_t off = 0;
     for (int l = 0; l < L; l++) {
         const int K = l == 0 ? obs_dim : H, Kp = l == 0 ? K0 : H;
-        for (int r = 0; r < H; r++)
-            for (int k = 0; k < K; k++) blob[(off + pl_operand_offset(H, r, k)) / 2] = f32_to_bf16(w[(size_t)r * K + k]);
+        if (l == 0 && mx) {
+            // header: the 2 N one-hot columns; link e's slot s at column 64 hdr_chunks + 128 nwv e + s; the rest stays zero
+            const int N2 = 2 * mx->nodes, hdr = 64 * mx->hdr_chunks, K0m = hdr + 128 * mx->nwv * mx->links;
+            blob0.assign((size_t)H * K0m, 0);
+            for (int r = 0; r < H; r++)
+                for (int k = 0; k < K; k++) {
+                    const int col = k < N2 ? k : hdr + 128 * mx->nwv * ((k - N2) / mx->slots) + (k - N2) % mx->slots;
+                    blob0[(size_t)pl_operand_offset(H, r, col) / 2] = f32_to_bf16(w[(size_t)r * K + k]);
+                }
+        } else {
+            for (int r = 0; r < H; r++)
+                for (int k = 0; k < K; k++) blob[(off + pl_operand_offset(H, r, k)) / 2] = f32_to_bf16(w[(size_t)r * K + k]);
+        }
         for (int r = 0; r < H; r++) bias[(size_t)l * H + r] = b[r];
         w += (size_t)H * K; b += H; off += (size_t)H * Kp * 2;
     }
@@ -1443,6 +1488,14 @@ static int policy_build(int device, int obs_dim, int H, int L, int n_actions, co
         cudaMemcpy(pol->w_dev, blob.data(), bytes, cudaMemcpyHostToDevice) != cudaSuccess ||
         cudaMemcpy(pol->b_dev, bias.data(), bias.size() * 4, cudaMemcpyHostToDevice) != cudaSuccess)
         return fail(ORLG_E_NOMEM, "policy weight upload failed");
+    if (mx) {
+        pol->matrix = true;
+        pol->mx = *mx;
+        if (cudaMalloc(&pol->w0_dev, blob0.size() * 2) != cudaSuccess ||
+            cudaMemcpy(pol->w0_dev, blob0.data(), blob0.size() * 2, cudaMemcpyHostToDevice) != cudaSuccess)
+            return fail(ORLG_E_NOMEM, "policy layer-0 weight upload failed");
+        pol->mx.w0 = reinterpret_cast<const uint4 *>(pol->w0_dev);
+    }
     pol->pp.w_blob = reinterpret_cast<const uint4 *>(pol->w_dev);
     pol->pp.w_bytes = (int)bytes;
     pol->pp.bias = reinterpret_cast<const float *>(pol->b_dev);
@@ -1451,6 +1504,7 @@ static int policy_build(int device, int obs_dim, int H, int L, int n_actions, co
     pol->smem = smem;
     // the attribute only raises a kernel's limit: a larger policy made earlier on this device keeps its launches valid
     for (auto kernel : {policy_kernel<false>(pol.get()), policy_kernel<true>(pol.get()), policy_kernel<true, true>(pol.get())}) {
+        if (!kernel) continue;
         cudaFuncAttributes fa;
         const int have = cudaFuncGetAttributes(&fa, kernel) == cudaSuccess ? fa.maxDynamicSharedSizeBytes : 0;
         if (have < (int)smem && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
@@ -1505,6 +1559,44 @@ int orlg_policy_create_wide(int device, int obs_dim, int hidden, int n_hidden_la
     return policy_build(device, obs_dim, H, L, n_actions, weights, biases, true, groups, out);
 }
 
+int orlg_policy_create_matrix(int device, int num_nodes, int num_links, int num_slots, int hidden, int n_hidden_layers, int n_actions,
+                              const float *weights, const float *biases, orlg_policy **out) {
+    if (!weights || !biases || !out) return fail(ORLG_E_INVALID, "null argument");
+    *out = nullptr;
+    if (hidden < 16 || hidden > PL_HMAX || hidden % 16)
+        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs a hidden width that is a multiple of 16 in 16..128; got " +
+                                            std::to_string(hidden));
+    if (n_hidden_layers < 1)
+        return fail(ORLG_E_UNSUPPORTED, "the fused policy kernel needs at least one hidden layer; got " + std::to_string(n_hidden_layers));
+    if (n_actions < 1 || n_actions + 1 > PL_NOUT)
+        return fail(ORLG_E_UNSUPPORTED, "the matrix policy kernel takes 1..15 actions; got " + std::to_string(n_actions));
+    if (num_nodes < 2 || num_nodes > 255)
+        return fail(ORLG_E_UNSUPPORTED, "the matrix policy kernel takes 2..255 nodes (one byte per node id); got " + std::to_string(num_nodes));
+    if (num_slots < 1 || num_slots > 512)
+        return fail(ORLG_E_UNSUPPORTED, "the matrix policy kernel takes 1..512 slots; got " + std::to_string(num_slots));
+    if (num_links < 1 || num_links > 4096)
+        return fail(ORLG_E_UNSUPPORTED, "the matrix policy kernel takes 1..4096 links; got " + std::to_string(num_links));
+    const int H = hidden, L = n_hidden_layers;
+    PolicyMatrix mx = {};
+    mx.nodes = num_nodes; mx.links = num_links; mx.slots = num_slots;
+    mx.nwv = (num_slots + 127) / 128;
+    mx.hdr_chunks = (2 * num_nodes + 63) / 64;
+    mx.link_chunks = (num_slots + 63) / 64;
+    // two tile groups if any ring fits next to them, else one; per group the deepest ring and the largest row stage that fit
+    static const int RING[][2] = {{6, 8}, {4, 8}, {3, 8}, {3, 4}, {3, 2}, {3, 1}};
+    int groups = 0;
+    for (int g = 2; g >= 1 && !groups; g--)
+        for (const auto &rs : RING)
+            if (pl_matrix_smem_bytes(H, L, g, rs[0], rs[1]) <= (size_t)PL_SMEM_MAX) { groups = g; mx.stages = rs[0]; mx.seg_q = rs[1]; break; }
+    if (!groups) {
+        const size_t smem = pl_matrix_smem_bytes(H, L, 1, 3, 1);
+        return fail(ORLG_E_UNSUPPORTED, "the matrix policy kernel needs " + std::to_string(smem) + " bytes of shared memory with one " +
+                                            "tile group, " + std::to_string(PL_SMEM_MAX) + " available, for " + std::to_string(L) +
+                                            " hidden layers of " + std::to_string(H));
+    }
+    return policy_build(device, 2 * num_nodes + num_links * num_slots, H, L, n_actions, weights, biases, false, groups, out, &mx);
+}
+
 int orlg_policy_tile_groups(const orlg_policy *pol) { return pol ? pol->groups : 0; }
 
 }  // extern "C"
@@ -1516,9 +1608,11 @@ static int launch_policy(const orlg_policy *pol, const float *obs_dev, int n, in
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, pol->device);
     const int pairs = ((n + PL_TILE - 1) / PL_TILE + pol->groups - 1) / pol->groups;
+    if (pol->matrix && (reinterpret_cast<uintptr_t>(obs_dev) & 15))
+        return fail(ORLG_E_INVALID, "a matrix policy reads packed rows from a 16-byte aligned buffer");
     cudaLaunchConfig_t cfg = pdl_config(pairs < sms ? pairs : sms, PL_WG * pol->groups, pol->smem, s);
     int *actions = actions_dev;
-    CUDA_OK(cudaLaunchKernelEx(&cfg, policy_kernel<SAMPLE, MASKED>(pol), pol->pp, obs_dev, n, actions, logits_dev, dr));
+    CUDA_OK(cudaLaunchKernelEx(&cfg, policy_kernel<SAMPLE, MASKED>(pol), pol->pp, obs_dev, n, actions, logits_dev, dr, pol->mx));
     return ORLG_OK;
 }
 
@@ -1558,6 +1652,7 @@ int orlg_policy_sample_masked(orlg_policy *pol, const float *obs_dev, int n, con
                               int32_t *actions_dev, float *log_prob_dev, float *value_dev, orlg_stream stream) {
     if (!pol || !obs_dev || !draw || n < 0) return fail(ORLG_E_INVALID, "null policy, observation buffer or draw");
     if (!mask_dev) return fail(ORLG_E_INVALID, "orlg_policy_sample_masked needs mask_dev (uint8 [n, n_actions])");
+    if (pol->matrix) return fail(ORLG_E_UNSUPPORTED, "a matrix policy has no masked sampling (PathOnlyFirstFitAction has no action masks)");
     if (n == 0) return ORLG_OK;
     DeviceGuard guard(pol->device);
     PolicyDraw dr = policy_draw(*draw, log_prob_dev, value_dev);
@@ -1567,21 +1662,45 @@ int orlg_policy_sample_masked(orlg_policy *pol, const float *obs_dev, int n, con
 
 }  // extern "C"
 
-// orlg_rollout_policy_info (masked = false) and orlg_rollout_policy_masked: the one loop of both
+// orlg_rollout_policy_info (masked = false) and orlg_rollout_policy_masked: the one loop of both.  DeepRMSA-v0: the policy reads
+// the env's float32 observation.  RMSA-v0 / RWA-v0: a matrix actor (orlg_policy_create_matrix) reads the packed matrix rows and
+// picks a path, PathOnlyFirstFitAction maps it to (path, first-fit slot) for the step.
 static int rollout_policy_impl(orlg_env *env, int steps, orlg_policy *actor, orlg_policy *critic, uint64_t seed, int deterministic,
                                float *obs_dev, int32_t *actions_dev, float *log_prob_dev, float *value_dev, float *reward_dev,
                                uint8_t *done_dev, bool masked, uint8_t *masks_dev, const orlg_info_out *info, orlg_stream stream) {
     if (!env || !actor) return fail(ORLG_E_INVALID, "null env or actor handle");
     const Params &p = env->p;
-    if (p.kind != ORLG_DEEPRMSA) return fail(ORLG_E_UNSUPPORTED, "orlg_rollout_policy drives DeepRMSA-v0 (the env kind with a tensor observation)");
-    if (p.obs_f64) return fail(ORLG_E_UNSUPPORTED, "orlg_rollout_policy needs float32 observations (the policy kernel reads float32)");
-    if (actor->pp.obs_dim != p.obs_dim)
-        return fail(ORLG_E_INVALID, "actor obs_dim " + std::to_string(actor->pp.obs_dim) + " != env obs_dim " + std::to_string(p.obs_dim));
-    const int n_act = p.k * p.J + p.allow_rejection;
-    if (actor->pp.n_actions != n_act)
-        return fail(ORLG_E_INVALID, "actor n_actions " + std::to_string(actor->pp.n_actions) + " != k * j + allow_rejection = " + std::to_string(n_act));
-    if (critic && critic->pp.obs_dim != p.obs_dim)
-        return fail(ORLG_E_INVALID, "critic obs_dim " + std::to_string(critic->pp.obs_dim) + " != env obs_dim " + std::to_string(p.obs_dim));
+    const bool matrix = p.kind == ORLG_RMSA || p.kind == ORLG_RWA;
+    int n_act;
+    if (matrix) {
+        if (masked) return fail(ORLG_E_UNSUPPORTED, "orlg_rollout_policy_masked drives DeepRMSA-v0 (PathOnlyFirstFitAction has no action masks)");
+        if (!actor->matrix || (critic && !critic->matrix))
+            return fail(ORLG_E_UNSUPPORTED, "on RMSA-v0 / RWA-v0 orlg_rollout_policy drives matrix-observation policies (orlg_policy_create_matrix) "
+                                            "through PathOnlyFirstFitAction; this one reads the DeepRMSA-v0 observation");
+        for (const orlg_policy *pol : {actor, critic})
+            if (pol && (pol->mx.nodes != p.N || pol->mx.links != p.E || pol->mx.slots != p.S))
+                return fail(ORLG_E_INVALID, std::string(pol == actor ? "actor" : "critic") + " matrix layout (" + std::to_string(pol->mx.nodes) +
+                                                " nodes, " + std::to_string(pol->mx.links) + " links, " + std::to_string(pol->mx.slots) +
+                                                " slots) != env (" + std::to_string(p.N) + ", " + std::to_string(p.E) + ", " + std::to_string(p.S) + ")");
+        n_act = p.k + p.allow_rejection;
+        if (actor->pp.n_actions != n_act)
+            return fail(ORLG_E_INVALID, "actor n_actions " + std::to_string(actor->pp.n_actions) + " != k + allow_rejection = " + std::to_string(n_act) +
+                                            " (PathOnlyFirstFitAction's Discrete(k + rej))");
+    } else {
+        if (p.kind != ORLG_DEEPRMSA)
+            return fail(ORLG_E_UNSUPPORTED, "orlg_rollout_policy drives DeepRMSA-v0 (the env kind with a tensor observation), and RMSA-v0 / "
+                                            "RWA-v0 through PathOnlyFirstFitAction");
+        if (actor->matrix || (critic && critic->matrix))
+            return fail(ORLG_E_UNSUPPORTED, "a matrix-observation policy reads RMSA-v0 / RWA-v0 rows, not the DeepRMSA-v0 observation");
+        if (p.obs_f64) return fail(ORLG_E_UNSUPPORTED, "orlg_rollout_policy needs float32 observations (the policy kernel reads float32)");
+        if (actor->pp.obs_dim != p.obs_dim)
+            return fail(ORLG_E_INVALID, "actor obs_dim " + std::to_string(actor->pp.obs_dim) + " != env obs_dim " + std::to_string(p.obs_dim));
+        n_act = p.k * p.J + p.allow_rejection;
+        if (actor->pp.n_actions != n_act)
+            return fail(ORLG_E_INVALID, "actor n_actions " + std::to_string(actor->pp.n_actions) + " != k * j + allow_rejection = " + std::to_string(n_act));
+        if (critic && critic->pp.obs_dim != p.obs_dim)
+            return fail(ORLG_E_INVALID, "critic obs_dim " + std::to_string(critic->pp.obs_dim) + " != env obs_dim " + std::to_string(p.obs_dim));
+    }
     if (actor->device != env->device || (critic && critic->device != env->device))
         return fail(ORLG_E_INVALID, "policy and env handles live on different devices");
     if (!obs_dev) return fail(ORLG_E_INVALID, "orlg_rollout_policy needs obs_dev (the policy reads it)");
@@ -1592,13 +1711,21 @@ static int rollout_policy_impl(orlg_env *env, int steps, orlg_policy *actor, orl
     DeviceGuard guard(env->device);
     cudaStream_t s = (cudaStream_t)stream;
     int rc = ensure_canonical(env, s);          // the handle may have been stepped by the persistent rollout kernel
-    if (!rc) rc = orlg_observation(env, obs_dev, stream);
+    if (!rc) rc = matrix ? launch_matrix_packed(env, reinterpret_cast<uint32_t *>(obs_dev), s) : orlg_observation(env, obs_dev, stream);
     if (rc) return rc;
     if (!actions_dev && steps > 0 && !env->ro_actions) {
-        rc = dev_alloc(env, &env->ro_actions, (size_t)p.n, false);
+        rc = dev_alloc(env, &env->ro_actions, (size_t)p.n * orlg_action_dim(env), false);
         if (rc) return rc;
     }
-    const size_t n = (size_t)p.n, row = n * (size_t)p.obs_dim;
+    if (matrix && steps > 0 && !env->ro_mapped) {
+        rc = dev_alloc(env, &env->ro_mapped, (size_t)p.n * 2, false);
+        if (rc) return rc;
+    }
+    // per step: actor, critic, [PathOnlyFirstFitAction], step, [packed rows of obs[t + 1]].  The policy kernel waits on its
+    // immediate predecessor only (programmatic dependent launch), so every kernel in between must not finish before the ones
+    // ahead of it: the critic (a policy launch) and matrix_observation_packed_kernel wait in every thread before they read or
+    // exit, path_only_first_fit_kernel and the step kernels are ordinary launches, which start after their predecessor ends.
+    const size_t n = (size_t)p.n, row = n * (size_t)(matrix ? orlg_matrix_obs_words(env) : p.obs_dim);
     orlg_policy_draw d;
     d.seed = seed; d.counter_dev = p.req_index; d.counter = 0; d.deterministic = deterministic; d.row_id_base = p.env_id_base;
     for (int t = 0; t < steps; t++) {
@@ -1614,10 +1741,15 @@ static int rollout_policy_impl(orlg_env *env, int steps, orlg_policy *actor, orl
             rc = launch_policy<true>(actor, o, p.n, a, nullptr, dr, s);
         }
         if (!rc && critic && v) rc = launch_policy<true>(critic, o, p.n, nullptr, nullptr, policy_draw(d, nullptr, v), s);
-        if (!rc) rc = step_impl(env, a, -1, nullptr, obs_dev + (size_t)(t + 1) * row, reward_dev ? reward_dev + (size_t)t * n : nullptr,
-                                done_dev ? done_dev + (size_t)t * n : nullptr, nullptr,
+        if (!rc && matrix) {
+            for_words(p.nwv, [&](auto W) { path_only_first_fit_kernel<decltype(W)::value><<<(p.n + 127) / 128, 128, 0, s>>>(p, a, env->ro_mapped); });
+            rc = cudaGetLastError() == cudaSuccess ? ORLG_OK : fail(ORLG_E_CUDA, "path_only_first_fit_kernel launch failed");
+        }
+        if (!rc) rc = step_impl(env, matrix ? env->ro_mapped : a, -1, nullptr, matrix ? nullptr : obs_dev + (size_t)(t + 1) * row,
+                                reward_dev ? reward_dev + (size_t)t * n : nullptr, done_dev ? done_dev + (size_t)t * n : nullptr, nullptr,
                                 info && info->counters_dev ? info->counters_dev + (size_t)t * n * 8 : nullptr, stream);
         if (!rc && info) rc = info_row(env, info, t, stream);
+        if (!rc && matrix) rc = launch_matrix_packed(env, reinterpret_cast<uint32_t *>(obs_dev + (size_t)(t + 1) * row), s);
         if (rc) return rc;
     }
     if (value_dev)                              // the bootstrap value of the last observation

@@ -36,6 +36,20 @@ struct PolicyParams {
     int H, L;                         // hidden width (multiple of 16, 16..128) and number of hidden layers (>= 1)
 };
 
+// MATRIX instances (orlg_policy_create_matrix): the agent reads SimpleMatrixObservation rows packed as bits (orlg_matrix_observation
+// _packed): uint32 [n, W], W = 4 + 4 NWV E, word 0 = min(src, dst) | max(src, dst) << 8, then per link NWV groups of 4 words,
+// bit b of word w of group v = slot 128 v + 32 w + b.  Layer 0 has K0 = 64 ceil(2 N / 64) + 128 NWV E columns: the one-hot
+// header, then link l's slots at 128 NWV l + s.  It does not fit in shared memory (360 KB at NSFNET / S = 100 / H = 64): it
+// stays in a device buffer and every tile streams it, 64 columns (H x 128 bytes) at a time, through a ring of `stages` buffers
+// per tile group; chunks whose 64 columns are all padding (slots >= S) are skipped.
+constexpr int PL_MX_RMAX = 6;         // most ring stages per tile group
+struct PolicyMatrix {
+    const uint4 *w0;                  // layer 0, bf16, [K0 / 64 chunks][H x 64 operand] (chunk c at c * H * 128 bytes); NULL = not MATRIX
+    int nodes, links, slots, nwv;     // N, E, S, 128-bit word groups per link (ceil(S / 128))
+    int hdr_chunks, link_chunks;      // ceil(2 N / 64); ceil(S / 64): the chunks of a link that hold slots
+    int stages, seg_q;                // ring stages per group (3..PL_MX_RMAX); 16-byte words per row of the row stage (1..8)
+};
+
 // bytes of weights and of dynamic shared memory of a policy with hidden width H, L hidden layers, layer 0 padded to K0 inputs
 // and G tile groups per CTA (the 2-argument forms: K0 = 64, G = 2, the instances of orlg_policy_create)
 inline size_t pl_weight_bytes(int H, int L, int K0) {
@@ -47,6 +61,11 @@ inline size_t pl_smem_bytes(int H, int L, int K0, int G) {
     return pl_weight_bytes(H, L, K0) + (size_t)G * PL_TILE * PL_HMAX * 2 + ((size_t)L * H + PL_NOUT) * 4 + 64;
 }
 inline size_t pl_smem_bytes(int H, int L) { return pl_smem_bytes(H, L, PL_K0, PL_GROUPS); }
+// a MATRIX handle: the resident weights are layers 1.. and the heads (K0 = 0), and each group adds its ring, its row stage and
+// 2 + PL_MX_RMAX mbarriers
+inline size_t pl_matrix_smem_bytes(int H, int L, int G, int stages, int seg_q) {
+    return pl_smem_bytes(H, L, 0, G) + (size_t)G * ((size_t)stages * H * 128 + (size_t)seg_q * PL_TILE * 16 + (2 + PL_MX_RMAX) * 8);
+}
 
 // The sampling epilogue (mlp_policy_kernel<true>, orlg_policy_sample): one Philox4x32-10 block per row, key = seed,
 // counter = (c0, 0, row_id_base + row, 3) -- stream 3 of DESIGN.md section 5 -- where c0 = counter_dev[row] (the env's
@@ -226,27 +245,38 @@ __device__ __forceinline__ void pl_group_sync(int group) {          // named bar
 // WIDE (run-time H, L only; orlg_policy_create_wide): observations up to 256 wide, any parity.  Layer 0 has K0 = obs_dim
 // rounded up to 16 inputs and runs in chunks of 64 columns through the A buffer (see the staging block), and the CTA has
 // G = blockDim.x / PL_WG tile groups (1 or 2: what fits in shared memory next to the larger layer-0 weights).
-template <bool SAMPLE, int HC, int LC, bool MASKED = false, bool WIDE = false>
+// MATRIX (run-time H, L, act and sample only; orlg_policy_create_matrix): `obs` is packed matrix rows (PolicyMatrix), layer 0
+// streamed through a ring (see the MATRIX block); G as for WIDE.  `mx` is read by the MATRIX instances only.
+template <bool SAMPLE, int HC, int LC, bool MASKED = false, bool WIDE = false, bool MATRIX = false>
 __global__ void __launch_bounds__(PL_WG * PL_GROUPS, 1)
 mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const int n, int *__restrict__ actions,
-                  float *__restrict__ logits_out /* [n, n_actions + 1] = logits + value, or NULL */, const PolicyDraw dr) {
+                  float *__restrict__ logits_out /* [n, n_actions + 1] = logits + value, or NULL */, const PolicyDraw dr,
+                  const PolicyMatrix mx) {
     extern __shared__ __align__(128) unsigned char psm[];
     const int H = HC ? HC : pp.H, L = LC ? LC : pp.L;
-    const int G = WIDE ? (int)(blockDim.x / PL_WG) : PL_GROUPS;                   // tile groups of this CTA
+    const int G = WIDE || MATRIX ? (int)(blockDim.x / PL_WG) : PL_GROUPS;         // tile groups of this CTA
     const int K0 = WIDE ? (pp.obs_dim + 15) & ~15 : PL_K0;                        // layer-0 inputs
     const int nch = WIDE ? (K0 + 63) >> 6 : 1;                                    // layer-0 chunks of 64 columns
     const int group = threadIdx.x / PL_WG, tid = threadIdx.x % PL_WG, warp = (tid >> 5) & 3;     // warp = TMEM lane quarter of this warp
     const int half = tid >> 7;        // which half of the H columns (K elements of the next layer) this thread produces
     unsigned char *s_w = psm;
     unsigned char *s_a = psm + pp.w_bytes + (size_t)group * PL_TILE * PL_HMAX * 2;
-    float *s_bias = reinterpret_cast<float *>(psm + pp.w_bytes + (size_t)G * PL_TILE * PL_HMAX * 2);
-    unsigned long long *bars = reinterpret_cast<unsigned long long *>(s_bias + L * H + PL_NOUT);   // [0] weights, [1 + g] mma of group g
-    unsigned *s_tmem = reinterpret_cast<unsigned *>(bars + 1 + G);
+    // MATRIX: [G][stages][H x 128 B] ring, then [G][seg_q][128 rows x 16 B] row stage, after the A buffers
+    const size_t mx_ring = MATRIX ? (size_t)mx.stages * H * 128 : 0, mx_stage = MATRIX ? (size_t)mx.seg_q * PL_TILE * 16 : 0;
+    unsigned char *s_ring = psm + pp.w_bytes + (size_t)G * PL_TILE * PL_HMAX * 2 + (size_t)group * mx_ring;
+    unsigned char *s_rows = psm + pp.w_bytes + (size_t)G * (PL_TILE * PL_HMAX * 2 + mx_ring) + (size_t)group * mx_stage;
+    float *s_bias = reinterpret_cast<float *>(psm + pp.w_bytes + (size_t)G * PL_TILE * PL_HMAX * 2 + (MATRIX ? (size_t)G * (mx_ring + mx_stage) : 0));
+    // [0] weights, [1 + g] mma of group g; MATRIX: [1 + G + (2 + PL_MX_RMAX) g ..] group g's A-half barriers, then its ring stages
+    unsigned long long *bars = reinterpret_cast<unsigned long long *>(s_bias + L * H + PL_NOUT);
+    const int nbars = 1 + G + (MATRIX ? G * (2 + PL_MX_RMAX) : 0);
+    unsigned *s_tmem = reinterpret_cast<unsigned *>(bars + 1 + G + (MATRIX ? G * (2 + PL_MX_RMAX) : 0));
 
     pdl_launch_dependents();
     if (threadIdx.x == 0) {
         mbar_init(&bars[0], 1);
         for (int g = 0; g < G; g++) mbar_init(&bars[1 + g], 1);
+        if (MATRIX)
+            for (int g = 1 + G; g < nbars; g++) mbar_init(&bars[g], 1);
         mbar_expect_tx(&bars[0], (unsigned)pp.w_bytes);
         // the weights do not depend on the previous kernel of the stream: requested before the dependency wait
         const unsigned chunk = 32768u;
@@ -268,6 +298,29 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const unsigned tmem = *s_tmem + (unsigned)group * 128u;           // this warpgroup's accumulator columns
     const unsigned t_lane = tmem + ((unsigned)(warp * 32) << 16);       // this warp's 32 TMEM lanes
+    // MATRIX: layer-0 chunk c of the compact chunk list (header chunks, then each link's chunks that hold slots) -> its first
+    // weight column; chunk gq of this group's stream (continuous over its tiles) goes to ring stage gq % stages
+    const int mnch = MATRIX ? mx.hdr_chunks + mx.links * mx.link_chunks : 0;
+    unsigned long long *abar = bars + 1 + G + (2 + PL_MX_RMAX) * group, *fullb = abar + 2;
+    auto mx_col = [&](int c) {
+        const int lc = c - mx.hdr_chunks;
+        return c < mx.hdr_chunks ? 64 * c : 64 * mx.hdr_chunks + 128 * mx.nwv * (lc / mx.link_chunks) + 64 * (lc % mx.link_chunks);
+    };
+    auto mx_fetch = [&](long long gq) {                                   // thread 0 of the group: chunk gq into its stage
+        const long long t = gq / mnch;
+        if ((long long)(blockIdx.x * G + group + t * gridDim.x * G) * PL_TILE >= n) return;  // past this group's last tile: never consumed
+        const unsigned bytes = (unsigned)H * 128u;
+        unsigned long long *fb = &fullb[gq % mx.stages];
+        mbar_expect_tx(fb, bytes);
+        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                     ::"r"((unsigned)__cvta_generic_to_shared(s_ring + (size_t)(gq % mx.stages) * bytes)),
+                       "l"(reinterpret_cast<const unsigned char *>(mx.w0) + (size_t)(mx_col((int)(gq % mnch)) >> 6) * bytes),
+                       "r"(bytes), "r"((unsigned)__cvta_generic_to_shared(fb)) : "memory");
+    };
+    if (MATRIX && tid == 0)           // the layer-0 weights do not depend on the previous kernel either
+        for (int gq = 0; gq < mx.stages - 2; gq++) mx_fetch(gq);
+    long long mx_gq = 0;
+    unsigned aph = 0u;                // bit h: phase parity of A-half barrier h
     mbar_wait(&bars[0], 0);           // weights have landed
     pdl_wait();                       // the observations come from the previous kernel of the stream
 
@@ -280,7 +333,85 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
     unsigned long long *bar = &bars[1 + group];
     for (int tile = blockIdx.x * G + group; tile * PL_TILE < n; tile += gridDim.x * G) {
         const int env = tile * PL_TILE + row;
-        if (WIDE) {
+        if (MATRIX) {
+            // ---- layer 0 of the MATRIX instance, in chunks of 64 columns.  Chunk c goes to half c & 1 of the A buffer as bf16
+            // 0.0 / 1.0: header chunks from the one-hot positions of word 0, link chunks from 64 bits of each row.  It waits
+            // for chunk c - 2's MMAs (which read that half and whose ring stage the refill below overwrites) on the half's
+            // barrier, so the expansion of chunk c overlaps the MMAs of chunk c - 1.  B is the chunk's ring stage.  The last two
+            // chunks commit nowhere: layer 0 of the layer loop (no MMA of its own) commits after them.
+            // Rows: the tile's 128 packed rows are one contiguous run; 16-byte words seg_q s .. seg_q s + seg_q - 1 of every row
+            // are loaded as consecutive uint4 of each row (coalesced) into the row stage, word qq of row r at
+            // qq * 2048 + ((r ^ qq) & 127) * 16 (consecutive rows on consecutive 16-byte slots for the reads; the XOR spreads the
+            // stores of one row's words over the banks).  A chunk needs one 16-byte word of its row (word 0 for the header).
+            const int U = 1 + mx.nwv * mx.links;                            // 16-byte words per packed row
+            const uint4 *rows4 = reinterpret_cast<const uint4 *>(obs);
+            int seg = -1;
+            for (int c = 0; c < mnch; c++, mx_gq++) {
+                const int h = c & 1;
+                const bool hdr = c < mx.hdr_chunks;
+                const int lc = c - mx.hdr_chunks, lj = hdr ? 0 : lc % mx.link_chunks;
+                const int q = hdr ? 0 : 1 + mx.nwv * (lc / mx.link_chunks) + (lj >> 1);
+                if (q / mx.seg_q != seg) {                                  // (the stage's last readers passed chunk c - 1's sync)
+                    seg = q / mx.seg_q;
+                    const int cnt = min(mx.seg_q, U - seg * mx.seg_q);
+                    uint4 v[4];
+#pragma unroll
+                    for (int i = 0; i < 4; i++) {
+                        const int e = tid + i * PL_WG, r = e / cnt, qq = e - r * cnt;
+                        v[i] = make_uint4(0u, 0u, 0u, 0u);
+                        if (e < PL_TILE * cnt && tile * PL_TILE + r < n) v[i] = rows4[(size_t)(tile * PL_TILE + r) * U + seg * mx.seg_q + qq];
+                    }
+#pragma unroll
+                    for (int i = 0; i < 4; i++) {
+                        const int e = tid + i * PL_WG, r = e / cnt, qq = e - r * cnt;
+                        if (e < PL_TILE * cnt) *reinterpret_cast<uint4 *>(s_rows + qq * 2048 + (((r ^ qq) & 127) << 4)) = v[i];
+                    }
+                    pl_group_sync(group);
+                }
+                if (c >= 2) {                                               // chunk c - 2's MMAs are done
+                    mbar_wait(&abar[h], (aph >> h) & 1u);
+                    aph ^= 1u << h;
+                }
+                if (tid == 0) mx_fetch(mx_gq + mx.stages - 2);              // into the stage chunk c - 2 read
+                const int qq = q - seg * mx.seg_q;
+                const uint4 x = *reinterpret_cast<const uint4 *>(s_rows + qq * 2048 + (((row ^ qq) & 127) << 4));
+                unsigned bits;
+                if (hdr) {                                                  // this thread's columns 64 c + 32 half .. + 31
+                    const int base = 64 * c + 32 * half, lo = (int)(x.x & 0xffu) - base, hi = mx.nodes + (int)((x.x >> 8) & 0xffu) - base;
+                    bits = (lo >= 0 && lo < 32 ? 1u << lo : 0u) | (hi >= 0 && hi < 32 ? 1u << hi : 0u);
+                } else {
+                    const int comp = 2 * (lj & 1) + half;                   // slots 64 lj + 32 half .. + 31 of the link
+                    bits = comp == 0 ? x.x : (comp == 1 ? x.y : (comp == 2 ? x.z : x.w));
+                }
+#pragma unroll
+                for (int j = 0; j < 4; j++) {                               // columns 8 j .. + 7 of this thread's 32
+                    unsigned w4[4];
+#pragma unroll
+                    for (int e = 0; e < 4; e++) {
+                        const unsigned b = bits >> (8 * j + 2 * e);
+                        w4[e] = ((b & 1u) ? 0x3F80u : 0u) | ((b & 2u) ? 0x3F800000u : 0u);
+                    }
+                    *reinterpret_cast<uint4 *>(a_row + (h * 8 + half * 4 + j) * 2048) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
+                }
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                pl_group_sync(group);
+                if (tid == 0) {
+                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    mbar_wait(&fullb[mx_gq % mx.stages], (unsigned)((mx_gq / mx.stages) & 1));
+                    const unsigned idesc = pl_instr_desc(PL_TILE, H);
+                    const unsigned a_lbo = (PL_TILE / 8) * 128, b_lbo = (unsigned)(H / 8) * 128;
+                    const unsigned b_addr = (unsigned)__cvta_generic_to_shared(s_ring + (size_t)(mx_gq % mx.stages) * H * 128);
+#pragma unroll 1
+                    for (int kk = 0; kk < 4; kk++) {
+                        const unsigned long long ad = pl_smem_desc(a_addr + (unsigned)(h * 8 + 2 * kk) * a_lbo, a_lbo, 128u);
+                        const unsigned long long bd = pl_smem_desc(b_addr + (unsigned)(2 * kk) * b_lbo, b_lbo, 128u);
+                        pl_mma(tmem, ad, bd, idesc, c > 0 || kk > 0 ? 1u : 0u);
+                    }
+                    if (c + 2 < mnch) pl_commit(&abar[h]);
+                }
+            }
+        } else if (WIDE) {
             // ---- layer-0 input of the WIDE instance, in chunks of 64 columns.  Chunk c (columns 64 c .. + 63) goes to half c & 1
             // of the A buffer (k blocks 8 (c & 1) .. + 7) as bf16; its fp32 rows are staged, 64 at a time, in the other half.  That
             // half is what chunk c - 1's MMAs read, so chunk c waits for them (their commit, on the group's mbarrier) before its
@@ -402,7 +533,7 @@ mlp_policy_kernel(const PolicyParams pp, const float *__restrict__ obs, const in
         }
         int w_off = 0;                 // byte offset of the current layer's weights in s_w
         for (int layer = 0; layer <= L; layer++) {
-            const int K = layer == 0 ? (WIDE ? K0 - 64 * (nch - 1) : PL_K0) : H;     // WIDE layer 0: its last chunk
+            const int K = layer == 0 ? (MATRIX ? 0 : WIDE ? K0 - 64 * (nch - 1) : PL_K0) : H;     // WIDE layer 0: its last chunk; MATRIX: none
             const int N = layer == L ? PL_NOUT : H;
             const bool chunked = WIDE && layer == 0 && nch > 1;
             // activations written by the generic proxy -> visible to the tensor core (async proxy); previous TMEM reads done

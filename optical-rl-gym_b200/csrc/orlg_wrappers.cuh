@@ -68,4 +68,32 @@ __global__ void matrix_observation_kernel(const Params p, unsigned char *out) {
     }
 }
 
+// The same observation packed as bits (RMSA-v0 / RWA-v0: one core), what the MATRIX policy instances read: uint32 [n, W] with
+// W = 4 + 4 nwv E.  Word 0 = min(src, dst) | max(src, dst) << 8 (the two one-hot positions), words 1..3 = 0; then link l's mask
+// words in link order, word 4 + 4 nwv l + 4 v + w = word w of its 128-bit group v (bit b = slot 128 v + 32 w + b; bits at and
+// above S are 0, as in the masks).  One thread per word, through mask_index: either mask layout.  Launched as a programmatic
+// dependent launch whose threads all wait first, so it may sit between a step kernel and a policy kernel that waits on it only.
+__global__ void matrix_observation_packed_kernel(const Params p, unsigned *out) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const int W = 4 + 4 * p.nwv * p.E;
+    const long long total = (long long)W * p.n;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += stride) {
+        const int env = (int)(idx / W);
+        const int w = (int)(idx - (long long)env * W);
+        unsigned v = 0u;
+        if (w == 0) {
+            const uint2 rq = p.cur_req[env];
+            const unsigned src = rq.x & 0xffu, dst = (rq.x >> 8) & 0xffu;
+            v = min(src, dst) | max(src, dst) << 8;
+        } else if (w >= 4) {
+            const int q = w - 4, l = q / (4 * p.nwv), r = q - l * 4 * p.nwv;
+            const uint4 m = p.masks[mask_index(p, l, r >> 2, env)];
+            v = (r & 3) == 0 ? m.x : ((r & 3) == 1 ? m.y : ((r & 3) == 2 ? m.z : m.w));
+        }
+        out[idx] = v;
+    }
+}
+
 }  // namespace orlg

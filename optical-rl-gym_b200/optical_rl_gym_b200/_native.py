@@ -124,6 +124,9 @@ def lib():
     L.orlg_rollout_policy_masked.argtypes = [vp, i32, vp, vp, C.c_uint64, i32, vp, vp, vp, vp, vp, vp, vp, C.POINTER(InfoOut), vp]
     L.orlg_policy_create_wide.argtypes = [i32, i32, i32, i32, i32, vp, vp, C.POINTER(vp)]
     L.orlg_policy_tile_groups.argtypes = [vp]
+    L.orlg_policy_create_matrix.argtypes = [i32, i32, i32, i32, i32, i32, i32, vp, vp, C.POINTER(vp)]
+    L.orlg_matrix_obs_words.argtypes = [vp]
+    L.orlg_matrix_observation_packed.argtypes = [vp, vp, vp]
     L.orlg_request_index.argtypes = [vp]
     L.orlg_request_index.restype = i64
     L.orlg_rollout_packed.argtypes = [vp, i32, i32, vp, vp, vp]
@@ -146,4 +149,5 @@ EXPORTED = ["orlg_create", "orlg_destroy", "orlg_last_error", "orlg_version", "o
             "orlg_path_only_first_fit", "orlg_rollout", "orlg_state_save_bytes", "orlg_state_save", "orlg_state_load", "orlg_policy_create", "orlg_policy_act", "orlg_policy_destroy", "orlg_rollout_packed", "orlg_expand_packed", "orlg_rollout_host", "orlg_action_hist_dim", "orlg_action_probability",
             "orlg_enable_link_stats", "orlg_link_stats", "orlg_policy_sample", "orlg_rollout_policy", "orlg_request_index",
             "orlg_rollout_info", "orlg_rollout_policy_info", "orlg_action_mask_dim", "orlg_action_masks",
-            "orlg_policy_sample_masked", "orlg_rollout_policy_masked", "orlg_policy_create_wide", "orlg_policy_tile_groups"]
+            "orlg_policy_sample_masked", "orlg_rollout_policy_masked", "orlg_policy_create_wide", "orlg_policy_tile_groups",
+            "orlg_policy_create_matrix", "orlg_matrix_obs_words", "orlg_matrix_observation_packed"]

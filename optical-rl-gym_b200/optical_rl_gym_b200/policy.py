@@ -16,6 +16,11 @@ The kernel takes any trunk of one width H (a multiple of 16 in 16..128) and any 
 (DeepRMSA on germany50 is 126 wide, on a 100-node topology with k = 10 251), the first layer in chunks of 64 inputs; its
 weights take more shared memory, so 5 x 128 fits up to 240 inputs.  At 64 inputs or fewer it gives the same results bit for
 bit.  It is opt-in: the default handles keep the kernel instances and the timing they have.
+``matrix_observation=(nodes, links, slots)`` (``env.matrix_layout``) builds them with ``orlg_policy_create_matrix``: the agent
+of ``PathOnlyFirstFitAction(SimpleMatrixObservation(env))`` on RMSA-v0 / RWA-v0, whose observation is ``2 nodes + links
+slots`` wide (2228 on NSFNET with 100 slots).  The native calls then read the packed rows of
+``env.packed_matrix_observation()`` (int32 ``[N, W]``), the first layer streamed from device memory; :meth:`forward` stays the
+float32 reference on unpacked rows (``env.unpack_matrix_observation``).
 :meth:`sample_native` is the same kernel with a sampling epilogue (``orlg_policy_sample``): sampled or argmax actions, their
 log-probabilities and the value estimate, as PPO's rollout collection needs them.  The native weights follow the module:
 an in-place update (``optimizer.step()``, ``load_state_dict``) rebuilds them at the next call.
@@ -31,9 +36,10 @@ import torch
 
 class MlpPolicy(torch.nn.Module):
     def __init__(self, obs_dim: int = 54, n_actions: int = 5, net_arch: Sequence[int] = (128,) * 5,
-                 wide_observations: bool = False):
+                 wide_observations: bool = False, matrix_observation=None):
         super().__init__()
         self.wide_observations = wide_observations      # native handles from orlg_policy_create_wide (see the module docstring)
+        self.matrix_observation = self._check_layout(matrix_observation, obs_dim, wide_observations)
         layers, d = [], obs_dim
         for width in net_arch:
             layers += [torch.nn.Linear(d, width), torch.nn.Tanh()]
@@ -43,21 +49,37 @@ class MlpPolicy(torch.nn.Module):
         self.value_net = torch.nn.Linear(d, 1)
         self.critic_net = None          # the critic's own trunk when the checkpoint has separate ones (SB3 >= 1.8)
 
+    @staticmethod
+    def _check_layout(layout, obs_dim, wide):
+        """``matrix_observation`` as a tuple of ints (or None), refused with ``ValueError`` when it does not fit."""
+        if layout is None:
+            return None
+        if wide:
+            raise ValueError("matrix_observation and wide_observations exclude each other (the matrix handles stream their "
+                             "first layer)")
+        nodes, links, slots = (int(x) for x in layout)
+        if obs_dim != 2 * nodes + links * slots:
+            raise ValueError("matrix_observation %s has 2 * %d + %d * %d = %d inputs, the policy's obs_dim is %d" % (
+                (nodes, links, slots), nodes, links, slots, 2 * nodes + links * slots, obs_dim))
+        return (nodes, links, slots)
+
     @classmethod
-    def from_state_dict(cls, sd, wide_observations: bool = False) -> "MlpPolicy":
+    def from_state_dict(cls, sd, wide_observations: bool = False, matrix_observation=None) -> "MlpPolicy":
         """``policy.pth`` of an SB3 ``ActorCriticPolicy`` with a shared trunk (keys ``mlp_extractor.shared_net.<2i>``)
         or with separate actor/critic trunks (``mlp_extractor.policy_net`` / ``mlp_extractor.value_net``, SB3 >= 1.8: the
         actor's trunk becomes ``shared_net``, the critic's is kept as ``critic_net``: ``forward``, :meth:`sample_native` and
         ``OpticalVecEnv.rollout_policy`` return its value (a second native handle evaluates it); the value column of
         :meth:`act_native`'s ``logits`` is the actor trunk's, or NaN when ``value_net`` does not fit the actor's trunk).
         ``value_net`` is sized from the checkpoint: with separate trunks it takes the critic's last width.
-        ``wide_observations``: as in the constructor, for the actor's and the critic's handle."""
+        ``wide_observations``, ``matrix_observation``: as in the constructor, for the actor's and the critic's handle (a
+        checkpoint whose observation width is not ``2 nodes + links slots`` is refused with ``ValueError``)."""
         shared = any(k.startswith("mlp_extractor.shared_net.") for k in sd)
         trunk = "mlp_extractor.shared_net." if shared else "mlp_extractor.policy_net."
         idx = sorted({int(k[len(trunk):].split(".")[0]) for k in sd if k.startswith(trunk)})
         widths = [sd["%s%d.weight" % (trunk, i)].shape[0] for i in idx]
         obs_dim = sd["%s%d.weight" % (trunk, idx[0])].shape[1]
-        pol = cls(obs_dim, sd["action_net.weight"].shape[0], widths, wide_observations=wide_observations)
+        pol = cls(obs_dim, sd["action_net.weight"].shape[0], widths, wide_observations=wide_observations,
+                  matrix_observation=matrix_observation)
         if sd["value_net.weight"].shape[1] != pol.value_net.in_features:
             pol.value_net = torch.nn.Linear(sd["value_net.weight"].shape[1], 1)
         mine = {}
@@ -80,10 +102,10 @@ class MlpPolicy(torch.nn.Module):
         return pol
 
     @classmethod
-    def from_sb3_zip(cls, path, device=None, wide_observations: bool = False) -> "MlpPolicy":
+    def from_sb3_zip(cls, path, device=None, wide_observations: bool = False, matrix_observation=None) -> "MlpPolicy":
         with zipfile.ZipFile(path) as z:
             sd = torch.load(io.BytesIO(z.read("policy.pth")), map_location="cpu", weights_only=True)
-        pol = cls.from_state_dict(sd, wide_observations=wide_observations)
+        pol = cls.from_state_dict(sd, wide_observations=wide_observations, matrix_observation=matrix_observation)
         return pol.to(device) if device is not None else pol
 
     # ------------------------------------------------------------------ fused native kernel (csrc/orlg_policy.cuh)
@@ -109,7 +131,7 @@ class MlpPolicy(torch.nn.Module):
         return specs
 
     @staticmethod
-    def _create_handle(device_index: int, spec, wide: bool = False):
+    def _create_handle(device_index: int, spec, wide: bool = False, matrix=None):
         import ctypes as C
 
         import numpy as np
@@ -130,6 +152,11 @@ class MlpPolicy(torch.nn.Module):
         w = np.concatenate([m.weight.detach().float().cpu().numpy().reshape(-1) for m in mats]).astype(np.float32)
         b = np.concatenate([m.bias.detach().float().cpu().numpy().reshape(-1) for m in mats]).astype(np.float32)
         h = C.c_void_p()
+        if matrix is not None:
+            MlpPolicy._check_layout(matrix, obs_dim, False)
+            nat.check(nat.lib().orlg_policy_create_matrix(device_index, *matrix, H, len(lins), heads[0].out_features,
+                                                          w.ctypes.data_as(C.c_void_p), b.ctypes.data_as(C.c_void_p), C.byref(h)))
+            return h
         create = nat.lib().orlg_policy_create_wide if wide else nat.lib().orlg_policy_create
         nat.check(create(device_index, obs_dim, H, len(lins), heads[0].out_features,
                          w.ctypes.data_as(C.c_void_p), b.ctypes.data_as(C.c_void_p), C.byref(h)))
@@ -164,10 +191,15 @@ class MlpPolicy(torch.nn.Module):
 
     def _native_handles(self, device_index: int):
         """(actor handle, critic handle | None) holding the CURRENT weights: rebuilt when a parameter was changed in place
-        (optimizer step, load_state_dict) or moved since the handles were made, or ``wide_observations`` was flipped."""
+        (optimizer step, load_state_dict) or moved since the handles were made, or ``wide_observations`` or
+        ``matrix_observation`` was changed."""
         cache = self.__dict__.setdefault("_native_cache", {})
         wide = bool(self.wide_observations)
-        key = (wide,) + self._weights_key()
+        matrix = self.matrix_observation
+        if matrix is not None and wide:
+            raise ValueError("matrix_observation and wide_observations exclude each other (the matrix handles stream their "
+                             "first layer)")
+        key = (wide, matrix) + self._weights_key()
         entry = cache.get(device_index)
         if entry is not None and entry[0] == key:
             return entry[1], entry[2]
@@ -175,9 +207,10 @@ class MlpPolicy(torch.nn.Module):
             del cache[device_index]
             self._destroy_handles(entry[1:], device_index)
         specs = self._native_specs()
-        actor = self._create_handle(device_index, specs["actor"], wide)
+        flags = (wide,) if matrix is None else (wide, matrix)
+        actor = self._create_handle(device_index, specs["actor"], *flags)
         try:
-            critic = None if specs["critic"] is None else self._create_handle(device_index, specs["critic"], wide)
+            critic = None if specs["critic"] is None else self._create_handle(device_index, specs["critic"], *flags)
         except Exception:
             self._destroy_handles((actor,), device_index)
             raise
@@ -198,6 +231,17 @@ class MlpPolicy(torch.nn.Module):
             pass
 
     def _check_obs(self, obs: torch.Tensor):
+        if self.matrix_observation is not None:           # packed rows (OpticalVecEnv.packed_matrix_observation)
+            from .vec_env import matrix_obs_words
+
+            W = matrix_obs_words(self.matrix_observation)
+            if not (torch.is_tensor(obs) and obs.is_cuda and obs.dtype == torch.int32 and obs.dim() == 2 and obs.shape[1] == W
+                    and obs.is_contiguous() and obs.data_ptr() % 16 == 0):
+                raise ValueError("a matrix_observation policy reads packed observations: a contiguous, 16-byte aligned int32 CUDA "
+                                 "tensor [N, %d] (env.packed_matrix_observation()), got %s %s %s" % (
+                                     W, tuple(obs.shape) if torch.is_tensor(obs) else type(obs).__name__,
+                                     getattr(obs, "dtype", ""), getattr(obs, "device", "")))
+            return obs.shape[0]
         d = self.shared_net[0].in_features
         if not (torch.is_tensor(obs) and obs.is_cuda and obs.dtype == torch.float32 and obs.dim() == 2 and obs.shape[1] == d
                 and obs.is_contiguous()):
@@ -249,6 +293,8 @@ class MlpPolicy(torch.nn.Module):
         from . import _native as nat
 
         n = self._check_obs(obs)
+        if action_masks is not None and self.matrix_observation is not None:
+            raise ValueError("a matrix_observation policy has no masked sampling (PathOnlyFirstFitAction has no action masks)")
         if out is None:
             out = (torch.empty((n, 1), dtype=torch.int32, device=obs.device), torch.empty(n, dtype=torch.float32, device=obs.device),
                    torch.empty(n, dtype=torch.float32, device=obs.device))

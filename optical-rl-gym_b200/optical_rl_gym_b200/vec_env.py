@@ -114,6 +114,32 @@ def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+def matrix_obs_words(layout) -> int:
+    """Words (uint32) of a packed matrix observation row for ``layout = (nodes, links, slots)``: 4 + 4 ceil(slots / 128) links."""
+    _, links, slots = (int(x) for x in layout)
+    return 4 + 4 * ((slots + 127) // 128) * links
+
+
+def unpack_matrix_observation(packed: torch.Tensor, layout, dtype=torch.uint8) -> torch.Tensor:
+    """Packed matrix rows (int32 ``[..., W]``, :meth:`OpticalVecEnv.packed_matrix_observation`) -> the
+    ``SimpleMatrixObservation`` rows ``[..., 2 nodes + links slots]`` of ``dtype``: one-hot(min(src, dst)), one-hot(max(src,
+    dst)), then ``available_slots`` link by link.  Plain torch bit operations on any device (for a learner's minibatches)."""
+    nodes, links, slots = (int(x) for x in layout)
+    W = matrix_obs_words(layout)
+    if packed.shape[-1] != W or packed.dtype != torch.int32:
+        raise ValueError("packed rows must be int32 [..., %d] for layout %s, got %s %s" % (W, (nodes, links, slots), packed.dtype,
+                                                                                         tuple(packed.shape)))
+    lead, dev = packed.shape[:-1], packed.device
+    w0 = packed[..., 0]
+    ids = torch.arange(nodes, device=dev, dtype=torch.int32)
+    lo = (ids == (w0 & 0xFF).unsqueeze(-1))
+    hi = (ids == ((w0 >> 8) & 0xFF).unsqueeze(-1))
+    words = packed[..., 4:].reshape(*lead, links, (W - 4) // links)
+    bits = (words.unsqueeze(-1) >> torch.arange(32, device=dev, dtype=torch.int32)) & 1
+    bits = bits.reshape(*lead, links, -1)[..., :slots].reshape(*lead, links * slots)
+    return torch.cat([lo.to(dtype), hi.to(dtype), bits.to(dtype)], -1)
+
+
 class OpticalVecEnv:
     """N batched environments of one kind on one GPU.
 
@@ -420,6 +446,32 @@ class OpticalVecEnv:
             nat.check(self._lib.orlg_rollout(self._h, T, pol, _ptr(obs), _ptr(reward), _ptr(done), _ptr(actions), self._stream()))
         return obs, reward, done, actions
 
+    @property
+    def matrix_layout(self):
+        """``(num_nodes, num_links, num_slots)`` of the matrix observation: the ``matrix_observation`` argument of an
+        :class:`~optical_rl_gym_b200.policy.MlpPolicy` that reads :meth:`packed_matrix_observation` rows."""
+        return (self.tables.num_nodes, self.tables.num_links, self.num_spectrum_resources)
+
+    def packed_matrix_observation(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """:meth:`matrix_observation` packed as bits, int32 ``[N, W]`` with ``W = 4 + 4 ceil(slots / 128) links`` (RMSA-v0 /
+        RWA-v0, ``orlg_matrix_observation_packed``): word 0 = ``min(src, dst) | max(src, dst) << 8``, words 1..3 = 0, then per
+        link ``ceil(slots / 128)`` groups of 4 words, bit ``b`` of word ``w`` of group ``v`` = slot ``128 v + 32 w + b``.  What a
+        ``MlpPolicy(..., matrix_observation=env.matrix_layout)`` reads; :meth:`unpack_matrix_observation` gives the uint8 rows."""
+        W = int(self._lib.orlg_matrix_obs_words(self._h))
+        if out is None:
+            out = torch.empty((self.num_envs, W), dtype=torch.int32, device=self.device)
+        elif (tuple(out.shape) != (self.num_envs, W) or out.dtype != torch.int32 or out.device != self.device
+              or not out.is_contiguous()):
+            raise ValueError("out must be a contiguous int32 tensor %s on %s, got %s %s %s" % (
+                (self.num_envs, W), self.device, tuple(out.shape), out.dtype, out.device))
+        nat.check(self._lib.orlg_matrix_observation_packed(self._h, _ptr(out), self._stream()))
+        return out
+
+    def unpack_matrix_observation(self, packed: torch.Tensor, dtype=torch.uint8) -> torch.Tensor:
+        """Packed rows ``[..., W]`` -> ``[..., 2 nodes + links slots]``, equal to :meth:`matrix_observation` (see the module
+        function ``unpack_matrix_observation``)."""
+        return unpack_matrix_observation(packed, self.matrix_layout, dtype)
+
     def rollout_policy(self, policy, steps: int, *, deterministic: bool = False, seed: Optional[int] = None,
                        out: Optional[PolicyRollout] = None, want_info: bool = False, action_masks: bool = False):
         """``steps`` iterations of ``a, log p(a), V(obs) = policy(obs); obs, r, done = env.step(a)`` in ONE native call
@@ -433,19 +485,26 @@ class OpticalVecEnv:
         ``action_masks=True`` draws every action from the masked distribution of sb3-contrib's ``MaskablePPO`` and appends
         the masks they were drawn under, ``torch.bool [T, N, A]`` (row t = :meth:`action_masks` of ``obs[t]``'s request):
         ``(PolicyRollout, masks)``, or ``(PolicyRollout, StepInfo, masks)`` with ``want_info=True``
-        (``orlg_rollout_policy_masked``)."""
+        (``orlg_rollout_policy_masked``).
+        RMSA-v0 / RWA-v0: the agent of ``PathOnlyFirstFitAction(SimpleMatrixObservation(env))``, a policy built with
+        ``matrix_observation=env.matrix_layout``.  ``obs`` is then the packed rows, int32 ``[T + 1, N, W]``
+        (:meth:`packed_matrix_observation`, :meth:`unpack_matrix_observation`), and ``actions`` the agent's path actions
+        ``[T, N]`` in ``Discrete(k + rej)``; each step maps them to (path, first-fit slot) as the wrapper does.  No action masks."""
         T, n, dev = int(steps), self.num_envs, self.device
         if T < 0:
             raise ValueError("steps must be >= 0")
         info, info_out = self._rollout_info(T) if want_info else (None, None)
+        matrix = getattr(policy, "matrix_observation", None) is not None and self.kind in (nat.KIND["RMSA-v0"], nat.KIND["RWA-v0"])
+        obs_shape, obs_dt = ((T + 1, n, int(self._lib.orlg_matrix_obs_words(self._h))), torch.int32) if matrix else \
+            ((T + 1, n, self.obs_dim), torch.float32)
         if out is None:
-            out = PolicyRollout(torch.empty((T + 1, n, self.obs_dim), dtype=torch.float32, device=dev),
+            out = PolicyRollout(torch.empty(obs_shape, dtype=obs_dt, device=dev),
                                 torch.empty((T, n), dtype=torch.int32, device=dev),
                                 torch.empty((T, n), dtype=torch.float32, device=dev),
                                 torch.empty((T + 1, n), dtype=torch.float32, device=dev),
                                 torch.empty((T, n), dtype=torch.float32, device=dev),
                                 torch.empty((T, n), dtype=torch.uint8, device=dev))
-        want = (((T + 1, n, self.obs_dim), torch.float32), ((T, n), torch.int32), ((T, n), torch.float32),
+        want = ((obs_shape, obs_dt), ((T, n), torch.int32), ((T, n), torch.float32),
                 ((T + 1, n), torch.float32), ((T, n), torch.float32), ((T, n), torch.uint8))
         for name, tns, (shape, dt) in zip(PolicyRollout._fields, out, want):
             if tuple(tns.shape) != shape or tns.dtype != dt or tns.device != dev or not tns.is_contiguous():
