@@ -643,12 +643,14 @@ int upload_fast_blob(orlg_env *env, const orlg_tables &t, const HostTables &h, i
     p.off_pair_count = put(h.pair_count.data(), h.pair_count.size());
     p.off_path_lm = put(h.linkmask.data(), h.linkmask.size() * 4);
     p.off_path_se = put(pse.data(), pse.size());
-    std::vector<unsigned long long> pll(P, 0ULL);      // hop list: 5 bits per link index, hop count in bits 60..63
+    // hop list: 5 bits per link index, hop count in bits 60..63; the fields past the last hop repeat hop 0, so that the rollout
+    // kernel walks a list four (or two) hops at a time without a select per hop (AND / OR / AND-NOT are idempotent)
+    std::vector<unsigned long long> pll(P, 0ULL);
     for (int r = 0; r < P; r++) {
         const int h0 = t.path_link_ptr[r], hn = t.path_link_ptr[r + 1] - h0;
         if (hn > 12) return ORLG_OK;
         unsigned long long v = (unsigned long long)hn << 60;
-        for (int i = 0; i < hn; i++) v |= (unsigned long long)(t.path_links[h0 + i] & 31) << (5 * i);
+        for (int i = 0; hn > 0 && i < 12; i++) v |= (unsigned long long)(t.path_links[h0 + (i < hn ? i : 0)] & 31) << (5 * i);
         pll[r] = v;
     }
     p.off_path_ll = put(pll.data(), pll.size() * 8);
@@ -670,6 +672,9 @@ int upload_fast_blob(orlg_env *env, const orlg_tables &t, const HostTables &h, i
         }
     }
     p.off_dbl = put(dbl.data(), dbl.size() * 4);
+    std::vector<float> br100(128);                              // bit rate / 100, the first observation entry (rates < 128)
+    for (int b = 0; b < 128; b++) br100[b] = (float)b / 100.0f;                     // IEEE f32 division == __fdiv_rn
+    p.off_br100 = put(br100.data(), br100.size() * 4);
     blob.resize((blob.size() + 127) / 128 * 128);          // the warp areas behind it are TMA destinations (128-byte aligned)
     if (blob.size() > 24 * 1024 || blob.size() + (size_t)FAST_THREADS * 16 * 32 > 100 * 1024) return ORLG_OK;
     std::vector<uint4> blob4(blob.size() / 16);

@@ -95,14 +95,19 @@ __device__ __forceinline__ int bits_ffs(const WBits<V> &a) {
         if (a.w[i]) r = 32 * i + __ffs(a.w[i]) - 1;
     return r;
 }
-// index of the highest set bit, or -1
+// index of the highest set bit, or -1: the highest non-zero word by selects, then one clz (an empty mask leaves x = 0,
+// base = 0, and 31 - clz(0) = -1)
 template <int V>
 __device__ __forceinline__ int bits_fls(const WBits<V> &a) {
-    int r = -1;
+    uint32_t x = 0;
+    int base = 0;
 #pragma unroll
-    for (int i = 0; i < 4 * V; i++)
-        if (a.w[i]) r = 32 * i + 31 - __clz(a.w[i]);
-    return r;
+    for (int i = 0; i < 4 * V; i++) {
+        const bool nz = a.w[i] != 0u;
+        x = nz ? a.w[i] : x;
+        base = nz ? 32 * i : base;
+    }
+    return base + 31 - __clz(x);
 }
 template <int V>
 __device__ __forceinline__ WBits<V> bits_clear_lowest(const WBits<V> &a) {
@@ -209,14 +214,18 @@ __device__ __forceinline__ Bits bits_range_short(int start, int n) {
 __device__ __forceinline__ Bits bits_range_auto(int start, int n) {
     return (n <= 32) ? bits_range_short(start, n) : bits_range(start, start + n);
 }
-// bits_ffs as a select chain instead of 4 dependent branches
+// bits_ffs without branches: the lowest non-zero word by selects, then one ffs (an empty mask leaves x = 0, base = 0,
+// and ffs(0) - 1 = -1).  One bit scan instead of four: BREV + FLO sit on the dependent chain of every caller.
 __device__ __forceinline__ int bits_ffs_flat(const Bits &a) {
-    const int p0 = __ffs(a.w[0]), p1 = __ffs(a.w[1]), p2 = __ffs(a.w[2]), p3 = __ffs(a.w[3]);
-    int r = p3 ? p3 + 95 : -1;
-    r = p2 ? p2 + 63 : r;
-    r = p1 ? p1 + 31 : r;
-    r = p0 ? p0 - 1 : r;
-    return r;
+    uint32_t x = 0;
+    int base = 0;
+#pragma unroll
+    for (int i = NW - 1; i >= 0; i--) {
+        const bool nz = a.w[i] != 0u;
+        x = nz ? a.w[i] : x;
+        base = nz ? 32 * i : base;
+    }
+    return base + __ffs(x) - 1;
 }
 
 // ---------------------------------------------------------------- Philox4x32-10 (counter-based traffic)

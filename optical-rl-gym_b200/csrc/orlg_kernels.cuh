@@ -44,7 +44,7 @@ struct Params {
     // packed copy of the small tables, staged in shared memory by the fast kernel (byte offsets)
     const uint4 *tab_blob;
     int tab_vec;                       // size in 16-byte units
-    int off_pair_first, off_pair_count, off_path_lm, off_path_se, off_path_ll, off_nslots, off_node_thr, off_pos, off_nsl, off_rcp4, off_dbl;
+    int off_pair_first, off_pair_count, off_path_lm, off_path_se, off_path_ll, off_nslots, off_node_thr, off_pos, off_nsl, off_rcp4, off_dbl, off_br100;
     int node_top_step;                 // highest power of two <= N-1 (binary search over the node CDF)
     int warp_area_bytes;               // fast kernel: shared-memory work area per warp (masks, then observation rows)
     unsigned lockstep_ridx;            // requests drawn so far by EVERY env (all envs reset and step together)

@@ -110,14 +110,13 @@ struct RolloutArgs {
     long long *info;             // [T][n][8]         the counters orlg_step's info_dev receives, every step (INFO instances)
 };
 
-// apply a release / an allocation to the path's links in the warp's shared-memory mask tile
+// apply a release / an allocation to the path's links in the warp's shared-memory mask tile.  `ll` is the path's hop list
+// (s_path_ll: 5 bits per link, hop count in bits 60..63, hop 0 repeated past the last hop): the link ids come out of shifts,
+// not out of a bit scan of the link mask, so both addresses of a pass are ready together
 template <bool SET>
-__device__ __forceinline__ void ro_path_update(uint4 *sm, unsigned lm, const Bits &rm) {
-    while (lm) {                         // two hops per pass: both loads in flight before either store (a repeated hop is harmless)
-        const int l0 = __ffs(lm) - 1;
-        lm &= lm - 1;
-        const int l1 = lm ? __ffs(lm) - 1 : l0;
-        lm &= lm - 1;
+__device__ __forceinline__ void ro_path_update(uint4 *sm, unsigned long long ll, const Bits &rm) {
+    for (int h = (int)(ll >> 60); h > 0; h -= 2, ll >>= 10) {   // two hops per pass: both loads in flight before either store (a repeated hop is harmless)
+        const int l0 = (int)(ll & 31u), l1 = (int)((ll >> 5) & 31u);
         uint4 v = sm[l0 * 32], u = sm[l1 * 32];
         if (SET) { v.x |= rm.w[0]; v.y |= rm.w[1]; v.z |= rm.w[2]; v.w |= rm.w[3]; u.x |= rm.w[0]; u.y |= rm.w[1]; u.z |= rm.w[2]; u.w |= rm.w[3]; }
         else { v.x &= ~rm.w[0]; v.y &= ~rm.w[1]; v.z &= ~rm.w[2]; v.w &= ~rm.w[3]; u.x &= ~rm.w[0]; u.y &= ~rm.w[1]; u.z &= ~rm.w[2]; u.w &= ~rm.w[3]; }
@@ -368,7 +367,6 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
     }
     const unsigned short *s_pair_first = reinterpret_cast<const unsigned short *>(smem + p.off_pair_first);
     const unsigned char *s_pair_count = smem + p.off_pair_count;
-    const unsigned *s_path_lm = reinterpret_cast<const unsigned *>(smem + p.off_path_lm);
     const unsigned char *s_path_se = smem + p.off_path_se;
     const unsigned long long *s_path_ll = reinterpret_cast<const unsigned long long *>(smem + p.off_path_ll);
     const unsigned char *s_nslots = smem + p.off_nslots;
@@ -377,6 +375,7 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
     const float *s_nsl = reinterpret_cast<const float *>(smem + p.off_nsl);
     const float *s_rcp4 = reinterpret_cast<const float *>(smem + p.off_rcp4);
     const unsigned *s_dbl = reinterpret_cast<const unsigned *>(smem + p.off_dbl);
+    const float *s_br100 = reinterpret_cast<const float *>(smem + p.off_br100);      // bit rate / 100 (== __fdiv_rn), rates < 128
     pdl_wait();                      // state is touched from here on
 
     // ---------------- state in: masks -> shared memory (cp.async, coalesced 512 B per link and warp), scalars -> registers
@@ -468,7 +467,7 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
 #define RO_POP_DUE()                                                                                              \
     while (head.t <= now) {                                                                                      \
         const int rs_ = svc_start(head.p);                                                                       \
-        ro_path_update<true>(sm, s_path_lm[svc_row(head.p)], bits_range_short(rs_, svc_slots(head.p)));          \
+        ro_path_update<true>(sm, s_path_ll[svc_row(head.p)], bits_range_short(rs_, svc_slots(head.p)));          \
         nlive--; wh++;                                                                                           \
         head = nxt;                                                                                              \
         if (wh + 1 < wn) nxt = win_load(win + (wh + 1) * 32); else nxt.t = ORLG_INF;                             \
@@ -583,7 +582,7 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
                 if (act < np_cur) {
                     const int a_row = s_pair_first[pair] + act;
                     const int a_n = KIND == ORLG_RWA ? 1 : s_nslots[s_path_se[a_row] * 128 + br];
-                    const unsigned a_lm = s_path_lm[a_row];
+                    const unsigned long long a_ll = s_path_ll[a_row];
                     bool fits;
                     if (KIND == ORLG_DEEPRMSA) {                 // the cached block start decides
                         const unsigned st = (unsigned)((candw >> (8 * act)) & 0xffu);
@@ -596,12 +595,8 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
                         fits = a_start + a_n <= p.S;
                         if (fits) {
                             Bits F = bits_ones();
-                            unsigned m = a_lm;
-                            while (m) {
-                                const int l = __ffs(m) - 1;
-                                m &= m - 1;
-                                F = bits_and(F, bits_from(sm[l * 32]));
-                            }
+                            unsigned long long m = a_ll;
+                            for (int h = (int)(m >> 60); h > 0; h--, m >>= 5) F = bits_and(F, bits_from(sm[(int)(m & 31u) * 32]));
                             fits = bits_contains(F, bits_range_short(a_start, a_n));
                         }
                     }
@@ -609,7 +604,7 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
                         if (nlive + 1 > (unsigned)p.heap_cap) {
                             err |= ORLG_ERR_HEAP_OVERFLOW;
                         } else {
-                            ro_path_update<false>(sm, a_lm, bits_range_short(a_start, a_n));      // _provision_path
+                            ro_path_update<false>(sm, a_ll, bits_range_short(a_start, a_n));      // _provision_path
                             const double rel = __dadd_rn(now, hold);
                             const unsigned long long pl = pack_service(a_row, a_start, a_n, 0, sid);
                             bool in_side = false;
@@ -657,7 +652,7 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
                     if (ts <= now) {
                         const unsigned long long pl = side_p[s * 32];
                         const int rs = svc_start(pl);
-                        ro_path_update<true>(sm, s_path_lm[svc_row(pl)], bits_range_short(rs, svc_slots(pl)));
+                        ro_path_update<true>(sm, s_path_ll[svc_row(pl)], bits_range_short(rs, svc_slots(pl)));
                         side_t[s * 32] = ORLG_INF;
                         nlive--;
                     } else {
@@ -718,17 +713,13 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
             for (int q = 0; q < KM; q++) {
                 const bool have = q < npaths;
                 const int row = have ? first + q : first;
-                unsigned lm = have ? s_path_lm[row] : 0u;
+                unsigned long long ll = s_path_ll[row];
+                const int nh = have ? (int)(ll >> 60) : 0;
                 Bits A = have ? bits_ones() : Bits{{0u, 0u, 0u, 0u}};
-                while (lm) {                     // four hops per pass, their loads in flight together (AND is idempotent: a short
-                    const int l0 = __ffs(lm) - 1;  // path repeats its first hop)
-                    lm &= lm - 1;
-                    const int l1 = lm ? __ffs(lm) - 1 : l0;
-                    lm &= lm - 1;
-                    const int l2 = lm ? __ffs(lm) - 1 : l0;
-                    lm &= lm - 1;
-                    const int l3 = lm ? __ffs(lm) - 1 : l0;
-                    lm &= lm - 1;
+                // four hops per pass off the hop list, their loads in flight together (AND is idempotent: past its last hop
+                // the list repeats the first)
+                for (int h = nh; h > 0; h -= 4, ll >>= 20) {
+                    const int l0 = (int)(ll & 31u), l1 = (int)((ll >> 5) & 31u), l2 = (int)((ll >> 10) & 31u), l3 = (int)((ll >> 15) & 31u);
                     const uint4 v0 = sm[l0 * 32], v1 = sm[l1 * 32], v2 = sm[l2 * 32], v3 = sm[l3 * 32];
                     A.w[0] &= v0.x & v1.x; A.w[1] &= v0.y & v1.y; A.w[2] &= v0.z & v1.z; A.w[3] &= v0.w & v1.w;
                     A.w[0] &= v2.x & v3.x; A.w[1] &= v2.y & v3.y; A.w[2] &= v2.z & v3.z; A.w[3] &= v2.w & v3.w;
@@ -747,7 +738,7 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
                     if (KIND == ORLG_RWA) {
                         if (POLICY == RO_POLICY_SAP_LF) { Bits L = A; L.w[0] &= ~1u; st = bits_fls(L); }     // range(W - 1, 0, -1): never wavelength 0
                         else st = bits_ffs_flat(A);
-                        if (have) hops_out |= (unsigned)(s_path_ll[row] >> 60) << (4 * q);
+                        hops_out |= (unsigned)nh << (4 * q);
                     } else {                                     // first fit over range(0, S - n): the last feasible start is never tried
                         const int n = s_nslots[s_path_se[row] * 128 + br];
                         const Bits B = bits_and(bits_runs_ge_sched(A, s_dbl[n]), bits_range(0, max(p.S - n, 0)));
@@ -800,7 +791,7 @@ deeprmsa_rollout_kernel(const Params p, const RolloutArgs ra) {
                 }
 #pragma unroll
                 for (int i = 0; i < (1 + 5 * KM + 1) / 2; i++) r2[p.N + i] = make_float2(v[2 * i], v[2 * i + 1]);
-                so32[0] = __fdiv_rn((float)br, 100.0f);
+                so32[0] = s_br100[br];
                 so32[1 + lo_n] = 1.0f;
                 if (hi_n != p.N - 1) so32[1 + p.N + hi_n] = 1.0f;
             }
